@@ -3,7 +3,7 @@
 bench.py -- ECG-ViT training-step throughput (BASELINE.json metric: train samples/s on synthetic 12x2500, bf16).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg4|cfg5]
-                    [--batch B | --global-batch G] [--no-graph] [--api-loop]
+                    [--batch B | --global-batch G] [--no-graph] [--api-loop] [--dump-outputs DIR]
 
 One "step" = zero_grad + forward + backward + (bucketed grad all-reduce) + clip_grad_norm(1.0) + AdamW on one batch of
 synthetic signals (seed 77), i.e. /root/reference/ecg_transformer/models/train.py:271-283 without its logging.
@@ -254,6 +254,21 @@ def run_reference_arm(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(path, model, trainer, loss, logits, n_sample=1 << 20):
+    """Writes what the timed step handed its caller, as float32 .npy files under `path`: the loss, the logits, the
+    gradient norm and a fixed sample of the updated parameters (seed 0, 2^20 indices into the parameters concatenated
+    in state_dict order, which does not depend on the library's internal flat layout).  Two builds run with the same
+    arguments start from the same weights and inputs, so their files can be compared one for one."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    params = torch.cat([v.detach().reshape(-1).float() for v in model.state_dict().values()])
+    idx = torch.from_numpy(np.random.default_rng(0).integers(0, params.numel(), n_sample)).to(params.device)
+    arrays = {'loss': loss, 'logits': logits, 'grad_norm': torch.tensor(trainer.grad_norm()), 'params_sample': params[idx]}
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def time_graph(torch, launch_all, reps):
     """device time per launch of `launch_all()` (which issues `reps` launches on the current stream): the batch is
     captured into a CUDA graph and the REPLAY is timed with CUDA events (launched one by one from Python, a 10-60 us
@@ -394,7 +409,13 @@ def main():
                     help='run clip + AdamW of step k beside the forward pass of step k + 1 (FusedTrainer(defer_optimizer=True)); '
                          'measured neutral at cfg2: the slices displace CTAs of the persistent forward GEMMs')
     ap.add_argument('--grad-reduce', default='auto', choices=['auto', 'fp32', 'bf16'], help='dtype of the gradient all-reduce')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='after the timed steps, write the outputs of the last one as DIR/<name>.npy (rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU step (--impl ours)')
     wl = WORKLOADS[args.config]
     MODEL_CFG = dict(wl['model'])
     MODEL_CFG['hidden_dropout_prob'] = MODEL_CFG['attention_probs_dropout_prob'] = args.dropout
@@ -472,9 +493,16 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    total_ms = timed(lambda: trainer.step(x, y), args.steps)
+    last = [None]
+
+    def train_step():
+        last[0] = trainer.step(x, y)
+
+    total_ms = timed(train_step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
     trainer.check_finite()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, trainer, *last[0])  # before later steps overwrite the step's buffers
     ms_per_step = total_ms / args.steps
     value = world * B / (ms_per_step / 1e3)
 

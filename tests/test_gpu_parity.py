@@ -8,7 +8,7 @@ from torch import nn
 
 pytestmark = pytest.mark.gpu
 
-from conftest import GOLDEN_CFG
+from conftest import GOLDEN_CFG, golden_sample
 import ecg_b200
 from ecg_b200 import EcgVit, EcgVitConfig, FusedTrainer, FusedAdamW, clip_grad_norm_
 from oracle.ecg_vit_oracle import OracleConfig, OracleEcgVit, OracleTrainer, synthetic_batch
@@ -54,9 +54,9 @@ def test_fp32_matches_golden_forward_backward(golden):
     assert rel(out.logits, torch.from_numpy(golden['logits'])) < FP32_TOL
     assert abs(float(out.loss) - float(golden['loss'])) < FP32_TOL * float(golden['loss'])
     for k, p in model.named_parameters():
-        g = torch.from_numpy(golden['grad/' + k])
-        assert rel(p.grad, g) < 2e-4, (k, rel(p.grad, g))
-        assert cosine(p.grad, g) > 0.999999, k
+        got, g = golden_sample(p.grad), torch.from_numpy(golden['grad/' + k])
+        assert rel(got, g) < 2e-4, (k, rel(got, g))
+        assert cosine(got, g) > 0.999999, k
 
 
 def test_fp32_matches_golden_three_steps(golden):
@@ -69,7 +69,8 @@ def test_fp32_matches_golden_three_steps(golden):
         assert abs(tr.grad_norm() - float(golden[f'norm{step}'])) < 1e-4 * float(golden[f'norm{step}'])
         if step in (1, 3):
             for k, v in model.state_dict().items():
-                assert rel(v, torch.from_numpy(golden[f'step{step}/' + k])) < FP32_TOL, (step, k)
+                got = golden_sample(v) if step == 1 else v
+                assert rel(got, torch.from_numpy(golden[f'step{step}/' + k])) < FP32_TOL, (step, k)
     tr.check_finite()
 
 

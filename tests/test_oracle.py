@@ -1,5 +1,5 @@
-"""CPU tier: pins the travelling oracle against (a) the committed golden vectors generated through the reference's
-own wrapper and (b), where /root/reference exists, the reference wrapper itself."""
+"""CPU tier: pins the travelling oracle against the committed golden vectors, which the reference's own wrapper,
+transform classes and metrics produced (tests/golden/make_golden*.py)."""
 import os
 
 import numpy as np
@@ -7,10 +7,8 @@ import pytest
 import torch
 from torch import nn
 
-from conftest import GOLDEN_CFG
-from oracle import ref_shim
-from oracle.ecg_vit_oracle import (OracleConfig, OracleEcgVit, OracleTrainer, NAMED_SIZES, lr_lambda, patch_matrix,
-                                   synthetic_batch)
+from conftest import GOLDEN_CFG, golden_sample
+from oracle.ecg_vit_oracle import OracleConfig, OracleEcgVit, OracleTrainer, NAMED_SIZES, lr_lambda, patch_matrix
 
 
 def _load_state(model, golden, prefix):
@@ -28,10 +26,23 @@ def test_oracle_reproduces_golden_forward_backward(golden):
     np.testing.assert_allclose(out.logits.detach().numpy(), golden['logits'], rtol=0, atol=1e-6)
     assert abs(out.loss.item() - float(golden['loss'])) < 1e-6
     for k, p in m.named_parameters():
-        np.testing.assert_allclose(p.grad.numpy(), golden['grad/' + k], rtol=0, atol=1e-7)
+        np.testing.assert_allclose(golden_sample(p.grad.numpy()), golden['grad/' + k], rtol=0, atol=1e-7)
 
 
-def test_oracle_reproduces_golden_three_steps(golden):
+@pytest.fixture
+def golden_threads():
+    """CPU reductions round according to how they are split over threads.  Where a weight's gradient cancels to the size
+    of AdamW's eps (1e-8), that rounding reaches its update: one patch-embedding weight moves by 1.6e-7 after three
+    steps with 1, 4 or 16 intra-op threads.  With 8 threads the oracle reproduces the golden vectors bit for bit, also
+    on machines with fewer or more cores.  The split is one input of the rounding; the CPU's vector width is another:
+    the vectors reproduce on AVX-512 CPUs, and a CPU with another vector width may still differ in the last bits."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(threads)
+
+
+def test_oracle_reproduces_golden_three_steps(golden, golden_threads):
     m = OracleEcgVit(config=OracleConfig(**GOLDEN_CFG))
     _load_state(m, golden, 'init/')
     m.train()
@@ -43,7 +54,8 @@ def test_oracle_reproduces_golden_three_steps(golden):
         assert abs(float(norm) - float(golden[f'norm{step}'])) < 1e-6
         if step in (1, 3):
             for k, v in m.state_dict().items():
-                np.testing.assert_allclose(v.numpy(), golden[f'step{step}/' + k], rtol=0, atol=1e-7)
+                got = golden_sample(v.numpy()) if step == 1 else v.numpy()
+                np.testing.assert_allclose(got, golden[f'step{step}/' + k], rtol=0, atol=1e-7)
 
 
 def test_oracle_eval_loss_none(golden):
@@ -85,29 +97,23 @@ def test_lr_lambda_matches_transformers():
             sch.step()
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='/root/reference only exists in the build container')
-def test_oracle_matches_reference_wrapper():
-    """the restated wrapper == the reference's verbatim `EcgVit` on the same weights and inputs (bit-exact)"""
-    EcgVit, EcgVitConfig, get_train_args, _ = ref_shim.load_reference()
-    kw = dict(GOLDEN_CFG, hidden_size=128, num_hidden_layers=3, num_attention_heads=8, intermediate_size=256)
-    torch.manual_seed(5)
-    ref = EcgVit(config=EcgVitConfig(**kw))
-    ours = OracleEcgVit(config=OracleConfig(**kw))
-    assert list(ref.state_dict().keys()) == list(ours.state_dict().keys())
-    ours.load_state_dict(ref.state_dict(), strict=True)
-    x, y = synthetic_batch(3, length=500, seed=11)
-    a, b = ref(sample_values=x, labels=y), ours(sample_values=x, labels=y)
-    assert torch.equal(a.logits, b.logits) and torch.equal(a.loss, b.loss)
-    a.loss.backward()
-    b.loss.backward()
-    for (k, p), (_, q) in zip(ref.named_parameters(), ours.named_parameters()):
-        assert torch.equal(p.grad, q.grad), k
-    # named sizes and trainer defaults
-    for size, dims in NAMED_SIZES.items():
-        c = EcgVitConfig.from_defined(f'ecg-vit-{size}')
-        assert (c.hidden_size, c.num_hidden_layers, c.num_attention_heads, c.intermediate_size) == dims
-    args = get_train_args()
-    assert (args['learning_rate'], args['weight_decay'], args['warmup_ratio'], args['schedule']) == (3e-4, 1e-2, 0.05, 'cosine')
+def test_oracle_matches_reference_wrapper(golden, golden_threads):
+    """The restated wrapper == the reference's verbatim `EcgVit`, bit for bit, through what that wrapper stored in the
+    golden vectors (tests/golden/make_golden.py): its state_dict keys in its order, its initial weights from the same
+    seed (parameter creation order and initialisers), and its logits, loss and gradients on those weights and inputs."""
+    torch.manual_seed(77)
+    ours = OracleEcgVit(config=OracleConfig(**GOLDEN_CFG))
+    ref_init = {k[len('init/'):]: v for k, v in golden.items() if k.startswith('init/')}
+    assert list(ours.state_dict().keys()) == list(ref_init.keys())
+    for k, v in ours.state_dict().items():
+        assert np.array_equal(v.numpy(), ref_init[k]), k
+    ours.train()
+    out = ours(sample_values=torch.from_numpy(golden['x']), labels=torch.from_numpy(golden['y']))
+    assert np.array_equal(out.logits.detach().numpy(), golden['logits']) and out.loss.item() == float(golden['loss'])
+    out.loss.backward()
+    assert [k for k, _ in ours.named_parameters()] == [k[len('grad/'):] for k in golden if k.startswith('grad/')]
+    for k, p in ours.named_parameters():
+        assert np.array_equal(golden_sample(p.grad.numpy()), golden['grad/' + k]), k
 
 
 # ---- input transforms (SURVEY 8f rank 1): oracle/transforms.py pinned by vectors the reference's own classes produced
@@ -130,24 +136,17 @@ def test_transform_oracle_matches_reference_vectors(transform_golden, case):
         assert got_eval.shape[-1] == rec.shape[-1] + k      # TimeEndPad pads a whole block when L % k == 0
 
 
-def test_transform_oracle_matches_reference_classes_live():
-    """when the reference tree is present (build container), run its classes directly against the restatement"""
-    if not os.path.isdir('/root/reference/ecg_transformer'):
-        pytest.skip('reference tree not present')
-    import importlib
+@pytest.mark.parametrize('case', ['ragged', 'full_block', 'long'])
+def test_transform_oracle_draws_time_out_like_reference_classes(transform_golden, case):
+    """The reference's `TimeOut` draws its span from torch's global RNG, one record after another, and the golden
+    `train` output is what its classes produced after torch.manual_seed(1234) (tests/golden/make_golden_transform.py).
+    `draw_time_out_span` must consume the RNG the same way: the same seed gives the same masked output, bit for bit."""
     from oracle import transforms
-    ref_shim.install()
-    T = importlib.import_module('ecg_transformer.preprocess.transform')
-    rng = np.random.default_rng(5)
-    rec = rng.standard_normal((12, 333)).astype(np.float32)
-    mean, std = rng.standard_normal(12) * 0.05, rng.random(12) * 0.3 + 0.1
-    want = T.TimeEndPad(64, pad_kwargs=dict(mode='constant', constant_values=0))(T.Normalize(mean=mean, std=std)(rec))
-    torch.manual_seed(9)
-    want_train = T.TimeOut()(want.copy())
-    torch.manual_seed(9)
-    s, l = transforms.draw_time_out_span(want.shape[-1])
-    got = transforms.pipeline(rec[None], mean, std, pad=64, spans=[(s, l)])[0]
-    assert np.array_equal(got, want_train)
+    g = transform_golden
+    rec, k = g[f'{case}/records'], int(g[f'{case}/k'])
+    torch.manual_seed(1234)
+    spans = [transforms.draw_time_out_span(g[f'{case}/eval'].shape[-1]) for _ in range(rec.shape[0])]
+    assert np.array_equal(transforms.pipeline(rec, g['mean'], g['std'], pad=k, spans=spans), g[f'{case}/train'])
 
 
 # ---- evaluation metrics (SURVEY 8f rank 2): oracle/metrics.py pinned by the reference's own get_accuracy outputs
@@ -176,7 +175,7 @@ def test_oracle_fp64_tie_breaker(golden):
     rel = float((out.logits.detach() - want).norm() / want.norm())
     assert rel < 1e-6, rel
     assert abs(out.loss.item() - float(golden['loss'])) < 1e-6 * float(golden['loss'])
-    worst = max(float((p.grad - torch.from_numpy(golden['grad/' + k]).double()).norm() /
+    worst = max(float((golden_sample(p.grad) - torch.from_numpy(golden['grad/' + k]).double()).norm() /
                       torch.from_numpy(golden['grad/' + k]).double().norm().clamp_min(1e-30))
                 for k, p in m.named_parameters())
     assert worst < 1e-5, worst
