@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(PKG_DIR, 'libecgvit_b200.so')
 F32, BF16, BF16_RES32 = 0, 1, 2  # BF16_RES32: bf16 mode whose residual-stream operand is fp32 (ecgvit_b200.h)
 STATS_FLOATS = 2052  # ECGVIT_STATS_FLOATS
 SUMSQ_MAX_BLOCKS = 2048  # partial slots of the gradient-norm scratch (stats[4:])
-EPI_STORE, EPI_BIAS_RES, EPI_BIAS_GELU, EPI_DGELU, EPI_ATOMIC_F32, EPI_BIAS_RES_F32 = 0, 1, 2, 3, 4, 5
+EPI_STORE, EPI_BIAS_RES, EPI_BIAS_GELU, EPI_DGELU, EPI_ATOMIC_F32, EPI_BIAS_RES_F32, EPI_BIAS_SUB_ROWSQ = 0, 1, 2, 3, 4, 5, 6
 REDUCTION = {'mean': 0, 'sum': 1, 'none': 2}
 
 
@@ -48,6 +48,16 @@ SIGNATURES = {
                               c_int, c_void_p],
     'ecgvit_embed_assemble_bwd': [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_int,
                                   c_void_p, c_int, c_void_p],
+    'ecgvit_mpm_mask': [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    'ecgvit_embed_assemble_masked': [c_void_p] * 6 + [c_int, c_int, c_int, c_float, c_int, c_void_p, c_int, c_void_p],
+    'ecgvit_embed_assemble_masked_bwd': [c_void_p] * 7 + [c_int, c_int, c_int, c_float, c_int, c_void_p, c_int,
+                                                          c_void_p],
+    'ecgvit_layernorm_patch_fwd': [c_void_p] * 6 + [c_int, c_int, c_int, c_float, c_int, c_void_p],
+    'ecgvit_layernorm_patch_bwd': [c_void_p] * 10 + [c_int, c_int, c_int, c_int, c_void_p],
+    'ecgvit_mpm_loss': [c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    'ecgvit_mpm_dpred': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_int,
+                         c_void_p],
+    'ecgvit_mpm_reconstruction': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
     'ecgvit_dropout_bwd_copy': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_float, c_int, c_void_p, c_int,
                                 c_void_p],
     'ecgvit_layernorm_fwd': [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float,
@@ -108,7 +118,7 @@ def last_error():
 
 
 # kernels launched per successful entry-point call (memsets are not kernels); feeds bench.py's `gpu_launches`
-KERNELS_PER_CALL = {'attention_bwd_flash': 3, 'head_fwd': 2, 'head_bwd': 3, 'layernorm_bwd': 2, 'layernorm_bwd_partial': 1, 'grad_sumsq': 2, 'eval_metrics': 3}
+KERNELS_PER_CALL = {'layernorm_patch_bwd': 3, 'attention_bwd_flash': 3, 'head_fwd': 2, 'head_bwd': 3, 'layernorm_bwd': 2, 'layernorm_bwd_partial': 1, 'grad_sumsq': 2, 'eval_metrics': 3}
 launch_counter = [0]
 
 
@@ -134,17 +144,9 @@ def ptr(t):
     return None if t is None else t.data_ptr()
 
 
-def dropout_keep_mask(seed, stream, p, index):
-    """host replica of the kernels' counter-based dropout (csrc/common.cuh `dropout_hash`, two multiply-and-fold rounds): multiplier (0 or
-    1/(1-p_q)) for every element index in the int64 tensor `index`; used by the tests to inject the SAME masks into the
-    CPU oracle"""
-    import torch
-    thr = min(int(p * 65536.0 + 0.5), 65535)
-    if thr == 0:
-        return torch.ones(index.shape, dtype=torch.float32)
+def counter_hash(seed, stream, pair):
+    """host replica of csrc/common.cuh `dropout_hash` (two multiply-and-fold rounds) over the int64 tensor `pair`"""
     m32 = 0xFFFFFFFF
-    idx = index.to(torch.int64)
-    pair = idx >> 1
     key = (seed ^ ((stream * 0x85EBCA77 + 0xC2B2AE3D) & m32)) & m32
 
     def mulfold(a, k):  # (a * k) as a 64-bit product, xor of its two 32-bit halves
@@ -157,10 +159,34 @@ def dropout_keep_mask(seed, stream, p, index):
         return lo ^ hi
 
     h = mulfold((pair ^ key) & m32, 0x9E3779B1)
-    h = mulfold(h, 0x7FEB352D)
+    return mulfold(h, 0x7FEB352D)
+
+
+def dropout_keep_mask(seed, stream, p, index):
+    """host replica of the kernels' counter-based dropout (csrc/common.cuh `dropout_hash`, two multiply-and-fold rounds): multiplier (0 or
+    1/(1-p_q)) for every element index in the int64 tensor `index`; used by the tests to inject the SAME masks into the
+    CPU oracle"""
+    import torch
+    thr = min(int(p * 65536.0 + 0.5), 65535)
+    if thr == 0:
+        return torch.ones(index.shape, dtype=torch.float32)
+    idx = index.to(torch.int64)
+    h = counter_hash(seed, stream, idx >> 1)
     bits = torch.where((idx & 1) == 1, h >> 16, h & 0xFFFF)
     scale = 1.0 / (1.0 - thr / 65536.0)
     return torch.where(bits >= thr, torch.tensor(scale, dtype=torch.float32), torch.tensor(0.0, dtype=torch.float32))
+
+
+def mpm_mask(seed, B, n, k, site):
+    """host replica of ecgvit_mpm_mask: bool [B, n], patch w of record b masked iff the rank of its key
+    counter_hash(seed, site, b*n + w) within record b is < k (ties broken by the lower index)"""
+    import torch
+    keys = counter_hash(seed, site, torch.arange(B * n, dtype=torch.int64)).reshape(B, n)
+    # stable sort on (key, index): the k first positions of every row are its masked patches
+    order = torch.sort(keys, dim=1, stable=True).indices
+    mask = torch.zeros(B, n, dtype=torch.bool)
+    mask.scatter_(1, order[:, :k], True)
+    return mask
 
 
 ADAMW_SLICE, ADAMW_FIRST_SLICE = 1, 2

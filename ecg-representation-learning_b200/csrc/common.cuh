@@ -341,6 +341,12 @@ __device__ __forceinline__ void epilogue_store(const EpiParams &p, int64_t row, 
         else load4(reinterpret_cast<const T *>(p.aux) + off, r);
 #pragma unroll
         for (int i = 0; i < NV; ++i) acc[i] += r[i];
+    } else if (MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) {   // acc keeps the fp32 residual for the caller's row sum
+        float t[NV];
+        if (NV == 8) load8(reinterpret_cast<const T *>(p.aux) + off, t);
+        else load4(reinterpret_cast<const T *>(p.aux) + off, t);
+#pragma unroll
+        for (int i = 0; i < NV; ++i) acc[i] -= t[i];
     } else if (MODE == ECGVIT_EPI_DGELU) {
         float u[NV];
         if (NV == 8) load8(reinterpret_cast<const T *>(p.aux) + off, u);

@@ -131,10 +131,12 @@ __global__ void unpad_add_kernel(const float *__restrict__ src, float *__restric
 
 // ---------------------------------------------------------------------------------------------------
 // tok[b,0,:] = cls + pos[0];  tok[b,1+w,:] = e[b*n+w,:] + pos[1+w,:]
-template <typename T, typename TO>
+// kMasked: rows with mask[b*n+w] != 0 take mask_token instead of e (masked-patch pre-training)
+template <typename T, typename TO, bool kMasked = false>
 __global__ void embed_assemble_kernel(const T *__restrict__ e, const float *__restrict__ cls,
                                       const float *__restrict__ pos, TO *__restrict__ tok, int B, int n_patch, int d,
-                                      DropoutParams drop) {
+                                      DropoutParams drop, const float *__restrict__ mask_token = nullptr,
+                                      const uint8_t *__restrict__ mask = nullptr) {
     const bool dropping = drop.threshold != 0;
     const uint32_t seed = dropping ? __ldg(drop.seed) : 0u;
     const int N = n_patch + 1;
@@ -148,6 +150,7 @@ __global__ void embed_assemble_kernel(const T *__restrict__ e, const float *__re
         float v[8], p[8];
         load8(pos + (int64_t)j * d + c, p);
         if (j == 0) load8(cls + c, v);
+        else if (kMasked && mask[b * n_patch + (j - 1)] != 0) load8(mask_token + c, v);
         else load8(e + (b * n_patch + (j - 1)) * d + c, v);
 #pragma unroll
         for (int k = 0; k < 8; ++k) v[k] += p[k];
@@ -159,21 +162,24 @@ __global__ void embed_assemble_kernel(const T *__restrict__ e, const float *__re
 // backward: grid (token position j, 256-column slab), block = 32 lanes x 8 columns each x 8 batch groups; the masked
 // gradient rows are copied to `de` on the way (16-byte accesses, one dropout hash per pair) and the batch sums are folded
 // through shared memory.  (One 2-byte element per thread with a hash per element was instruction bound: 22 us for 40 MB.)
-template <typename T>
+// kMasked: masked rows (mask[b*n+w] != 0) send their gradient to dmask_token instead of de / dbias (de rows are zeroed)
+template <typename T, bool kMasked = false>
 __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__restrict__ dtok, T *__restrict__ de,
                                                                   float *__restrict__ dcls, float *__restrict__ dpos,
                                                                   float *__restrict__ dbias, int B, int n_patch, int d,
-                                                                  DropoutParams drop) {
-    __shared__ float red[8][256 + 8];
+                                                                  DropoutParams drop,
+                                                                  const uint8_t *__restrict__ mask = nullptr,
+                                                                  float *__restrict__ dmask_token = nullptr) {
+    __shared__ float red[kMasked ? 16 : 8][256 + 8];
     const int N = n_patch + 1;
     const int j = blockIdx.x;
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const int col = (blockIdx.y * 32 + tx) * 8;
     const bool dropping = drop.threshold != 0;
     const uint32_t seed = dropping ? __ldg(drop.seed) : 0u;
-    float s[8];
+    float s[8], sm[8];   // sums of the visible rows (all rows without kMasked) / of the masked rows
 #pragma unroll
-    for (int k = 0; k < 8; ++k) s[k] = 0.f;
+    for (int k = 0; k < 8; ++k) s[k] = sm[k] = 0.f;
     if (col < d) {
         // two samples in flight per thread (rows N * d elements apart)
         for (int b0 = ty; b0 < B; b0 += 16) {
@@ -186,10 +192,18 @@ __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__rest
                 if (b < B) {
                     const int64_t idx = ((int64_t)b * N + j) * d + col;
                     if (dropping) dropout_apply<8>(drop, seed, static_cast<uint32_t>(idx), gv[q]);
+                    if (kMasked && j > 0 && mask[(int64_t)b * n_patch + (j - 1)] != 0) {
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) {
-                        gv[q][k] = to_f32(from_f32<T>(gv[q][k]));   // the sums are those of the rounded rows
-                        s[k] += gv[q][k];
+                        for (int k = 0; k < 8; ++k) {
+                            sm[k] += to_f32(from_f32<T>(gv[q][k]));
+                            gv[q][k] = 0.f;
+                        }
+                    } else {
+#pragma unroll
+                        for (int k = 0; k < 8; ++k) {
+                            gv[q][k] = to_f32(from_f32<T>(gv[q][k]));   // the sums are those of the rounded rows
+                            s[k] += gv[q][k];
+                        }
                     }
                     if (j > 0) store8(de + ((int64_t)b * n_patch + (j - 1)) * d + col, gv[q]);
                 }
@@ -198,16 +212,39 @@ __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__rest
     }
 #pragma unroll
     for (int k = 0; k < 8; ++k) red[ty][tx * 8 + k] = s[k];
+    if (kMasked) {
+#pragma unroll
+        for (int k = 0; k < 8; ++k) red[8 + ty][tx * 8 + k] = sm[k];
+    }
     __syncthreads();
     const int c = blockIdx.y * 256 + threadIdx.x;   // one column per thread for the fold
     if (c < d) {
         float t = 0.f;
 #pragma unroll
         for (int y = 0; y < 8; ++y) t += red[y][threadIdx.x];
-        dpos[(int64_t)j * d + c] += t;
-        if (j == 0) dcls[c] += t;
-        else atomicAdd(dbias + c, t);
+        if (kMasked) {
+            float tm = 0.f;
+#pragma unroll
+            for (int y = 0; y < 8; ++y) tm += red[8 + y][threadIdx.x];
+            dpos[(int64_t)j * d + c] += t + tm;
+            if (j == 0) dcls[c] += t;
+            else {
+                atomicAdd(dbias + c, t);
+                atomicAdd(dmask_token + c, tm);
+            }
+        } else {
+            dpos[(int64_t)j * d + c] += t;
+            if (j == 0) dcls[c] += t;
+            else atomicAdd(dbias + c, t);
+        }
     }
+}
+
+// zeros the CLS rows (b * N, b = 0..B-1) of a token-shaped [B*N, d] matrix
+template <typename T>
+__global__ void zero_cls_rows_kernel(T *__restrict__ tok, int B, int N, int d) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (int64_t)B * d; i += (int64_t)gridDim.x * blockDim.x)
+        tok[(i / d) * N * d + (i % d)] = from_f32<T>(0.f);
 }
 
 constexpr int LN_MAXV = 4;  // 4 x 8 elements per lane
@@ -270,11 +307,12 @@ __device__ __forceinline__ float pair_sum(uint64_t v) {
 // gamma / beta held in registers for the whole kernel and the NEXT row's loads in flight while the current row is reduced
 // (the kernel is latency bound: a row is load -> two shuffle reductions -> store, and the first version re-read gamma /
 // beta from L1 for every row and had nothing in flight during the reductions: 19.5 us for 40 MB in the round-1 profile).
-template <typename T, int NV, int R, int MINB, typename TX = T>
+// kPatch: output row i reads input row i + i / n_patch + 1 (the patch rows of a [B*(n_patch+1), d] token matrix)
+template <typename T, int NV, int R, int MINB, typename TX = T, bool kPatch = false>
 __global__ void __launch_bounds__(256, MINB) layernorm_fwd_kernel(const TX *__restrict__ x, const float *__restrict__ gamma,
                                                              const float *__restrict__ beta, T *__restrict__ y,
                                                              float *__restrict__ mean_out, float *__restrict__ rstd_out,
-                                                             int M, int d, float eps) {
+                                                             int M, int d, float eps, int n_patch) {
     pdl_launch_dependents();
     const int lane = threadIdx.x & 31;
     const int warps_per_block = blockDim.x >> 5;
@@ -298,7 +336,7 @@ __global__ void __launch_bounds__(256, MINB) layernorm_fwd_kernel(const TX *__re
 #pragma unroll
         for (int i = 0; i < NV; ++i) {
             const int c = (i * 32 + lane) * 8;
-            if (c < d) ld_packed(cur[i], x + row * d + c);
+            if (c < d) ld_packed(cur[i], x + (kPatch ? row + row / n_patch + 1 : row) * d + c);
         }
     }
     for (; row < M; row += total_warps) {
@@ -307,7 +345,7 @@ __global__ void __launch_bounds__(256, MINB) layernorm_fwd_kernel(const TX *__re
 #pragma unroll
             for (int i = 0; i < NV; ++i) {
                 const int c = (i * 32 + lane) * 8;
-                if (c < d) ld_packed(nxt[i], x + row_n * d + c);
+                if (c < d) ld_packed(nxt[i], x + (kPatch ? row_n + row_n / n_patch + 1 : row_n) * d + c);
             }
         }
         uint64_t v[NV][4];
@@ -365,14 +403,16 @@ __global__ void __launch_bounds__(256, MINB) layernorm_fwd_kernel(const TX *__re
 //   with s1 = mean_c(dy * gamma), s2 = mean_c(dy * gamma * xhat)
 // kDrop: dx feeds a Linear through a dropout (to_out[1] / net[4] of the block below): additionally write
 // dxm = mask * dx / (1 - p) (that Linear's dgrad / wgrad operand) and make the column sums those of dxm (its bias grad).
-template <typename T, int NV, bool kDrop, typename TX = T>
+// kPatch: dy / mean / rstd are compact patch rows; x is read from, and dx written to, token row i + i / n_patch + 1
+template <typename T, int NV, bool kDrop, typename TX = T, bool kPatch = false>
 __global__ void __launch_bounds__(256, 1) layernorm_bwd_kernel(const T *__restrict__ dy, const TX *__restrict__ x,
                                                                 const float *__restrict__ gamma,
                                                                 const float *__restrict__ mean_in,
                                                                 const float *__restrict__ rstd_in, const T *dres, T *dx,
                                                                 float *__restrict__ dgamma, float *__restrict__ dbeta,
                                                                 float *__restrict__ dcolsum, float *__restrict__ partial,
-                                                                int M, int d, T *__restrict__ dxm, DropoutParams drop) {
+                                                                int M, int d, T *__restrict__ dxm, DropoutParams drop,
+                                                                int n_patch) {
     extern __shared__ float red[];  // [warps][3][d] column partials, then [NV * 256] permuted gamma
     pdl_launch_dependents();
     pdl_wait();
@@ -410,7 +450,7 @@ __global__ void __launch_bounds__(256, 1) layernorm_bwd_kernel(const T *__restri
             const int c = (i * 32 + lane) * 8;
             if (c < d) {
                 ld_packed(a[i], dy + r_ * d + c);
-                ld_packed(b[i], x + r_ * d + c);
+                ld_packed(b[i], x + (kPatch ? r_ + r_ / n_patch + 1 : r_) * d + c);
                 if (dres != nullptr) ld_packed(c_[i], dres + r_ * d + c);
             }
         }
@@ -468,7 +508,7 @@ __global__ void __launch_bounds__(256, 1) layernorm_bwd_kernel(const T *__restri
 #pragma unroll
                     for (int k = 0; k < 4; ++k) o2[k] = add2(o2[k], r2[k]);
                 }
-                store_pairs(dx + row * d + c, o2);
+                store_pairs(dx + (kPatch ? row + row / n_patch + 1 : row) * d + c, o2);
                 if (kDrop) {
                     const uint32_t seed = __ldg(drop.seed);
                     const uint32_t e0 = static_cast<uint32_t>(row * d + c);
@@ -757,6 +797,72 @@ int ecgvit_embed_assemble_bwd(const void *dtok, void *de, float *dcls, float *dp
     return check_launch("embed_assemble_bwd");
 }
 
+int ecgvit_embed_assemble_masked(const void *e, const float *cls, const float *pos, const float *mask_token,
+                                 const uint8_t *mask, void *tok, int B, int n_patch, int d, float dropout_p,
+                                 int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream) {
+    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    ECGVIT_REQUIRE(e && cls && pos && mask_token && mask && tok && B > 0 && n_patch > 0,
+                   "embed_assemble_masked: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "embed_assemble_masked: d=%d must be a multiple of 8", d);
+    const int64_t total = (int64_t)B * (n_patch + 1) * (d / 8);
+    const int grid = grid_for(total, 256);
+    cudaStream_t st = as_stream(stream);
+    if (dtype == ECGVIT_BF16)
+        embed_assemble_kernel<bf16, bf16, true><<<grid, 256, 0, st>>>((const bf16 *)e, cls, pos, (bf16 *)tok, B, n_patch, d, drop, mask_token, mask);
+    else if (dtype == ECGVIT_BF16_RES32)
+        embed_assemble_kernel<bf16, float, true><<<grid, 256, 0, st>>>((const bf16 *)e, cls, pos, (float *)tok, B, n_patch, d, drop, mask_token, mask);
+    else if (dtype == ECGVIT_F32)
+        embed_assemble_kernel<float, float, true><<<grid, 256, 0, st>>>((const float *)e, cls, pos, (float *)tok, B, n_patch, d, drop, mask_token, mask);
+    else return fail(-1, "embed_assemble_masked: unknown dtype %d", dtype);
+    return check_launch("embed_assemble_masked");
+}
+
+int ecgvit_embed_assemble_masked_bwd(const void *dtok, const uint8_t *mask, void *de, float *dcls, float *dpos,
+                                     float *dbias, float *dmask_token, int B, int n_patch, int d, float dropout_p,
+                                     int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream) {
+    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    ECGVIT_REQUIRE(dtok && mask && de && dcls && dpos && dbias && dmask_token && B > 0 && n_patch > 0 && d > 0,
+                   "embed_assemble_masked_bwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "embed_assemble_masked_bwd: d=%d must be a multiple of 8", d);
+    dim3 grid(n_patch + 1, (d + 255) / 256);
+    cudaStream_t st = as_stream(stream);
+    if (dtype == ECGVIT_BF16)
+        embed_assemble_bwd_kernel<bf16, true><<<grid, 256, 0, st>>>((const bf16 *)dtok, (bf16 *)de, dcls, dpos, dbias, B, n_patch, d, drop, mask, dmask_token);
+    else if (dtype == ECGVIT_F32)
+        embed_assemble_bwd_kernel<float, true><<<grid, 256, 0, st>>>((const float *)dtok, (float *)de, dcls, dpos, dbias, B, n_patch, d, drop, mask, dmask_token);
+    else return fail(-1, "embed_assemble_masked_bwd: unknown dtype %d", dtype);
+    return check_launch("embed_assemble_masked_bwd");
+}
+
+int ecgvit_layernorm_patch_fwd(const void *tok, const float *gamma, const float *beta, void *y, float *mean,
+                               float *rstd, int B, int n_patch, int d, float eps, int dtype, void *stream) {
+    ECGVIT_REQUIRE(tok && gamma && beta && y && B > 0 && n_patch > 0, "layernorm_patch_fwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0 && d <= 8 * 32 * LN_MAXV, "layernorm_patch_fwd: d=%d must be a multiple of 8 and <= %d", d,
+                   8 * 32 * LN_MAXV);
+    const int M = B * n_patch;
+    const int nv = (d + 255) / 256;
+    cudaStream_t st = as_stream(stream);
+    int grid = grid_for((int64_t)M * 32, 256);
+    if (grid > sm_count() * 2) grid = sm_count() * 2;
+#define ECGVIT_LNP_FWD(TT, NVV, TXX)                                                                                    \
+    launch_pdl(layernorm_fwd_kernel<TT, NVV, 1, 2, TXX, true>, dim3(grid), dim3(256), 0, st, (const TXX *)tok, gamma, \
+               beta, (TT *)y, mean, rstd, M, d, eps, n_patch)
+#define ECGVIT_LNP_FWD_NV(TT, TXX)                   \
+    switch (nv) {                                    \
+        case 1: ECGVIT_LNP_FWD(TT, 1, TXX); break;   \
+        case 2: ECGVIT_LNP_FWD(TT, 2, TXX); break;   \
+        case 3: ECGVIT_LNP_FWD(TT, 3, TXX); break;   \
+        default: ECGVIT_LNP_FWD(TT, 4, TXX); break;  \
+    }
+    if (dtype == ECGVIT_BF16) { ECGVIT_LNP_FWD_NV(bf16, bf16) }
+    else if (dtype == ECGVIT_BF16_RES32) { ECGVIT_LNP_FWD_NV(bf16, float) }
+    else if (dtype == ECGVIT_F32) { ECGVIT_LNP_FWD_NV(float, float) }
+    else return fail(-1, "layernorm_patch_fwd: unknown dtype %d", dtype);
+#undef ECGVIT_LNP_FWD_NV
+#undef ECGVIT_LNP_FWD
+    return check_launch("layernorm_patch_fwd");
+}
+
 int ecgvit_layernorm_fwd(const void *x, const float *gamma, const float *beta, void *y, float *mean, float *rstd,
                          int M, int d, float eps, int dtype, void *stream) {
     ECGVIT_REQUIRE(x && gamma && beta && y && M > 0, "layernorm_fwd: bad arguments");
@@ -770,7 +876,7 @@ int ecgvit_layernorm_fwd(const void *x, const float *gamma, const float *beta, v
     if (grid > sm_count() * 2) grid = sm_count() * 2;
 #define ECGVIT_LN_FWD(TT, NVV)                                                                                          \
     launch_pdl(layernorm_fwd_kernel<TT, NVV, 1, 2>, dim3(grid), dim3(256), 0, st, (const TT *)x, gamma, beta, (TT *)y,   \
-               mean, rstd, M, d, eps)
+               mean, rstd, M, d, eps, 1)
     if (dtype == ECGVIT_BF16) {
         switch (nv) {
             case 1: ECGVIT_LN_FWD(bf16, 1); break;
@@ -781,7 +887,7 @@ int ecgvit_layernorm_fwd(const void *x, const float *gamma, const float *beta, v
     } else if (dtype == ECGVIT_BF16_RES32) {   // fp32 residual stream in, bf16 operand out
 #define ECGVIT_LN_FWD_R(NVV)                                                                                            \
     launch_pdl(layernorm_fwd_kernel<bf16, NVV, 1, 2, float>, dim3(grid), dim3(256), 0, st, (const float *)x, gamma, beta, \
-               (bf16 *)y, mean, rstd, M, d, eps)
+               (bf16 *)y, mean, rstd, M, d, eps, 1)
         switch (nv) {
             case 1: ECGVIT_LN_FWD_R(1); break;
             case 2: ECGVIT_LN_FWD_R(2); break;
@@ -840,7 +946,7 @@ int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, cons
         }                                                                                                              \
         launch_pdl(layernorm_bwd_kernel<TT, NVV, DROP, TXX>, dim3(grid), dim3(256), smem, st, (const TT *)dy,         \
                    (const TXX *)x, gamma, mean, rstd, (const TT *)dres, (TT *)dx, dgamma, dbeta, dcolsum, scratch, M, d, \
-                   (TT *)dxm, drop);                                                                                   \
+                   (TT *)dxm, drop, 1);                                                                                \
     } while (0)
 #define ECGVIT_LN_BWD(TT, NVV) do { if (dropping) ECGVIT_LN_BWD2(TT, NVV, true, TT); else ECGVIT_LN_BWD2(TT, NVV, false, TT); } while (0)
 #define ECGVIT_LN_BWD_R(NVV) do { if (dropping) ECGVIT_LN_BWD2(bf16, NVV, true, float); else ECGVIT_LN_BWD2(bf16, NVV, false, float); } while (0)
@@ -871,6 +977,53 @@ int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, cons
 #undef ECGVIT_LN_BWD2
     int rc = check_launch("layernorm_bwd");
     if (rc || defer_finalize) return rc;
+    return ecgvit_layernorm_bwd_finalize(scratch, dgamma, dbeta, dcolsum, M, d, stream);
+}
+
+int ecgvit_layernorm_patch_bwd(const void *dy, const void *tok, const float *gamma, const float *mean,
+                               const float *rstd, void *dtok, float *dgamma, float *dbeta, float *dcolsum,
+                               float *scratch, int B, int n_patch, int d, int dtype, void *stream) {
+    ECGVIT_REQUIRE(dy && tok && gamma && mean && rstd && dtok && dgamma && dbeta && scratch && B > 0 && n_patch > 0,
+                   "layernorm_patch_bwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0 && d <= 8 * 32 * LN_MAXV, "layernorm_patch_bwd: d=%d must be a multiple of 8 and <= %d", d,
+                   8 * 32 * LN_MAXV);
+    const int M = B * n_patch;
+    const int grid = ln_bwd_blocks(M);
+    const int nv = (d + 255) / 256;
+    const size_t smem = (8 * 3 * (size_t)d + (size_t)nv * 256) * sizeof(float);
+    cudaStream_t st = as_stream(stream);
+    const DropoutParams nodrop = make_dropout(0.f, 0, nullptr);
+    const bool bf = dtype == ECGVIT_BF16 || dtype == ECGVIT_BF16_RES32;
+    if (!bf && dtype != ECGVIT_F32) return fail(-1, "layernorm_patch_bwd: unknown dtype %d", dtype);
+    const int zgrid = grid_for((int64_t)B * d, 256);
+    if (bf) zero_cls_rows_kernel<bf16><<<zgrid, 256, 0, st>>>((bf16 *)dtok, B, n_patch + 1, d);
+    else zero_cls_rows_kernel<float><<<zgrid, 256, 0, st>>>((float *)dtok, B, n_patch + 1, d);
+#define ECGVIT_LNP_BWD(TT, NVV, TXX)                                                                                   \
+    do {                                                                                                               \
+        static bool attr_set = false;                                                                                  \
+        if (!attr_set) {                                                                                               \
+            cudaFuncSetAttribute(layernorm_bwd_kernel<TT, NVV, false, TXX, true>,                                      \
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 25 * 1024 * 4);                          \
+            attr_set = true;                                                                                           \
+        }                                                                                                              \
+        launch_pdl(layernorm_bwd_kernel<TT, NVV, false, TXX, true>, dim3(grid), dim3(256), smem, st, (const TT *)dy,  \
+                   (const TXX *)tok, gamma, mean, rstd, (const TT *)nullptr, (TT *)dtok, dgamma, dbeta, dcolsum,       \
+                   scratch, M, d, (TT *)nullptr, nodrop, n_patch);                                                     \
+    } while (0)
+#define ECGVIT_LNP_BWD_NV(TT, TXX)                   \
+    switch (nv) {                                    \
+        case 1: ECGVIT_LNP_BWD(TT, 1, TXX); break;   \
+        case 2: ECGVIT_LNP_BWD(TT, 2, TXX); break;   \
+        case 3: ECGVIT_LNP_BWD(TT, 3, TXX); break;   \
+        default: ECGVIT_LNP_BWD(TT, 4, TXX); break;  \
+    }
+    if (dtype == ECGVIT_BF16) { ECGVIT_LNP_BWD_NV(bf16, bf16) }
+    else if (dtype == ECGVIT_BF16_RES32) { ECGVIT_LNP_BWD_NV(bf16, float) }
+    else { ECGVIT_LNP_BWD_NV(float, float) }
+#undef ECGVIT_LNP_BWD_NV
+#undef ECGVIT_LNP_BWD
+    const int rc = check_launch("layernorm_patch_bwd");
+    if (rc) return rc;
     return ecgvit_layernorm_bwd_finalize(scratch, dgamma, dbeta, dcolsum, M, d, stream);
 }
 

@@ -56,6 +56,24 @@ __global__ void __launch_bounds__(256) gemm_ffma_kernel(const float *__restrict_
         __syncthreads();
     }
     const int col = n0 + tx * 4;
+    if (MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) {
+        // row partial of r^2 over this 64-column tile: the 16 threads of a row (tx, one half-warp) fold in a fixed order
+        float *rowsq = reinterpret_cast<float *>(ep.out2);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const int row = m0 + ty * 4 + i;
+            float s = 0.f;
+            if (col < N && row < M) {
+                epilogue_store<MODE, float, 4, true>(ep, row, col, acc[i]);
+#pragma unroll
+                for (int j = 0; j < 4; ++j) s = fmaf(acc[i][j], acc[i][j], s);
+            }
+#pragma unroll
+            for (int o = 8; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+            if (tx == 0 && row < M) rowsq[(int64_t)blockIdx.x * M + row] = s;
+        }
+        return;
+    }
     if (col < N) {
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -72,6 +90,8 @@ int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream) {
     ECGVIT_REQUIRE(g->N % 4 == 0 && g->ldo % 4 == 0, "gemm(f32): N=%d and ldo=%lld must be multiples of 4", g->N,
                    (long long)g->ldo);
     ECGVIT_REQUIRE((reinterpret_cast<uintptr_t>(g->out) & 15) == 0, "gemm(f32): out must be 16-byte aligned");
+    ECGVIT_REQUIRE(g->epilogue != ECGVIT_EPI_BIAS_SUB_ROWSQ || (g->aux != nullptr && g->out2 != nullptr),
+                   "gemm(f32): the row-square epilogue needs aux (target) and out2 (row partials)");
     const float *A = reinterpret_cast<const float *>(g->A), *B = reinterpret_cast<const float *>(g->B);
     const int64_t sAm = g->a_kmajor ? g->lda : 1, sAk = g->a_kmajor ? 1 : g->lda;
     const int64_t sBn = g->b_kmajor ? g->ldb : 1, sBk = g->b_kmajor ? 1 : g->ldb;
@@ -85,6 +105,7 @@ int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream) {
         ECGVIT_CASE(ECGVIT_EPI_BIAS_GELU)
         ECGVIT_CASE(ECGVIT_EPI_DGELU)
         ECGVIT_CASE(ECGVIT_EPI_ATOMIC_F32)
+        ECGVIT_CASE(ECGVIT_EPI_BIAS_SUB_ROWSQ)
 #undef ECGVIT_CASE
         default: return fail(-1, "gemm(f32): unknown epilogue %d", g->epilogue);
     }

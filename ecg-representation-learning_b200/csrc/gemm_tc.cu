@@ -109,7 +109,7 @@ int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream) {
         if ((rc = make_tmap(&to, g->out, g->N, g->M, g->ldo, 32, 32, CU_TENSOR_MAP_SWIZZLE_64B))) return rc;
         if (MODE == ECGVIT_EPI_BIAS_GELU &&
             (rc = make_tmap(&to2, g->out2, g->N, g->M, g->ldo, 32, 32, CU_TENSOR_MAP_SWIZZLE_64B))) return rc;
-        if ((MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU) &&
+        if ((MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) &&
             (rc = make_tmap(&tx, g->aux, g->N, g->M, g->ldo, 32, 32, CU_TENSOR_MAP_SWIZZLE_64B))) return rc;
     }
     auto kern = gemm_tc2_kernel<BN, A_MN, B_MN, MODE>;
@@ -141,6 +141,7 @@ template <int BN> int dispatch_pair(const ecgvit_gemm_args *g, int split_k, cuda
     ECGVIT_CASE(false, false, ECGVIT_EPI_STORE)
     ECGVIT_CASE(false, false, ECGVIT_EPI_BIAS_RES)
     ECGVIT_CASE(false, false, ECGVIT_EPI_BIAS_GELU)
+    ECGVIT_CASE(false, false, ECGVIT_EPI_BIAS_SUB_ROWSQ)
     ECGVIT_CASE(false, true, ECGVIT_EPI_STORE)
     ECGVIT_CASE(false, true, ECGVIT_EPI_DGELU)
     ECGVIT_CASE(true, true, ECGVIT_EPI_ATOMIC_F32)
@@ -172,6 +173,8 @@ int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream) {
     ECGVIT_REQUIRE((reinterpret_cast<uintptr_t>(g->bias) & 15) == 0, "gemm(bf16): bias must be 16-byte aligned");
     ECGVIT_REQUIRE(g->epilogue != ECGVIT_EPI_BIAS_RES_F32 || (g->aux != nullptr && g->a_kmajor && g->b_kmajor),
                    "gemm(bf16): the fp32-residual epilogue needs aux and K-major operands");
+    ECGVIT_REQUIRE(g->epilogue != ECGVIT_EPI_BIAS_SUB_ROWSQ || (g->aux != nullptr && g->out2 != nullptr),
+                   "gemm(bf16): the row-square epilogue needs aux (target) and out2 (row partials)");
     const int sms = sm_count();
     const int kb_total = (g->K + BK - 1) / BK;
     int split_k = g->split_k > 1 ? g->split_k : 1;

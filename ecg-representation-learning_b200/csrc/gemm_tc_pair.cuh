@@ -64,10 +64,11 @@ __device__ __forceinline__ uint32_t sw64_offset(int lane, int j) {
 // the warp's swizzled staging tile(s); for BIAS_RES / DGELU the tile already holds the aux operand (residual /
 // pre-activation), fetched by TMA while the mainloop was still running, and is updated in place.
 // The caller then issues one TMA store per tile (TMA clips rows >= M and columns >= N, so there are no guards here).
+// BIAS_SUB_ROWSQ: the tile holds the target; out = acc + bias - target, and `sq` accumulates the fp32 squares.
 template <int MODE>
 __device__ __forceinline__ void epilogue_half16(const EpiParams &ep, int64_t row, int col_base, int jbase,
                                                 const uint32_t r[16], uint8_t *tile0, uint8_t *tile1, int lane,
-                                                int n_cols) {
+                                                int n_cols, float &sq) {
     const bool drop = ep.drop.threshold != 0;  // kernel-uniform
     const uint32_t seed = drop ? __ldg(ep.drop.seed) : 0u;
 #pragma unroll
@@ -88,7 +89,7 @@ __device__ __forceinline__ void epilogue_half16(const EpiParams &ep, int64_t row
         const uint32_t soff = sw64_offset(lane, j);
         const uint32_t eidx = static_cast<uint32_t>(row * ep.ldo + col);  // element index of v[0] (even)
         if (drop && (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU)) dropout_apply<8>(ep.drop, seed, eidx, v);
-        if (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU) {
+        if (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) {
             const uint4 a4 = *reinterpret_cast<const uint4 *>(tile0 + soff);
             float a[8];
             unpack_bf16x2(a4.x, a[0], a[1]); unpack_bf16x2(a4.y, a[2], a[3]);
@@ -96,6 +97,13 @@ __device__ __forceinline__ void epilogue_half16(const EpiParams &ep, int64_t row
             if (MODE == ECGVIT_EPI_BIAS_RES) {
 #pragma unroll
                 for (int i = 0; i < 8; ++i) v[i] += a[i];
+            } else if (MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) {
+                // columns >= N hold zeros on both sides (zero-filled B rows and target columns, no bias): they add 0
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    v[i] -= a[i];
+                    sq = fmaf(v[i], v[i], sq);
+                }
             } else {
 #pragma unroll
                 for (int i = 0; i < 8; i += 2) {
@@ -160,7 +168,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                 int *__restrict__ sched_ctr, int dynamic) {
     constexpr bool kWide = MODE == ECGVIT_EPI_BIAS_RES_F32;   // (the split-K epilogue has its own fp32 path below)
     using Cfg = PairCfgFor<BN, B_MN, MODE>;
-    constexpr bool kHasAux = (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || kWide);
+    constexpr bool kRowSq = MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ;
+    constexpr bool kHasAux = (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || kWide || kRowSq);
     constexpr int STAGES = Cfg::STAGES;
     constexpr int BM2 = 2 * BM;  // rows of the pair tile
 
@@ -414,6 +423,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                 // TMEM loads are software-pipelined over the 16-column halves: the load of half s + 1 is in flight
                 // while half s is being computed (two register buffers)
                 uint32_t ra[16], rb[16];
+                float sq = 0.f;   // BIAS_SUB_ROWSQ: this row's squares over the warp's 64 columns
                 if (n_units > 0) ptx::tmem_ld_32x16(taddr0, ra);
 #pragma unroll 1
                 for (int i = 0; i < n_units; ++i) {
@@ -437,11 +447,11 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                         __syncwarp();
                     }
                     if (kWide) epilogue_half16_f32(ep, row, col_base, 0, ra, t0, lane, N);
-                    else epilogue_half16<MODE>(ep, row, col_base, 0, ra, t0, t1, lane, N);
+                    else epilogue_half16<MODE>(ep, row, col_base, 0, ra, t0, t1, lane, N, sq);
                     ptx::tmem_ld_wait_bind(rb);
                     if (i + 1 < n_units) ptx::tmem_ld_32x16(taddr0 + 32 * (i + 1), ra);
                     if (kWide) epilogue_half16_f32(ep, row, col_base, 1, rb, t0, lane, N);
-                    else epilogue_half16<MODE>(ep, row, col_base, 2, rb, t0, t1, lane, N);
+                    else epilogue_half16<MODE>(ep, row, col_base, 2, rb, t0, t1, lane, N, sq);
                     ptx::fence_proxy_async_smem();  // generic-proxy smem writes -> visible to the TMA (async proxy)
                     __syncwarp();
                     if (lane == 0) {
@@ -450,6 +460,10 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                         ptx::tma_store_commit();
                     }
                 }
+                // one fp32 partial per (64-column group, row): tiles are multiples of 64 columns wide, so the group index
+                // is global and every (group, row) has exactly one writer
+                if (kRowSq && n_units > 0 && row < M)
+                    reinterpret_cast<float *>(ep.out2)[static_cast<int64_t>(col_warp >> 6) * M + row] = sq;
             }
             ptx::tcgen05_fence_before();
             __syncwarp();

@@ -27,7 +27,7 @@ import torch
 
 from . import _lib
 from ._lib import (GemmArgs, F32, BF16, EPI_STORE, EPI_BIAS_RES, EPI_BIAS_GELU, EPI_DGELU, EPI_ATOMIC_F32,
-                   EPI_BIAS_RES_F32)
+                   EPI_BIAS_RES_F32, EPI_BIAS_SUB_ROWSQ)
 
 LN_EPS = 1e-5  # nn.LayerNorm default
 
@@ -238,16 +238,31 @@ class StepEngine:
         self._gemm(B * n, d, Kp, w.a_patch, Kp, 1, w_embed, Kp, 1, EPI_STORE, w.e, d, bias=pf['embed.b'])
         p_emb, p_blk = self._dropout_probs()
         w.p_emb, w.p_blk = p_emb, p_blk
-        seed_ptr = self.rng.data_ptr()
-        _lib.check(lib.ecgvit_embed_assemble(w.e.data_ptr(), pf['cls'].data_ptr(), pf['pos'].data_ptr(),
-                                             w.x[0].data_ptr(), B, n, d, p_emb, 0, seed_ptr if p_emb > 0 else None,
-                                             rdt, st), 'embed_assemble')
+        self._assemble(w)
         for l in range(c.num_hidden_layers):
             if hook is not None:
                 hook(l)
             self._block_forward(l, w, record_attention=record_attention)
         if hook is not None:
             hook(c.num_hidden_layers)   # head
+        return self._head_forward(w, labels, reduction)
+
+    def _assemble(self, w):
+        """token matrix x[0] = [cls | e] + pos (embedding dropout)"""
+        m, lib, st = self.model, self.lib, self._stream
+        pf = m._params_f32()
+        seed_ptr = self.rng.data_ptr()
+        _lib.check(lib.ecgvit_embed_assemble(w.e.data_ptr(), pf['cls'].data_ptr(), pf['pos'].data_ptr(),
+                                             w.x[0].data_ptr(), w.B, w.n, m.config.hidden_size, w.p_emb, 0,
+                                             seed_ptr if w.p_emb > 0 else None, m._res_code, st), 'embed_assemble')
+
+    def _head_forward(self, w, labels, reduction):
+        """CLS pool + mlp_head + BCE: (loss | None, logits)"""
+        m, lib, st = self.model, self.lib, self._stream
+        c = m.config
+        rdt = m._res_code
+        pf = m._params_f32()
+        B, N, d = w.B, w.N, c.hidden_size
         red = _lib.REDUCTION[reduction]
         loss_buf = None
         if labels is not None:
@@ -357,13 +372,7 @@ class StepEngine:
         top = (depth - 1) & 1
         # with dropout between net[3] / to_out[0] and the residual add, the Linear sees mask * dz / (1 - p): its operand
         # and its bias gradient come from the masked copy, so the producers must not pre-sum the unmasked gradient
-        _lib.check(lib.ecgvit_head_bwd(
-            w.x[depth].data_ptr(), pf['head.ln.w'].data_ptr(), pf['head.w'].data_ptr(), w.labels.data_ptr(),
-            *self._loss_weight_table(), w.xn.data_ptr(), w.hstat[0].data_ptr(), w.hstat[1].data_ptr(), w.logits.data_ptr(),
-            w.dz[top].data_ptr(),
-            gr['head.w'].data_ptr(), gr['head.b'].data_ptr(), gr['head.ln.w'].data_ptr(), gr['head.ln.b'].data_ptr(),
-            gr[last + 'ff2.b'].data_ptr() if p_blk == 0 else None, w.head_scratch.data_ptr(), B, N, d, m.num_class,
-            _lib.REDUCTION[w.reduction], float(grad_scale), _lib.ptr(grad_scale_dev), rdt, st), 'head_bwd')
+        self._head_backward(w, w.dz[top], gr[last + 'ff2.b'] if p_blk == 0 else None, grad_scale, grad_scale_dev)
         scale = float(dh) ** -0.5
 
         main, side = torch.cuda.current_stream(), self.side_stream
@@ -491,9 +500,7 @@ class StepEngine:
             before_overwrite(ev)
         dz = w.dz[(-1) & 1]   # gradient w.r.t. the token matrix (input of block 0)
         # ---- embedding: tok = [cls | a_patch We^T + be] + pos
-        _lib.check(lib.ecgvit_embed_assemble_bwd(dz.data_ptr(), w.de.data_ptr(), gr['cls'].data_ptr(),
-                                                 gr['pos'].data_ptr(), gr['embed.b'].data_ptr(), B, n, d, p_emb, 0,
-                                                 seed_ptr if p_emb > 0 else None, dt, st), 'embed_assemble_bwd')
+        self._assemble_backward(w, dz)
         if w.Kp == w.K:
             self._gemm(d, w.K, B * n, w.de, d, 0, w.a_patch, w.K, 0, EPI_ATOMIC_F32, gr['embed.w'], w.K, split_k=0)
         else:
@@ -503,3 +510,196 @@ class StepEngine:
                        'unpad_add')
         if m._after_layer_backward is not None:
             m._after_layer_backward(-1)
+
+    def _head_backward(self, w, dtok, dcolsum, grad_scale, grad_scale_dev):
+        """backward of `_head_forward`: writes the whole token-shaped gradient `dtok` of the encoder output and adds its
+        column sum into `dcolsum` (the top block's ff2 bias gradient, when not None)"""
+        m, lib, st = self.model, self.lib, self._stream
+        c = m.config
+        pf, gr = m._params_f32(), m._grads_f32()
+        _lib.check(lib.ecgvit_head_bwd(
+            w.x[c.num_hidden_layers].data_ptr(), pf['head.ln.w'].data_ptr(), pf['head.w'].data_ptr(), w.labels.data_ptr(),
+            *self._loss_weight_table(), w.xn.data_ptr(), w.hstat[0].data_ptr(), w.hstat[1].data_ptr(), w.logits.data_ptr(),
+            dtok.data_ptr(),
+            gr['head.w'].data_ptr(), gr['head.b'].data_ptr(), gr['head.ln.w'].data_ptr(), gr['head.ln.b'].data_ptr(),
+            _lib.ptr(dcolsum), w.head_scratch.data_ptr(), w.B, w.N, c.hidden_size, m.num_class,
+            _lib.REDUCTION[w.reduction], float(grad_scale), _lib.ptr(grad_scale_dev), m._res_code, st), 'head_bwd')
+
+    def _assemble_backward(self, w, dz):
+        """backward of `_assemble`: de, and the cls / pos / embedding-bias gradients"""
+        m, lib, st = self.model, self.lib, self._stream
+        gr = m._grads_f32()
+        p_emb = w.p_emb
+        _lib.check(lib.ecgvit_embed_assemble_bwd(dz.data_ptr(), w.de.data_ptr(), gr['cls'].data_ptr(),
+                                                 gr['pos'].data_ptr(), gr['embed.b'].data_ptr(), w.B, w.n,
+                                                 m.config.hidden_size, p_emb, 0,
+                                                 self.rng.data_ptr() if p_emb > 0 else None, m._dtype_code, st),
+                   'embed_assemble_bwd')
+
+
+class MaskedPatchEngine(StepEngine):
+    """StepEngine of `EcgVitForMaskedPatchModeling`: the same encoder sequence; the token assembly puts the learned
+    mask token on the masked patches and the head is the reconstruction objective
+
+        pred = LN_r(z[:, 1:]) Wr^T + br;  loss = sum over masked patches of (pred - a_patch)^2 / (n_masked * K)
+
+    Forward: mask draw (or count of the caller's mask) -> masked assembly -> blocks -> patch-row LayerNorm -> one GEMM
+    whose epilogue writes r = pred - a_patch and fp32 row partials of r^2 -> one-CTA loss fold.  Backward: dpred =
+    upstream * 2 * mask * r / (count * K) -> recon weight / bias gradients -> dgrad -> patch-row LayerNorm' into the
+    top block's gradient.  With per-lead tokens (K = P not a multiple of 8) the recon weight rows and bias are padded
+    to Kp like the embedding weight; the padded target columns are zero, so they add nothing to the loss."""
+
+    EVAL_SEED = 0x5EED5   # mask seed in eval mode: the same batch always gets the same mask
+
+    def __init__(self, model):
+        super().__init__(model)
+        self._eval_seed = torch.tensor([self.EVAL_SEED, 0], device=self.device, dtype=torch.int32)
+        self._user_mask = None
+
+    @property
+    def mask_site(self):
+        """counter-hash site of the mask keys: the dropout sites are 0 .. 4 * depth"""
+        return 4 * self.model.config.num_hidden_layers + 1
+
+    def workspace(self, B, L):
+        w = super().workspace(B, L)
+        if hasattr(w, 'mask'):
+            return w
+        m = self.model
+        d = m.config.hidden_size
+        T = m._act_dtype
+        rows, K, Kp = B * w.n, w.K, w.Kp
+        dev = self.device
+        w.mask = torch.zeros(rows, device=dev, dtype=torch.uint8)
+        w.counts = torch.zeros(B, device=dev, dtype=torch.int32)
+        w.ln_r = torch.empty(rows, d, device=dev, dtype=T)
+        w.rstat = torch.empty(2, rows, device=dev, dtype=torch.float32)
+        w.r = torch.empty(rows, Kp, device=dev, dtype=T)        # pred - target
+        w.dpred = torch.empty(rows, Kp, device=dev, dtype=T)
+        w.n_groups = (Kp + 63) // 64
+        w.rowsq = torch.empty(w.n_groups, rows, device=dev, dtype=torch.float32)
+        w.mloss = torch.zeros(1, device=dev, dtype=torch.float32)
+        w.mcount = torch.zeros(1, device=dev, dtype=torch.float32)
+        w.dln_r = torch.empty(rows, d, device=dev, dtype=T)
+        if Kp != K:
+            w.recon_wpad = torch.zeros(Kp, d, device=dev, dtype=T)
+            w.recon_bpad = torch.zeros(Kp, device=dev, dtype=torch.float32)
+            w.recon_gpad = torch.zeros(Kp * d + Kp, device=dev, dtype=torch.float32)
+        return w
+
+    def forward(self, sample_values, labels=None, reduction='mean', record_attention=False, bool_masked_pos=None):
+        """(loss, None); the loss is a view of a workspace buffer.  bool_masked_pos: optional bool [B, n_patch] (any
+        number of masked patches per record); drawn on the device when None (see `_assemble`)."""
+        assert labels is None, 'masked-patch pre-training takes no labels'
+        assert reduction == 'mean', "the masked-patch loss is a mean ('mean' reduction only)"
+        self._user_mask = bool_masked_pos
+        try:
+            return super().forward(sample_values, None, reduction, record_attention)
+        finally:
+            self._user_mask = None
+
+    def _assemble(self, w):
+        m, lib, st = self.model, self.lib, self._stream
+        pf = m._params_f32()
+        B, n = w.B, w.n
+        user = self._user_mask
+        if user is not None:
+            assert tuple(user.shape) == (B, n), f'bool_masked_pos must be [{B}, {n}], got {tuple(user.shape)}'
+            w.mask.view(B, n).copy_(user, non_blocking=True)
+            seed = None
+        else:
+            k = int(round(m.mask_ratio * n))
+            # training: the step's device seed (refreshed per forward, read at replay by a captured graph); eval: fixed
+            seed = (self.rng if m.training else self._eval_seed).data_ptr()
+        _lib.check(lib.ecgvit_mpm_mask(seed, B, n, k if user is None else 0, self.mask_site, w.mask.data_ptr(),
+                                       w.counts.data_ptr(), st), 'mpm_mask')
+        _lib.check(lib.ecgvit_embed_assemble_masked(
+            w.e.data_ptr(), pf['cls'].data_ptr(), pf['pos'].data_ptr(), pf['mask'].data_ptr(), w.mask.data_ptr(),
+            w.x[0].data_ptr(), B, n, m.config.hidden_size, w.p_emb, 0, self.rng.data_ptr() if w.p_emb > 0 else None,
+            m._res_code, st), 'embed_assemble_masked')
+
+    def _recon_params(self, w):
+        """(weight, bias) operands of the recon GEMM: padded to Kp rows in per-lead mode"""
+        m = self.model
+        wt, pf = m._weights(), m._params_f32()
+        if w.Kp == w.K:
+            return wt['recon.w'], pf['recon.b']
+        return w.recon_wpad, w.recon_bpad
+
+    def _head_forward(self, w, labels, reduction):
+        m, lib, st = self.model, self.lib, self._stream
+        c = m.config
+        d = c.hidden_size
+        pf, wt = m._params_f32(), m._weights()
+        B, n, K, Kp = w.B, w.n, w.K, w.Kp
+        rows = B * n
+        if Kp != K:
+            # rows K..Kp-1 of the padded copies stay zero (allocation)
+            _lib.check(lib.ecgvit_pad_cols(wt['recon.w'].data_ptr(), w.recon_wpad.data_ptr(), 1, K * d, Kp * d,
+                                           m._dtype_code, st), 'pad_cols')
+            _lib.check(lib.ecgvit_pad_cols(pf['recon.b'].data_ptr(), w.recon_bpad.data_ptr(), 1, K, Kp, _lib.F32, st),
+                       'pad_cols')
+        w_r, b_r = self._recon_params(w)
+        _lib.check(lib.ecgvit_layernorm_patch_fwd(
+            w.x[c.num_hidden_layers].data_ptr(), pf['recon.ln.w'].data_ptr(), pf['recon.ln.b'].data_ptr(),
+            w.ln_r.data_ptr(), w.rstat[0].data_ptr(), w.rstat[1].data_ptr(), B, n, d, LN_EPS, m._res_code, st),
+            'layernorm_patch_fwd')
+        self._gemm(rows, Kp, d, w.ln_r, d, 1, w_r, d, 1, EPI_BIAS_SUB_ROWSQ, w.r, Kp, out2=w.rowsq, aux=w.a_patch,
+                   bias=b_r)
+        _lib.check(lib.ecgvit_mpm_loss(w.rowsq.data_ptr(), w.n_groups, w.mask.data_ptr(), w.counts.data_ptr(), B, n, K,
+                                       w.mloss.data_ptr(), w.mcount.data_ptr(), st), 'mpm_loss')
+        w.reduction = reduction
+        return w.mloss[0], None
+
+    def reconstruction(self):
+        """fp32 [B, n_patch, K] prediction of the last forward (patch-matrix feature order)"""
+        w = self._cur
+        out = torch.empty(w.B, w.n, w.K, device=self.device, dtype=torch.float32)
+        _lib.check(self.lib.ecgvit_mpm_reconstruction(w.r.data_ptr(), w.a_patch.data_ptr(), out.data_ptr(), w.B * w.n,
+                                                      w.Kp, w.K, self.model._dtype_code, self._stream),
+                   'mpm_reconstruction')
+        return out
+
+    def mask(self):
+        """bool [B, n_patch] mask of the last forward (a copy)"""
+        w = self._cur
+        return w.mask.view(w.B, w.n).bool()
+
+    def _head_backward(self, w, dtok, dcolsum, grad_scale, grad_scale_dev):
+        m, lib, st = self.model, self.lib, self._stream
+        c = m.config
+        d = c.hidden_size
+        dt = m._dtype_code
+        pf, gr = m._params_f32(), m._grads_f32()
+        B, n, K, Kp = w.B, w.n, w.K, w.Kp
+        rows = B * n
+        _lib.check(lib.ecgvit_mpm_dpred(w.r.data_ptr(), w.mask.data_ptr(), w.mcount.data_ptr(), rows, Kp, K,
+                                        float(grad_scale), _lib.ptr(grad_scale_dev), w.dpred.data_ptr(), dt, st),
+                   'mpm_dpred')
+        # recon weight gradient dWr = dpred^T ln_r (split-K) and bias gradient colsum(dpred)
+        if Kp == K:
+            self._gemm(Kp, d, rows, w.dpred, Kp, 0, w.ln_r, d, 0, EPI_ATOMIC_F32, gr['recon.w'], d, split_k=0)
+            _lib.check(lib.ecgvit_colsum(w.dpred.data_ptr(), gr['recon.b'].data_ptr(), rows, K, Kp, dt, st), 'colsum')
+        else:
+            w.recon_gpad.zero_()
+            gw, gb = w.recon_gpad[:Kp * d], w.recon_gpad[Kp * d:]
+            self._gemm(Kp, d, rows, w.dpred, Kp, 0, w.ln_r, d, 0, EPI_ATOMIC_F32, gw, d, split_k=0)
+            _lib.check(lib.ecgvit_colsum(w.dpred.data_ptr(), gb.data_ptr(), rows, Kp, Kp, dt, st), 'colsum')
+            _lib.check(lib.ecgvit_unpad_add_f32(gw.data_ptr(), gr['recon.w'].data_ptr(), 1, K * d, Kp * d, st),
+                       'unpad_add')
+            _lib.check(lib.ecgvit_unpad_add_f32(gb.data_ptr(), gr['recon.b'].data_ptr(), 1, K, Kp, st), 'unpad_add')
+        w_r, _ = self._recon_params(w)
+        self._gemm(rows, d, Kp, w.dpred, Kp, 1, w_r, d, 0, EPI_STORE, w.dln_r, d)
+        _lib.check(lib.ecgvit_layernorm_patch_bwd(
+            w.dln_r.data_ptr(), w.x[c.num_hidden_layers].data_ptr(), pf['recon.ln.w'].data_ptr(), w.rstat[0].data_ptr(),
+            w.rstat[1].data_ptr(), dtok.data_ptr(), gr['recon.ln.w'].data_ptr(), gr['recon.ln.b'].data_ptr(),
+            _lib.ptr(dcolsum), w.ln_scratch[0].data_ptr(), B, n, d, m._res_code, st), 'layernorm_patch_bwd')
+
+    def _assemble_backward(self, w, dz):
+        m, lib, st = self.model, self.lib, self._stream
+        gr = m._grads_f32()
+        p_emb = w.p_emb
+        _lib.check(lib.ecgvit_embed_assemble_masked_bwd(
+            dz.data_ptr(), w.mask.data_ptr(), w.de.data_ptr(), gr['cls'].data_ptr(), gr['pos'].data_ptr(),
+            gr['embed.b'].data_ptr(), gr['mask'].data_ptr(), w.B, w.n, m.config.hidden_size, p_emb, 0,
+            self.rng.data_ptr() if p_emb > 0 else None, m._dtype_code, st), 'embed_assemble_masked_bwd')

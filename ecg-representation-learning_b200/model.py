@@ -17,9 +17,10 @@ from torch import nn
 
 from . import _lib
 from .config import EcgVitConfig
-from .engine import StepEngine
+from .engine import StepEngine, MaskedPatchEngine
 
 ModelOutput = namedtuple('ModelOutput', ['loss', 'logits'])  # reference: util/models.py:3
+MaskedPatchOutput = namedtuple('MaskedPatchOutput', ['loss', 'reconstruction', 'bool_masked_pos'])
 
 _ALIGN = 64  # elements: every tensor starts on a 256-byte boundary of the flat buffers
 
@@ -78,10 +79,13 @@ class Transformer(nn.Module):
 
 
 class ViT(nn.Module):
-    """parameter container with vit_pytorch.ViT's attribute names / init distributions"""
+    """parameter container with vit_pytorch.ViT's attribute names / init distributions.
+    head=False leaves out `mlp_head`; mask_token=True adds the zero-initialised `mask_token` [1, 1, dim] of masked-patch
+    pre-training, registered right after `cls_token`: the flat buffers follow registration order, so its gradient
+    (produced last, by the embedding backward) sits with the other pre-block parameters in the last gradient bucket."""
 
     def __init__(self, *, signal_length, patch_size, num_classes, dim, depth, heads, mlp_dim, channels, dim_head,
-                 dropout, emb_dropout, per_lead=False):
+                 dropout, emb_dropout, per_lead=False, head=True, mask_token=False):
         super().__init__()
         assert signal_length % patch_size == 0, 'Image dimensions must be divisible by the patch size.'
         n_patch = signal_length // patch_size * (channels if per_lead else 1)
@@ -90,11 +94,14 @@ class ViT(nn.Module):
                                                 nn.Linear(patch_dim, dim))
         self.pos_embedding = nn.Parameter(torch.randn(1, n_patch + 1, dim))
         self.cls_token = nn.Parameter(torch.randn(1, 1, dim))
+        if mask_token:
+            self.mask_token = nn.Parameter(torch.zeros(1, 1, dim))
         self.dropout = _Slot(f'Dropout(p={emb_dropout})')
         self.transformer = Transformer(dim, depth, heads, dim_head, mlp_dim, dropout)
         self.pool = 'cls'
         self.to_latent = nn.Identity()
-        self.mlp_head = nn.Sequential(nn.LayerNorm(dim), nn.Linear(dim, num_classes))
+        if head:
+            self.mlp_head = nn.Sequential(nn.LayerNorm(dim), nn.Linear(dim, num_classes))
     forward = _no_eager
 
 
@@ -114,7 +121,7 @@ class _EcgVitFunction(torch.autograd.Function):
         return loss, logits
 
     @staticmethod
-    def backward(ctx, grad_loss, _grad_logits):
+    def backward(ctx, grad_loss, *_grad_outputs):
         model = ctx.model
         eng = model._engine
         if ctx.ws.fwd_id != ctx.fwd_id:
@@ -148,6 +155,9 @@ class _EcgVitFunction(torch.autograd.Function):
 
 
 class EcgVit(nn.Module):
+    _classification_head = True   # ViT container with `mlp_head` and no mask token
+    _engine_class = StepEngine
+
     def __init__(self, num_class: int = 71, config: EcgVitConfig = None, loss_reduction: str = 'mean'):
         super().__init__()
         config = config if config is not None else EcgVitConfig()
@@ -160,7 +170,8 @@ class EcgVit(nn.Module):
                        channels=config.num_channels, dim_head=hd_sz // n_head,
                        dropout=config.hidden_dropout_prob,              # attention + feed-forward (ecg_vit.py:113)
                        emb_dropout=config.attention_probs_dropout_prob,  # embedding (ecg_vit.py:114)
-                       per_lead=bool(getattr(config, 'per_lead_tokens', False)))
+                       per_lead=bool(getattr(config, 'per_lead_tokens', False)),
+                       head=self._classification_head, mask_token=not self._classification_head)
         self.vit._owner = weakref.ref(self)  # lets `Recorder(model.vit)` reach the kernels (not a module: no cycle)
         self._loss_reduction = loss_reduction
         self.loss_weight = None
@@ -224,7 +235,7 @@ class EcgVit(nn.Module):
                 time_out_spans = pipe.draw_spans(sample_values.shape[0], pipe.padded_length(sample_values.shape[2]))
             self._engine.set_spans(time_out_spans)
         need_grad = torch.is_grad_enabled() and labels is not None and any(p.requires_grad for p in self.parameters())
-        if self.training and (self.config.hidden_dropout_prob > 0 or self.config.attention_probs_dropout_prob > 0):
+        if self._draws_step_seed():
             self._engine.new_dropout_seed()  # masks of this forward; its backward regenerates them from the same seed
         if need_grad:
             loss, logits = _EcgVitFunction.apply(self, sample_values, labels, *self._param_list())
@@ -233,6 +244,10 @@ class EcgVit(nn.Module):
             loss = None if loss is None else loss.clone()
             logits = logits.clone()
         return ModelOutput(loss=loss, logits=logits)
+
+    def _draws_step_seed(self):
+        """whether a training forward needs a fresh device seed (dropout masks)"""
+        return self.training and (self.config.hidden_dropout_prob > 0 or self.config.attention_probs_dropout_prob > 0)
 
     # ---- flat storage ------------------------------------------------------------------------------
     def _param_list(self):
@@ -243,10 +258,15 @@ class EcgVit(nn.Module):
         out = OrderedDict()
         for name, _ in self.named_parameters():
             parts = name.split('.')
-            if name == 'vit.pos_embedding':
+            wb = 'w' if parts[-1] == 'weight' else 'b'
+            if parts[0] == 'recon_head':
+                k = ('recon.ln.' if parts[1] == '0' else 'recon.') + wb
+            elif name == 'vit.pos_embedding':
                 k = 'pos'
             elif name == 'vit.cls_token':
                 k = 'cls'
+            elif name == 'vit.mask_token':
+                k = 'mask'
             elif parts[1] == 'to_patch_embedding':
                 k = 'embed.' + ('w' if parts[-1] == 'weight' else 'b')
             elif parts[1] == 'mlp_head':
@@ -285,7 +305,7 @@ class EcgVit(nn.Module):
         self._views_w = self._views_p if self._shadow is None else \
             {k: self._shadow[o:o + n].view(shape) for k, (o, n, shape, _) in layout.items()}
         self._shadow_versions = None
-        self._engine = StepEngine(self)
+        self._engine = self._engine_class(self)
 
     def _is_flat(self, device):
         if self._flat_p is None or self._flat_p.device != device:
@@ -330,6 +350,101 @@ class EcgVit(nn.Module):
     def _grad_views(self):
         names = self._short_names()
         return [self._views_g[k] for k in names.values()]
+
+
+class _MaskedPatchFunction(_EcgVitFunction):
+    """autograd bridge of `EcgVitForMaskedPatchModeling` (`loss.backward()` then e.g. `FusedAdamW`); backward, with its
+    workspace / seed guards, is `_EcgVitFunction`'s"""
+
+    @staticmethod
+    def forward(ctx, model, sample_values, bool_masked_pos, *params):
+        eng = model._engine
+        loss, _ = eng.forward(sample_values, bool_masked_pos=bool_masked_pos)
+        ctx.model = model
+        ctx.ws = eng._cur
+        ctx.fwd_id = ctx.ws.fwd_id
+        ctx.seed = eng.last_seed
+        recon, mask = eng.reconstruction(), eng.mask()
+        ctx.mark_non_differentiable(recon, mask)
+        return loss.clone(), recon, mask
+
+
+class EcgVitForMaskedPatchModeling(EcgVit):
+    """SimMIM-style masked-patch pre-training of the `EcgVit` encoder on unlabelled records.
+
+    Masked patches keep their place in the sequence (the encoder's shapes do not change) and enter it as the learned
+    `vit.mask_token`; `recon_head` = LayerNorm + Linear(d, patch_dim) predicts every patch from its encoder output, and
+    the loss is the mean squared error over the masked patches:
+
+        loss = sum_{masked (b, w), k < K} (pred - a)^2 / (n_masked * K),   a = the patch matrix (the embedding's input)
+
+    `forward(sample_values, bool_masked_pos=None)` -> `MaskedPatchOutput(loss, reconstruction, bool_masked_pos)`:
+    `reconstruction` is fp32 [B, n, patch_dim] in the patch matrix's feature order (`t*C + c`, or `t` with per-lead
+    tokens; `unpatchify` maps it back to [B, C, L]).  It is rebuilt as r + a from the residual r = pred - a that the
+    loss GEMM stores, so in bf16 mode it carries r's bf16 rounding (relative error up to ~1e-2): an output to look
+    at, not the loss's own prediction; `bool_masked_pos` [B, n] is the mask used.  Without one, exactly
+    round(mask_ratio * n) patches per record are masked: in training mode drawn afresh every forward from the step's
+    device seed (a captured training step draws new masks on every replay), in eval mode from a fixed seed (the same
+    batch always gets the same mask).
+
+    `encoder_state_dict()` hands the encoder over to fine-tuning:
+    `EcgVit(config=...).load_state_dict(pre.encoder_state_dict(), strict=False)` misses only `vit.mlp_head.*`."""
+    _classification_head = False
+    _engine_class = MaskedPatchEngine
+
+    def __init__(self, config: EcgVitConfig = None, mask_ratio: float = 0.5):
+        if not 0.0 <= float(mask_ratio) <= 1.0:
+            raise ValueError(f'mask_ratio must lie in [0, 1], got {mask_ratio}')
+        super().__init__(num_class=0, config=config)
+        c = self.config
+        per_lead = bool(getattr(c, 'per_lead_tokens', False))
+        patch_dim = c.patch_size if per_lead else c.patch_size * c.num_channels
+        if not per_lead and patch_dim % 8 != 0:
+            # the residual / its gradient share the patch matrix's row length, and their column kernels read 8 elements
+            # at a time (per-lead rows are padded to a multiple of 8 instead)
+            raise ValueError(f'masked-patch pre-training needs patch_size * num_channels = {patch_dim} to be a multiple '
+                             f'of 8')
+        self.recon_head = nn.Sequential(nn.LayerNorm(c.hidden_size), nn.Linear(c.hidden_size, patch_dim))
+        self.mask_ratio = float(mask_ratio)
+
+    def _draws_step_seed(self):
+        return self.training   # the mask is drawn afresh every training forward
+
+    def encoder_state_dict(self):
+        """the `vit.*` entries an `EcgVit` loads (everything but the mask token)"""
+        return OrderedDict((k, v) for k, v in self.state_dict().items()
+                           if k.startswith('vit.') and k != 'vit.mask_token')
+
+    def unpatchify(self, reconstruction):
+        """[B, n, patch_dim] in patch-matrix feature order -> [B, C, L] (the inverse of the patch gather)"""
+        c = self.config
+        B, n, K = reconstruction.shape
+        P, C = c.patch_size, c.num_channels
+        if bool(getattr(c, 'per_lead_tokens', False)):
+            return reconstruction.reshape(B, C, (n // C) * P)
+        return reconstruction.reshape(B, n, P, C).permute(0, 3, 1, 2).reshape(B, C, n * P)
+
+    def forward(self, sample_values: torch.FloatTensor, bool_masked_pos: torch.BoolTensor = None, time_out_spans=None):
+        if self._flush_pending is not None:
+            self._flush_pending()
+        self._prepare(sample_values.device)
+        pipe = self.input_pipeline
+        if pipe is not None and pipe.timeout is not None and self.training:
+            if time_out_spans is None:
+                time_out_spans = pipe.draw_spans(sample_values.shape[0], pipe.padded_length(sample_values.shape[2]))
+            self._engine.set_spans(time_out_spans)
+        if bool_masked_pos is not None:
+            bool_masked_pos = bool_masked_pos.to(device=sample_values.device, dtype=torch.bool)
+        if self._draws_step_seed():
+            self._engine.new_dropout_seed()   # mask and dropout of this forward; backward reuses both
+        need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters())
+        if need_grad:
+            loss, recon, mask = _MaskedPatchFunction.apply(self, sample_values, bool_masked_pos, *self._param_list())
+        else:
+            eng = self._engine
+            loss, _ = eng.forward(sample_values, bool_masked_pos=bool_masked_pos)
+            loss, recon, mask = loss.clone(), eng.reconstruction(), eng.mask()
+        return MaskedPatchOutput(loss=loss, reconstruction=recon, bool_masked_pos=mask)
 
 
 class Recorder(nn.Module):

@@ -223,7 +223,8 @@ class FusedTrainer:
         before block 0 (pos, cls, patch embedding), l = block l, depth = the head"""
         m = self.model
         depth = m.config.num_hidden_layers
-        starts = [m._layout[f'l{l}.ln1.w'][0] for l in range(depth)] + [m._layout['head.ln.w'][0]]
+        head = 'head.ln.w' if 'head.ln.w' in m._layout else 'recon.ln.w'   # classification or reconstruction head
+        starts = [m._layout[f'l{l}.ln1.w'][0] for l in range(depth)] + [m._layout[head][0]]
         n = m._flat_p.numel()
         out = [(-1, 0, starts[0])]
         for l in range(depth):
@@ -273,11 +274,15 @@ class FusedTrainer:
         self._hyper_ring.upload(self.hyper, self._hyper_values(t))
         self._apply_update(torch.cuda.current_stream())
 
-    def step(self, sample_values, labels, time_out_spans=None):
+    def step(self, sample_values, labels=None, time_out_spans=None):
         """One optimisation step on device-resident fp32 inputs; returns (loss, logits) device tensors (no sync).
 
         The returned tensors are views of workspace buffers: valid until the next step.  With an `input_pipeline` on
-        the model, `sample_values` are raw records; `time_out_spans` as in `EcgVit.forward`."""
+        the model, `sample_values` are raw records; `time_out_spans` as in `EcgVit.forward`.
+        An `EcgVitForMaskedPatchModeling` takes no labels (its masks are drawn on the device) and returns (loss, None)."""
+        pretrain = getattr(self.model, 'mask_ratio', None) is not None
+        if (labels is None) != pretrain:
+            raise ValueError('a masked-patch model trains without labels' if pretrain else 'EcgVit.step needs labels')
         self._ensure_state(sample_values.device)
         self._upload_hyper()
         pipe = self.model.input_pipeline
@@ -285,8 +290,7 @@ class FusedTrainer:
             if time_out_spans is None:
                 time_out_spans = pipe.draw_spans(sample_values.shape[0], pipe.padded_length(sample_values.shape[2]))
             self.model._engine.set_spans(time_out_spans)  # a persistent device buffer: the captured graph reads it
-        cfg = self.model.config
-        if self.model.training and (cfg.hidden_dropout_prob > 0 or cfg.attention_probs_dropout_prob > 0):
+        if self.model._draws_step_seed():
             self.model._engine.new_dropout_seed()  # a device scalar: the captured graph reads the fresh value
         if self.use_cuda_graph:
             out = self._graph_step(sample_values, labels)
@@ -307,15 +311,19 @@ class FusedTrainer:
         cfg = self.model.config
         # everything the capture bakes in: shapes, loss weighting / reduction, train vs eval (dropout on or off and its
         # probabilities), the input pipeline, and the flat buffers the kernels point at
-        key = (tuple(sample_values.shape), tuple(labels.shape), tuple(float(v) for v in lw) if lw else None,
+        # (a masked-patch model: no labels, and its mask ratio sets how many patches the captured mask draw takes)
+        key = (tuple(sample_values.shape), None if labels is None else tuple(labels.shape),
+               tuple(float(v) for v in lw) if lw else None,
                self.model.training, float(cfg.hidden_dropout_prob), float(cfg.attention_probs_dropout_prob),
                self.model.loss_reduction, self.model._flat_p.data_ptr(),
-               None if pipe is None else (id(pipe), pipe.pad, pipe.timeout))
+               None if pipe is None else (id(pipe), pipe.pad, pipe.timeout), getattr(self.model, 'mask_ratio', None))
         if self._graph is None or self._graph_key != key:
             self._static_x = torch.empty_like(sample_values)
-            self._static_y = torch.empty(labels.shape, device=labels.device, dtype=torch.float32)
+            self._static_y = None if labels is None else \
+                torch.empty(labels.shape, device=labels.device, dtype=torch.float32)
             self._static_x.copy_(sample_values)
-            self._static_y.copy_(labels)
+            if labels is not None:
+                self._static_y.copy_(labels)
             # eager warm-up (sets function attributes, allocates workspaces) on a side stream, then capture;
             # parameters/optimizer state are snapshotted so the warm-up does not count as a step
             self.flush()   # the warm-up below must not apply a pending update twice
@@ -335,7 +343,8 @@ class FusedTrainer:
             self.launches_per_step = _lib.launch_counter[0] - n0  # kernels of ours replayed by every graph launch
             self._graph, self._graph_key = g, key
         self._static_x.copy_(sample_values, non_blocking=True)
-        self._static_y.copy_(labels, non_blocking=True)
+        if labels is not None:
+            self._static_y.copy_(labels, non_blocking=True)
         self._graph.replay()
         return self._graph_out
 

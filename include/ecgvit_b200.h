@@ -41,7 +41,13 @@ enum {
     ECGVIT_EPI_BIAS_GELU = 2,  /* out = acc + bias ; out2 = gelu_erf(out)                         */
     ECGVIT_EPI_DGELU = 3,      /* out = acc * gelu_erf'(aux)                                      */
     ECGVIT_EPI_ATOMIC_F32 = 4, /* out(fp32) += acc                (weight gradients, split-K)     */
-    ECGVIT_EPI_BIAS_RES_F32 = 5 /* out(fp32) = acc + bias + aux(fp32)  (bf16 GEMM, fp32 residual stream) */
+    ECGVIT_EPI_BIAS_RES_F32 = 5, /* out(fp32) = acc + bias + aux(fp32)  (bf16 GEMM, fp32 residual stream) */
+    /* out = acc + bias - aux  (the residual of a prediction against the target `aux`, same dtype / ld as out) and
+     * out2 = fp32 [ceil(N / 64), M] row partials of its square: out2[g * M + m] = sum over the columns
+     * 64g .. min(64g + 64, N) - 1 of (acc + bias - aux)^2, taken in fp32 before out is rounded to dtype.  Plain stores,
+     * no atomics, so the partials (and a loss folded from them in a fixed order) are bit-identical from run to run.
+     * K-major A and B only; no dropout. */
+    ECGVIT_EPI_BIAS_SUB_ROWSQ = 6
 };
 
 enum { ECGVIT_REDUCTION_MEAN = 0, ECGVIT_REDUCTION_SUM = 1, ECGVIT_REDUCTION_NONE = 2 };
@@ -90,6 +96,50 @@ int ecgvit_embed_assemble(const void *e, const float *cls, const float *pos, voi
 int ecgvit_embed_assemble_bwd(const void *dtok, void *de, float *dcls, float *dpos, float *dbias, int B,
                               int n_patch, int d, float dropout_p, int dropout_stream,
                               const uint32_t *dropout_seed, int dtype, void *stream);
+
+/* ---- masked-patch pre-training (SimMIM-style: masked patches keep their place in the sequence).
+ *      Added in ABI version 7 without changing any earlier entry point, so the version number stays 7.
+ *
+ *      Mask draw: patch w of record b is masked iff the rank of its key hash(seed, site, b*n_patch + w) (the 32-bit
+ *      counter hash of the dropout masks, csrc/common.cuh) among the n_patch keys of its record is < k, ties broken by
+ *      the lower index: exactly k masked patches per record.  `site` keeps the keys apart from the dropout sites
+ *      (0 .. 4*depth).  mask: uint8 [B, n_patch]; counts: int32 [B], the masked patches of every record.
+ *      seed == NULL: `mask` already holds a caller-supplied mask (any count per record) and is only counted.
+ *      One CTA per record, the keys in shared memory (n_patch <= 12000); O(n_patch^2) compares per record. */
+int ecgvit_mpm_mask(const uint32_t *seed, int B, int n_patch, int k, int site, uint8_t *mask, int *counts,
+                    void *stream);
+/* tok[b,0,:] = cls + pos[0];  tok[b,1+w,:] = (mask[b*n_patch+w] ? mask_token : e[b*n_patch+w,:]) + pos[1+w]
+ * (ecgvit_embed_assemble with masked patches replaced by the learned token; dropout / dtype as there) */
+int ecgvit_embed_assemble_masked(const void *e, const float *cls, const float *pos, const float *mask_token,
+                                 const uint8_t *mask, void *tok, int B, int n_patch, int d, float dropout_p,
+                                 int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream);
+/* backward of the above: de = g[:,1:,:] on visible rows and 0 on masked rows; dpos += sum_b g; dcls += sum_b g[:,0];
+ * dbias += sum over visible rows; dmask_token += sum over masked rows */
+int ecgvit_embed_assemble_masked_bwd(const void *dtok, const uint8_t *mask, void *de, float *dcls, float *dpos,
+                                     float *dbias, float *dmask_token, int B, int n_patch, int d, float dropout_p,
+                                     int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream);
+/* LayerNorm over the PATCH rows of a token matrix tok [B*(n_patch+1), d]: y[b*n_patch+w] = LN(tok[b*(n_patch+1)+1+w]);
+ * y, mean and rstd are compact ([B*n_patch, d], [B*n_patch]).  dtype ECGVIT_BF16_RES32: tok is fp32, y bf16. */
+int ecgvit_layernorm_patch_fwd(const void *tok, const float *gamma, const float *beta, void *y, float *mean,
+                               float *rstd, int B, int n_patch, int d, float eps, int dtype, void *stream);
+/* its backward: dtok (token-shaped, dtype of dy) is FULLY written: LN'(dy) on the patch rows, zeros on the CLS rows;
+ * dgamma += ..; dbeta += ..; dcolsum (optional) += colsum(dtok).  scratch as for ecgvit_layernorm_bwd. */
+int ecgvit_layernorm_patch_bwd(const void *dy, const void *tok, const float *gamma, const float *mean,
+                               const float *rstd, void *dtok, float *dgamma, float *dbeta, float *dcolsum,
+                               float *scratch, int B, int n_patch, int d, int dtype, void *stream);
+/* Masked-patch MSE from the row partials of ECGVIT_EPI_BIAS_SUB_ROWSQ (rowsq fp32 [n_groups, B*n_patch]):
+ *      count[0] = sum_b counts[b];  loss[0] = sum over masked rows, in a fixed order, of their partials / (count * K).
+ *      One CTA: bit-identical from run to run.  count 0 gives NaN, as torch's mean over an empty selection. */
+int ecgvit_mpm_loss(const float *rowsq, int n_groups, const uint8_t *mask, const int *counts, int B, int n_patch,
+                    int K, float *loss, float *count, void *stream);
+/* gradient of that loss w.r.t. the prediction: dpred = r * mask_row * 2 * grad_scale (* *grad_scale_dev) / (count * K)
+ * for r [rows, ld] (dtype), mask [rows], count the device scalar written by ecgvit_mpm_loss; no host sync */
+int ecgvit_mpm_dpred(const void *r, const uint8_t *mask, const float *count, int rows, int ld, int K,
+                     float grad_scale, const float *grad_scale_dev, void *dpred, int dtype, void *stream);
+/* reconstruction = r + target as fp32 [rows, K] (r, target: [rows, ld] in dtype).  In bf16 mode r is the stored bf16
+ * residual, so this is bf16(pred - target) + target: an inspection output, not the exact prediction. */
+int ecgvit_mpm_reconstruction(const void *r, const void *target, float *out, int rows, int ld, int K, int dtype,
+                              void *stream);
 
 /* ---- nn.LayerNorm(d, eps) forward (PreNorm.norm / mlp_head[0]); saves per-row mean and rstd (fp32) */
 int ecgvit_layernorm_fwd(const void *x, const float *gamma, const float *beta, void *y, float *mean,
