@@ -6,7 +6,8 @@ The directory name follows the build contract (`ecg-representation-learning_b200
 through the shim at the repo root.
 """
 from .config import EcgVitConfig
-from .model import EcgVit, ModelOutput, Recorder, EcgVitForMaskedPatchModeling, MaskedPatchOutput
+from .model import EcgVit, ModelOutput, Recorder, EcgVitForMaskedPatchModeling, MaskedPatchOutput, \
+    EcgVitForMaskedAutoencoding
 from .trainer import FusedTrainer, fused_train_step, get_train_args, lr_multiplier
 from .optim import FusedAdamW, clip_grad_norm_
 from .transform import InputPipeline
@@ -14,5 +15,6 @@ from .metrics import get_accuracy, evaluate
 from .synthetic import synthetic_batch
 from . import _lib
 
-__all__ = ['EcgVitConfig', 'EcgVit', 'ModelOutput', 'EcgVitForMaskedPatchModeling', 'MaskedPatchOutput', 'FusedTrainer', 'fused_train_step', 'FusedAdamW', 'clip_grad_norm_',
+__all__ = ['EcgVitConfig', 'EcgVit', 'ModelOutput', 'EcgVitForMaskedPatchModeling', 'EcgVitForMaskedAutoencoding',
+           'MaskedPatchOutput', 'FusedTrainer', 'fused_train_step', 'FusedAdamW', 'clip_grad_norm_',
            'get_train_args', 'lr_multiplier', 'InputPipeline', 'Recorder', 'get_accuracy', 'evaluate', 'synthetic_batch']

@@ -58,6 +58,13 @@ SIGNATURES = {
     'ecgvit_mpm_dpred': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_float, c_void_p, c_void_p, c_int,
                          c_void_p],
     'ecgvit_mpm_reconstruction': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
+    'ecgvit_mae_index': [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p],
+    'ecgvit_row_gather': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p],
+    'ecgvit_embed_assemble_visible': [c_void_p] * 5 + [c_int, c_int, c_int, c_float, c_int, c_void_p, c_int, c_void_p],
+    'ecgvit_embed_assemble_visible_bwd': [c_void_p] * 7 + [c_int, c_int, c_int, c_int, c_float, c_int, c_void_p, c_int,
+                                                           c_void_p],
+    'ecgvit_mae_unshuffle': [c_void_p] * 5 + [c_int, c_int, c_int, c_int, c_int, c_void_p],
+    'ecgvit_mae_unshuffle_bwd': [c_void_p] * 6 + [c_int, c_int, c_int, c_int, c_int, c_void_p],
     'ecgvit_dropout_bwd_copy': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_float, c_int, c_void_p, c_int,
                                 c_void_p],
     'ecgvit_layernorm_fwd': [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float,
@@ -118,7 +125,8 @@ def last_error():
 
 
 # kernels launched per successful entry-point call (memsets are not kernels); feeds bench.py's `gpu_launches`
-KERNELS_PER_CALL = {'layernorm_patch_bwd': 3, 'attention_bwd_flash': 3, 'head_fwd': 2, 'head_bwd': 3, 'layernorm_bwd': 2, 'layernorm_bwd_partial': 1, 'grad_sumsq': 2, 'eval_metrics': 3}
+KERNELS_PER_CALL = {'layernorm_patch_bwd': 3, 'attention_bwd_flash': 3, 'head_fwd': 2, 'head_bwd': 3, 'layernorm_bwd': 2, 'layernorm_bwd_partial': 1, 'grad_sumsq': 2, 'eval_metrics': 3,
+                    'embed_assemble_visible_bwd': 3, 'mae_unshuffle_bwd': 3}
 launch_counter = [0]
 
 

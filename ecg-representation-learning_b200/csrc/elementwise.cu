@@ -132,11 +132,18 @@ __global__ void unpad_add_kernel(const float *__restrict__ src, float *__restric
 // ---------------------------------------------------------------------------------------------------
 // tok[b,0,:] = cls + pos[0];  tok[b,1+w,:] = e[b*n+w,:] + pos[1+w,:]
 // kMasked: rows with mask[b*n+w] != 0 take mask_token instead of e (masked-patch pre-training)
-template <typename T, typename TO, bool kMasked = false>
+// kVisible: n_patch is the number of VISIBLE patches of every record (MAE encoder); row 1+j of record b takes
+// e[b*n_patch+j] and pos[1 + vis_idx[b*n_patch+j]]
+template <typename T, typename TO, bool kMasked = false, bool kVisible = false>
 __global__ void embed_assemble_kernel(const T *__restrict__ e, const float *__restrict__ cls,
                                       const float *__restrict__ pos, TO *__restrict__ tok, int B, int n_patch, int d,
                                       DropoutParams drop, const float *__restrict__ mask_token = nullptr,
-                                      const uint8_t *__restrict__ mask = nullptr) {
+                                      const uint8_t *__restrict__ mask = nullptr,
+                                      const int *__restrict__ vis_idx = nullptr) {
+    if constexpr (kVisible) {
+        pdl_launch_dependents();
+        pdl_wait();
+    }
     const bool dropping = drop.threshold != 0;
     const uint32_t seed = dropping ? __ldg(drop.seed) : 0u;
     const int N = n_patch + 1;
@@ -148,7 +155,8 @@ __global__ void embed_assemble_kernel(const T *__restrict__ e, const float *__re
         const int j = (int)(r % N);
         const int64_t b = r / N;
         float v[8], p[8];
-        load8(pos + (int64_t)j * d + c, p);
+        if constexpr (kVisible) load8(pos + (int64_t)(j == 0 ? 0 : 1 + vis_idx[b * n_patch + (j - 1)]) * d + c, p);
+        else load8(pos + (int64_t)j * d + c, p);
         if (j == 0) load8(cls + c, v);
         else if (kMasked && mask[b * n_patch + (j - 1)] != 0) load8(mask_token + c, v);
         else load8(e + (b * n_patch + (j - 1)) * d + c, v);
@@ -163,16 +171,33 @@ __global__ void embed_assemble_kernel(const T *__restrict__ e, const float *__re
 // gradient rows are copied to `de` on the way (16-byte accesses, one dropout hash per pair) and the batch sums are folded
 // through shared memory.  (One 2-byte element per thread with a hash per element was instruction bound: 22 us for 40 MB.)
 // kMasked: masked rows (mask[b*n+w] != 0) send their gradient to dmask_token instead of de / dbias (de rows are zeroed)
-template <typename T, bool kMasked = false>
+// kVisible (MAE encoder, n_vis visible patches per record, dtok [B*(n_vis+1), d], de [B*n_vis, d]): blockIdx.x is the
+// patch POSITION p (0 = CLS); record b contributes its token row 1 + slot[b*n_patch+p-1] when that patch is visible.
+// Instead of the atomic bias add, the position's sum goes to pos_sums[p-1] for a fixed-order fold (no float atomics).
+template <typename T, bool kMasked = false, bool kVisible = false>
 __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__restrict__ dtok, T *__restrict__ de,
                                                                   float *__restrict__ dcls, float *__restrict__ dpos,
                                                                   float *__restrict__ dbias, int B, int n_patch, int d,
                                                                   DropoutParams drop,
                                                                   const uint8_t *__restrict__ mask = nullptr,
-                                                                  float *__restrict__ dmask_token = nullptr) {
+                                                                  float *__restrict__ dmask_token = nullptr,
+                                                                  const int *__restrict__ slot = nullptr, int n_vis = 0,
+                                                                  float *__restrict__ pos_sums = nullptr) {
     __shared__ float red[kMasked ? 16 : 8][256 + 8];
-    const int N = n_patch + 1;
-    const int j = blockIdx.x;
+    if constexpr (kVisible) {
+        pdl_launch_dependents();
+        pdl_wait();
+    }
+    const int N = kVisible ? n_vis + 1 : n_patch + 1;
+    const int n_e = kVisible ? n_vis : n_patch;   // rows of de per record
+    const int p_blk = blockIdx.x;
+    const int j = kVisible ? 0 : p_blk;   // token row (per record under kVisible, see row_of)
+    // token row of record b at this block's position, -1 when the patch is masked
+    auto row_of = [&](int b) -> int {
+        if constexpr (kVisible) return p_blk == 0 ? 0 : (slot[(int64_t)b * n_patch + (p_blk - 1)] >= 0 ?
+                                                         1 + slot[(int64_t)b * n_patch + (p_blk - 1)] : -1);
+        else return j;
+    };
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const int col = (blockIdx.y * 32 + tx) * 8;
     const bool dropping = drop.threshold != 0;
@@ -184,12 +209,18 @@ __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__rest
         // two samples in flight per thread (rows N * d elements apart)
         for (int b0 = ty; b0 < B; b0 += 16) {
             float gv[2][8];
+            int jq[2];
 #pragma unroll
-            for (int q = 0; q < 2; ++q) load8(dtok + ((int64_t)min(b0 + 8 * q, B - 1) * N + j) * d + col, gv[q]);
+            for (int q = 0; q < 2; ++q) {
+                const int bq = min(b0 + 8 * q, B - 1);
+                jq[q] = row_of(bq);
+                if (!kVisible || jq[q] >= 0) load8(dtok + ((int64_t)bq * N + jq[q]) * d + col, gv[q]);
+            }
 #pragma unroll
             for (int q = 0; q < 2; ++q) {
                 const int b = b0 + 8 * q;
-                if (b < B) {
+                if (b < B && (!kVisible || jq[q] >= 0)) {
+                    const int j = jq[q];
                     const int64_t idx = ((int64_t)b * N + j) * d + col;
                     if (dropping) dropout_apply<8>(drop, seed, static_cast<uint32_t>(idx), gv[q]);
                     if (kMasked && j > 0 && mask[(int64_t)b * n_patch + (j - 1)] != 0) {
@@ -205,7 +236,7 @@ __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__rest
                             s[k] += gv[q][k];
                         }
                     }
-                    if (j > 0) store8(de + ((int64_t)b * n_patch + (j - 1)) * d + col, gv[q]);
+                    if (j > 0) store8(de + ((int64_t)b * n_e + (j - 1)) * d + col, gv[q]);
                 }
             }
         }
@@ -232,11 +263,126 @@ __global__ void __launch_bounds__(256) embed_assemble_bwd_kernel(const T *__rest
                 atomicAdd(dbias + c, t);
                 atomicAdd(dmask_token + c, tm);
             }
+        } else if constexpr (kVisible) {
+            dpos[(int64_t)p_blk * d + c] += t;
+            if (p_blk == 0) dcls[c] += t;
+            else pos_sums[(int64_t)(p_blk - 1) * d + c] = t;
         } else {
             dpos[(int64_t)j * d + c] += t;
             if (j == 0) dcls[c] += t;
             else atomicAdd(dbias + c, t);
         }
+    }
+}
+
+// Column sums of an fp32 [rows, d] scratch in a fixed order, in two launches (bit-identical from launch to launch; the
+// deterministic second half of the visible-assemble and unshuffle backward):
+//   chunk pass: CTA (column slab x, chunk g) sums rows [g * kFoldChunk, (g + 1) * kFoldChunk) over 32 row groups and
+//               a fixed fold, and writes the sum over the chunk's FIRST row (only this CTA reads that chunk);
+//   final pass: one CTA per column slab folds the chunk sums (rows 0, kFoldChunk, 2 kFoldChunk, ...) into out.
+// fold_rows_kernel is both: rows are r * row_stride, and out == nullptr selects the chunk pass.
+constexpr int kFoldGroups = 32;
+constexpr int kFoldChunk = 128;
+__global__ void __launch_bounds__(32 * kFoldGroups) fold_rows_kernel(float *__restrict__ S, int rows, int row_stride,
+                                                                     int d, float *__restrict__ out) {
+    __shared__ float red[kFoldGroups][33];
+    pdl_launch_dependents();
+    pdl_wait();
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int c = blockIdx.x * 32 + tx;
+    const int r0 = out == nullptr ? blockIdx.y * kFoldChunk : 0;
+    const int r1 = out == nullptr ? min(r0 + kFoldChunk, rows) : rows;
+    float s = 0.f;
+    if (c < d)
+        for (int r = r0 + ty; r < r1; r += kFoldGroups) s += S[(int64_t)r * row_stride * d + c];
+    red[ty][tx] = s;
+    __syncthreads();
+    if (ty == 0 && c < d) {
+        float t = 0.f;
+#pragma unroll
+        for (int y = 0; y < kFoldGroups; ++y) t += red[y][tx];
+        if (out == nullptr) S[(int64_t)r0 * d + c] = t;
+        else out[c] += t;
+    }
+}
+
+// MAE decoder input: u[b, 0] = t[b, 0] + pos[0]; u[b, 1+p] = (slot[b, p] >= 0 ? t[b, 1 + slot[b, p]] : mask_token)
+// + pos[1+p], with t [B*(n_vis+1), d] and u [B*(n_patch+1), d]
+template <typename T, typename TO>
+__global__ void mae_unshuffle_kernel(const T *__restrict__ t, const float *__restrict__ mask_token,
+                                     const float *__restrict__ pos, const int *__restrict__ slot, TO *__restrict__ u,
+                                     int B, int n_patch, int n_vis, int d) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int N = n_patch + 1, Nv = n_vis + 1;
+    const int vec_per_row = d / 8;
+    const int64_t total = (int64_t)B * N * vec_per_row;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int c = (int)(i % vec_per_row) * 8;
+        const int64_t r = i / vec_per_row;
+        const int p = (int)(r % N);
+        const int64_t b = r / N;
+        float v[8], q[8];
+        load8(pos + (int64_t)p * d + c, q);
+        const int s = p == 0 ? -1 : slot[b * n_patch + (p - 1)];
+        if (p == 0) load8(t + b * Nv * d + c, v);
+        else if (s >= 0) load8(t + (b * Nv + 1 + s) * d + c, v);
+        else load8(mask_token + c, v);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) v[k] += q[k];
+        store8(u + r * d + c, v);
+    }
+}
+
+// its backward: grid (position p, 256-column slab), block = 32 lanes x 8 columns x 8 record groups.  dt rows are
+// copied from du (every row of t feeds exactly one row of u); dpos[p] += sum_b du[b, p]; the masked rows' sum of
+// position p goes to mask_sums[p-1] for the fixed-order fold into the mask-token gradient.
+template <typename T>
+__global__ void __launch_bounds__(256) mae_unshuffle_bwd_kernel(const T *__restrict__ du, const int *__restrict__ slot,
+                                                                 T *__restrict__ dt, float *__restrict__ dpos,
+                                                                 float *__restrict__ mask_sums, int B, int n_patch,
+                                                                 int n_vis, int d) {
+    __shared__ float red[16][256 + 8];
+    pdl_launch_dependents();
+    pdl_wait();
+    const int N = n_patch + 1, Nv = n_vis + 1;
+    const int p = blockIdx.x;
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int col = (blockIdx.y * 32 + tx) * 8;
+    float s[8], sm[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) s[k] = sm[k] = 0.f;
+    if (col < d) {
+        for (int b = ty; b < B; b += 8) {
+            float g[8];
+            load8(du + ((int64_t)b * N + p) * d + col, g);
+            const int sl = p == 0 ? 0 : slot[(int64_t)b * n_patch + (p - 1)];
+#pragma unroll
+            for (int k = 0; k < 8; ++k) s[k] += g[k];
+            if (p == 0) store8(dt + (int64_t)b * Nv * d + col, g);
+            else if (sl >= 0) store8(dt + ((int64_t)b * Nv + 1 + sl) * d + col, g);
+            else {
+#pragma unroll
+                for (int k = 0; k < 8; ++k) sm[k] += g[k];
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+        red[ty][tx * 8 + k] = s[k];
+        red[8 + ty][tx * 8 + k] = sm[k];
+    }
+    __syncthreads();
+    const int c = blockIdx.y * 256 + threadIdx.x;
+    if (c < d) {
+        float a = 0.f, am = 0.f;
+#pragma unroll
+        for (int y = 0; y < 8; ++y) {
+            a += red[y][threadIdx.x];
+            am += red[8 + y][threadIdx.x];
+        }
+        dpos[(int64_t)p * d + c] += a;
+        if (p > 0) mask_sums[(int64_t)(p - 1) * d + c] = am;
     }
 }
 
@@ -691,6 +837,15 @@ static int patchify_group(int n_patch, int P, int C) {
     return wg < 1 ? 1 : wg;
 }
 
+// fixed-order column sums of scratch [rows, d] into out (two launches, see fold_rows_kernel); scratch is overwritten
+static void fold_rows(float *scratch, int rows, int d, float *out, cudaStream_t st) {
+    const int chunks = (rows + kFoldChunk - 1) / kFoldChunk;
+    launch_pdl(fold_rows_kernel, dim3((d + 31) / 32, chunks), dim3(32 * kFoldGroups), 0, st, scratch, rows, 1, d,
+               (float *)nullptr);
+    launch_pdl(fold_rows_kernel, dim3((d + 31) / 32, 1), dim3(32 * kFoldGroups), 0, st, scratch, chunks, kFoldChunk, d,
+               out);
+}
+
 extern "C" {
 
 int ecgvit_patchify(const float *x, void *a, int B, int C, int64_t x_ld, int n_patch, int P, int dtype,
@@ -832,6 +987,93 @@ int ecgvit_embed_assemble_masked_bwd(const void *dtok, const uint8_t *mask, void
         embed_assemble_bwd_kernel<float, true><<<grid, 256, 0, st>>>((const float *)dtok, (float *)de, dcls, dpos, dbias, B, n_patch, d, drop, mask, dmask_token);
     else return fail(-1, "embed_assemble_masked_bwd: unknown dtype %d", dtype);
     return check_launch("embed_assemble_masked_bwd");
+}
+
+int ecgvit_embed_assemble_visible(const void *e, const float *cls, const float *pos, const int *vis_idx, void *tok,
+                                  int B, int n_vis, int d, float dropout_p, int dropout_stream,
+                                  const uint32_t *dropout_seed, int dtype, void *stream) {
+    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    ECGVIT_REQUIRE(e && cls && pos && vis_idx && tok && B > 0 && n_vis > 0, "embed_assemble_visible: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "embed_assemble_visible: d=%d must be a multiple of 8", d);
+    const int64_t total = (int64_t)B * (n_vis + 1) * (d / 8);
+    const dim3 grid(grid_for(total, 256));
+    cudaStream_t st = as_stream(stream);
+    if (dtype == ECGVIT_BF16)
+        launch_pdl(embed_assemble_kernel<bf16, bf16, false, true>, grid, dim3(256), 0, st, (const bf16 *)e, cls, pos,
+                   (bf16 *)tok, B, n_vis, d, drop, (const float *)nullptr, (const uint8_t *)nullptr, vis_idx);
+    else if (dtype == ECGVIT_BF16_RES32)
+        launch_pdl(embed_assemble_kernel<bf16, float, false, true>, grid, dim3(256), 0, st, (const bf16 *)e, cls, pos,
+                   (float *)tok, B, n_vis, d, drop, (const float *)nullptr, (const uint8_t *)nullptr, vis_idx);
+    else if (dtype == ECGVIT_F32)
+        launch_pdl(embed_assemble_kernel<float, float, false, true>, grid, dim3(256), 0, st, (const float *)e, cls, pos,
+                   (float *)tok, B, n_vis, d, drop, (const float *)nullptr, (const uint8_t *)nullptr, vis_idx);
+    else return fail(-1, "embed_assemble_visible: unknown dtype %d", dtype);
+    return check_launch("embed_assemble_visible");
+}
+
+int ecgvit_embed_assemble_visible_bwd(const void *dtok, const int *slot, void *de, float *dcls, float *dpos,
+                                      float *dbias, float *scratch, int B, int n_patch, int n_vis, int d,
+                                      float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int dtype,
+                                      void *stream) {
+    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    ECGVIT_REQUIRE(dtok && slot && de && dcls && dpos && dbias && scratch && B > 0 && n_vis > 0 && n_vis <= n_patch &&
+                   d > 0, "embed_assemble_visible_bwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "embed_assemble_visible_bwd: d=%d must be a multiple of 8", d);
+    const dim3 grid(n_patch + 1, (d + 255) / 256);
+    cudaStream_t st = as_stream(stream);
+    if (dtype == ECGVIT_BF16)
+        launch_pdl(embed_assemble_bwd_kernel<bf16, false, true>, grid, dim3(256), 0, st, (const bf16 *)dtok, (bf16 *)de,
+                   dcls, dpos, dbias, B, n_patch, d, drop, (const uint8_t *)nullptr, (float *)nullptr, slot, n_vis,
+                   scratch);
+    else if (dtype == ECGVIT_F32)
+        launch_pdl(embed_assemble_bwd_kernel<float, false, true>, grid, dim3(256), 0, st, (const float *)dtok,
+                   (float *)de, dcls, dpos, dbias, B, n_patch, d, drop, (const uint8_t *)nullptr, (float *)nullptr, slot,
+                   n_vis, scratch);
+    else return fail(-1, "embed_assemble_visible_bwd: unknown dtype %d", dtype);
+    int rc = check_launch("embed_assemble_visible_bwd");
+    if (rc) return rc;
+    fold_rows(scratch, n_patch, d, dbias, st);
+    return check_launch("embed_assemble_visible_bwd");
+}
+
+int ecgvit_mae_unshuffle(const void *t, const float *mask_token, const float *pos, const int *slot, void *u, int B,
+                         int n_patch, int n_vis, int d, int dtype, void *stream) {
+    ECGVIT_REQUIRE(t && mask_token && pos && slot && u && B > 0 && n_vis > 0 && n_vis <= n_patch,
+                   "mae_unshuffle: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "mae_unshuffle: d=%d must be a multiple of 8", d);
+    const dim3 grid(grid_for((int64_t)B * (n_patch + 1) * (d / 8), 256));
+    cudaStream_t st = as_stream(stream);
+    if (dtype == ECGVIT_BF16)
+        launch_pdl(mae_unshuffle_kernel<bf16, bf16>, grid, dim3(256), 0, st, (const bf16 *)t, mask_token, pos, slot,
+                   (bf16 *)u, B, n_patch, n_vis, d);
+    else if (dtype == ECGVIT_BF16_RES32)
+        launch_pdl(mae_unshuffle_kernel<bf16, float>, grid, dim3(256), 0, st, (const bf16 *)t, mask_token, pos, slot,
+                   (float *)u, B, n_patch, n_vis, d);
+    else if (dtype == ECGVIT_F32)
+        launch_pdl(mae_unshuffle_kernel<float, float>, grid, dim3(256), 0, st, (const float *)t, mask_token, pos, slot,
+                   (float *)u, B, n_patch, n_vis, d);
+    else return fail(-1, "mae_unshuffle: unknown dtype %d", dtype);
+    return check_launch("mae_unshuffle");
+}
+
+int ecgvit_mae_unshuffle_bwd(const void *du, const int *slot, void *dt, float *dpos, float *dmask_token,
+                             float *scratch, int B, int n_patch, int n_vis, int d, int dtype, void *stream) {
+    ECGVIT_REQUIRE(du && slot && dt && dpos && dmask_token && scratch && B > 0 && n_vis > 0 && n_vis <= n_patch,
+                   "mae_unshuffle_bwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "mae_unshuffle_bwd: d=%d must be a multiple of 8", d);
+    const dim3 grid(n_patch + 1, (d + 255) / 256);
+    cudaStream_t st = as_stream(stream);
+    if (dtype == ECGVIT_BF16)
+        launch_pdl(mae_unshuffle_bwd_kernel<bf16>, grid, dim3(256), 0, st, (const bf16 *)du, slot, (bf16 *)dt, dpos,
+                   scratch, B, n_patch, n_vis, d);
+    else if (dtype == ECGVIT_F32)
+        launch_pdl(mae_unshuffle_bwd_kernel<float>, grid, dim3(256), 0, st, (const float *)du, slot, (float *)dt, dpos,
+                   scratch, B, n_patch, n_vis, d);
+    else return fail(-1, "mae_unshuffle_bwd: unknown dtype %d", dtype);
+    int rc = check_launch("mae_unshuffle_bwd");
+    if (rc) return rc;
+    fold_rows(scratch, n_patch, d, dmask_token, st);
+    return check_launch("mae_unshuffle_bwd");
 }
 
 int ecgvit_layernorm_patch_fwd(const void *tok, const float *gamma, const float *beta, void *y, float *mean,

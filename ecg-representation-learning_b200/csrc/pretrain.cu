@@ -1,4 +1,4 @@
-// Masked-patch pre-training (SimMIM-style): the mask draw, the loss fold of the reconstruction GEMM's row partials
+// Masked-patch pre-training (SimMIM-style): the mask draw, the MAE index build and row gather, the loss fold of the reconstruction GEMM's row partials
 // (ECGVIT_EPI_BIAS_SUB_ROWSQ), the gradient of that loss w.r.t. the prediction, and the fp32 reconstruction output.
 // The encoder, the masked token assembly and the patch-row LayerNorm live in elementwise.cu; the GEMMs in gemm_*.cu.
 #include "common.cuh"
@@ -123,6 +123,57 @@ __global__ void mpm_reconstruction_kernel(const T *__restrict__ r, const T *__re
     }
 }
 
+// MAE index build, one CTA per record: a block prefix sum over the visible flags.  Thread t owns the contiguous chunk
+// [t * chunk, (t + 1) * chunk) of the record's patches; a warp scan of the chunk counts, then a scan of the warp totals.
+constexpr int kIndexThreads = 256;
+__global__ void __launch_bounds__(kIndexThreads) mae_index_kernel(const uint8_t *__restrict__ mask, int n, int n_vis,
+                                                                   int *__restrict__ vis_idx, int *__restrict__ slot) {
+    __shared__ int warp_tot[kIndexThreads / 32];
+    pdl_launch_dependents();
+    pdl_wait();
+    const int b = blockIdx.x;
+    const uint8_t *m = mask + (int64_t)b * n;
+    const int chunk = (n + kIndexThreads - 1) / kIndexThreads;
+    const int lo = min(threadIdx.x * chunk, n), hi = min(lo + chunk, n);
+    int cnt = 0;
+    for (int i = lo; i < hi; ++i) cnt += m[i] == 0;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) warp_tot[warp] = incl;
+    __syncthreads();
+    int run = incl - cnt;
+    for (int w = 0; w < warp; ++w) run += warp_tot[w];
+    int *sl = slot + (int64_t)b * n;
+    int *vi = vis_idx + (int64_t)b * n_vis;
+    for (int i = lo; i < hi; ++i) {
+        if (m[i] == 0) {
+            sl[i] = run;
+            if (run < n_vis) vi[run] = i;   // a mask with more visible patches than n_vis cannot write past the row
+            ++run;
+        } else {
+            sl[i] = -1;
+        }
+    }
+}
+
+// dst row b*n_dst + j = src row b*n_src + idx[b*n_dst + j]; rows of vec 16-byte words
+__global__ void row_gather_kernel(const uint4 *__restrict__ src, uint4 *__restrict__ dst, const int *__restrict__ idx,
+                                  int n_src, int n_dst, int64_t rows, int vec) {
+    pdl_launch_dependents();
+    pdl_wait();
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < rows * vec; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t r = i / vec;
+        const int v = (int)(i - r * vec);
+        const int64_t s = (r / n_dst) * n_src + idx[r];
+        dst[i] = src[s * vec + v];
+    }
+}
+
 inline int grid_cap(int64_t items, int threads) {
     int64_t g = (items + threads - 1) / threads;
     const int64_t cap = (int64_t)sm_count() * 8;
@@ -146,6 +197,29 @@ int ecgvit_mpm_mask(const uint32_t *seed, int B, int n_patch, int k, int site, u
     mpm_mask_kernel<<<B, kMaskThreads, smem, as_stream(stream)>>>(seed, n_patch, k, static_cast<uint32_t>(site), mask,
                                                                   counts);
     return check_launch("mpm_mask");
+}
+
+int ecgvit_mae_index(const uint8_t *mask, int B, int n_patch, int n_vis, int *vis_idx, int *slot, void *stream) {
+    ECGVIT_REQUIRE(mask && vis_idx && slot && B > 0 && n_patch > 0 && n_vis > 0 && n_vis <= n_patch,
+                   "mae_index: bad arguments");
+    ECGVIT_REQUIRE(n_patch <= kMaxMaskPatches, "mae_index: n_patch=%d exceeds %d", n_patch, kMaxMaskPatches);
+    launch_pdl(mae_index_kernel, dim3(B), dim3(kIndexThreads), 0, as_stream(stream), mask, n_patch, n_vis, vis_idx, slot);
+    return check_launch("mae_index");
+}
+
+int ecgvit_row_gather(const void *src, void *dst, const int *idx, int B, int n_src, int n_dst, int ld, int dtype,
+                      void *stream) {
+    ECGVIT_REQUIRE(src && dst && idx && B > 0 && n_src > 0 && n_dst > 0 && ld > 0, "row_gather: bad arguments");
+    int esz;
+    if (dtype == ECGVIT_BF16) esz = 2;
+    else if (dtype == ECGVIT_F32) esz = 4;
+    else return fail(-1, "row_gather: unknown dtype %d", dtype);
+    ECGVIT_REQUIRE(((int64_t)ld * esz) % 16 == 0, "row_gather: rows of %d elements are not 16-byte multiples", ld);
+    const int vec = (int)((int64_t)ld * esz / 16);
+    const int64_t rows = (int64_t)B * n_dst;
+    launch_pdl(row_gather_kernel, dim3(grid_cap(rows * vec, 256)), dim3(256), 0, as_stream(stream), (const uint4 *)src,
+               (uint4 *)dst, idx, n_src, n_dst, rows, vec);
+    return check_launch("row_gather");
 }
 
 int ecgvit_mpm_loss(const float *rowsq, int n_groups, const uint8_t *mask, const int *counts, int B, int n_patch,

@@ -96,8 +96,9 @@ class StepEngine:
             _lib.profile_meta[0] = (M, N, K, epi, a_k, b_k, keep)
         _lib.check(self.lib.ecgvit_gemm(ctypes.byref(g), self._stream), 'gemm')
 
-    def workspace(self, B, L):
-        key = (B, L)
+    def workspace(self, B, L, n_vis=None):
+        """activations of one (batch, length) shape; n_vis: the patches the encoder sees per record (all when None)"""
+        key = (B, L, n_vis)
         w = self.ws.get(key)
         if w is not None:
             return w
@@ -107,7 +108,6 @@ class StepEngine:
         T = m._act_dtype
         P, C, d, mlp = c.patch_size, c.num_channels, c.hidden_size, c.intermediate_size
         H = c.num_attention_heads
-        inner = d  # dim_head = d // heads (ecg_vit.py:100)
         assert L % P == 0, f'signal length {L} must be a multiple of patch_size {P}'
         per_lead = bool(getattr(c, 'per_lead_tokens', False))
         n = L // P * (C if per_lead else 1)
@@ -115,44 +115,30 @@ class StepEngine:
         Kp = (K + 7) // 8 * 8 if per_lead else K  # row length of the patch matrix (16-byte aligned rows for TMA)
         assert n + 1 <= m.vit.pos_embedding.shape[1], \
             f'{n} patches exceed the positional table ({m.vit.pos_embedding.shape[1] - 1})'
-        N = n + 1
+        nv = n if n_vis is None else n_vis
+        N = nv + 1
         M = B * N
         depth = c.num_hidden_layers
         w = _Workspace()
         w.B, w.L, w.n, w.N, w.M = B, L, n, N, M
+        w.n_vis = nv
         w.per_lead, w.K, w.Kp = per_lead, K, Kp
 
         def buf(*shape, dtype=T):
             return torch.empty(*shape, device=dev, dtype=dtype)
 
         w.a_patch = buf(B * n, Kp)
+        w.a_emb = w.a_patch    # the embedding GEMM's operand: the rows of the patches the encoder sees
         # per-lead tokens with P % 8 != 0: zero-padded copies of the embedding weight and of its gradient
         w.embed_wpad = buf(d, Kp) if Kp != K else None
         w.embed_gpad = buf(d, Kp, dtype=torch.float32) if Kp != K else None
-        w.e = buf(B * n, d)
-        RT = m._res_dtype  # residual stream: fp32 for deep models in bf16 mode (config.residual_dtype)
-        w.x = [buf(M, d, dtype=RT) for _ in range(depth + 1)]  # x[l] = input of block l; x[depth] = encoder output
+        w.e = buf(B * nv, d)
         # Activation checkpointing (config.activation_checkpointing; BASELINE.json configs[4]): only the block inputs x[l]
         # are kept per layer; everything inside a block lives in TWO buffer sets used alternately (layer l -> set l % 2)
         # and is recomputed from x[l] in backward.  Two sets, so that the weight-gradient GEMMs of layer l (side stream)
         # can still read their operands while layer l - 1 is being recomputed into the other set.
-        w.ckpt = bool(getattr(c, 'activation_checkpointing', False)) and depth > 2
-        n_sets = 2 if w.ckpt else depth
-
-        def per_layer(make):
-            sets = [make() for _ in range(n_sets)]
-            return [sets[l % n_sets] for l in range(depth)]
-
-        w.ln1 = per_layer(lambda: buf(M, d))
-        w.ln2 = per_layer(lambda: buf(M, d))
-        w.stat1 = per_layer(lambda: buf(2, M, dtype=torch.float32))
-        w.stat2 = per_layer(lambda: buf(2, M, dtype=torch.float32))
-        w.qkv = per_layer(lambda: buf(M, 3 * inner))
-        w.lse = per_layer(lambda: buf(B, H, N, dtype=torch.float32))
-        w.o = per_layer(lambda: buf(M, inner))
-        w.y = per_layer(lambda: buf(M, d, dtype=RT))
-        w.u = per_layer(lambda: buf(M, mlp))
-        w.h = per_layer(lambda: buf(M, mlp))
+        ckpt = bool(getattr(c, 'activation_checkpointing', False)) and depth > 2
+        self._alloc_stack(w, 'l', B, N, d, mlp, H, depth, ckpt)
         # head
         n_class = m.num_class
         w.xn = buf(B, d, dtype=torch.float32)
@@ -162,25 +148,60 @@ class StepEngine:
         w.loss_none = buf(B, n_class, dtype=torch.float32)
         w.head_scratch = buf(B * d + B * n_class, dtype=torch.float32)
         w.labels = buf(B, n_class, dtype=torch.float32)
+        w.de = buf(B * nv, d)
+        self.ws[key] = w
+        return w
+
+    def _alloc_stack(self, s, prefix, B, N, d, mlp, H, depth, ckpt):
+        """a block stack on the object s: `depth` blocks of width d over B sequences of N tokens, parameters keyed
+        `{prefix}{l}.`, its dims, activations and backward scratch.  Only the encoder stack (prefix 'l') calls the layer
+        hooks; p_blk is its block dropout probability, set by the forward pass."""
+        m = self.model
+        dev = m._flat_p.device
+        T = m._act_dtype
+        M = B * N
+        inner = d  # dim_head = d // heads (ecg_vit.py:100)
+        s.prefix, s.d, s.mlp, s.H, s.depth, s.ckpt, s.hooks = prefix, d, mlp, H, depth, ckpt, prefix == 'l'
+        s.B, s.N, s.M = B, N, M
+        s.p_blk = 0.0
+
+        def buf(*shape, dtype=T):
+            return torch.empty(*shape, device=dev, dtype=dtype)
+
+        RT = m._res_dtype  # residual stream: fp32 for deep models in bf16 mode (config.residual_dtype)
+        s.x = [buf(M, d, dtype=RT) for _ in range(depth + 1)]  # x[l] = input of block l; x[depth] = stack output
+        n_sets = 2 if ckpt else depth
+
+        def per_layer(make):
+            sets = [make() for _ in range(n_sets)]
+            return [sets[l % n_sets] for l in range(depth)]
+
+        s.ln1 = per_layer(lambda: buf(M, d))
+        s.ln2 = per_layer(lambda: buf(M, d))
+        s.stat1 = per_layer(lambda: buf(2, M, dtype=torch.float32))
+        s.stat2 = per_layer(lambda: buf(2, M, dtype=torch.float32))
+        s.qkv = per_layer(lambda: buf(M, 3 * inner))
+        s.lse = per_layer(lambda: buf(B, H, N, dtype=torch.float32))
+        s.o = per_layer(lambda: buf(M, inner))
+        s.y = per_layer(lambda: buf(M, d, dtype=RT))
+        s.u = per_layer(lambda: buf(M, mlp))
+        s.h = per_layer(lambda: buf(M, mlp))
         # backward scratch
         # Every scratch buffer that a side-stream weight-gradient GEMM reads exists TWICE, indexed by layer parity: the main
         # chain of layer l - 1 then never has to wait for the weight gradients of layer l (it waits for those of layer
         # l + 1, a whole layer old), so the side stream is free to lag and fill whatever the chain leaves idle
-        w.dz = [buf(M, d), buf(M, d)]          # gradient w.r.t. a block's output (input of its backward)
-        w.dy = [buf(M, d), buf(M, d)]          # gradient w.r.t. the block's middle residual sum y
-        w.dln = buf(M, d)
-        w.d_o = buf(M, inner)
-        w.dqkv = [buf(M, 3 * inner), buf(M, 3 * inner)]
-        w.du = [buf(M, mlp), buf(M, mlp)]
-        w.de = buf(B * n, d)
+        s.dz = [buf(M, d), buf(M, d)]          # gradient w.r.t. a block's output (input of its backward)
+        s.dy = [buf(M, d), buf(M, d)]          # gradient w.r.t. the block's middle residual sum y
+        s.dln = buf(M, d)
+        s.d_o = buf(M, inner)
+        s.dqkv = [buf(M, 3 * inner), buf(M, 3 * inner)]
+        s.du = [buf(M, mlp), buf(M, mlp)]
         # dropout-masked copies of the residual-stream gradients (only used when p > 0): one per site of a block
-        w.dzm = [[buf(M, d), buf(M, d)], [buf(M, d), buf(M, d)]]   # [site 0 = after net[3], 1 = after to_out][parity]
+        s.dzm = [[buf(M, d), buf(M, d)], [buf(M, d), buf(M, d)]]   # [site 0 = after net[3], 1 = after to_out][parity]
         # two partial-row scratch buffers (one per LayerNorm of a block): their fold runs off the critical chain
-        w.ln_scratch = [buf(int(self.lib.ecgvit_layernorm_bwd_scratch_floats(d)), dtype=torch.float32) for _ in range(2)]
+        s.ln_scratch = [buf(int(self.lib.ecgvit_layernorm_bwd_scratch_floats(d)), dtype=torch.float32) for _ in range(2)]
         n_attn = int(self.lib.ecgvit_attention_bwd_scratch_floats(B, N, H, d // H, m._dtype_code))
-        w.attn_scratch = buf(n_attn, dtype=torch.float32) if n_attn > 0 else None
-        self.ws[key] = w
-        return w
+        s.attn_scratch = buf(n_attn, dtype=torch.float32) if n_attn > 0 else None
 
     # ---- forward ---------------------------------------------------------------------------------
     def forward(self, sample_values, labels=None, reduction='mean', record_attention=False):
@@ -227,15 +248,16 @@ class StepEngine:
             _lib.check(lib.ecgvit_patchify_transform(x.data_ptr(), _lib.ptr(mean), _lib.ptr(std), _lib.ptr(spans),
                                                      w.a_patch.data_ptr(), B, C, x.stride(1), L_in, n, P, dt, st),
                        'patchify_transform')
+        self._select_patches(w)
         hook = m._before_layer_forward
         if hook is not None:
             hook(-1)   # embedding weights, cls, pos
-        # e = a_patch @ We^T + be
+        # e = a_emb @ We^T + be
         w_embed = wt['embed.w']
         if Kp != K:
             _lib.check(lib.ecgvit_pad_cols(w_embed.data_ptr(), w.embed_wpad.data_ptr(), d, K, Kp, dt, st), 'pad_cols')
             w_embed = w.embed_wpad
-        self._gemm(B * n, d, Kp, w.a_patch, Kp, 1, w_embed, Kp, 1, EPI_STORE, w.e, d, bias=pf['embed.b'])
+        self._gemm(B * w.n_vis, d, Kp, w.a_emb, Kp, 1, w_embed, Kp, 1, EPI_STORE, w.e, d, bias=pf['embed.b'])
         p_emb, p_blk = self._dropout_probs()
         w.p_emb, w.p_blk = p_emb, p_blk
         self._assemble(w)
@@ -246,6 +268,9 @@ class StepEngine:
         if hook is not None:
             hook(c.num_hidden_layers)   # head
         return self._head_forward(w, labels, reduction)
+
+    def _select_patches(self, w):
+        """the rows of the patch matrix the encoder embeds (`w.a_emb`, `w.n_vis` per record): all of them here"""
 
     def _assemble(self, w):
         """token matrix x[0] = [cls | e] + pos (embedding dropout)"""
@@ -280,48 +305,47 @@ class StepEngine:
             loss = w.loss_none if reduction == 'none' else w.loss[0]
         return loss, w.logits
 
-    def _block_forward(self, l, w, record_attention=False, recompute=False):
-        """block l: x[l] -> x[l + 1] (PreNorm attention + residual, PreNorm feed-forward + residual).
+    def _block_forward(self, l, s, record_attention=False, recompute=False):
+        """block l of the stack s (the encoder's is the workspace itself): x[l] -> x[l + 1] (PreNorm attention +
+        residual, PreNorm feed-forward + residual).
         recompute=True (activation checkpointing, from backward): rebuild what backward reads of the block -- ln1, qkv,
         lse, o, y, ln2, u, h -- from x[l]; the last Linear (whose output x[l + 1] is kept) is skipped.  Dropout masks are
         a function of (seed, site, element), so the recomputed tensors are bit-identical to the forward pass's."""
         m, lib, st = self.model, self.lib, self._stream
-        c = m.config
         dt, rdt = m._dtype_code, m._res_code
         epi_res = EPI_BIAS_RES_F32 if m._res_f32 else EPI_BIAS_RES
-        d, mlp, H = c.hidden_size, c.intermediate_size, c.num_attention_heads
+        d, mlp, H = s.d, s.mlp, s.H
         inner, dh = d, d // H
-        B, N, M = w.B, w.N, w.M
+        B, N, M = s.B, s.N, s.M
         wt, pf = m._weights(), m._params_f32()
-        p_blk = w.p_blk
+        p_blk = s.p_blk
         scale = float(dh) ** -0.5
         blk_seed = self.rng.data_ptr() if p_blk > 0 else None
-        p = f'l{l}.'
+        p = f'{s.prefix}{l}.'
         # dropout sites of block l: 1+4l attention probabilities, 2+4l after to_out, 3+4l after GELU, 4+4l after net[3]
         s_att, s_out, s_act, s_ff2 = 1 + 4 * l, 2 + 4 * l, 3 + 4 * l, 4 + 4 * l
-        _lib.check(lib.ecgvit_layernorm_fwd(w.x[l].data_ptr(), pf[p + 'ln1.w'].data_ptr(), pf[p + 'ln1.b'].data_ptr(),
-                                            w.ln1[l].data_ptr(), w.stat1[l][0].data_ptr(), w.stat1[l][1].data_ptr(),
+        _lib.check(lib.ecgvit_layernorm_fwd(s.x[l].data_ptr(), pf[p + 'ln1.w'].data_ptr(), pf[p + 'ln1.b'].data_ptr(),
+                                            s.ln1[l].data_ptr(), s.stat1[l][0].data_ptr(), s.stat1[l][1].data_ptr(),
                                             M, d, LN_EPS, rdt, st), 'layernorm_fwd')
-        self._gemm(M, 3 * inner, d, w.ln1[l], d, 1, wt[p + 'qkv.w'], d, 1, EPI_STORE, w.qkv[l], 3 * inner)
+        self._gemm(M, 3 * inner, d, s.ln1[l], d, 1, wt[p + 'qkv.w'], d, 1, EPI_STORE, s.qkv[l], 3 * inner)
         if record_attention:
             if l == 0:
-                self.recorded_attention = torch.empty(B, c.num_hidden_layers, H, N, N, device=self.device,
-                                                      dtype=torch.float32)
+                self.recorded_attention = torch.empty(B, s.depth, H, N, N, device=self.device, dtype=torch.float32)
             rec = self.recorded_attention
-            _lib.check(lib.ecgvit_attention_probs(w.qkv[l].data_ptr(), rec[:, l].data_ptr(), B, N, H, dh, scale,
+            _lib.check(lib.ecgvit_attention_probs(s.qkv[l].data_ptr(), rec[:, l].data_ptr(), B, N, H, dh, scale,
                                                   rec.stride(0), dt, st), 'attention_probs')
-        _lib.check(lib.ecgvit_attention_fwd(w.qkv[l].data_ptr(), w.o[l].data_ptr(), w.lse[l].data_ptr(), B, N, H, dh,
+        _lib.check(lib.ecgvit_attention_fwd(s.qkv[l].data_ptr(), s.o[l].data_ptr(), s.lse[l].data_ptr(), B, N, H, dh,
                                             scale, p_blk, s_att, blk_seed, dt, st), 'attention_fwd')
-        self._gemm(M, d, inner, w.o[l], inner, 1, wt[p + 'out.w'], inner, 1, epi_res, w.y[l], d,
-                   aux=w.x[l], bias=pf[p + 'out.b'], drop=(p_blk, s_out))
-        _lib.check(lib.ecgvit_layernorm_fwd(w.y[l].data_ptr(), pf[p + 'ln2.w'].data_ptr(), pf[p + 'ln2.b'].data_ptr(),
-                                            w.ln2[l].data_ptr(), w.stat2[l][0].data_ptr(), w.stat2[l][1].data_ptr(),
+        self._gemm(M, d, inner, s.o[l], inner, 1, wt[p + 'out.w'], inner, 1, epi_res, s.y[l], d,
+                   aux=s.x[l], bias=pf[p + 'out.b'], drop=(p_blk, s_out))
+        _lib.check(lib.ecgvit_layernorm_fwd(s.y[l].data_ptr(), pf[p + 'ln2.w'].data_ptr(), pf[p + 'ln2.b'].data_ptr(),
+                                            s.ln2[l].data_ptr(), s.stat2[l][0].data_ptr(), s.stat2[l][1].data_ptr(),
                                             M, d, LN_EPS, rdt, st), 'layernorm_fwd')
-        self._gemm(M, mlp, d, w.ln2[l], d, 1, wt[p + 'ff1.w'], d, 1, EPI_BIAS_GELU, w.u[l], mlp,
-                   out2=w.h[l], bias=pf[p + 'ff1.b'], drop=(p_blk, s_act))
+        self._gemm(M, mlp, d, s.ln2[l], d, 1, wt[p + 'ff1.w'], d, 1, EPI_BIAS_GELU, s.u[l], mlp,
+                   out2=s.h[l], bias=pf[p + 'ff1.b'], drop=(p_blk, s_act))
         if not recompute:
-            self._gemm(M, d, mlp, w.h[l], mlp, 1, wt[p + 'ff2.w'], mlp, 1, epi_res, w.x[l + 1], d,
-                       aux=w.y[l], bias=pf[p + 'ff2.b'], drop=(p_blk, s_ff2))
+            self._gemm(M, d, mlp, s.h[l], mlp, 1, wt[p + 'ff2.w'], mlp, 1, epi_res, s.x[l + 1], d,
+                       aux=s.y[l], bias=pf[p + 'ff2.b'], drop=(p_blk, s_ff2))
 
     def span_buffer(self, B):
         """device int32 [B, 2] (start, length) of the TimeOut span of every record; a persistent buffer, so a captured
@@ -353,26 +377,51 @@ class StepEngine:
         grad_scale_dev: optional fp32 CUDA scalar multiplied into the upstream gradient on the device (no host sync)."""
         m, lib, st = self.model, self.lib, self._stream
         c = m.config
-        dt = m._dtype_code
-        rdt = m._res_code
         w = self._cur
         assert w is not None, 'backward before forward'
         assert w.reduction in ('mean', 'sum'), "backward needs loss_reduction 'mean' or 'sum'"
-        B, n, N, M = w.B, w.n, w.N, w.M
-        P, C, d, mlp, H = c.patch_size, c.num_channels, c.hidden_size, c.intermediate_size, c.num_attention_heads
-        inner, dh = d, d // H
+        B, d = w.B, c.hidden_size
         depth = c.num_hidden_layers
-        wt, pf, gr = m._weights(), m._params_f32(), m._grads_f32()
+        gr = m._grads_f32()
         if zero_grads:
             m._flat_g.zero_()
-        p_emb, p_blk = w.p_emb, w.p_blk
-        seed_ptr = self.rng.data_ptr()
-        blk_seed = seed_ptr if p_blk > 0 else None
         last = f'l{depth - 1}.'
         top = (depth - 1) & 1
         # with dropout between net[3] / to_out[0] and the residual add, the Linear sees mask * dz / (1 - p): its operand
         # and its bias gradient come from the masked copy, so the producers must not pre-sum the unmasked gradient
-        self._head_backward(w, w.dz[top], gr[last + 'ff2.b'] if p_blk == 0 else None, grad_scale, grad_scale_dev)
+        self._head_backward(w, w.dz[top], gr[last + 'ff2.b'] if w.p_blk == 0 else None, grad_scale, grad_scale_dev)
+        self._stack_backward(w)
+        dz = w.dz[(-1) & 1]   # gradient w.r.t. the token matrix (input of block 0)
+        # ---- embedding: tok = [cls | a_emb We^T + be] + pos
+        self._assemble_backward(w, dz)
+        rows = B * w.n_vis
+        if w.Kp == w.K:
+            self._gemm(d, w.K, rows, w.de, d, 0, w.a_emb, w.K, 0, EPI_ATOMIC_F32, gr['embed.w'], w.K, split_k=0)
+        else:
+            w.embed_gpad.zero_()
+            self._gemm(d, w.Kp, rows, w.de, d, 0, w.a_emb, w.Kp, 0, EPI_ATOMIC_F32, w.embed_gpad, w.Kp, split_k=0)
+            _lib.check(lib.ecgvit_unpad_add_f32(w.embed_gpad.data_ptr(), gr['embed.w'].data_ptr(), d, w.K, w.Kp, st),
+                       'unpad_add')
+        if m._after_layer_backward is not None:
+            m._after_layer_backward(-1)
+
+    def _stack_backward(self, s):
+        """backward through the blocks of the stack s, from the gradient of its output in s.dz[(depth - 1) & 1] (its
+        column sum already added to the top ff2 bias gradient when p = 0) to that of its input in s.dz[1]; the weight
+        gradients run on the side stream, which is joined at the end"""
+        m, lib, st = self.model, self.lib, self._stream
+        dt = m._dtype_code
+        rdt = m._res_code
+        M, d, mlp, H = s.M, s.d, s.mlp, s.H
+        B, N = s.B, s.N
+        inner, dh = d, d // H
+        depth = s.depth
+        wt, pf, gr = m._weights(), m._params_f32(), m._grads_f32()
+        p_blk = s.p_blk
+        seed_ptr = self.rng.data_ptr()
+        blk_seed = seed_ptr if p_blk > 0 else None
+        last = f'{s.prefix}{depth - 1}.'
+        top = (depth - 1) & 1
         scale = float(dh) ** -0.5
 
         main, side = torch.cuda.current_stream(), self.side_stream
@@ -402,7 +451,7 @@ class StepEngine:
         def layernorm_bwd(which, dln, x_in, gamma, stat, dres, dx, dgamma, dbeta, dcol, dxm, p_drop, site):
             """dx = dres + LN'(dln) (+ the dropout-masked copy dxm) on the main stream; the fold of the per-CTA partial rows
             into dgamma / dbeta / dcol feeds nothing in the chain and runs on the side stream"""
-            scr = w.ln_scratch[which]
+            scr = s.ln_scratch[which]
             before_overwrite(ev_fold[which])  # the fold of this scratch's previous user
             seed = blk_seed if (dxm is not None and p_drop > 0) else None
             _lib.check(lib.ecgvit_layernorm_bwd(
@@ -425,26 +474,26 @@ class StepEngine:
         evs = {}
         if p_blk > 0:
             # the top block's input gradient comes from the head, not from a LayerNorm': mask it here
-            _lib.check(lib.ecgvit_dropout_bwd_copy(w.dz[top].data_ptr(), w.dzm[0][top].data_ptr(),
+            _lib.check(lib.ecgvit_dropout_bwd_copy(s.dz[top].data_ptr(), s.dzm[0][top].data_ptr(),
                                                    gr[last + 'ff2.b'].data_ptr(), M, d, d, p_blk, 4 * depth, seed_ptr, dt, st),
                        'dropout_bwd_copy')
         for l in range(depth - 1, -1, -1):
-            p = f'l{l}.'
+            p = f'{s.prefix}{l}.'
             q, qn = l & 1, (l - 1) & 1      # buffer parity of this layer / of the layer below
             s_att, s_out, s_act, s_ff2 = 1 + 4 * l, 2 + 4 * l, 3 + 4 * l, 4 + 4 * l
             old = evs.pop(l + 2, {})        # the previous users of this parity's buffers (a whole layer ago)
-            if w.ckpt and l < depth - 2:
+            if s.ckpt and l < depth - 2:
                 # the activation set of layer l was last used by layer l + 2: its weight gradients must have read it
                 for ev in old.values():
                     before_overwrite(ev)
-                self._block_forward(l, w, recompute=True)
+                self._block_forward(l, s, recompute=True)
             e = evs.setdefault(l, {})
-            dz, dy, du, dqkv = w.dz[q], w.dy[q], w.du[q], w.dqkv[q]
-            dzl = w.dzm[0][q] if p_blk > 0 else dz      # what net[3] saw: mask * dz / (1 - p)
+            dz, dy, du, dqkv = s.dz[q], s.dy[q], s.du[q], s.dqkv[q]
+            dzl = s.dzm[0][q] if p_blk > 0 else dz      # what net[3] saw: mask * dz / (1 - p)
             # ---- feed-forward branch: x[l+1] = y + drop(W2 drop(gelu(W1 ln2(y) + b1)) + b2)
-            e['ff2'] = wgrad(d, mlp, M, dzl, d, 0, w.h[l], mlp, 0, EPI_ATOMIC_F32, gr[p + 'ff2.w'], mlp, split_k=0)
+            e['ff2'] = wgrad(d, mlp, M, dzl, d, 0, s.h[l], mlp, 0, EPI_ATOMIC_F32, gr[p + 'ff2.w'], mlp, split_k=0)
             before_overwrite(old.get('ff1'))   # du of this parity
-            self._gemm(M, mlp, d, dzl, d, 1, wt[p + 'ff2.w'], mlp, 0, EPI_DGELU, du, mlp, aux=w.u[l], drop=(p_blk, s_act))
+            self._gemm(M, mlp, d, dzl, d, 1, wt[p + 'ff2.w'], mlp, 0, EPI_DGELU, du, mlp, aux=s.u[l], drop=(p_blk, s_act))
             # FF1's bias gradient (column sums of du) feeds nothing in the chain: it rides on the side stream in front of
             # FF1's weight gradient (same operand, so the event that guards `du` covers both)
             if side is None:
@@ -456,31 +505,31 @@ class StepEngine:
                 with torch.cuda.stream(side):
                     _lib.check(lib.ecgvit_colsum(du.data_ptr(), gr[p + 'ff1.b'].data_ptr(), M, mlp, mlp, dt,
                                                  side.cuda_stream), 'colsum')
-            e['ff1'] = wgrad(mlp, d, M, du, mlp, 0, w.ln2[l], d, 0, EPI_ATOMIC_F32, gr[p + 'ff1.w'], d, split_k=0)
-            self._gemm(M, d, mlp, du, mlp, 1, wt[p + 'ff1.w'], d, 0, EPI_STORE, w.dln, d)
+            e['ff1'] = wgrad(mlp, d, M, du, mlp, 0, s.ln2[l], d, 0, EPI_ATOMIC_F32, gr[p + 'ff1.w'], d, split_k=0)
+            self._gemm(M, d, mlp, du, mlp, 1, wt[p + 'ff1.w'], d, 0, EPI_STORE, s.dln, d)
             before_overwrite(old.get('out'))   # dy / its masked copy of this parity
-            dyl = w.dzm[1][q] if p_blk > 0 else dy
-            layernorm_bwd(0, w.dln, w.y[l], pf[p + 'ln2.w'], w.stat2[l], dz, dy, gr[p + 'ln2.w'], gr[p + 'ln2.b'],
+            dyl = s.dzm[1][q] if p_blk > 0 else dy
+            layernorm_bwd(0, s.dln, s.y[l], pf[p + 'ln2.w'], s.stat2[l], dz, dy, gr[p + 'ln2.w'], gr[p + 'ln2.b'],
                           gr[p + 'out.b'], dyl if p_blk > 0 else None, p_blk, s_out)
             # ---- attention branch: y = x + drop(Wo attn(Wqkv ln1(x)) + bo); dyl = mask * dy / (1 - p)
-            e['out'] = wgrad(d, inner, M, dyl, d, 0, w.o[l], inner, 0, EPI_ATOMIC_F32, gr[p + 'out.w'], inner, split_k=0)
-            self._gemm(M, inner, d, dyl, d, 1, wt[p + 'out.w'], inner, 0, EPI_STORE, w.d_o, inner)
+            e['out'] = wgrad(d, inner, M, dyl, d, 0, s.o[l], inner, 0, EPI_ATOMIC_F32, gr[p + 'out.w'], inner, split_k=0)
+            self._gemm(M, inner, d, dyl, d, 1, wt[p + 'out.w'], inner, 0, EPI_STORE, s.d_o, inner)
             before_overwrite(old.get('qkv'))   # dqkv of this parity
-            _lib.check(lib.ecgvit_attention_bwd(w.qkv[l].data_ptr(), w.o[l].data_ptr(), w.d_o.data_ptr(),
-                                                w.lse[l].data_ptr(), dqkv.data_ptr(), _lib.ptr(w.attn_scratch), B, N,
+            _lib.check(lib.ecgvit_attention_bwd(s.qkv[l].data_ptr(), s.o[l].data_ptr(), s.d_o.data_ptr(),
+                                                s.lse[l].data_ptr(), dqkv.data_ptr(), _lib.ptr(s.attn_scratch), B, N,
                                                 H, dh, scale, p_blk, s_att, blk_seed, dt, st),
-                       'attention_bwd' if w.attn_scratch is None else 'attention_bwd_flash')
-            e['qkv'] = wgrad(3 * inner, d, M, dqkv, 3 * inner, 0, w.ln1[l], d, 0, EPI_ATOMIC_F32, gr[p + 'qkv.w'], d,
+                       'attention_bwd' if s.attn_scratch is None else 'attention_bwd_flash')
+            e['qkv'] = wgrad(3 * inner, d, M, dqkv, 3 * inner, 0, s.ln1[l], d, 0, EPI_ATOMIC_F32, gr[p + 'qkv.w'], d,
                              split_k=0)
-            self._gemm(M, d, 3 * inner, dqkv, 3 * inner, 1, wt[p + 'qkv.w'], d, 0, EPI_STORE, w.dln, d)
-            below_bias = gr[f'l{l - 1}.ff2.b'] if l > 0 else None
+            self._gemm(M, d, 3 * inner, dqkv, 3 * inner, 1, wt[p + 'qkv.w'], d, 0, EPI_STORE, s.dln, d)
+            below_bias = gr[f'{s.prefix}{l - 1}.ff2.b'] if l > 0 else None
             drop_below = p_blk > 0 and l > 0
             # LayerNorm' writes the input gradient of layer l - 1 into the OTHER parity, last read by the ff2 weight
             # gradient of layer l + 1
             before_overwrite(evs.get(l + 1, {}).get('ff2'))
-            layernorm_bwd(1, w.dln, w.x[l], pf[p + 'ln1.w'], w.stat1[l], dy, w.dz[qn], gr[p + 'ln1.w'], gr[p + 'ln1.b'],
-                          below_bias, w.dzm[0][qn] if drop_below else None, p_blk if drop_below else 0.0, s_ff2 - 4)
-            if m._after_layer_backward is not None:
+            layernorm_bwd(1, s.dln, s.x[l], pf[p + 'ln1.w'], s.stat1[l], dy, s.dz[qn], gr[p + 'ln1.w'], gr[p + 'ln1.b'],
+                          below_bias, s.dzm[0][qn] if drop_below else None, p_blk if drop_below else 0.0, s_ff2 - 4)
+            if s.hooks and m._after_layer_backward is not None:
                 # the gradient bucket of layer l is complete once its side-stream wgrads AND everything the main stream
                 # has issued so far (LayerNorm / bias gradients) are done.  The collective is therefore issued from the
                 # side stream after it has waited for the main stream's current point: c10d orders the NCCL kernel
@@ -498,18 +547,6 @@ class StepEngine:
                 before_overwrite(ev)  # join the side stream
         for ev in ev_fold:
             before_overwrite(ev)
-        dz = w.dz[(-1) & 1]   # gradient w.r.t. the token matrix (input of block 0)
-        # ---- embedding: tok = [cls | a_patch We^T + be] + pos
-        self._assemble_backward(w, dz)
-        if w.Kp == w.K:
-            self._gemm(d, w.K, B * n, w.de, d, 0, w.a_patch, w.K, 0, EPI_ATOMIC_F32, gr['embed.w'], w.K, split_k=0)
-        else:
-            w.embed_gpad.zero_()
-            self._gemm(d, w.Kp, B * n, w.de, d, 0, w.a_patch, w.Kp, 0, EPI_ATOMIC_F32, w.embed_gpad, w.Kp, split_k=0)
-            _lib.check(lib.ecgvit_unpad_add_f32(w.embed_gpad.data_ptr(), gr['embed.w'].data_ptr(), d, w.K, w.Kp, st),
-                       'unpad_add')
-        if m._after_layer_backward is not None:
-            m._after_layer_backward(-1)
 
     def _head_backward(self, w, dtok, dcolsum, grad_scale, grad_scale_dev):
         """backward of `_head_forward`: writes the whole token-shaped gradient `dtok` of the encoder output and adds its
@@ -561,12 +598,12 @@ class MaskedPatchEngine(StepEngine):
         """counter-hash site of the mask keys: the dropout sites are 0 .. 4 * depth"""
         return 4 * self.model.config.num_hidden_layers + 1
 
-    def workspace(self, B, L):
-        w = super().workspace(B, L)
+    def workspace(self, B, L, n_vis=None):
+        w = super().workspace(B, L, n_vis)
         if hasattr(w, 'mask'):
             return w
         m = self.model
-        d = m.config.hidden_size
+        d = m.recon_head[0].normalized_shape[0]   # width of the token matrix the head reads
         T = m._act_dtype
         rows, K, Kp = B * w.n, w.K, w.Kp
         dev = self.device
@@ -598,9 +635,9 @@ class MaskedPatchEngine(StepEngine):
         finally:
             self._user_mask = None
 
-    def _assemble(self, w):
+    def _draw_mask(self, w):
+        """w.mask / w.counts: the caller's mask, or round(mask_ratio * n) patches per record drawn on the device"""
         m, lib, st = self.model, self.lib, self._stream
-        pf = m._params_f32()
         B, n = w.B, w.n
         user = self._user_mask
         if user is not None:
@@ -613,6 +650,12 @@ class MaskedPatchEngine(StepEngine):
             seed = (self.rng if m.training else self._eval_seed).data_ptr()
         _lib.check(lib.ecgvit_mpm_mask(seed, B, n, k if user is None else 0, self.mask_site, w.mask.data_ptr(),
                                        w.counts.data_ptr(), st), 'mpm_mask')
+
+    def _assemble(self, w):
+        m, lib, st = self.model, self.lib, self._stream
+        pf = m._params_f32()
+        B, n = w.B, w.n
+        self._draw_mask(w)
         _lib.check(lib.ecgvit_embed_assemble_masked(
             w.e.data_ptr(), pf['cls'].data_ptr(), pf['pos'].data_ptr(), pf['mask'].data_ptr(), w.mask.data_ptr(),
             w.x[0].data_ptr(), B, n, m.config.hidden_size, w.p_emb, 0, self.rng.data_ptr() if w.p_emb > 0 else None,
@@ -626,10 +669,14 @@ class MaskedPatchEngine(StepEngine):
             return wt['recon.w'], pf['recon.b']
         return w.recon_wpad, w.recon_bpad
 
+    def _head_stack(self, w):
+        """the block stack whose output the reconstruction head reads: the encoder"""
+        return w
+
     def _head_forward(self, w, labels, reduction):
         m, lib, st = self.model, self.lib, self._stream
-        c = m.config
-        d = c.hidden_size
+        hs = self._head_stack(w)
+        d = hs.d
         pf, wt = m._params_f32(), m._weights()
         B, n, K, Kp = w.B, w.n, w.K, w.Kp
         rows = B * n
@@ -641,7 +688,7 @@ class MaskedPatchEngine(StepEngine):
                        'pad_cols')
         w_r, b_r = self._recon_params(w)
         _lib.check(lib.ecgvit_layernorm_patch_fwd(
-            w.x[c.num_hidden_layers].data_ptr(), pf['recon.ln.w'].data_ptr(), pf['recon.ln.b'].data_ptr(),
+            hs.x[hs.depth].data_ptr(), pf['recon.ln.w'].data_ptr(), pf['recon.ln.b'].data_ptr(),
             w.ln_r.data_ptr(), w.rstat[0].data_ptr(), w.rstat[1].data_ptr(), B, n, d, LN_EPS, m._res_code, st),
             'layernorm_patch_fwd')
         self._gemm(rows, Kp, d, w.ln_r, d, 1, w_r, d, 1, EPI_BIAS_SUB_ROWSQ, w.r, Kp, out2=w.rowsq, aux=w.a_patch,
@@ -667,8 +714,8 @@ class MaskedPatchEngine(StepEngine):
 
     def _head_backward(self, w, dtok, dcolsum, grad_scale, grad_scale_dev):
         m, lib, st = self.model, self.lib, self._stream
-        c = m.config
-        d = c.hidden_size
+        hs = self._head_stack(w)
+        d = hs.d
         dt = m._dtype_code
         pf, gr = m._params_f32(), m._grads_f32()
         B, n, K, Kp = w.B, w.n, w.K, w.Kp
@@ -691,9 +738,9 @@ class MaskedPatchEngine(StepEngine):
         w_r, _ = self._recon_params(w)
         self._gemm(rows, d, Kp, w.dpred, Kp, 1, w_r, d, 0, EPI_STORE, w.dln_r, d)
         _lib.check(lib.ecgvit_layernorm_patch_bwd(
-            w.dln_r.data_ptr(), w.x[c.num_hidden_layers].data_ptr(), pf['recon.ln.w'].data_ptr(), w.rstat[0].data_ptr(),
+            w.dln_r.data_ptr(), hs.x[hs.depth].data_ptr(), pf['recon.ln.w'].data_ptr(), w.rstat[0].data_ptr(),
             w.rstat[1].data_ptr(), dtok.data_ptr(), gr['recon.ln.w'].data_ptr(), gr['recon.ln.b'].data_ptr(),
-            _lib.ptr(dcolsum), w.ln_scratch[0].data_ptr(), B, n, d, m._res_code, st), 'layernorm_patch_bwd')
+            _lib.ptr(dcolsum), hs.ln_scratch[0].data_ptr(), B, n, d, m._res_code, st), 'layernorm_patch_bwd')
 
     def _assemble_backward(self, w, dz):
         m, lib, st = self.model, self.lib, self._stream
@@ -703,3 +750,117 @@ class MaskedPatchEngine(StepEngine):
             dz.data_ptr(), w.mask.data_ptr(), w.de.data_ptr(), gr['cls'].data_ptr(), gr['pos'].data_ptr(),
             gr['embed.b'].data_ptr(), gr['mask'].data_ptr(), w.B, w.n, m.config.hidden_size, p_emb, 0,
             self.rng.data_ptr() if p_emb > 0 else None, m._dtype_code, st), 'embed_assemble_masked_bwd')
+
+
+class MaskedAutoencoderEngine(MaskedPatchEngine):
+    """StepEngine of `EcgVitForMaskedAutoencoding` (MAE): the encoder sees only the n_vis visible patches of every
+    record; a second, narrower block stack (the decoder, keys `dec{i}.`) runs over all n + 1 positions and the head and
+    loss are `MaskedPatchEngine`'s, at the decoder's width.
+
+    Forward: patchify -> mask draw -> index build (vis_idx [B, n_vis], slot [B, n]) -> row gather of the visible patch
+    rows -> embedding GEMM on B * n_vis rows -> visible assemble (pos at the patches' positions) -> encoder blocks over
+    n_vis + 1 tokens -> LayerNorm + decoder embedding GEMM -> unshuffle (mask token at the masked positions, + decoder pos)
+    -> decoder blocks over n + 1 tokens -> reconstruction head.  Backward runs the same path in reverse."""
+
+    def workspace(self, B, L, n_vis=None):
+        m = self.model
+        c = m.config
+        if n_vis is None:
+            n = L // c.patch_size * (c.num_channels if getattr(c, 'per_lead_tokens', False) else 1)
+            k = self._user_k if self._user_mask is not None else int(round(m.mask_ratio * n))
+            n_vis = n - k
+        w = super().workspace(B, L, n_vis)
+        if hasattr(w, 'dec'):
+            return w
+        dev, T = self.device, m._act_dtype
+        d, dd = c.hidden_size, m.decoder_hidden_size
+        n, nv, Kp, M = w.n, w.n_vis, w.Kp, w.M
+        w.vis_idx = torch.empty(B, nv, device=dev, dtype=torch.int32)
+        w.slot = torch.empty(B, n, device=dev, dtype=torch.int32)
+        w.a_vis = torch.empty(B * nv, Kp, device=dev, dtype=T)
+        w.a_emb = w.a_vis
+        w.ln_t = torch.empty(M, d, device=dev, dtype=T)            # decoder.norm(encoder output)
+        w.stat_t = torch.empty(2, M, device=dev, dtype=torch.float32)
+        w.t = torch.empty(M, dd, device=dev, dtype=T)              # decoder.embed(ln_t)
+        w.dt = torch.empty(M, dd, device=dev, dtype=T)
+        w.dln_t = torch.empty(M, d, device=dev, dtype=T)
+        # per-position partial sums of the two deterministic backward folds (used one after the other)
+        w.pos_scratch = torch.empty(n * max(d, dd), device=dev, dtype=torch.float32)
+        w.dec = _Workspace()
+        self._alloc_stack(w.dec, 'dec', B, n + 1, dd, m.decoder_intermediate_size, m.decoder_num_attention_heads,
+                          m.decoder_num_hidden_layers, False)
+        return w
+
+    def forward(self, sample_values, labels=None, reduction='mean', record_attention=False, bool_masked_pos=None):
+        # the caller's mask sets the encoder's token count: its per-record count (equal in every record, checked by the
+        # model) is read on the host
+        self._user_k = None if bool_masked_pos is None else int(bool_masked_pos[0].sum())
+        return super().forward(sample_values, labels, reduction, record_attention, bool_masked_pos)
+
+    def _select_patches(self, w):
+        lib, st = self.lib, self._stream
+        self._draw_mask(w)
+        _lib.check(lib.ecgvit_mae_index(w.mask.data_ptr(), w.B, w.n, w.n_vis, w.vis_idx.data_ptr(), w.slot.data_ptr(),
+                                        st), 'mae_index')
+        _lib.check(lib.ecgvit_row_gather(w.a_patch.data_ptr(), w.a_vis.data_ptr(), w.vis_idx.data_ptr(), w.B, w.n,
+                                         w.n_vis, w.Kp, self.model._dtype_code, st), 'row_gather')
+
+    def _assemble(self, w):
+        m, lib, st = self.model, self.lib, self._stream
+        pf = m._params_f32()
+        _lib.check(lib.ecgvit_embed_assemble_visible(
+            w.e.data_ptr(), pf['cls'].data_ptr(), pf['pos'].data_ptr(), w.vis_idx.data_ptr(), w.x[0].data_ptr(), w.B,
+            w.n_vis, m.config.hidden_size, w.p_emb, 0, self.rng.data_ptr() if w.p_emb > 0 else None, m._res_code, st),
+            'embed_assemble_visible')
+
+    def _head_stack(self, w):
+        return w.dec
+
+    def _head_forward(self, w, labels, reduction):
+        m, lib, st = self.model, self.lib, self._stream
+        c = m.config
+        pf, wt = m._params_f32(), m._weights()
+        d, dec = c.hidden_size, w.dec
+        _lib.check(lib.ecgvit_layernorm_fwd(w.x[c.num_hidden_layers].data_ptr(), pf['dec.ln.w'].data_ptr(),
+                                            pf['dec.ln.b'].data_ptr(), w.ln_t.data_ptr(), w.stat_t[0].data_ptr(),
+                                            w.stat_t[1].data_ptr(), w.M, d, LN_EPS, m._res_code, st), 'layernorm_fwd')
+        self._gemm(w.M, dec.d, d, w.ln_t, d, 1, wt['dec.embed.w'], d, 1, EPI_STORE, w.t, dec.d, bias=pf['dec.embed.b'])
+        _lib.check(lib.ecgvit_mae_unshuffle(w.t.data_ptr(), pf['dec.mask'].data_ptr(), pf['dec.pos'].data_ptr(),
+                                            w.slot.data_ptr(), dec.x[0].data_ptr(), w.B, w.n, w.n_vis, dec.d,
+                                            m._res_code, st), 'mae_unshuffle')
+        for l in range(dec.depth):
+            self._block_forward(l, dec)
+        return super()._head_forward(w, labels, reduction)
+
+    def _head_backward(self, w, dtok, dcolsum, grad_scale, grad_scale_dev):
+        m, lib, st = self.model, self.lib, self._stream
+        c = m.config
+        dt = m._dtype_code
+        wt, pf, gr = m._weights(), m._params_f32(), m._grads_f32()
+        d, dec, M = c.hidden_size, w.dec, w.M
+        super()._head_backward(w, dec.dz[(dec.depth - 1) & 1], gr[f'dec{dec.depth - 1}.ff2.b'], grad_scale,
+                               grad_scale_dev)
+        self._stack_backward(dec)
+        _lib.check(lib.ecgvit_mae_unshuffle_bwd(dec.dz[1].data_ptr(), w.slot.data_ptr(), w.dt.data_ptr(),
+                                                gr['dec.pos'].data_ptr(), gr['dec.mask'].data_ptr(),
+                                                w.pos_scratch.data_ptr(), w.B, w.n, w.n_vis, dec.d, dt, st),
+                   'mae_unshuffle_bwd')
+        # decoder.embed: weight gradient dt^T ln_t, bias gradient colsum(dt), input gradient dt We
+        self._gemm(dec.d, d, M, w.dt, dec.d, 0, w.ln_t, d, 0, EPI_ATOMIC_F32, gr['dec.embed.w'], d, split_k=0)
+        _lib.check(lib.ecgvit_colsum(w.dt.data_ptr(), gr['dec.embed.b'].data_ptr(), M, dec.d, dec.d, dt, st), 'colsum')
+        self._gemm(M, d, dec.d, w.dt, dec.d, 1, wt['dec.embed.w'], d, 0, EPI_STORE, w.dln_t, d)
+        # decoder.norm': the whole gradient of the encoder output (no residual term), its column sum into the top block's
+        # ff2 bias gradient when that block has no dropout
+        _lib.check(lib.ecgvit_layernorm_bwd(
+            w.dln_t.data_ptr(), w.x[c.num_hidden_layers].data_ptr(), pf['dec.ln.w'].data_ptr(), w.stat_t[0].data_ptr(),
+            w.stat_t[1].data_ptr(), None, dtok.data_ptr(), gr['dec.ln.w'].data_ptr(), gr['dec.ln.b'].data_ptr(),
+            _lib.ptr(dcolsum), w.ln_scratch[0].data_ptr(), None, 0.0, 0, None, M, d, 0, m._res_code, st),
+            'layernorm_bwd')
+
+    def _assemble_backward(self, w, dz):
+        m, lib, st = self.model, self.lib, self._stream
+        gr = m._grads_f32()
+        _lib.check(lib.ecgvit_embed_assemble_visible_bwd(
+            dz.data_ptr(), w.slot.data_ptr(), w.de.data_ptr(), gr['cls'].data_ptr(), gr['pos'].data_ptr(),
+            gr['embed.b'].data_ptr(), w.pos_scratch.data_ptr(), w.B, w.n, w.n_vis, m.config.hidden_size, w.p_emb, 0,
+            self.rng.data_ptr() if w.p_emb > 0 else None, m._dtype_code, st), 'embed_assemble_visible_bwd')

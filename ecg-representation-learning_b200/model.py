@@ -17,7 +17,7 @@ from torch import nn
 
 from . import _lib
 from .config import EcgVitConfig
-from .engine import StepEngine, MaskedPatchEngine
+from .engine import StepEngine, MaskedPatchEngine, MaskedAutoencoderEngine
 
 ModelOutput = namedtuple('ModelOutput', ['loss', 'logits'])  # reference: util/models.py:3
 MaskedPatchOutput = namedtuple('MaskedPatchOutput', ['loss', 'reconstruction', 'bool_masked_pos'])
@@ -155,7 +155,8 @@ class _EcgVitFunction(torch.autograd.Function):
 
 
 class EcgVit(nn.Module):
-    _classification_head = True   # ViT container with `mlp_head` and no mask token
+    _classification_head = True   # ViT container with `mlp_head`
+    _encoder_mask_token = False   # ... and without `mask_token`
     _engine_class = StepEngine
 
     def __init__(self, num_class: int = 71, config: EcgVitConfig = None, loss_reduction: str = 'mean'):
@@ -171,7 +172,7 @@ class EcgVit(nn.Module):
                        dropout=config.hidden_dropout_prob,              # attention + feed-forward (ecg_vit.py:113)
                        emb_dropout=config.attention_probs_dropout_prob,  # embedding (ecg_vit.py:114)
                        per_lead=bool(getattr(config, 'per_lead_tokens', False)),
-                       head=self._classification_head, mask_token=not self._classification_head)
+                       head=self._classification_head, mask_token=self._encoder_mask_token)
         self.vit._owner = weakref.ref(self)  # lets `Recorder(model.vit)` reach the kernels (not a module: no cycle)
         self._loss_reduction = loss_reduction
         self.loss_weight = None
@@ -261,6 +262,9 @@ class EcgVit(nn.Module):
             wb = 'w' if parts[-1] == 'weight' else 'b'
             if parts[0] == 'recon_head':
                 k = ('recon.ln.' if parts[1] == '0' else 'recon.') + wb
+            elif parts[0] == 'decoder' and parts[1] != 'transformer':
+                k = {'norm': 'dec.ln.' + wb, 'embed': 'dec.embed.' + wb, 'mask_token': 'dec.mask',
+                     'pos_embedding': 'dec.pos'}[parts[1]]
             elif name == 'vit.pos_embedding':
                 k = 'pos'
             elif name == 'vit.cls_token':
@@ -271,15 +275,16 @@ class EcgVit(nn.Module):
                 k = 'embed.' + ('w' if parts[-1] == 'weight' else 'b')
             elif parts[1] == 'mlp_head':
                 k = ('head.ln.' if parts[2] == '0' else 'head.') + ('w' if parts[-1] == 'weight' else 'b')
-            else:  # vit.transformer.layers.{i}.{0|1}.(norm|fn)...
+            else:  # (vit|decoder).transformer.layers.{i}.{0|1}.(norm|fn)...
                 i, branch = int(parts[3]), int(parts[4])
                 wb = 'w' if parts[-1] == 'weight' else 'b'
+                L = 'dec' if parts[0] == 'decoder' else 'l'
                 if parts[5] == 'norm':
-                    k = f'l{i}.ln{branch + 1}.{wb}'
+                    k = f'{L}{i}.ln{branch + 1}.{wb}'
                 elif branch == 0:
-                    k = f'l{i}.qkv.{wb}' if parts[6] == 'to_qkv' else f'l{i}.out.{wb}'
+                    k = f'{L}{i}.qkv.{wb}' if parts[6] == 'to_qkv' else f'{L}{i}.out.{wb}'
                 else:
-                    k = f'l{i}.ff1.{wb}' if parts[7] == '0' else f'l{i}.ff2.{wb}'
+                    k = f'{L}{i}.ff1.{wb}' if parts[7] == '0' else f'{L}{i}.ff2.{wb}'
             out[name] = k
         return out
 
@@ -352,6 +357,19 @@ class EcgVit(nn.Module):
         return [self._views_g[k] for k in names.values()]
 
 
+def _recon_patch_dim(c):
+    """features of one patch, the reconstruction target's width; rejects the widths the reconstruction kernels cannot
+    read"""
+    per_lead = bool(getattr(c, 'per_lead_tokens', False))
+    patch_dim = c.patch_size if per_lead else c.patch_size * c.num_channels
+    if not per_lead and patch_dim % 8 != 0:
+        # the residual / its gradient share the patch matrix's row length, and their column kernels read 8 elements
+        # at a time (per-lead rows are padded to a multiple of 8 instead)
+        raise ValueError(f'masked-patch pre-training needs patch_size * num_channels = {patch_dim} to be a multiple '
+                         f'of 8')
+    return patch_dim
+
+
 class _MaskedPatchFunction(_EcgVitFunction):
     """autograd bridge of `EcgVitForMaskedPatchModeling` (`loss.backward()` then e.g. `FusedAdamW`); backward, with its
     workspace / seed guards, is `_EcgVitFunction`'s"""
@@ -390,6 +408,7 @@ class EcgVitForMaskedPatchModeling(EcgVit):
     `encoder_state_dict()` hands the encoder over to fine-tuning:
     `EcgVit(config=...).load_state_dict(pre.encoder_state_dict(), strict=False)` misses only `vit.mlp_head.*`."""
     _classification_head = False
+    _encoder_mask_token = True
     _engine_class = MaskedPatchEngine
 
     def __init__(self, config: EcgVitConfig = None, mask_ratio: float = 0.5):
@@ -397,14 +416,7 @@ class EcgVitForMaskedPatchModeling(EcgVit):
             raise ValueError(f'mask_ratio must lie in [0, 1], got {mask_ratio}')
         super().__init__(num_class=0, config=config)
         c = self.config
-        per_lead = bool(getattr(c, 'per_lead_tokens', False))
-        patch_dim = c.patch_size if per_lead else c.patch_size * c.num_channels
-        if not per_lead and patch_dim % 8 != 0:
-            # the residual / its gradient share the patch matrix's row length, and their column kernels read 8 elements
-            # at a time (per-lead rows are padded to a multiple of 8 instead)
-            raise ValueError(f'masked-patch pre-training needs patch_size * num_channels = {patch_dim} to be a multiple '
-                             f'of 8')
-        self.recon_head = nn.Sequential(nn.LayerNorm(c.hidden_size), nn.Linear(c.hidden_size, patch_dim))
+        self.recon_head = nn.Sequential(nn.LayerNorm(c.hidden_size), nn.Linear(c.hidden_size, _recon_patch_dim(c)))
         self.mask_ratio = float(mask_ratio)
 
     def _draws_step_seed(self):
@@ -445,6 +457,76 @@ class EcgVitForMaskedPatchModeling(EcgVit):
             loss, _ = eng.forward(sample_values, bool_masked_pos=bool_masked_pos)
             loss, recon, mask = loss.clone(), eng.reconstruction(), eng.mask()
         return MaskedPatchOutput(loss=loss, reconstruction=recon, bool_masked_pos=mask)
+
+
+class _Decoder(nn.Module):
+    """MAE decoder parameters: `norm` (the LayerNorm MAE puts at the end of its encoder; here, so that the encoder keys
+    stay those of `EcgVit`), `embed` Linear(d -> d_dec), `mask_token` [1, 1, d_dec], the learned `pos_embedding`
+    [1, n + 1, d_dec] and `transformer`, blocks with the encoder's structure and no dropout"""
+
+    def __init__(self, dim, n_patch, dec_dim, depth, heads, mlp_dim):
+        super().__init__()
+        self.norm = nn.LayerNorm(dim)
+        self.embed = nn.Linear(dim, dec_dim)
+        self.mask_token = nn.Parameter(torch.zeros(1, 1, dec_dim))
+        self.pos_embedding = nn.Parameter(torch.randn(1, n_patch + 1, dec_dim))
+        self.transformer = Transformer(dec_dim, depth, heads, dec_dim // heads, mlp_dim, 0.0)
+    forward = _no_eager
+
+
+class EcgVitForMaskedAutoencoding(EcgVitForMaskedPatchModeling):
+    """MAE-style pre-training of the `EcgVit` encoder on unlabelled records.
+
+    The encoder runs over the CLS token and the visible patches only (their embeddings plus the positional embedding of
+    their own positions).  `decoder` normalises and embeds its output at the decoder width, puts `decoder.mask_token` on
+    every masked position, adds `decoder.pos_embedding` and runs its own, narrower blocks over all n + 1 positions;
+    `recon_head` = LayerNorm + Linear(d_dec, patch_dim) predicts every patch.  The loss is the mean squared error over
+    the masked patches, as in `EcgVitForMaskedPatchModeling`, whose interface this model shares: `forward` returns
+    `MaskedPatchOutput(loss, reconstruction [B, n, patch_dim], bool_masked_pos)`, and `encoder_state_dict()` /
+    `unpatchify()` behave the same.
+
+    Exactly k = round(mask_ratio * n) patches of every record are masked (training: a fresh mask every forward, eval: a
+    fixed one).  A caller's `bool_masked_pos` must mask the same number of patches, between 1 and n - 1, in every
+    record (the encoder's token count depends on it); it is checked on the host.  The decoder has no dropout and never
+    checkpoints; the encoder follows the config."""
+    _encoder_mask_token = False
+    _engine_class = MaskedAutoencoderEngine
+
+    def __init__(self, config: EcgVitConfig = None, mask_ratio: float = 0.75, decoder_hidden_size: int = 256,
+                 decoder_num_hidden_layers: int = 4, decoder_num_attention_heads: int = 4,
+                 decoder_intermediate_size: int = 1024):
+        EcgVit.__init__(self, num_class=0, config=config)
+        c = self.config
+        n = c.max_signal_length // c.patch_size * (c.num_channels if getattr(c, 'per_lead_tokens', False) else 1)
+        k = int(round(float(mask_ratio) * n))
+        if not 1 <= k <= n - 1:
+            raise ValueError(f'mask_ratio {mask_ratio} masks {k} of {n} patches: MAE needs at least one masked and one '
+                             f'visible patch')
+        dd, dh = int(decoder_hidden_size), int(decoder_num_attention_heads)
+        if dh < 1 or dd % dh != 0:
+            raise ValueError(f'decoder_hidden_size {dd} is not a multiple of decoder_num_attention_heads {dh}')
+        if (dd // dh) % 8 != 0:
+            raise ValueError(f'decoder head dim {dd // dh} must be a multiple of 8')
+        if int(decoder_intermediate_size) < 8 or int(decoder_intermediate_size) % 8 != 0:
+            # the decoder's MLP width is a GEMM row length: 16-byte aligned rows
+            raise ValueError(f'decoder_intermediate_size {decoder_intermediate_size} must be a positive multiple of 8')
+        if int(decoder_num_hidden_layers) < 1:
+            raise ValueError('the decoder needs at least one block')
+        patch_dim = _recon_patch_dim(c)
+        self.decoder = _Decoder(c.hidden_size, n, dd, int(decoder_num_hidden_layers), dh, int(decoder_intermediate_size))
+        self.recon_head = nn.Sequential(nn.LayerNorm(dd), nn.Linear(dd, patch_dim))
+        self.mask_ratio = float(mask_ratio)
+        self.decoder_hidden_size, self.decoder_num_hidden_layers = dd, int(decoder_num_hidden_layers)
+        self.decoder_num_attention_heads, self.decoder_intermediate_size = dh, int(decoder_intermediate_size)
+
+    def forward(self, sample_values: torch.FloatTensor, bool_masked_pos: torch.BoolTensor = None, time_out_spans=None):
+        if bool_masked_pos is not None:
+            counts = bool_masked_pos.reshape(bool_masked_pos.shape[0], -1).sum(1).cpu()
+            n = self.vit.pos_embedding.shape[1] - 1
+            if not (counts == counts[0]).all() or not 1 <= int(counts[0]) <= n - 1:
+                raise ValueError(f'bool_masked_pos must mask the same number of patches, between 1 and {n - 1}, in every '
+                                 f'record; got counts {counts.tolist()}')
+        return super().forward(sample_values, bool_masked_pos, time_out_spans)
 
 
 class Recorder(nn.Module):

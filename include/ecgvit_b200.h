@@ -141,6 +141,40 @@ int ecgvit_mpm_dpred(const void *r, const uint8_t *mask, const float *count, int
 int ecgvit_mpm_reconstruction(const void *r, const void *target, float *out, int rows, int ld, int K, int dtype,
                               void *stream);
 
+/* ---- MAE-style pre-training (the encoder sees only the visible patches; a second, narrower block stack decodes).
+ *      Added in ABI version 7 without changing any earlier entry point, so the version number stays 7.
+ *
+ *      Index build, one CTA per record (n_patch <= 12000): from mask uint8 [B, n_patch] (n_vis patches with mask 0 in
+ *      every record) vis_idx int32 [B, n_vis] = the ascending positions of the visible patches, and slot int32
+ *      [B, n_patch] = a patch's index among them, or -1 when it is masked. */
+int ecgvit_mae_index(const uint8_t *mask, int B, int n_patch, int n_vis, int *vis_idx, int *slot, void *stream);
+/* dst[b*n_dst + j, :] = src[b*n_src + idx[b*n_dst + j], :] for rows of ld elements (dtype BF16 / F32); the row length
+ * must be a multiple of 16 bytes */
+int ecgvit_row_gather(const void *src, void *dst, const int *idx, int B, int n_src, int n_dst, int ld, int dtype,
+                      void *stream);
+/* tok[b,0,:] = cls + pos[0];  tok[b,1+j,:] = e[b*n_vis+j,:] + pos[1 + vis_idx[b*n_vis+j]]; tok is [B*(n_vis+1), d].
+ * Dropout (element index = position in tok) and dtype as ecgvit_embed_assemble. */
+int ecgvit_embed_assemble_visible(const void *e, const float *cls, const float *pos, const int *vis_idx, void *tok,
+                                  int B, int n_vis, int d, float dropout_p, int dropout_stream,
+                                  const uint32_t *dropout_seed, int dtype, void *stream);
+/* backward of the above (g = dropout mask applied to dtok): de = g[:,1:,:]; dcls += sum_b g[:,0]; dpos[0] += the same;
+ * dpos[1+p] += sum over the records where patch p is visible of g[b, 1+slot[b,p]]; dbias += sum_{b,j} g[:,1:].
+ * scratch: fp32 [n_patch, d].  Every sum runs in a fixed record order without float atomics: bit-identical from launch
+ * to launch.  Three kernels: the position sums, then a two-pass fixed-order fold of them. */
+int ecgvit_embed_assemble_visible_bwd(const void *dtok, const int *slot, void *de, float *dcls, float *dpos,
+                                      float *dbias, float *scratch, int B, int n_patch, int n_vis, int d,
+                                      float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int dtype,
+                                      void *stream);
+/* decoder input u [B*(n_patch+1), d] from the embedded encoder output t [B*(n_vis+1), d]:
+ * u[b,0] = t[b,0] + pos[0];  u[b,1+p] = (slot[b,p] >= 0 ? t[b, 1+slot[b,p]] : mask_token) + pos[1+p].
+ * dtype ECGVIT_BF16_RES32: t bf16, u fp32. */
+int ecgvit_mae_unshuffle(const void *t, const float *mask_token, const float *pos, const int *slot, void *u, int B,
+                         int n_patch, int n_vis, int d, int dtype, void *stream);
+/* its backward: dt (fully written) = the rows of du that t fed; dpos += sum_b du; dmask_token += sum of the masked rows.
+ * scratch: fp32 [n_patch, d].  Fixed record order, no float atomics; three kernels, as the visible-assemble backward. */
+int ecgvit_mae_unshuffle_bwd(const void *du, const int *slot, void *dt, float *dpos, float *dmask_token,
+                             float *scratch, int B, int n_patch, int n_vis, int d, int dtype, void *stream);
+
 /* ---- nn.LayerNorm(d, eps) forward (PreNorm.norm / mlp_head[0]); saves per-row mean and rstd (fp32) */
 int ecgvit_layernorm_fwd(const void *x, const float *gamma, const float *beta, void *y, float *mean,
                          float *rstd, int M, int d, float eps, int dtype, void *stream);
