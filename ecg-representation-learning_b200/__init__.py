@@ -9,12 +9,12 @@ from .config import EcgVitConfig
 from .model import EcgVit, ModelOutput, Recorder, EcgVitForMaskedPatchModeling, MaskedPatchOutput, \
     EcgVitForMaskedAutoencoding
 from .trainer import FusedTrainer, fused_train_step, get_train_args, lr_multiplier
-from .optim import FusedAdamW, clip_grad_norm_
+from .optim import FusedAdamW, clip_grad_norm_, param_groups_lrd
 from .transform import InputPipeline
 from .metrics import get_accuracy, evaluate
 from .synthetic import synthetic_batch
 from . import _lib
 
 __all__ = ['EcgVitConfig', 'EcgVit', 'ModelOutput', 'EcgVitForMaskedPatchModeling', 'EcgVitForMaskedAutoencoding',
-           'MaskedPatchOutput', 'FusedTrainer', 'fused_train_step', 'FusedAdamW', 'clip_grad_norm_',
+           'MaskedPatchOutput', 'FusedTrainer', 'fused_train_step', 'FusedAdamW', 'clip_grad_norm_', 'param_groups_lrd',
            'get_train_args', 'lr_multiplier', 'InputPipeline', 'Recorder', 'get_accuracy', 'evaluate', 'synthetic_batch']

@@ -87,12 +87,16 @@ SIGNATURES = {
                                                                      c_void_p],
     'ecgvit_head_bwd': [c_void_p] * 5 + [c_int] + [c_void_p] * 11 + [c_int, c_int, c_int, c_int, c_int, c_float, c_void_p,
                                                                       c_int, c_void_p],
+    'ecgvit_token_mean': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
+    'ecgvit_token_mean_bwd': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
     'ecgvit_colsum': [c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_void_p],
     'ecgvit_grad_sumsq': [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p],
     'ecgvit_grad_sumsq_partial': [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p],
     'ecgvit_grad_sumsq_finalize': [c_void_p, c_int, c_void_p],
     'ecgvit_adamw_step': [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int,
                           c_void_p],
+    'ecgvit_adamw_step_grouped': [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_void_p,
+                                  c_void_p, c_void_p, c_int, c_void_p],
     'ecgvit_grad_scale_by_clip': [c_void_p, c_int64, c_void_p, c_void_p, c_void_p],
     'ecgvit_cast_f32_to_bf16': [c_void_p, c_void_p, c_int64, c_void_p],
 }

@@ -25,7 +25,7 @@ class EcgVitConfig(PretrainedConfig):
                  intermediate_size: int = 2048, hidden_dropout_prob: float = 0.1,
                  attention_probs_dropout_prob: float = 0.1, num_class: int = 71,
                  compute_dtype: str = 'bf16', per_lead_tokens: bool = False, residual_dtype: str = 'auto',
-                 activation_checkpointing: bool = False, **kwargs):
+                 activation_checkpointing: bool = False, pool: str = 'cls', **kwargs):
         self.max_signal_length = max_signal_length
         self.patch_size = patch_size
         self.num_channels = num_channels
@@ -51,6 +51,12 @@ class EcgVitConfig(PretrainedConfig):
         # Costs one extra block forward per layer (minus the last Linear); 'large' at 512 records per GPU fits 180 GB
         # without it (33.5 GB), so it is off by default
         self.activation_checkpointing = activation_checkpointing
+        # classification pooling, vit_pytorch's `pool`: 'cls' = the CLS token's output (the reference's), 'mean' = the
+        # mean over all tokens, CLS included (the usual head for fine-tuning MAE-style encoders).  The pre-training
+        # models ignore it: their heads read every patch token
+        if pool not in ('cls', 'mean'):
+            raise ValueError(f"pool must be 'cls' or 'mean', got {pool!r}")
+        self.pool = pool
         super().__init__(**kwargs)
         self.size = None
 

@@ -348,6 +348,62 @@ __global__ void __launch_bounds__(256) head_bwd_weight_kernel(const float *__res
     }
 }
 
+// Mean pool (vit_pytorch pool='mean'): out[b, k] = sum_t tok[b, t, k] / N over all N tokens, CLS included.
+// One CTA = one record x 256 columns; thread (tx, ty) sums 8 columns over the rows t = ty, ty + 8, ... in order, and the
+// 8 row groups are folded in order: a fixed summation order, no atomics, so the result is bit-identical run to run.
+constexpr int MEAN_ROWG = 8;
+template <typename T>
+__global__ void __launch_bounds__(32 * MEAN_ROWG) token_mean_kernel(const T *__restrict__ tok, float *__restrict__ out,
+                                                                     int N, int d) {
+    __shared__ float red[MEAN_ROWG][256 + 8];
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    const int b = blockIdx.y;
+    const int c = blockIdx.x * 256 + tx * 8;
+    float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    if (c < d) {
+        const T *xr = tok + (int64_t)b * N * d + c;
+        for (int t = ty; t < N; t += MEAN_ROWG) {
+            float v[8];
+            load8(xr + (int64_t)t * d, v);
+#pragma unroll
+            for (int k = 0; k < 8; ++k) s[k] += v[k];
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) red[ty][tx * 8 + k] = s[k];
+    __syncthreads();
+    if (ty == 0 && c < d) {
+        float o[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+            float a = red[0][tx * 8 + k];
+#pragma unroll
+            for (int y = 1; y < MEAN_ROWG; ++y) a += red[y][tx * 8 + k];
+            o[k] = a / (float)N;
+        }
+        store8(out + (int64_t)b * d + c, o);
+    }
+}
+
+// its backward: dtok[b, t, :] = dpool[b, :] / N for every token t
+template <typename T>
+__global__ void __launch_bounds__(256) token_mean_bwd_kernel(const float *__restrict__ dpool, T *__restrict__ dtok,
+                                                              int B, int N, int d) {
+    const int dv = d / 8;
+    const int64_t total = (int64_t)B * N * dv;
+    const float inv = 1.0f / (float)N;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int c = (int)(i % dv) * 8;
+        const int64_t row = i / dv;
+        const int b = (int)(row / N);
+        float v[8];
+        load8(dpool + (int64_t)b * d + c, v);
+#pragma unroll
+        for (int k = 0; k < 8; ++k) v[k] *= inv;
+        store8(dtok + row * d + c, v);
+    }
+}
+
 }  // namespace
 }  // namespace ecgvit
 
@@ -426,6 +482,31 @@ int ecgvit_head_bwd(const void *tok, const float *gamma, const float *w, const f
     dim3 gw((d + 31) / 32, n_class);
     head_bwd_weight_kernel<<<gw, 256, 0, s>>>(dlog, xn, dw, db, B, d, n_class);
     return check_launch("head_bwd");
+}
+
+int ecgvit_token_mean(const void *tok, float *out, int B, int N, int d, int dtype, void *stream) {
+    ECGVIT_REQUIRE(tok && out && B > 0 && N > 0 && d > 0, "token_mean: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "token_mean: d=%d must be a multiple of 8", d);
+    const dim3 grid((d + 255) / 256, B);
+    if (dtype == ECGVIT_BF16)
+        token_mean_kernel<bf16><<<grid, 32 * MEAN_ROWG, 0, as_stream(stream)>>>((const bf16 *)tok, out, N, d);
+    else if (dtype == ECGVIT_F32 || dtype == ECGVIT_BF16_RES32)   // fp32 tokens (parity mode / fp32 residual stream)
+        token_mean_kernel<float><<<grid, 32 * MEAN_ROWG, 0, as_stream(stream)>>>((const float *)tok, out, N, d);
+    else return fail(-1, "token_mean: unknown dtype %d", dtype);
+    return check_launch("token_mean");
+}
+
+int ecgvit_token_mean_bwd(const float *dpool, void *dtok, int B, int N, int d, int dtype, void *stream) {
+    ECGVIT_REQUIRE(dpool && dtok && B > 0 && N > 0 && d > 0, "token_mean_bwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0, "token_mean_bwd: d=%d must be a multiple of 8", d);
+    const int64_t vecs = (int64_t)B * N * (d / 8);
+    const int grid = (int)std::min<int64_t>((vecs + 255) / 256, (int64_t)sm_count() * 8);
+    if (dtype == ECGVIT_BF16 || dtype == ECGVIT_BF16_RES32)   // the token-shaped gradient is bf16 in both bf16 modes
+        token_mean_bwd_kernel<bf16><<<grid, 256, 0, as_stream(stream)>>>(dpool, (bf16 *)dtok, B, N, d);
+    else if (dtype == ECGVIT_F32)
+        token_mean_bwd_kernel<float><<<grid, 256, 0, as_stream(stream)>>>(dpool, (float *)dtok, B, N, d);
+    else return fail(-1, "token_mean_bwd: unknown dtype %d", dtype);
+    return check_launch("token_mean_bwd");
 }
 
 }  // extern "C"

@@ -78,12 +78,19 @@ __device__ __forceinline__ float clip_coef_from(const float *hyper, const float 
     return fminf(max_norm / (total_norm + 1e-6f), 1.0f);
 }
 
-template <bool kShadow, typename TG>
+// kGrouped: per-parameter-group learning rate / weight decay.  gmap holds one group id per 64-element block of the
+// flat buffers (every tensor starts on a 64-element boundary); gtable[2 * id] = 1 - lr_g * wd_g and
+// gtable[2 * id + 1] = lr_g / (1 - beta1^t) replace hyper's decay / step size; id ADAMW_UNGROUPED leaves p, m, v and
+// the shadow untouched.  Everything else (clip, skip, the non-finite counter, the update itself) is shared.
+constexpr uint8_t ADAMW_UNGROUPED = 255;
+
+template <bool kShadow, typename TG, bool kGrouped = false>
 __global__ void __launch_bounds__(256) adamw_kernel(float *__restrict__ p, float *__restrict__ m,
                                                      float *__restrict__ v, const TG *__restrict__ g,
                                                      bf16 *__restrict__ shadow, int64_t n,
                                                      const float *__restrict__ hyper, float *__restrict__ stats,
-                                                     bool count_skips) {
+                                                     bool count_skips, const uint8_t *__restrict__ gmap = nullptr,
+                                                     const float *__restrict__ gtable = nullptr) {
     if (hyper[H_SKIP] != 0.f) return;   // a deferred-update slot with nothing pending (first step, or just flushed)
     float total_norm;
     const float clip = clip_coef_from(hyper, stats, total_norm);
@@ -98,10 +105,17 @@ __global__ void __launch_bounds__(256) adamw_kernel(float *__restrict__ p, float
     // (1 - beta in fp32 differs from fp32(1 - beta) by 1.3e-5 relative for beta2 = 0.999)
     const float beta2 = hyper[H_BETA2], eps = hyper[H_EPS];
     const float one_m_b1 = hyper[H_ONE_MINUS_B1], one_m_b2 = hyper[H_ONE_MINUS_B2];
-    const float decay = hyper[H_DECAY], step_size = hyper[H_STEP_SIZE], bc2_sqrt = hyper[H_BC2_SQRT];
+    float decay = hyper[H_DECAY], step_size = hyper[H_STEP_SIZE];
+    const float bc2_sqrt = hyper[H_BC2_SQRT];
     const float gmul = hyper[H_GSCALE] * clip;
     const int64_t n4 = n / 4;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+        if (kGrouped) {
+            const uint8_t id = __ldg(gmap + (i >> 4));   // 16 float4 = one 64-element block
+            if (id == ADAMW_UNGROUPED) continue;
+            decay = __ldg(gtable + 2 * id);
+            step_size = __ldg(gtable + 2 * id + 1);
+        }
         const float4 g4 = load_grad4(g, i);
         float4 p4 = reinterpret_cast<float4 *>(p)[i], m4 = reinterpret_cast<float4 *>(m)[i],
                v4 = reinterpret_cast<float4 *>(v)[i];
@@ -219,6 +233,35 @@ int ecgvit_adamw_step(float *p, float *m, float *v, const void *g, int grad_dtyp
         else adamw_kernel<false, bf16><<<grid, 256, 0, s>>>(p, m, v, (const bf16 *)g, nullptr, n, hyper, stats, count);
     }
     return check_launch("adamw_step");
+}
+
+int ecgvit_adamw_step_grouped(float *p, float *m, float *v, const void *g, int grad_dtype, void *shadow_bf16, int64_t n,
+                              const uint8_t *group_map, const float *group_table, const float *hyper, float *stats,
+                              int flags, void *stream) {
+    ECGVIT_REQUIRE(p && m && v && g && group_map && group_table && hyper && stats && n > 0,
+                   "adamw_step_grouped: bad arguments");
+    ECGVIT_REQUIRE(n % 64 == 0, "adamw_step_grouped: length %lld must be a multiple of 64 (one group id per 64 elements)",
+                   (long long)n);
+    ECGVIT_REQUIRE(((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v) |
+                     reinterpret_cast<uintptr_t>(g)) & 15) == 0,
+                   "adamw_step_grouped: buffers must be 16-byte aligned");
+    ECGVIT_REQUIRE(grad_dtype == ECGVIT_F32 || grad_dtype == ECGVIT_BF16, "adamw_step_grouped: unknown gradient dtype %d",
+                   grad_dtype);
+    cudaStream_t s = as_stream(stream);
+    const bool slice = (flags & ECGVIT_ADAMW_SLICE) != 0;
+    const bool count = !slice || (flags & ECGVIT_ADAMW_FIRST_SLICE) != 0;
+    const int grid = slice ? (int)((n / 4 + 255) / 256) : flat_grid(n);
+    bf16 *sh = (bf16 *)shadow_bf16;
+    const uint8_t *gm = group_map;
+    const float *gt = group_table;
+    if (grad_dtype == ECGVIT_F32) {
+        if (sh) adamw_kernel<true, float, true><<<grid, 256, 0, s>>>(p, m, v, (const float *)g, sh, n, hyper, stats, count, gm, gt);
+        else adamw_kernel<false, float, true><<<grid, 256, 0, s>>>(p, m, v, (const float *)g, nullptr, n, hyper, stats, count, gm, gt);
+    } else {
+        if (sh) adamw_kernel<true, bf16, true><<<grid, 256, 0, s>>>(p, m, v, (const bf16 *)g, sh, n, hyper, stats, count, gm, gt);
+        else adamw_kernel<false, bf16, true><<<grid, 256, 0, s>>>(p, m, v, (const bf16 *)g, nullptr, n, hyper, stats, count, gm, gt);
+    }
+    return check_launch("adamw_step_grouped");
 }
 
 int ecgvit_grad_scale_by_clip(float *g, int64_t n, const float *hyper, float *stats, void *stream) {

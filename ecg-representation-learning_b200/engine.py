@@ -148,6 +148,9 @@ class StepEngine:
         w.loss_none = buf(B, n_class, dtype=torch.float32)
         w.head_scratch = buf(B * d + B * n_class, dtype=torch.float32)
         w.labels = buf(B, n_class, dtype=torch.float32)
+        # pool='mean': the pooled rows and their gradient, fp32 [B, d] (the head kernels read them as N = 1 tokens)
+        w.pooled = buf(B, d, dtype=torch.float32) if m._mean_pool else None
+        w.dpool = buf(B, d, dtype=torch.float32) if m._mean_pool else None
         w.de = buf(B * nv, d)
         self.ws[key] = w
         return w
@@ -282,12 +285,17 @@ class StepEngine:
                                              seed_ptr if w.p_emb > 0 else None, m._res_code, st), 'embed_assemble')
 
     def _head_forward(self, w, labels, reduction):
-        """CLS pool + mlp_head + BCE: (loss | None, logits)"""
+        """CLS (or mean) pool + mlp_head + BCE: (loss | None, logits)"""
         m, lib, st = self.model, self.lib, self._stream
         c = m.config
         rdt = m._res_code
         pf = m._params_f32()
         B, N, d = w.B, w.N, c.hidden_size
+        tok = w.x[c.num_hidden_layers]
+        if m._mean_pool:
+            # pool='mean': fp32 token means, then the CLS head over them as one fp32 token per record
+            _lib.check(lib.ecgvit_token_mean(tok.data_ptr(), w.pooled.data_ptr(), B, N, d, rdt, st), 'token_mean')
+            tok, N, rdt = w.pooled, 1, F32
         red = _lib.REDUCTION[reduction]
         loss_buf = None
         if labels is not None:
@@ -295,7 +303,7 @@ class StepEngine:
             w.labels.copy_(labels, non_blocking=True)  # also casts (the reference passes float multi-hot)
             loss_buf = w.loss_none if reduction == 'none' else w.loss
         _lib.check(lib.ecgvit_head_fwd(
-            w.x[c.num_hidden_layers].data_ptr(), pf['head.ln.w'].data_ptr(), pf['head.ln.b'].data_ptr(),
+            tok.data_ptr(), pf['head.ln.w'].data_ptr(), pf['head.ln.b'].data_ptr(),
             pf['head.w'].data_ptr(), pf['head.b'].data_ptr(), w.labels.data_ptr() if labels is not None else None,
             *self._loss_weight_table(), w.xn.data_ptr(), w.hstat[0].data_ptr(), w.hstat[1].data_ptr(), w.logits.data_ptr(),
             _lib.ptr(loss_buf), B, N, d, m.num_class, red, LN_EPS, rdt, st), 'head_fwd')
@@ -554,13 +562,21 @@ class StepEngine:
         m, lib, st = self.model, self.lib, self._stream
         c = m.config
         pf, gr = m._params_f32(), m._grads_f32()
+        tok, dhead, N, rdt = w.x[c.num_hidden_layers], dtok, w.N, m._res_code
+        if m._mean_pool:
+            # the head's backward over the pooled rows writes the fp32 pooled gradient, and its dcolsum
+            # sum_b dpool[b] is already the column sum of the broadcast gradient below
+            tok, dhead, N, rdt = w.pooled, w.dpool, 1, F32
         _lib.check(lib.ecgvit_head_bwd(
-            w.x[c.num_hidden_layers].data_ptr(), pf['head.ln.w'].data_ptr(), pf['head.w'].data_ptr(), w.labels.data_ptr(),
+            tok.data_ptr(), pf['head.ln.w'].data_ptr(), pf['head.w'].data_ptr(), w.labels.data_ptr(),
             *self._loss_weight_table(), w.xn.data_ptr(), w.hstat[0].data_ptr(), w.hstat[1].data_ptr(), w.logits.data_ptr(),
-            dtok.data_ptr(),
+            dhead.data_ptr(),
             gr['head.w'].data_ptr(), gr['head.b'].data_ptr(), gr['head.ln.w'].data_ptr(), gr['head.ln.b'].data_ptr(),
-            _lib.ptr(dcolsum), w.head_scratch.data_ptr(), w.B, w.N, c.hidden_size, m.num_class,
-            _lib.REDUCTION[w.reduction], float(grad_scale), _lib.ptr(grad_scale_dev), m._res_code, st), 'head_bwd')
+            _lib.ptr(dcolsum), w.head_scratch.data_ptr(), w.B, N, c.hidden_size, m.num_class,
+            _lib.REDUCTION[w.reduction], float(grad_scale), _lib.ptr(grad_scale_dev), rdt, st), 'head_bwd')
+        if m._mean_pool:
+            _lib.check(lib.ecgvit_token_mean_bwd(w.dpool.data_ptr(), dtok.data_ptr(), w.B, w.N, c.hidden_size,
+                                                 m._dtype_code, st), 'token_mean_bwd')
 
     def _assemble_backward(self, w, dz):
         """backward of `_assemble`: de, and the cls / pos / embedding-bias gradients"""

@@ -85,7 +85,7 @@ class ViT(nn.Module):
     (produced last, by the embedding backward) sits with the other pre-block parameters in the last gradient bucket."""
 
     def __init__(self, *, signal_length, patch_size, num_classes, dim, depth, heads, mlp_dim, channels, dim_head,
-                 dropout, emb_dropout, per_lead=False, head=True, mask_token=False):
+                 dropout, emb_dropout, per_lead=False, head=True, mask_token=False, pool='cls'):
         super().__init__()
         assert signal_length % patch_size == 0, 'Image dimensions must be divisible by the patch size.'
         n_patch = signal_length // patch_size * (channels if per_lead else 1)
@@ -98,7 +98,7 @@ class ViT(nn.Module):
             self.mask_token = nn.Parameter(torch.zeros(1, 1, dim))
         self.dropout = _Slot(f'Dropout(p={emb_dropout})')
         self.transformer = Transformer(dim, depth, heads, dim_head, mlp_dim, dropout)
-        self.pool = 'cls'
+        self.pool = pool
         self.to_latent = nn.Identity()
         if head:
             self.mlp_head = nn.Sequential(nn.LayerNorm(dim), nn.Linear(dim, num_classes))
@@ -164,6 +164,11 @@ class EcgVit(nn.Module):
         config = config if config is not None else EcgVitConfig()
         hd_sz, n_head = config.hidden_size, config.num_attention_heads
         assert hd_sz % n_head == 0  # ecg_vit.py:99
+        pool = getattr(config, 'pool', 'cls')
+        if pool not in ('cls', 'mean'):
+            raise ValueError(f"pool must be 'cls' or 'mean', got {pool!r}")
+        # only the classification head pools; the pre-training heads read every patch token and ignore `pool`
+        self._mean_pool = pool == 'mean' and self._classification_head
         self.config = config
         self.num_class = num_class  # the reference builds the head from the ctor arg, not config.num_class (:105)
         self.vit = ViT(signal_length=config.max_signal_length, patch_size=config.patch_size, num_classes=num_class,
@@ -172,7 +177,8 @@ class EcgVit(nn.Module):
                        dropout=config.hidden_dropout_prob,              # attention + feed-forward (ecg_vit.py:113)
                        emb_dropout=config.attention_probs_dropout_prob,  # embedding (ecg_vit.py:114)
                        per_lead=bool(getattr(config, 'per_lead_tokens', False)),
-                       head=self._classification_head, mask_token=self._encoder_mask_token)
+                       head=self._classification_head, mask_token=self._encoder_mask_token,
+                       pool='mean' if self._mean_pool else 'cls')
         self.vit._owner = weakref.ref(self)  # lets `Recorder(model.vit)` reach the kernels (not a module: no cycle)
         self._loss_reduction = loss_reduction
         self.loss_weight = None
@@ -288,15 +294,20 @@ class EcgVit(nn.Module):
             out[name] = k
         return out
 
-    def _flatten(self, device):
-        names = self._short_names()
+    def _flat_layout(self):
+        """(layout, total): flat-buffer key -> (offset, numel, shape, parameter name), every offset a multiple of
+        _ALIGN elements, in `named_parameters()` order"""
         params = dict(self.named_parameters())
         layout, off = OrderedDict(), 0
-        for name, key in names.items():
+        for name, key in self._short_names().items():
             n = params[name].numel()
             layout[key] = (off, n, tuple(params[name].shape), name)
             off += (n + _ALIGN - 1) // _ALIGN * _ALIGN
-        total = off
+        return layout, off
+
+    def _flatten(self, device):
+        params = dict(self.named_parameters())
+        layout, total = self._flat_layout()
         flat = torch.zeros(total, device=device, dtype=torch.float32)
         for key, (o, n, shape, name) in layout.items():
             flat[o:o + n].copy_(params[name].detach().reshape(-1))
@@ -406,7 +417,8 @@ class EcgVitForMaskedPatchModeling(EcgVit):
     batch always gets the same mask).
 
     `encoder_state_dict()` hands the encoder over to fine-tuning:
-    `EcgVit(config=...).load_state_dict(pre.encoder_state_dict(), strict=False)` misses only `vit.mlp_head.*`."""
+    `EcgVit(config=...).load_state_dict(pre.encoder_state_dict(), strict=False)` misses only `vit.mlp_head.*`.
+    `config.pool` is ignored here (the head reads every patch token); it applies to the `EcgVit` that is fine-tuned."""
     _classification_head = False
     _encoder_mask_token = True
     _engine_class = MaskedPatchEngine

@@ -16,6 +16,90 @@ from . import _lib
 
 
 
+UNGROUPED = 255   # group id of the parameters in no group: the grouped AdamW leaves them untouched
+MAX_GROUPS = 255
+NO_WEIGHT_DECAY = ('vit.pos_embedding', 'vit.cls_token', 'vit.mask_token', 'decoder.mask_token')
+
+
+def _layer_id(name, depth):
+    """MAE's `get_layer_id_for_vit` over this model's names: 0 = embedding, CLS, positions and mask token, i + 1 = encoder
+    block i, depth + 1 = everything else (the classification head, or the pre-training decoder and head)"""
+    if name.startswith('vit.to_patch_embedding.') or name in ('vit.pos_embedding', 'vit.cls_token', 'vit.mask_token'):
+        return 0
+    if name.startswith('vit.transformer.layers.'):
+        return int(name.split('.')[3]) + 1
+    return depth + 1
+
+
+def param_groups_lrd(model, weight_decay=0.05, layer_decay=0.75, no_weight_decay=NO_WEIGHT_DECAY):
+    """Parameter groups for fine-tuning with layer-wise learning-rate decay (MAE's `param_groups_lrd`): encoder block i
+    gets lr * layer_decay^(depth - i), the embedding layer_decay^(depth + 1), the head the full lr; 1-D tensors (biases,
+    LayerNorms) and the `no_weight_decay` parameter names get no weight decay.  Returns one
+    `{'params', 'lr_scale', 'weight_decay'}` dict per (layer, decay or not), in order of first appearance, for
+    `FusedAdamW(..., param_groups=...)`, `FusedTrainer(..., param_groups=...)` or `torch.optim.AdamW`.
+    layer_decay=1.0 gives the plain decay / no-decay split."""
+    depth = model.config.num_hidden_layers
+    no_wd = set(no_weight_decay)
+    groups = {}
+    for name, p in model.named_parameters():
+        if not p.requires_grad:
+            continue
+        decay = not (p.ndim == 1 or name in no_wd)
+        lid = _layer_id(name, depth)
+        g = groups.get((lid, decay))
+        if g is None:
+            g = groups[(lid, decay)] = {'params': [], 'lr_scale': float(layer_decay) ** (depth + 1 - lid),
+                                        'weight_decay': float(weight_decay) if decay else 0.0}
+        g['params'].append(p)
+    return list(groups.values())
+
+
+def group_names(model, param_groups):
+    """the parameter names of every group (`model.named_parameters()` names); raises on a tensor that is not one of the
+    model's parameters or that sits in two groups"""
+    names = {id(p): n for n, p in model.named_parameters()}
+    seen, out = set(), []
+    for g in param_groups:
+        ps = g['params']
+        ps = [ps] if isinstance(ps, torch.Tensor) else list(ps)
+        row = []
+        for p in ps:
+            if id(p) not in names:
+                raise ValueError('a parameter group holds a tensor that is not a parameter of the model')
+            if id(p) in seen:
+                raise ValueError('some parameters appear in more than one parameter group')
+            seen.add(id(p))
+            row.append(names[id(p)])
+        out.append(tuple(row))
+    if len(out) > MAX_GROUPS:
+        raise ValueError(f'at most {MAX_GROUPS} parameter groups, got {len(out)}')
+    return out
+
+
+def group_map(model, names_per_group):
+    """uint8 [flat length / 64] (host): the group id of every 64-element block of the model's flat buffers, UNGROUPED
+    for parameters in no group (every tensor starts on a 64-element boundary, so a block never straddles two)"""
+    from .model import _ALIGN
+    layout, total = (model._layout, model._flat_p.numel()) if model._layout is not None else model._flat_layout()
+    where = {name: (o, n) for o, n, _, name in layout.values()}
+    gm = torch.full((total // _ALIGN,), UNGROUPED, dtype=torch.uint8)
+    for gid, names in enumerate(names_per_group):
+        for name in names:
+            o, n = where[name]
+            gm[o // _ALIGN:(o + n + _ALIGN - 1) // _ALIGN] = gid
+    return gm
+
+
+def group_table(lrs, weight_decays, beta1, step):
+    """the grouped AdamW's per-group scalars [1 - lr * wd, lr / (1 - beta1^t)] in double precision, as
+    `adamw_hyper` derives hyper's own"""
+    bc1 = 1.0 - beta1 ** step
+    out = []
+    for lr, wd in zip(lrs, weight_decays):
+        out += [1.0 - lr * wd, lr / bc1]
+    return out
+
+
 def _flat_grads(model):
     """make `model._flat_g` hold the current `.grad` of every parameter and return it"""
     views = model._grad_views()
@@ -73,17 +157,41 @@ def clip_grad_norm_(model, max_norm, norm_type=2.0, error_if_nonfinite=False):
 
 
 class FusedAdamW(torch.optim.Optimizer):
-    """AdamW over the model's flat parameter buffer; one group, decay on everything (train.py:242-244).
+    """AdamW over the model's flat parameter buffer; by default one group, decay on everything (train.py:242-244).
+
+    `param_groups` (e.g. from `param_groups_lrd`): a list of `{'params', 'lr_scale', 'weight_decay', ...}` dicts.  A
+    group's `lr` defaults to `lr * lr_scale`, so `LambdaLR` and transformers' schedulers scale every group as they do
+    for `torch.optim.AdamW`; `step()` reads every group's current `lr` and `weight_decay`.  Parameters in no group are
+    not updated.  All groups share the constructor's betas and eps (a group with others raises `ValueError`).
 
     `state_dict()` / `load_state_dict()` carry the moments and the step count (as flat tensors under `state['flat']`),
     so the usual `torch.save(optimizer.state_dict())` checkpoint resumes exactly.  Parameters whose `.grad` is None are
     left untouched (value and moments), as torch.optim.AdamW leaves them."""
 
-    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
+    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, param_groups=None):
         self.model = model
-        super().__init__(model.parameters(), dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+        self._grouped = param_groups is not None
+        params = model.parameters()
+        if self._grouped:
+            params = []
+            for g in param_groups:
+                g = dict(g)
+                g.setdefault('lr', lr * float(g.get('lr_scale', 1.0)))
+                params.append(g)
+        super().__init__(params, dict(lr=lr, betas=betas, eps=eps, weight_decay=weight_decay))
+        if self._grouped:
+            self._check_groups()
         self._step = 0
         self._m = self._v = None
+        self._gmap = self._gmap_key = None
+        self._ghyper = self._gring = None
+
+    def _check_groups(self):
+        b, e = tuple(self.defaults['betas']), self.defaults['eps']
+        for g in self.param_groups:
+            if tuple(g['betas']) != b or g['eps'] != e:
+                raise ValueError(f'FusedAdamW: every parameter group shares betas {b} and eps {e}; a group has '
+                                 f'betas {tuple(g["betas"])}, eps {g["eps"]}')
 
     def _ensure_moments(self, g):
         n = g.numel()
@@ -112,13 +220,17 @@ class FusedAdamW(torch.optim.Optimizer):
         self._step += 1
         hyper, stats = _scratch(model)
         b1, b2 = grp['betas']
-        # max_norm 0: clipping is a separate call in the reference loop
-        _upload(model, hyper, _lib.adamw_hyper(grp['lr'], b1, b2, grp['eps'], grp['weight_decay'], self._step, 0.0, 1.0))
-        stats.zero_()
         st = torch.cuda.current_stream().cuda_stream
-        _lib.check(_lib.load().ecgvit_adamw_step(model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(),
-                                                 g.data_ptr(), _lib.F32, _lib.ptr(model._shadow), n, hyper.data_ptr(),
-                                                 stats.data_ptr(), 0, st), 'adamw_step')
+        if self._grouped:
+            self._grouped_step(g, stats, st)
+        else:
+            # max_norm 0: clipping is a separate call in the reference loop
+            _upload(model, hyper, _lib.adamw_hyper(grp['lr'], b1, b2, grp['eps'], grp['weight_decay'], self._step, 0.0,
+                                                   1.0))
+            stats.zero_()
+            _lib.check(_lib.load().ecgvit_adamw_step(model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(),
+                                                     g.data_ptr(), _lib.F32, _lib.ptr(model._shadow), n,
+                                                     hyper.data_ptr(), stats.data_ptr(), 0, st), 'adamw_step')
         for o, cnt, p0, m0, v0 in keep:
             model._flat_p[o:o + cnt].copy_(p0)
             self._m[o:o + cnt].copy_(m0)
@@ -126,6 +238,30 @@ class FusedAdamW(torch.optim.Optimizer):
         if keep:
             model.sync_shadow(force=True)
         return loss
+
+    def _grouped_step(self, g, stats, st):
+        """ecgvit_adamw_step_grouped with every group's current lr / weight decay; the group map is rebuilt when the
+        membership or the flat layout changes"""
+        model = self.model
+        self._check_groups()
+        names = group_names(model, self.param_groups)
+        key = (tuple(names), model._flat_p.data_ptr())
+        if self._gmap_key != key:
+            self._gmap = group_map(model, names).to(model._flat_p.device)
+            self._gmap_key = key
+        b1, b2 = self.defaults['betas']
+        vals = _lib.adamw_hyper(0.0, b1, b2, self.defaults['eps'], 0.0, self._step, 0.0, 1.0)
+        vals += group_table([grp['lr'] for grp in self.param_groups], [grp['weight_decay'] for grp in self.param_groups],
+                            b1, self._step)
+        if self._ghyper is None or self._ghyper.numel() != len(vals) or self._ghyper.device != g.device:
+            self._ghyper = torch.zeros(len(vals), device=g.device)
+            self._gring = _lib.PinnedRing(len(vals), torch.float32)
+        self._gring.upload(self._ghyper, vals)   # hyper block, then the group table right behind it
+        stats.zero_()
+        _lib.check(_lib.load().ecgvit_adamw_step_grouped(
+            model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(), g.data_ptr(), _lib.F32,
+            _lib.ptr(model._shadow), g.numel(), self._gmap.data_ptr(), self._ghyper.data_ptr() + 64,
+            self._ghyper.data_ptr(), stats.data_ptr(), 0, st), 'adamw_step_grouped')
 
     # ---- checkpointing: torch.optim.Optimizer.state is empty here (the moments are flat), so carry them explicitly ----
     def state_dict(self):

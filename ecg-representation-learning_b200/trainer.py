@@ -50,7 +50,7 @@ class FusedTrainer:
     def __init__(self, model, learning_rate=3e-4, weight_decay=1e-2, betas=(0.9, 0.999), eps=1e-8,
                  schedule='constant', n_warmup=0, n_step=1 << 30, max_grad_norm=1.0, process_group=None,
                  bucket_layers=1, use_cuda_graph=False, data_parallel=True, grad_reduce_dtype='auto',
-                 defer_optimizer=False):
+                 defer_optimizer=False, param_groups=None):
         self.model = model
         self._flat_ptr = None
         self.lr, self.wd, self.betas, self.eps = learning_rate, weight_decay, betas, eps
@@ -84,6 +84,20 @@ class FusedTrainer:
         self._reducer = None
         self.launches_per_step = None
         self._step_done = collections.deque(maxlen=2)
+        # param_groups (e.g. `param_groups_lrd(model)`): per group lr = learning_rate * schedule * lr_scale and its own
+        # weight decay (the trainer's when the group has none); parameters in no group are not updated.  Without groups
+        # the step issues exactly the ungrouped kernels
+        self.param_groups = None
+        if param_groups is not None:
+            from .optim import group_names
+            self._group_names = group_names(model, param_groups)
+            self.param_groups = []
+            for g in param_groups:
+                if tuple(g.get('betas', betas)) != tuple(betas) or g.get('eps', eps) != eps:
+                    raise ValueError(f'FusedTrainer: every parameter group shares betas {tuple(betas)} and eps {eps}')
+                wd = g.get('weight_decay')
+                self.param_groups.append({'lr_scale': float(g.get('lr_scale', 1.0)),
+                                          'weight_decay': None if wd is None else float(wd)})
 
     # ---- lazily created device state ---------------------------------------------------------------
     def _ensure_state(self, device):
@@ -101,7 +115,13 @@ class FusedTrainer:
         if old is not None:
             self.exp_avg.copy_(old[0])
             self.exp_avg_sq.copy_(old[1])
-        self.hyper = torch.zeros(16, device=device, dtype=torch.float32)
+        # with groups, the group table sits right behind the 16-float hyper block: one upload per step feeds both
+        n_hyper = 16 + (2 * len(self.param_groups) if self.param_groups is not None else 0)
+        self.hyper = torch.zeros(n_hyper, device=device, dtype=torch.float32)
+        self._gmap = None
+        if self.param_groups is not None:
+            from .optim import group_map
+            self._gmap = group_map(m, self._group_names).to(device)   # once per flat layout
         self.stats = torch.zeros(_lib.STATS_FLOATS, device=device, dtype=torch.float32)
         self._flat_ptr = m._flat_p.data_ptr()
         self._graph = None   # a captured graph points at the old flat buffers
@@ -147,9 +167,29 @@ class FusedTrainer:
         b1, b2 = self.betas
         mg = self.max_grad_norm if self.max_grad_norm is not None else 0.0
         if t is None:
-            return _lib.adamw_hyper(0.0, b1, b2, self.eps, self.wd, 1, mg, 1.0 / self.world, skip=True)
+            vals = _lib.adamw_hyper(0.0, b1, b2, self.eps, self.wd, 1, mg, 1.0 / self.world, skip=True)
+            return vals if self.param_groups is None else vals + [1.0, 0.0] * len(self.param_groups)
         lr = self.lr * lr_multiplier(self.schedule, t - 1, self.n_warmup, self.n_step)
-        return _lib.adamw_hyper(lr, b1, b2, self.eps, self.wd, t, mg, 1.0 / self.world)
+        vals = _lib.adamw_hyper(lr, b1, b2, self.eps, self.wd, t, mg, 1.0 / self.world)
+        if self.param_groups is None:
+            return vals
+        from .optim import group_table
+        return vals + group_table([lr * g['lr_scale'] for g in self.param_groups],
+                                  [self.wd if g['weight_decay'] is None else g['weight_decay'] for g in self.param_groups],
+                                  b1, t)
+
+    def _adamw(self, p, m, v, g, g_code, shadow, lo, n, flags, stream):
+        """AdamW over [lo, lo + n) of the flat buffers (the base pointers are passed; the slice offsets them)"""
+        esz = 4 if g_code == _lib.F32 else 2
+        args = (p + 4 * lo, m + 4 * lo, v + 4 * lo, g + esz * lo, g_code, None if shadow is None else shadow + 2 * lo, n)
+        if self.param_groups is None:
+            _lib.check(self.lib.ecgvit_adamw_step(*args, self.hyper.data_ptr(), self.stats.data_ptr(), flags, stream),
+                       'adamw_step')
+        else:
+            from .model import _ALIGN
+            _lib.check(self.lib.ecgvit_adamw_step_grouped(*args, self._gmap.data_ptr() + lo // _ALIGN,
+                                                          self.hyper.data_ptr() + 64, self.hyper.data_ptr(),
+                                                          self.stats.data_ptr(), flags, stream), 'adamw_step_grouped')
 
     def _upload_hyper(self):
         # immediate mode: this replay applies update step_count + 1; deferred mode: it applies the PENDING update (or none)
@@ -212,9 +252,8 @@ class FusedTrainer:
             _lib.check(self.lib.ecgvit_grad_sumsq(g.data_ptr(), g_code, n, self.hyper.data_ptr(), self.stats.data_ptr(), st),
                        'grad_sumsq')
         if not self.defer_optimizer:
-            _lib.check(self.lib.ecgvit_adamw_step(m._flat_p.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(),
-                                                  g.data_ptr(), g_code, _lib.ptr(m._shadow), n, self.hyper.data_ptr(),
-                                                  self.stats.data_ptr(), 0, st), 'adamw_step')
+            self._adamw(m._flat_p.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), g.data_ptr(), g_code,
+                        _lib.ptr(m._shadow), 0, n, 0, st)
         return loss, logits
 
     # ---- deferred optimizer --------------------------------------------------------------------------------------
@@ -238,14 +277,11 @@ class FusedTrainer:
         m = self.model
         g, g_code = (m._flat_g, _lib.F32) if self._reducer is None or self._reducer.flat_g16 is None \
             else (self._reducer.flat_g16, _lib.BF16)
-        esz = 4 if g_code == _lib.F32 else 2
         with torch.cuda.stream(stream):
             for i, (pos, lo, hi) in enumerate(self._update_slices()):
                 flags = _lib.ADAMW_SLICE | (_lib.ADAMW_FIRST_SLICE if i == 0 else 0)
-                _lib.check(self.lib.ecgvit_adamw_step(
-                    m._flat_p.data_ptr() + 4 * lo, self.exp_avg.data_ptr() + 4 * lo, self.exp_avg_sq.data_ptr() + 4 * lo,
-                    g.data_ptr() + esz * lo, g_code, None if m._shadow is None else m._shadow.data_ptr() + 2 * lo, hi - lo,
-                    self.hyper.data_ptr(), self.stats.data_ptr(), flags, stream.cuda_stream), 'adamw_step')
+                self._adamw(m._flat_p.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), g.data_ptr(),
+                            g_code, _lib.ptr(m._shadow), lo, hi - lo, flags, stream.cuda_stream)
                 m._flat_g[lo:hi].zero_()
                 if events is not None:
                     ev = torch.cuda.Event()
@@ -316,7 +352,8 @@ class FusedTrainer:
                tuple(float(v) for v in lw) if lw else None,
                self.model.training, float(cfg.hidden_dropout_prob), float(cfg.attention_probs_dropout_prob),
                self.model.loss_reduction, self.model._flat_p.data_ptr(),
-               None if pipe is None else (id(pipe), pipe.pad, pipe.timeout), getattr(self.model, 'mask_ratio', None))
+               None if pipe is None else (id(pipe), pipe.pad, pipe.timeout), getattr(self.model, 'mask_ratio', None),
+               None if self.param_groups is None else (tuple(self._group_names), self._gmap.data_ptr()))
         if self._graph is None or self._graph_key != key:
             self._static_x = torch.empty_like(sample_values)
             self._static_y = None if labels is None else \
@@ -402,9 +439,20 @@ class FusedTrainer:
         return {'step': self.step_count, 'exp_avg': self.exp_avg.clone(), 'exp_avg_sq': self.exp_avg_sq.clone(),
                 'dropout_counter': eng._seed_counter, 'dropout_base_seed': eng.base_seed,  # rank-independent
                 'schedule': self.schedule, 'n_warmup': self.n_warmup, 'n_step': self.n_step, 'lr': self.lr,
-                'weight_decay': self.wd, 'betas': tuple(self.betas), 'eps': self.eps, 'max_grad_norm': self.max_grad_norm}
+                'weight_decay': self.wd, 'betas': tuple(self.betas), 'eps': self.eps, 'max_grad_norm': self.max_grad_norm,
+                **({} if self.param_groups is None else {'param_groups': self._groups_state()})}
+
+    def _groups_state(self):
+        """the groups as [(parameter names, lr_scale, weight_decay)]"""
+        return [(names, g['lr_scale'], g['weight_decay']) for names, g in zip(self._group_names, self.param_groups)]
 
     def load_state_dict(self, sd):
+        mine = None if self.param_groups is None else self._groups_state()
+        theirs = sd.get('param_groups')
+        theirs = None if theirs is None else [(tuple(n), float(s), None if w is None else float(w)) for n, s, w in theirs]
+        if theirs != mine:
+            raise ValueError('FusedTrainer.load_state_dict: the checkpoint\'s parameter groups differ from this '
+                             'trainer\'s (build the trainer with the same param_groups)')
         self._ensure_state(next(self.model.parameters()).device)
         self._pending_step = None
         self.step_count = sd['step']

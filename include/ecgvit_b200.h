@@ -263,6 +263,15 @@ int ecgvit_head_bwd(const void *tok, const float *gamma, const float *w, const f
                     float *dbeta, float *dcolsum, float *scratch, int B, int N, int d, int n_class, int reduction,
                     float grad_scale, const float *grad_scale_dev, int dtype, void *stream);
 
+/* ---- mean pool of vit_pytorch's ViT(pool='mean'): out[b, :] = mean over all N tokens (CLS included) of tok[b, :, :].
+ *      tok [B*N, d] in the stream dtype (ECGVIT_BF16_RES32: fp32 tokens); out fp32 [B, d].  Each column is summed in
+ *      a fixed order without atomics: bit-identical from run to run.  The pooled rows feed ecgvit_head_fwd /
+ *      ecgvit_head_bwd as fp32 tokens with N = 1; the head's dcolsum is then sum_b dpool[b, :], the column sum of the
+ *      broadcast gradient. */
+int ecgvit_token_mean(const void *tok, float *out, int B, int N, int d, int dtype, void *stream);
+/* its backward: dtok[b, t, :] = dpool[b, :] / N for every token t (dtok is FULLY written; bf16 in both bf16 modes) */
+int ecgvit_token_mean_bwd(const float *dpool, void *dtok, int B, int N, int d, int dtype, void *stream);
+
 /* ---- evaluation metrics on the device (SURVEY 8f rank 2): replaces the sklearn calls of
  *      ecg_transformer/util/train.py:12-56 `get_accuracy(preds, labels)`.
  *      preds (probabilities, fp32) and labels (multi-hot fp32) are [n_rows, n_class] device arrays.
@@ -321,6 +330,16 @@ int ecgvit_grad_sumsq_finalize(float *stats, int n_blocks, void *stream);
 #define ECGVIT_ADAMW_FIRST_SLICE 2
 int ecgvit_adamw_step(float *p, float *m, float *v, const void *g, int grad_dtype, void *shadow_bf16, int64_t n,
                       const float *hyper, float *stats, int flags, void *stream);
+/* ecgvit_adamw_step with per-parameter-group learning rate and weight decay (layer-wise LR decay, no-decay sets).
+ *      group_map (device uint8[n / 64]): the group id of every 64-element block of the flat buffers (every tensor
+ *      starts on a 64-element boundary); id 255 leaves p, m, v and the shadow untouched (parameters in no group).
+ *      group_table (device fp32[2 * n_groups], n_groups <= 255): [2i] = 1 - lr_i * weight_decay_i,
+ *      [2i + 1] = lr_i / (1 - beta1^t), derived by the host in double precision; they replace hyper[11] / hyper[12].
+ *      Everything else of hyper and stats (betas, eps, clipping, skip, the skipped-update counter) and the flags are
+ *      those of ecgvit_adamw_step.  A slice offsets group_map by its first element / 64 (n must be a multiple of 64). */
+int ecgvit_adamw_step_grouped(float *p, float *m, float *v, const void *g, int grad_dtype, void *shadow_bf16, int64_t n,
+                              const uint8_t *group_map, const float *group_table, const float *hyper, float *stats,
+                              int flags, void *stream);
 /* in-place  g *= clip_coef  for API-compatible clip_grad_norm_ on a flat buffer */
 int ecgvit_grad_scale_by_clip(float *g, int64_t n, const float *hyper, float *stats, void *stream);
 
