@@ -75,6 +75,12 @@ SIGNATURES = {
                              c_void_p],
     'ecgvit_layernorm_bwd_finalize': [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p],
     'ecgvit_gemm': [POINTER(GemmArgs), c_void_p],
+    # drop path: the plain arguments (without the stream), then path_p, path_stream, rows_per_record, stream
+    'ecgvit_gemm_drop_path': [POINTER(GemmArgs), c_float, c_int, c_int, c_void_p],
+    'ecgvit_layernorm_bwd_drop_path': [c_void_p] * 12 + [c_float, c_int, c_void_p, c_int, c_int, c_int, c_int, c_float,
+                                                         c_int, c_int, c_void_p],
+    'ecgvit_dropout_bwd_copy_drop_path': [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_float, c_int, c_void_p,
+                                          c_int, c_float, c_int, c_int, c_void_p],
     'ecgvit_attention_probs': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_int64, c_int, c_void_p],
     'ecgvit_eval_metrics_scratch_bytes': [c_int],
     'ecgvit_eval_metrics': [c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p],

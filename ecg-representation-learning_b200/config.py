@@ -17,6 +17,19 @@ _DEFINED_SIZES = {
 }
 
 
+def check_drop_path_rate(rate):
+    if not 0.0 <= float(rate) < 1.0:
+        raise ValueError(f'drop_path_rate must lie in [0, 1), got {rate}')
+
+
+def drop_path_rates(config):
+    """per-block drop-path rates of the encoder: torch.linspace(0, drop_path_rate, depth), as timm's ViT builds them"""
+    import torch
+    rate, depth = float(getattr(config, 'drop_path_rate', 0.0)), config.num_hidden_layers
+    check_drop_path_rate(rate)
+    return [float(r) for r in torch.linspace(0.0, rate, depth)]
+
+
 class EcgVitConfig(PretrainedConfig):
     pattern_model_name = re.compile(r'^(?P<name>\S+)-(?P<size>\S+)$')
 
@@ -25,7 +38,7 @@ class EcgVitConfig(PretrainedConfig):
                  intermediate_size: int = 2048, hidden_dropout_prob: float = 0.1,
                  attention_probs_dropout_prob: float = 0.1, num_class: int = 71,
                  compute_dtype: str = 'bf16', per_lead_tokens: bool = False, residual_dtype: str = 'auto',
-                 activation_checkpointing: bool = False, pool: str = 'cls', **kwargs):
+                 activation_checkpointing: bool = False, pool: str = 'cls', drop_path_rate: float = 0.0, **kwargs):
         self.max_signal_length = max_signal_length
         self.patch_size = patch_size
         self.num_channels = num_channels
@@ -57,6 +70,11 @@ class EcgVitConfig(PretrainedConfig):
         if pool not in ('cls', 'mean'):
             raise ValueError(f"pool must be 'cls' or 'mean', got {pool!r}")
         self.pool = pool
+        # stochastic depth (timm's DropPath) on the encoder blocks in training mode: block l of D drops each of its two
+        # residual branches for a whole record with probability drop_path_rate * l / (D - 1) (torch.linspace(0, rate, D))
+        # and scales kept branches by 1 / (1 - that rate).  Rates are quantised to multiples of 1/65536, as dropout's are
+        check_drop_path_rate(drop_path_rate)
+        self.drop_path_rate = float(drop_path_rate)
         super().__init__(**kwargs)
         self.size = None
 

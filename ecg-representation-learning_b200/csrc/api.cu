@@ -30,8 +30,9 @@ bool pdl_enabled() {
     return v == 1;
 }
 
-int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream);   // gemm_tc.cu
-int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream);  // gemm_simt.cu
+// path: drop-path factor of the residual epilogues, or nullptr
+int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream, const PathParams *path = nullptr);   // gemm_tc.cu
+int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream, const PathParams *path = nullptr);  // gemm_simt.cu
 
 }  // namespace ecgvit
 
@@ -58,6 +59,25 @@ int ecgvit_gemm(const ecgvit_gemm_args *g, void *stream) {
         return ecgvit::fail(-1, "gemm: the fp32-residual epilogue belongs to bf16 mode (fp32 mode uses BIAS_RES)");
     if (g->dtype == ECGVIT_BF16) return ecgvit::gemm_bf16_tc(g, ecgvit::as_stream(stream));
     if (g->dtype == ECGVIT_F32) return ecgvit::gemm_f32_ffma(g, ecgvit::as_stream(stream));
+    return ecgvit::fail(-1, "gemm: unknown dtype %d", g->dtype);
+}
+
+int ecgvit_gemm_drop_path(const ecgvit_gemm_args *g, float path_p, int path_stream, int rows_per_record, void *stream) {
+    if (g == nullptr) return ecgvit::fail(-1, "gemm_drop_path: null argument block");
+    ecgvit::PathParams pp;
+    if (int rc = ecgvit::make_path("gemm_drop_path", path_p, path_stream, rows_per_record, g->dropout_seed, pp)) return rc;
+    if (path_p > 0.f && g->epilogue != ECGVIT_EPI_BIAS_RES && g->epilogue != ECGVIT_EPI_BIAS_RES_F32)
+        return ecgvit::fail(-1, "gemm_drop_path: drop path needs epilogue BIAS_RES or BIAS_RES_F32, got %d", g->epilogue);
+    if (pp.drop.threshold == 0) return ecgvit_gemm(g, stream);
+    if (g->A == nullptr || g->B == nullptr || g->out == nullptr || g->aux == nullptr)
+        return ecgvit::fail(-1, "gemm_drop_path: null operand");
+    if (g->epilogue == ECGVIT_EPI_BIAS_RES_F32 && g->dtype != ECGVIT_BF16)
+        return ecgvit::fail(-1, "gemm: the fp32-residual epilogue belongs to bf16 mode (fp32 mode uses BIAS_RES)");
+    if (g->dtype == ECGVIT_BF16) return ecgvit::gemm_bf16_tc(g, ecgvit::as_stream(stream), &pp);
+    if (g->dtype == ECGVIT_F32) {
+        if (g->epilogue != ECGVIT_EPI_BIAS_RES) return ecgvit::fail(-1, "gemm_drop_path(f32): epilogue must be BIAS_RES");
+        return ecgvit::gemm_f32_ffma(g, ecgvit::as_stream(stream), &pp);
+    }
     return ecgvit::fail(-1, "gemm: unknown dtype %d", g->dtype);
 }
 

@@ -5,6 +5,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
+#include <type_traits>
 
 #include "../../include/ecgvit_b200.h"
 
@@ -299,6 +300,33 @@ inline DropoutParams make_dropout(float p, int stream, const uint32_t *seed) {
     return d;
 }
 
+// ---- drop path (stochastic depth) -------------------------------------------------------------------
+// One keep decision per RECORD for a residual branch: record b = row / rows_per_record of a [B * N, d] token matrix
+// draws dropout_one(drop, seed, b) (0 or 1 / (1 - r)) from the counter hash above, so forward, backward and an
+// activation-checkpointing recompute all see the same factor without a stored mask.  Kernels instantiated with a
+// PathParams always have drop.threshold > 0 (the entry points run the plain kernels otherwise).
+struct PathParams {
+    DropoutParams drop;
+    int rows_per_record;
+};
+__device__ __forceinline__ float path_factor(const PathParams &pp, int64_t row) {
+    return dropout_one(pp.drop, __ldg(pp.drop.seed), static_cast<uint32_t>(row / pp.rows_per_record));
+}
+// element dropout and drop path of one branch together (the drop-path variants of the backward masked copies)
+struct DropoutPathParams : DropoutParams {
+    PathParams path;
+};
+template <bool kPath> using DropParamsFor = typename std::conditional<kPath, DropoutPathParams, DropoutParams>::type;
+// host: checks the drop-path arguments of a *_drop_path entry point.  The rate is quantised like dropout's
+// (round(p * 65536)); pp.drop.threshold == 0 means the call is the plain entry point's.  The seed is the dropout seed.
+inline int make_path(const char *what, float p, int stream, int rows_per_record, const uint32_t *seed, PathParams &pp) {
+    if (!(p >= 0.f && p < 1.f)) return fail(-1, "%s: drop-path rate %g outside [0, 1)", what, (double)p);
+    if (rows_per_record <= 0) return fail(-1, "%s: rows_per_record=%d must be positive", what, rows_per_record);
+    if (p > 0.f && seed == nullptr) return fail(-1, "%s: drop path needs a dropout seed", what);
+    pp = PathParams{make_dropout(p, stream, seed), rows_per_record};
+    return 0;
+}
+
 // ---- GEMM epilogue parameters shared by the tcgen05 and FFMA kernels -----------------------------
 struct EpiParams {
     void *out;
@@ -308,11 +336,16 @@ struct EpiParams {
     int64_t ldo;
     DropoutParams drop;  // BIAS_RES: on (acc + bias); BIAS_GELU: on gelu(out); DGELU: on acc
 };
+// BIAS_RES / BIAS_RES_F32 with drop path: out = s[row / rows_per_record] * drop(acc + bias) + aux
+struct EpiPathParams : EpiParams {
+    PathParams path;
+};
 
 // Applies epilogue MODE to NV (4 or 8) consecutive accumulator columns of one row and stores them.
 // `col` is a multiple of NV and the caller guarantees row/col are in bounds.
-template <int MODE, typename T, int NV, bool kExactGelu>
-__device__ __forceinline__ void epilogue_store(const EpiParams &p, int64_t row, int col, float acc[NV]) {
+// EP = EpiPathParams (BIAS_RES only) scales the dropped branch by the row's drop-path factor before the residual add.
+template <int MODE, typename T, int NV, bool kExactGelu, typename EP>
+__device__ __forceinline__ void epilogue_store(const EP &p, int64_t row, int col, float acc[NV]) {
     const int64_t off = row * p.ldo + col;
     if (MODE == ECGVIT_EPI_ATOMIC_F32) {
         float *o = reinterpret_cast<float *>(p.out) + off;
@@ -335,6 +368,12 @@ __device__ __forceinline__ void epilogue_store(const EpiParams &p, int64_t row, 
     const uint32_t seed = drop ? __ldg(p.drop.seed) : 0u;
     if (drop && (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU))
         dropout_apply<NV>(p.drop, seed, static_cast<uint32_t>(off), acc);
+    if constexpr (std::is_same<EP, EpiPathParams>::value) {
+        static_assert(MODE == ECGVIT_EPI_BIAS_RES, "drop path belongs to the residual epilogue");
+        const float s = path_factor(p.path, row);
+#pragma unroll
+        for (int i = 0; i < NV; ++i) acc[i] *= s;
+    }
     if (MODE == ECGVIT_EPI_BIAS_RES) {
         float r[NV];
         if (NV == 8) load8(reinterpret_cast<const T *>(p.aux) + off, r);

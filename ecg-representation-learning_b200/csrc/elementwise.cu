@@ -550,15 +550,17 @@ __global__ void __launch_bounds__(256, MINB) layernorm_fwd_kernel(const TX *__re
 // kDrop: dx feeds a Linear through a dropout (to_out[1] / net[4] of the block below): additionally write
 // dxm = mask * dx / (1 - p) (that Linear's dgrad / wgrad operand) and make the column sums those of dxm (its bias grad).
 // kPatch: dy / mean / rstd are compact patch rows; x is read from, and dx written to, token row i + i / n_patch + 1
-template <typename T, int NV, bool kDrop, typename TX = T, bool kPatch = false>
+// kPath (with kDrop): drop path on the branch as well: dxm = s[row / rows_per_record] * mask * dx, where the element mask
+// is all ones when drop.threshold == 0
+template <typename T, int NV, bool kDrop, typename TX = T, bool kPatch = false, bool kPath = false>
 __global__ void __launch_bounds__(256, 1) layernorm_bwd_kernel(const T *__restrict__ dy, const TX *__restrict__ x,
                                                                 const float *__restrict__ gamma,
                                                                 const float *__restrict__ mean_in,
                                                                 const float *__restrict__ rstd_in, const T *dres, T *dx,
                                                                 float *__restrict__ dgamma, float *__restrict__ dbeta,
                                                                 float *__restrict__ dcolsum, float *__restrict__ partial,
-                                                                int M, int d, T *__restrict__ dxm, DropoutParams drop,
-                                                                int n_patch) {
+                                                                int M, int d, T *__restrict__ dxm,
+                                                                DropParamsFor<kPath> drop, int n_patch) {
     extern __shared__ float red[];  // [warps][3][d] column partials, then [NV * 256] permuted gamma
     pdl_launch_dependents();
     pdl_wait();
@@ -638,6 +640,8 @@ __global__ void __launch_bounds__(256, 1) layernorm_bwd_kernel(const T *__restri
         const float s1 = warp_sum(pair_sum(s1_2)) * inv_d;
         const float s2 = warp_sum(pair_sum(s2_2)) * inv_d;
         const uint64_t B2 = splat2(-rstd * rstd * s2), C2 = splat2(rstd * (mean * rstd * s2 - s1));
+        uint64_t rs2 = 0ull;
+        if constexpr (kPath) rs2 = splat2(path_factor(drop.path, row));
 #pragma unroll
         for (int i = 0; i < NV; ++i) {
             const int c = (i * 32 + lane) * 8;
@@ -655,7 +659,21 @@ __global__ void __launch_bounds__(256, 1) layernorm_bwd_kernel(const T *__restri
                     for (int k = 0; k < 4; ++k) o2[k] = add2(o2[k], r2[k]);
                 }
                 store_pairs(dx + (kPatch ? row + row / n_patch + 1 : row) * d + c, o2);
-                if (kDrop) {
+                if constexpr (kPath) {
+                    const uint32_t seed = __ldg(drop.path.drop.seed);
+                    const uint32_t e0 = static_cast<uint32_t>(row * d + c);
+                    if (drop.threshold != 0) {
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) {
+                            float m0, m1;
+                            dropout_pair(drop, seed, e0 + 2 * k, m0, m1);
+                            o2[k] = mul2(o2[k], pack2(m0, m1));
+                        }
+                    }
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) o2[k] = mul2(o2[k], rs2);
+                    store_pairs(dxm + row * d + c, o2);
+                } else if (kDrop) {
                     const uint32_t seed = __ldg(drop.seed);
                     const uint32_t e0 = static_cast<uint32_t>(row * d + c);
 #pragma unroll
@@ -734,10 +752,11 @@ constexpr int LN_BWD_MAX_BLOCKS = 2 * 160;  // scratch rows; the kernel runs one
 
 // ---------------------------------------------------------------------------------------------------
 // dym = mask * dy / (1 - p);  dcolsum[n] += sum_m dym[m, n].  Same block shape as colsum_kernel.
-template <typename T>
+// kPath: dym = s[row / rows_per_record] * mask * dy, the element mask all ones when drop.threshold == 0
+template <typename T, bool kPath = false>
 __global__ void __launch_bounds__(256) dropout_bwd_copy_kernel(const T *__restrict__ dy, T *__restrict__ dym,
                                                                 float *__restrict__ dcolsum, int M, int N, int64_t ld,
-                                                                int rows_per_block, DropoutParams drop) {
+                                                                int rows_per_block, DropParamsFor<kPath> drop) {
     __shared__ float red[8][32 * 8 + 1];
     pdl_launch_dependents();
     pdl_wait();
@@ -745,7 +764,9 @@ __global__ void __launch_bounds__(256) dropout_bwd_copy_kernel(const T *__restri
     const int c = (blockIdx.x * 32 + tx) * 8;
     const int r0 = blockIdx.y * rows_per_block;
     const int r1 = min(r0 + rows_per_block, M);
-    const uint32_t seed = __ldg(drop.seed);
+    uint32_t seed;
+    if constexpr (kPath) seed = __ldg(drop.path.drop.seed);
+    else seed = __ldg(drop.seed);
     float acc[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) acc[k] = 0.f;
@@ -753,7 +774,14 @@ __global__ void __launch_bounds__(256) dropout_bwd_copy_kernel(const T *__restri
         for (int r = r0 + ty; r < r1; r += 8) {
             float v[8];
             load8(dy + (int64_t)r * ld + c, v);
-            dropout_apply<8>(drop, seed, static_cast<uint32_t>((int64_t)r * ld + c), v);
+            if constexpr (kPath) {
+                if (drop.threshold != 0) dropout_apply<8>(drop, seed, static_cast<uint32_t>((int64_t)r * ld + c), v);
+                const float rs = path_factor(drop.path, r);
+#pragma unroll
+                for (int k = 0; k < 8; ++k) v[k] *= rs;
+            } else {
+                dropout_apply<8>(drop, seed, static_cast<uint32_t>((int64_t)r * ld + c), v);
+            }
             store8(dym + (int64_t)r * ld + c, v);
 #pragma unroll
             for (int k = 0; k < 8; ++k) acc[k] += to_f32(from_f32<T>(v[k]));
@@ -1164,16 +1192,14 @@ int ecgvit_layernorm_bwd_finalize(const float *scratch, float *dgamma, float *db
     return check_launch("layernorm_bwd_finalize");
 }
 
-int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, const float *mean, const float *rstd,
-                         const void *dres, void *dx, float *dgamma, float *dbeta, float *dcolsum, float *scratch,
-                         void *dxm, float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int M, int d,
-                         int defer_finalize, int dtype, void *stream) {
-    ECGVIT_REQUIRE(dy && x && gamma && mean && rstd && dx && dgamma && dbeta && scratch && M > 0,
-                   "layernorm_bwd: bad arguments");
-    ECGVIT_REQUIRE(d % 8 == 0 && d <= 8 * 32 * LN_MAXV, "layernorm_bwd: d=%d must be a multiple of 8 and <= %d", d,
-                   8 * 32 * LN_MAXV);
-    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
-    const bool dropping = drop.threshold != 0 && dxm != nullptr;
+}  // extern "C"
+
+// dxm (when `dropping`) = mask * dx, or with kPath s[row / rows_per_record] * mask * dx
+template <bool kPath>
+static int layernorm_bwd_launch(const void *dy, const void *x, const float *gamma, const float *mean, const float *rstd,
+                                const void *dres, void *dx, float *dgamma, float *dbeta, float *dcolsum, float *scratch,
+                                void *dxm, const DropParamsFor<kPath> &drop, bool dropping, int M, int d,
+                                int defer_finalize, int dtype, void *stream) {
     const int grid = ln_bwd_blocks(M);
     const int nv = (d + 255) / 256;
     const size_t smem = (8 * 3 * (size_t)d + (size_t)nv * 256) * sizeof(float);  // warp slabs + permuted gamma
@@ -1182,16 +1208,17 @@ int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, cons
     do {                                                                                                               \
         static bool attr_set = false;                                                                                  \
         if (!attr_set) {                                                                                               \
-            cudaFuncSetAttribute(layernorm_bwd_kernel<TT, NVV, DROP, TXX>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                 25 * 1024 * 4);                                                                       \
+            cudaFuncSetAttribute(layernorm_bwd_kernel<TT, NVV, DROP, TXX, false, kPath>,                               \
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 25 * 1024 * 4);                          \
             attr_set = true;                                                                                           \
         }                                                                                                              \
-        launch_pdl(layernorm_bwd_kernel<TT, NVV, DROP, TXX>, dim3(grid), dim3(256), smem, st, (const TT *)dy,         \
-                   (const TXX *)x, gamma, mean, rstd, (const TT *)dres, (TT *)dx, dgamma, dbeta, dcolsum, scratch, M, d, \
-                   (TT *)dxm, drop, 1);                                                                                \
+        launch_pdl(layernorm_bwd_kernel<TT, NVV, DROP, TXX, false, kPath>, dim3(grid), dim3(256), smem, st,            \
+                   (const TT *)dy, (const TXX *)x, gamma, mean, rstd, (const TT *)dres, (TT *)dx, dgamma, dbeta,       \
+                   dcolsum, scratch, M, d, (TT *)dxm, drop, 1);                                                        \
     } while (0)
-#define ECGVIT_LN_BWD(TT, NVV) do { if (dropping) ECGVIT_LN_BWD2(TT, NVV, true, TT); else ECGVIT_LN_BWD2(TT, NVV, false, TT); } while (0)
-#define ECGVIT_LN_BWD_R(NVV) do { if (dropping) ECGVIT_LN_BWD2(bf16, NVV, true, float); else ECGVIT_LN_BWD2(bf16, NVV, false, float); } while (0)
+    // (the drop-path kernels always write dxm)
+#define ECGVIT_LN_BWD(TT, NVV) do { if constexpr (kPath) ECGVIT_LN_BWD2(TT, NVV, true, TT); else if (dropping) ECGVIT_LN_BWD2(TT, NVV, true, TT); else ECGVIT_LN_BWD2(TT, NVV, false, TT); } while (0)
+#define ECGVIT_LN_BWD_R(NVV) do { if constexpr (kPath) ECGVIT_LN_BWD2(bf16, NVV, true, float); else if (dropping) ECGVIT_LN_BWD2(bf16, NVV, true, float); else ECGVIT_LN_BWD2(bf16, NVV, false, float); } while (0)
     if (dtype == ECGVIT_BF16) {
         switch (nv) {
             case 1: ECGVIT_LN_BWD(bf16, 1); break;
@@ -1220,6 +1247,43 @@ int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, cons
     int rc = check_launch("layernorm_bwd");
     if (rc || defer_finalize) return rc;
     return ecgvit_layernorm_bwd_finalize(scratch, dgamma, dbeta, dcolsum, M, d, stream);
+}
+
+extern "C" {
+
+int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, const float *mean, const float *rstd,
+                         const void *dres, void *dx, float *dgamma, float *dbeta, float *dcolsum, float *scratch,
+                         void *dxm, float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int M, int d,
+                         int defer_finalize, int dtype, void *stream) {
+    ECGVIT_REQUIRE(dy && x && gamma && mean && rstd && dx && dgamma && dbeta && scratch && M > 0,
+                   "layernorm_bwd: bad arguments");
+    ECGVIT_REQUIRE(d % 8 == 0 && d <= 8 * 32 * LN_MAXV, "layernorm_bwd: d=%d must be a multiple of 8 and <= %d", d,
+                   8 * 32 * LN_MAXV);
+    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    const bool dropping = drop.threshold != 0 && dxm != nullptr;
+    return layernorm_bwd_launch<false>(dy, x, gamma, mean, rstd, dres, dx, dgamma, dbeta, dcolsum, scratch, dxm, drop,
+                                       dropping, M, d, defer_finalize, dtype, stream);
+}
+
+int ecgvit_layernorm_bwd_drop_path(const void *dy, const void *x, const float *gamma, const float *mean,
+                                   const float *rstd, const void *dres, void *dx, float *dgamma, float *dbeta,
+                                   float *dcolsum, float *scratch, void *dxm, float dropout_p, int dropout_stream,
+                                   const uint32_t *dropout_seed, int M, int d, int defer_finalize, int dtype,
+                                   float path_p, int path_stream, int rows_per_record, void *stream) {
+    PathParams pp;
+    if (int rc = make_path("layernorm_bwd_drop_path", path_p, path_stream, rows_per_record, dropout_seed, pp)) return rc;
+    if (pp.drop.threshold == 0)
+        return ecgvit_layernorm_bwd(dy, x, gamma, mean, rstd, dres, dx, dgamma, dbeta, dcolsum, scratch, dxm, dropout_p,
+                                    dropout_stream, dropout_seed, M, d, defer_finalize, dtype, stream);
+    ECGVIT_REQUIRE(dy && x && gamma && mean && rstd && dx && dgamma && dbeta && scratch && dxm && M > 0,
+                   "layernorm_bwd_drop_path: bad arguments (drop path writes dxm)");
+    ECGVIT_REQUIRE(d % 8 == 0 && d <= 8 * 32 * LN_MAXV, "layernorm_bwd: d=%d must be a multiple of 8 and <= %d", d,
+                   8 * 32 * LN_MAXV);
+    DropoutPathParams drop;
+    static_cast<DropoutParams &>(drop) = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    drop.path = pp;
+    return layernorm_bwd_launch<true>(dy, x, gamma, mean, rstd, dres, dx, dgamma, dbeta, dcolsum, scratch, dxm, drop,
+                                      true, M, d, defer_finalize, dtype, stream);
 }
 
 int ecgvit_layernorm_patch_bwd(const void *dy, const void *tok, const float *gamma, const float *mean,
@@ -1286,12 +1350,11 @@ int ecgvit_colsum(const void *x, float *out, int M, int N, int64_t ld, int dtype
     return check_launch("colsum");
 }
 
-int ecgvit_dropout_bwd_copy(const void *dy, void *dym, float *dcolsum, int M, int N, int64_t ld, float dropout_p,
-                            int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream) {
-    ECGVIT_REQUIRE(dy && dym && M > 0 && N > 0, "dropout_bwd_copy: bad arguments");
-    ECGVIT_REQUIRE(N % 8 == 0 && ld % 8 == 0, "dropout_bwd_copy: N=%d and ld=%lld must be multiples of 8", N, (long long)ld);
-    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
-    ECGVIT_REQUIRE(drop.threshold != 0, "dropout_bwd_copy: needs p > 0 and a seed");
+}  // extern "C"
+
+template <bool kPath>
+static int dropout_bwd_copy_launch(const void *dy, void *dym, float *dcolsum, int M, int N, int64_t ld,
+                                   const DropParamsFor<kPath> &drop, int dtype, void *stream) {
     const int col_blocks = (N + 255) / 256;
     int row_blocks = (sm_count() * 4 + col_blocks - 1) / col_blocks;
     if (row_blocks > (M + 63) / 64) row_blocks = (M + 63) / 64;
@@ -1299,11 +1362,38 @@ int ecgvit_dropout_bwd_copy(const void *dy, void *dym, float *dcolsum, int M, in
     const int rows_per_block = (M + row_blocks - 1) / row_blocks;
     dim3 grid(col_blocks, (M + rows_per_block - 1) / rows_per_block);
     if (dtype == ECGVIT_BF16)
-        launch_pdl(dropout_bwd_copy_kernel<bf16>, grid, dim3(256), 0, as_stream(stream), (const bf16 *)dy, (bf16 *)dym, dcolsum, M, N, ld, rows_per_block, drop);
+        launch_pdl(dropout_bwd_copy_kernel<bf16, kPath>, grid, dim3(256), 0, as_stream(stream), (const bf16 *)dy, (bf16 *)dym, dcolsum, M, N, ld, rows_per_block, drop);
     else if (dtype == ECGVIT_F32)
-        dropout_bwd_copy_kernel<float><<<grid, 256, 0, as_stream(stream)>>>((const float *)dy, (float *)dym, dcolsum, M, N, ld, rows_per_block, drop);
+        dropout_bwd_copy_kernel<float, kPath><<<grid, 256, 0, as_stream(stream)>>>((const float *)dy, (float *)dym, dcolsum, M, N, ld, rows_per_block, drop);
     else return fail(-1, "dropout_bwd_copy: unknown dtype %d", dtype);
     return check_launch("dropout_bwd_copy");
+}
+
+extern "C" {
+
+int ecgvit_dropout_bwd_copy(const void *dy, void *dym, float *dcolsum, int M, int N, int64_t ld, float dropout_p,
+                            int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream) {
+    ECGVIT_REQUIRE(dy && dym && M > 0 && N > 0, "dropout_bwd_copy: bad arguments");
+    ECGVIT_REQUIRE(N % 8 == 0 && ld % 8 == 0, "dropout_bwd_copy: N=%d and ld=%lld must be multiples of 8", N, (long long)ld);
+    const DropoutParams drop = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    ECGVIT_REQUIRE(drop.threshold != 0, "dropout_bwd_copy: needs p > 0 and a seed");
+    return dropout_bwd_copy_launch<false>(dy, dym, dcolsum, M, N, ld, drop, dtype, stream);
+}
+
+int ecgvit_dropout_bwd_copy_drop_path(const void *dy, void *dym, float *dcolsum, int M, int N, int64_t ld,
+                                      float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int dtype,
+                                      float path_p, int path_stream, int rows_per_record, void *stream) {
+    PathParams pp;
+    if (int rc = make_path("dropout_bwd_copy_drop_path", path_p, path_stream, rows_per_record, dropout_seed, pp))
+        return rc;
+    if (pp.drop.threshold == 0)
+        return ecgvit_dropout_bwd_copy(dy, dym, dcolsum, M, N, ld, dropout_p, dropout_stream, dropout_seed, dtype, stream);
+    ECGVIT_REQUIRE(dy && dym && M > 0 && N > 0, "dropout_bwd_copy_drop_path: bad arguments");
+    ECGVIT_REQUIRE(N % 8 == 0 && ld % 8 == 0, "dropout_bwd_copy: N=%d and ld=%lld must be multiples of 8", N, (long long)ld);
+    DropoutPathParams drop;
+    static_cast<DropoutParams &>(drop) = make_dropout(dropout_p, dropout_stream, dropout_seed);
+    drop.path = pp;
+    return dropout_bwd_copy_launch<true>(dy, dym, dcolsum, M, N, ld, drop, dtype, stream);
 }
 
 int ecgvit_cast_f32_to_bf16(const float *src, void *dst, int64_t n, void *stream) {

@@ -10,10 +10,10 @@ namespace {
 
 constexpr int TM = 64, TN = 64, TK = 16;
 
-template <int MODE>
+template <int MODE, typename EP = EpiParams>
 __global__ void __launch_bounds__(256) gemm_ffma_kernel(const float *__restrict__ A, int64_t sAm, int64_t sAk,
                                                          const float *__restrict__ B, int64_t sBn, int64_t sBk,
-                                                         int M, int N, int K, EpiParams ep) {
+                                                         int M, int N, int K, EP ep) {
     __shared__ float As[TK][TM + 4];
     __shared__ float Bs[TK][TN + 4];
     const int tid = threadIdx.x;
@@ -85,7 +85,7 @@ __global__ void __launch_bounds__(256) gemm_ffma_kernel(const float *__restrict_
 
 }  // namespace
 
-int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream) {
+int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream, const PathParams *path) {
     ECGVIT_REQUIRE(g->M > 0 && g->N > 0 && g->K > 0, "gemm: empty problem M=%d N=%d K=%d", g->M, g->N, g->K);
     ECGVIT_REQUIRE(g->N % 4 == 0 && g->ldo % 4 == 0, "gemm(f32): N=%d and ldo=%lld must be multiples of 4", g->N,
                    (long long)g->ldo);
@@ -97,6 +97,14 @@ int gemm_f32_ffma(const ecgvit_gemm_args *g, cudaStream_t stream) {
     const int64_t sBn = g->b_kmajor ? g->ldb : 1, sBk = g->b_kmajor ? 1 : g->ldb;
     EpiParams ep{g->out, g->out2, g->aux, g->bias, g->ldo, make_dropout(g->dropout_p, g->dropout_stream, g->dropout_seed)};
     dim3 grid((g->N + TN - 1) / TN, (g->M + TM - 1) / TM);
+    if (path != nullptr) {   // drop path: the residual epilogue only (checked by the entry point)
+        EpiPathParams epp;
+        static_cast<EpiParams &>(epp) = ep;
+        epp.path = *path;
+        gemm_ffma_kernel<ECGVIT_EPI_BIAS_RES, EpiPathParams><<<grid, 256, 0, stream>>>(A, sAm, sAk, B, sBn, sBk, g->M, g->N,
+                                                                                     g->K, epp);
+        return check_launch("gemm_ffma_drop_path");
+    }
     switch (g->epilogue) {
 #define ECGVIT_CASE(MODE) \
     case MODE: gemm_ffma_kernel<MODE><<<grid, 256, 0, stream>>>(A, sAm, sAk, B, sBn, sBk, g->M, g->N, g->K, ep); break;

@@ -84,8 +84,8 @@ int *next_sched_slot() {
     return base + 2 * (__atomic_fetch_add(&next, 1u, __ATOMIC_RELAXED) % kSchedSlots);
 }
 
-template <int BN, bool A_MN, bool B_MN, int MODE>
-int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream) {
+template <int BN, bool A_MN, bool B_MN, int MODE, bool kPath = false>
+int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream, const PathParams *path = nullptr) {
     constexpr bool kWide = MODE == ECGVIT_EPI_BIAS_RES_F32;   // fp32 residual stream: 128-byte staging rows
     using Cfg = PairCfgFor<BN, B_MN, MODE>;
     CUtensorMap ta, tb;
@@ -112,7 +112,7 @@ int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream) {
         if ((MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) &&
             (rc = make_tmap(&tx, g->aux, g->N, g->M, g->ldo, 32, 32, CU_TENSOR_MAP_SWIZZLE_64B))) return rc;
     }
-    auto kern = gemm_tc2_kernel<BN, A_MN, B_MN, MODE>;
+    auto kern = gemm_tc2_kernel<BN, A_MN, B_MN, MODE, kPath>;
     static bool attr_set = false;
     if (!attr_set) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES);
@@ -123,7 +123,10 @@ int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream) {
     const int units = tiles_m * tiles_n * split_k;
     const int clusters = gemm_clusters();
     const int grid = 2 * (units < clusters ? units : clusters);
-    EpiParams ep{g->out, g->out2, g->aux, g->bias, g->ldo, make_dropout(g->dropout_p, g->dropout_stream, g->dropout_seed)};
+    EpiParamsFor<kPath> ep;
+    static_cast<EpiParams &>(ep) =
+        EpiParams{g->out, g->out2, g->aux, g->bias, g->ldo, make_dropout(g->dropout_p, g->dropout_stream, g->dropout_seed)};
+    if constexpr (kPath) ep.path = *path;
     static const int dynamic = [] { const char *e = getenv("ECGVIT_GEMM_DYNAMIC"); return e == nullptr || atoi(e) != 0; }();
     int *sched = next_sched_slot();
     if (sched == nullptr) return fail(-4, "gemm_tc2: cannot resolve the scheduler counters");
@@ -133,9 +136,18 @@ int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream) {
     return check_launch("gemm_tc2");
 }
 
-template <int BN> int dispatch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t s) {
+template <int BN> int dispatch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t s, const PathParams *path) {
     const bool a_mn = !g->a_kmajor, b_mn = !g->b_kmajor;
     const int mode = g->epilogue;
+    if (path != nullptr) {   // drop path: the K-major residual epilogues only (the entry point checked the epilogue)
+        if (a_mn || b_mn) return fail(-1, "gemm(bf16): drop path needs K-major operands");
+        if (mode == ECGVIT_EPI_BIAS_RES) return launch_pair<BN, false, false, ECGVIT_EPI_BIAS_RES, true>(g, split_k, s, path);
+        if (BN < 256 && mode == ECGVIT_EPI_BIAS_RES_F32) {
+            constexpr int BNW = BN < 256 ? BN : 192;
+            return launch_pair<BNW, false, false, ECGVIT_EPI_BIAS_RES_F32, true>(g, split_k, s, path);
+        }
+        return fail(-1, "gemm(bf16): drop path needs a residual epilogue (got %d)", mode);
+    }
 #define ECGVIT_CASE(AM, BMN, MODE) \
     if (a_mn == AM && b_mn == BMN && mode == MODE) return launch_pair<BN, AM, BMN, MODE>(g, split_k, s);
     ECGVIT_CASE(false, false, ECGVIT_EPI_STORE)
@@ -161,7 +173,7 @@ inline double b_kmajor_eff(int b_kmajor) { return b_kmajor ? 0.88 : 0.82; }  // 
 
 }  // namespace
 
-int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream) {
+int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream, const PathParams *path) {
     ECGVIT_REQUIRE(g->M > 0 && g->N > 0 && g->K > 0, "gemm: empty problem M=%d N=%d K=%d", g->M, g->N, g->K);
     ECGVIT_REQUIRE(g->N % 8 == 0, "gemm(bf16): N=%d must be a multiple of 8", g->N);
     ECGVIT_REQUIRE(g->lda % 8 == 0 && g->ldb % 8 == 0, "gemm(bf16): lda=%lld ldb=%lld must be multiples of 8",
@@ -215,13 +227,13 @@ int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream) {
     };
     const bool wide_ok = g->epilogue != ECGVIT_EPI_BIAS_RES_F32;   // see dispatch_pair
     static const int forced_bn = [] { const char *e = getenv("ECGVIT_GEMM_BN"); return e != nullptr ? atoi(e) : 0; }();
-    if (forced_bn == 128) return dispatch_pair<128>(g, split_k, stream);   // experiments only
-    if (forced_bn == 192) return dispatch_pair<192>(g, split_k, stream);
-    if (forced_bn == 256 && wide_ok) return dispatch_pair<256>(g, split_k, stream);
+    if (forced_bn == 128) return dispatch_pair<128>(g, split_k, stream, path);   // experiments only
+    if (forced_bn == 192) return dispatch_pair<192>(g, split_k, stream, path);
+    if (forced_bn == 256 && wide_ok) return dispatch_pair<256>(g, split_k, stream, path);
     const double s256 = wide_ok ? score(256, 1.0) : 1e30, s192 = score(192, b_kmajor_eff(g->b_kmajor)), s128 = score(128, 0.67);
-    if (g->N <= 128 || (s128 < s256 && s128 < s192)) return dispatch_pair<128>(g, split_k, stream);
-    if (s192 < s256) return dispatch_pair<192>(g, split_k, stream);
-    return dispatch_pair<256>(g, split_k, stream);
+    if (g->N <= 128 || (s128 < s256 && s128 < s192)) return dispatch_pair<128>(g, split_k, stream, path);
+    if (s192 < s256) return dispatch_pair<192>(g, split_k, stream, path);
+    return dispatch_pair<256>(g, split_k, stream, path);
 }
 
 }  // namespace ecgvit

@@ -65,10 +65,11 @@ __device__ __forceinline__ uint32_t sw64_offset(int lane, int j) {
 // pre-activation), fetched by TMA while the mainloop was still running, and is updated in place.
 // The caller then issues one TMA store per tile (TMA clips rows >= M and columns >= N, so there are no guards here).
 // BIAS_SUB_ROWSQ: the tile holds the target; out = acc + bias - target, and `sq` accumulates the fp32 squares.
-template <int MODE>
+// kPath (BIAS_RES): the dropped branch is scaled by the row's drop-path factor `rs` before the residual add.
+template <int MODE, bool kPath = false>
 __device__ __forceinline__ void epilogue_half16(const EpiParams &ep, int64_t row, int col_base, int jbase,
                                                 const uint32_t r[16], uint8_t *tile0, uint8_t *tile1, int lane,
-                                                int n_cols, float &sq) {
+                                                int n_cols, float &sq, float rs = 1.f) {
     const bool drop = ep.drop.threshold != 0;  // kernel-uniform
     const uint32_t seed = drop ? __ldg(ep.drop.seed) : 0u;
 #pragma unroll
@@ -89,6 +90,10 @@ __device__ __forceinline__ void epilogue_half16(const EpiParams &ep, int64_t row
         const uint32_t soff = sw64_offset(lane, j);
         const uint32_t eidx = static_cast<uint32_t>(row * ep.ldo + col);  // element index of v[0] (even)
         if (drop && (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU)) dropout_apply<8>(ep.drop, seed, eidx, v);
+        if (kPath) {
+#pragma unroll
+            for (int i = 0; i < 8; ++i) v[i] *= rs;
+        }
         if (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ) {
             const uint4 a4 = *reinterpret_cast<const uint4 *>(tile0 + soff);
             float a[8];
@@ -135,8 +140,11 @@ __device__ __forceinline__ void epilogue_half16(const EpiParams &ep, int64_t row
 
 // fp32 residual stream (ECGVIT_EPI_BIAS_RES_F32): out = drop(acc + bias) + aux with aux / out fp32.  The warp's staging
 // tile is 32 rows x 128 bytes (SWIZZLE_128B) and already holds the residual; 16 columns = four 16-byte pieces per call.
+// kPath: out = rs * drop(acc + bias) + aux with the row's drop-path factor rs.
+template <bool kPath = false>
 __device__ __forceinline__ void epilogue_half16_f32(const EpiParams &ep, int64_t row, int col_base, int half,
-                                                    const uint32_t r[16], uint8_t *tile, int lane, int n_cols) {
+                                                    const uint32_t r[16], uint8_t *tile, int lane, int n_cols,
+                                                    float rs = 1.f) {
     const bool drop = ep.drop.threshold != 0;  // kernel-uniform
     const uint32_t seed = drop ? __ldg(ep.drop.seed) : 0u;
 #pragma unroll
@@ -151,6 +159,10 @@ __device__ __forceinline__ void epilogue_half16_f32(const EpiParams &ep, int64_t
             v[0] += b.x; v[1] += b.y; v[2] += b.z; v[3] += b.w;
         }
         if (drop) dropout_apply<4>(ep.drop, seed, static_cast<uint32_t>(row * ep.ldo + col), v);
+        if (kPath) {
+#pragma unroll
+            for (int i = 0; i < 4; ++i) v[i] *= rs;
+        }
         float4 *p = reinterpret_cast<float4 *>(tile + static_cast<uint32_t>(lane) * 128u +
                                                (static_cast<uint32_t>(jc ^ (lane & 7)) << 4));
         float4 a = *p;
@@ -159,12 +171,15 @@ __device__ __forceinline__ void epilogue_half16_f32(const EpiParams &ep, int64_t
     }
 }
 
-template <int BN, bool A_MN, bool B_MN, int MODE>
+// kPath: the drop-path variant of the residual epilogues (BIAS_RES / BIAS_RES_F32), whose `ep` is an EpiPathParams
+template <bool kPath> using EpiParamsFor = typename std::conditional<kPath, EpiPathParams, EpiParams>::type;
+
+template <int BN, bool A_MN, bool B_MN, int MODE, bool kPath = false>
 __global__ void __cluster_dims__(2, 1, 1)
 __launch_bounds__(PairCfgFor<BN, B_MN, MODE>::THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                 const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_out2,
-                const __grid_constant__ CUtensorMap tmap_aux, int M, int N, int K, int split_k, EpiParams ep,
+                const __grid_constant__ CUtensorMap tmap_aux, int M, int N, int K, int split_k, EpiParamsFor<kPath> ep,
                 int *__restrict__ sched_ctr, int dynamic) {
     constexpr bool kWide = MODE == ECGVIT_EPI_BIAS_RES_F32;   // (the split-K epilogue has its own fp32 path below)
     using Cfg = PairCfgFor<BN, B_MN, MODE>;
@@ -172,6 +187,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
     constexpr bool kHasAux = (MODE == ECGVIT_EPI_BIAS_RES || MODE == ECGVIT_EPI_DGELU || kWide || kRowSq);
     constexpr int STAGES = Cfg::STAGES;
     constexpr int BM2 = 2 * BM;  // rows of the pair tile
+    static_assert(!kPath || MODE == ECGVIT_EPI_BIAS_RES || kWide, "drop path belongs to the residual epilogues");
 
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -424,6 +440,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                 // while half s is being computed (two register buffers)
                 uint32_t ra[16], rb[16];
                 float sq = 0.f;   // BIAS_SUB_ROWSQ: this row's squares over the warp's 64 columns
+                float rs = 1.f;   // kPath: this row's drop-path factor (one hash per row and tile)
+                if constexpr (kPath) rs = path_factor(ep.path, row);
                 if (n_units > 0) ptx::tmem_ld_32x16(taddr0, ra);
 #pragma unroll 1
                 for (int i = 0; i < n_units; ++i) {
@@ -446,12 +464,12 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
                         if (lane == 0) ptx::tma_store_wait_read<0>();
                         __syncwarp();
                     }
-                    if (kWide) epilogue_half16_f32(ep, row, col_base, 0, ra, t0, lane, N);
-                    else epilogue_half16<MODE>(ep, row, col_base, 0, ra, t0, t1, lane, N, sq);
+                    if (kWide) epilogue_half16_f32<kPath>(ep, row, col_base, 0, ra, t0, lane, N, rs);
+                    else epilogue_half16<MODE, kPath>(ep, row, col_base, 0, ra, t0, t1, lane, N, sq, rs);
                     ptx::tmem_ld_wait_bind(rb);
                     if (i + 1 < n_units) ptx::tmem_ld_32x16(taddr0 + 32 * (i + 1), ra);
-                    if (kWide) epilogue_half16_f32(ep, row, col_base, 1, rb, t0, lane, N);
-                    else epilogue_half16<MODE>(ep, row, col_base, 2, rb, t0, t1, lane, N, sq);
+                    if (kWide) epilogue_half16_f32<kPath>(ep, row, col_base, 1, rb, t0, lane, N, rs);
+                    else epilogue_half16<MODE, kPath>(ep, row, col_base, 2, rb, t0, t1, lane, N, sq, rs);
                     ptx::fence_proxy_async_smem();  // generic-proxy smem writes -> visible to the TMA (async proxy)
                     __syncwarp();
                     if (lane == 0) {

@@ -26,6 +26,7 @@ import os
 import torch
 
 from . import _lib
+from .config import drop_path_rates
 from ._lib import (GemmArgs, F32, BF16, EPI_STORE, EPI_BIAS_RES, EPI_BIAS_GELU, EPI_DGELU, EPI_ATOMIC_F32,
                    EPI_BIAS_RES_F32, EPI_BIAS_SUB_ROWSQ)
 
@@ -80,21 +81,32 @@ class StepEngine:
             return 0.0, 0.0
         return float(m.config.attention_probs_dropout_prob), float(m.config.hidden_dropout_prob)
 
+    def _drop_path_rates(self):
+        """per-block drop-path rates of the encoder (config.drop_path_rate); zero in eval mode"""
+        m = self.model
+        depth = m.config.num_hidden_layers
+        return drop_path_rates(m.config) if m.training else [0.0] * depth
+
     # ---- helpers ---------------------------------------------------------------------------------
     @property
     def _stream(self):
         return torch.cuda.current_stream().cuda_stream
 
     def _gemm(self, M, N, K, A, lda, a_k, B, ldb, b_k, epi, out, ldo, out2=None, aux=None, bias=None, split_k=1,
-              drop=None):
+              drop=None, path=None):
+        """path: (rate, site, rows per record) of a drop-path residual epilogue, or None"""
         p, stream = drop if drop is not None else (0.0, 0)
+        r = path[0] if path is not None else 0.0
         g = GemmArgs(M, N, K, A.data_ptr(), lda, a_k, B.data_ptr(), ldb, b_k, epi, out.data_ptr(), ldo,
                      _lib.ptr(out2), _lib.ptr(aux), _lib.ptr(bias), self.model._dtype_code, split_k,
-                     stream, p, self.rng.data_ptr() if p > 0 else None)
+                     stream, p, self.rng.data_ptr() if p > 0 or r > 0 else None)
         if _lib.profile[0] is not None:
             keep = GemmArgs.from_buffer_copy(g)  # lets bench.py re-launch exactly this call when timing the kernel
             _lib.profile_meta[0] = (M, N, K, epi, a_k, b_k, keep)
-        _lib.check(self.lib.ecgvit_gemm(ctypes.byref(g), self._stream), 'gemm')
+        if r > 0:
+            _lib.check(self.lib.ecgvit_gemm_drop_path(ctypes.byref(g), r, path[1], path[2], self._stream), 'gemm')
+        else:
+            _lib.check(self.lib.ecgvit_gemm(ctypes.byref(g), self._stream), 'gemm')
 
     def workspace(self, B, L, n_vis=None):
         """activations of one (batch, length) shape; n_vis: the patches the encoder sees per record (all when None)"""
@@ -158,7 +170,9 @@ class StepEngine:
     def _alloc_stack(self, s, prefix, B, N, d, mlp, H, depth, ckpt):
         """a block stack on the object s: `depth` blocks of width d over B sequences of N tokens, parameters keyed
         `{prefix}{l}.`, its dims, activations and backward scratch.  Only the encoder stack (prefix 'l') calls the layer
-        hooks; p_blk is its block dropout probability, set by the forward pass."""
+        hooks; p_blk is its block dropout probability and r_path its per-block drop-path rates, both set by the forward
+        pass (the encoder's; a decoder keeps zeros).  Drop-path site of branch j (0 attention, 1 feed-forward) of block l:
+        path_site + 2 * l + j, after the dropout sites 0 .. 4 * depth and the mask site 4 * depth + 1."""
         m = self.model
         dev = m._flat_p.device
         T = m._act_dtype
@@ -167,6 +181,8 @@ class StepEngine:
         s.prefix, s.d, s.mlp, s.H, s.depth, s.ckpt, s.hooks = prefix, d, mlp, H, depth, ckpt, prefix == 'l'
         s.B, s.N, s.M = B, N, M
         s.p_blk = 0.0
+        s.r_path = [0.0] * depth
+        s.path_site = 4 * depth + 2
 
         def buf(*shape, dtype=T):
             return torch.empty(*shape, device=dev, dtype=dtype)
@@ -263,6 +279,7 @@ class StepEngine:
         self._gemm(B * w.n_vis, d, Kp, w.a_emb, Kp, 1, w_embed, Kp, 1, EPI_STORE, w.e, d, bias=pf['embed.b'])
         p_emb, p_blk = self._dropout_probs()
         w.p_emb, w.p_blk = p_emb, p_blk
+        w.r_path = self._drop_path_rates()
         self._assemble(w)
         for l in range(c.num_hidden_layers):
             if hook is not None:
@@ -345,7 +362,7 @@ class StepEngine:
         _lib.check(lib.ecgvit_attention_fwd(s.qkv[l].data_ptr(), s.o[l].data_ptr(), s.lse[l].data_ptr(), B, N, H, dh,
                                             scale, p_blk, s_att, blk_seed, dt, st), 'attention_fwd')
         self._gemm(M, d, inner, s.o[l], inner, 1, wt[p + 'out.w'], inner, 1, epi_res, s.y[l], d,
-                   aux=s.x[l], bias=pf[p + 'out.b'], drop=(p_blk, s_out))
+                   aux=s.x[l], bias=pf[p + 'out.b'], drop=(p_blk, s_out), path=(s.r_path[l], s.path_site + 2 * l, N))
         _lib.check(lib.ecgvit_layernorm_fwd(s.y[l].data_ptr(), pf[p + 'ln2.w'].data_ptr(), pf[p + 'ln2.b'].data_ptr(),
                                             s.ln2[l].data_ptr(), s.stat2[l][0].data_ptr(), s.stat2[l][1].data_ptr(),
                                             M, d, LN_EPS, rdt, st), 'layernorm_fwd')
@@ -353,7 +370,8 @@ class StepEngine:
                    out2=s.h[l], bias=pf[p + 'ff1.b'], drop=(p_blk, s_act))
         if not recompute:
             self._gemm(M, d, mlp, s.h[l], mlp, 1, wt[p + 'ff2.w'], mlp, 1, epi_res, s.x[l + 1], d,
-                       aux=s.y[l], bias=pf[p + 'ff2.b'], drop=(p_blk, s_ff2))
+                       aux=s.y[l], bias=pf[p + 'ff2.b'], drop=(p_blk, s_ff2),
+                       path=(s.r_path[l], s.path_site + 2 * l + 1, N))
 
     def span_buffer(self, B):
         """device int32 [B, 2] (start, length) of the TimeOut span of every record; a persistent buffer, so a captured
@@ -395,9 +413,11 @@ class StepEngine:
             m._flat_g.zero_()
         last = f'l{depth - 1}.'
         top = (depth - 1) & 1
-        # with dropout between net[3] / to_out[0] and the residual add, the Linear sees mask * dz / (1 - p): its operand
-        # and its bias gradient come from the masked copy, so the producers must not pre-sum the unmasked gradient
-        self._head_backward(w, w.dz[top], gr[last + 'ff2.b'] if w.p_blk == 0 else None, grad_scale, grad_scale_dev)
+        # with dropout or drop path between net[3] / to_out[0] and the residual add, the Linear sees s * mask * dz / (1 - p):
+        # its operand and its bias gradient come from the masked copy, so the producers must not pre-sum the unmasked
+        # gradient
+        self._head_backward(w, w.dz[top], None if self._masked(w, depth - 1) else gr[last + 'ff2.b'], grad_scale,
+                            grad_scale_dev)
         self._stack_backward(w)
         dz = w.dz[(-1) & 1]   # gradient w.r.t. the token matrix (input of block 0)
         # ---- embedding: tok = [cls | a_emb We^T + be] + pos
@@ -413,10 +433,16 @@ class StepEngine:
         if m._after_layer_backward is not None:
             m._after_layer_backward(-1)
 
+    @staticmethod
+    def _masked(s, l):
+        """whether the residual branches of block l of stack s are masked (element dropout or drop path): their
+        Linears then read a masked copy of the residual-stream gradient"""
+        return s.p_blk > 0 or s.r_path[l] > 0
+
     def _stack_backward(self, s):
         """backward through the blocks of the stack s, from the gradient of its output in s.dz[(depth - 1) & 1] (its
-        column sum already added to the top ff2 bias gradient when p = 0) to that of its input in s.dz[1]; the weight
-        gradients run on the side stream, which is joined at the end"""
+        column sum already added to the top ff2 bias gradient when the top block is not masked) to that of its input in
+        s.dz[1]; the weight gradients run on the side stream, which is joined at the end"""
         m, lib, st = self.model, self.lib, self._stream
         dt = m._dtype_code
         rdt = m._res_code
@@ -456,17 +482,22 @@ class StepEngine:
 
         ev_fold = [None, None]
 
-        def layernorm_bwd(which, dln, x_in, gamma, stat, dres, dx, dgamma, dbeta, dcol, dxm, p_drop, site):
-            """dx = dres + LN'(dln) (+ the dropout-masked copy dxm) on the main stream; the fold of the per-CTA partial rows
-            into dgamma / dbeta / dcol feeds nothing in the chain and runs on the side stream"""
+        def layernorm_bwd(which, dln, x_in, gamma, stat, dres, dx, dgamma, dbeta, dcol, dxm, p_drop, site,
+                          r_path=0.0, path_site=0):
+            """dx = dres + LN'(dln) (+ the masked copy dxm: dropout p_drop at `site`, drop path r_path at `path_site`) on
+            the main stream; the fold of the per-CTA partial rows into dgamma / dbeta / dcol feeds nothing in the chain and
+            runs on the side stream"""
             scr = s.ln_scratch[which]
             before_overwrite(ev_fold[which])  # the fold of this scratch's previous user
-            seed = blk_seed if (dxm is not None and p_drop > 0) else None
-            _lib.check(lib.ecgvit_layernorm_bwd(
-                dln.data_ptr(), x_in.data_ptr(), gamma.data_ptr(), stat[0].data_ptr(), stat[1].data_ptr(),
-                dres.data_ptr(), dx.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), _lib.ptr(dcol), scr.data_ptr(),
-                _lib.ptr(dxm), p_drop, site, seed, M, d, 0 if side is None else 1, rdt, st),
-                'layernorm_bwd' if side is None else 'layernorm_bwd_partial')
+            seed = seed_ptr if (dxm is not None and (p_drop > 0 or r_path > 0)) else None
+            args = (dln.data_ptr(), x_in.data_ptr(), gamma.data_ptr(), stat[0].data_ptr(), stat[1].data_ptr(),
+                    dres.data_ptr(), dx.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), _lib.ptr(dcol), scr.data_ptr(),
+                    _lib.ptr(dxm), p_drop, site, seed, M, d, 0 if side is None else 1, rdt)
+            what = 'layernorm_bwd' if side is None else 'layernorm_bwd_partial'
+            if r_path > 0:
+                _lib.check(lib.ecgvit_layernorm_bwd_drop_path(*args, r_path, path_site, N, st), what)
+            else:
+                _lib.check(lib.ecgvit_layernorm_bwd(*args, st), what)
             if side is not None:
                 ready = torch.cuda.Event()
                 ready.record(main)
@@ -480,11 +511,16 @@ class StepEngine:
 
         # side-stream events per layer: ev[l] = {'ff2', 'ff1', 'out', 'qkv'} -> completion of that weight gradient
         evs = {}
-        if p_blk > 0:
+        if self._masked(s, depth - 1):
             # the top block's input gradient comes from the head, not from a LayerNorm': mask it here
-            _lib.check(lib.ecgvit_dropout_bwd_copy(s.dz[top].data_ptr(), s.dzm[0][top].data_ptr(),
-                                                   gr[last + 'ff2.b'].data_ptr(), M, d, d, p_blk, 4 * depth, seed_ptr, dt, st),
-                       'dropout_bwd_copy')
+            args = (s.dz[top].data_ptr(), s.dzm[0][top].data_ptr(), gr[last + 'ff2.b'].data_ptr(), M, d, d, p_blk,
+                    4 * depth, seed_ptr, dt)
+            r_top = s.r_path[depth - 1]
+            if r_top > 0:
+                _lib.check(lib.ecgvit_dropout_bwd_copy_drop_path(*args, r_top, s.path_site + 2 * (depth - 1) + 1, N, st),
+                           'dropout_bwd_copy')
+            else:
+                _lib.check(lib.ecgvit_dropout_bwd_copy(*args, st), 'dropout_bwd_copy')
         for l in range(depth - 1, -1, -1):
             p = f'{s.prefix}{l}.'
             q, qn = l & 1, (l - 1) & 1      # buffer parity of this layer / of the layer below
@@ -497,7 +533,8 @@ class StepEngine:
                 self._block_forward(l, s, recompute=True)
             e = evs.setdefault(l, {})
             dz, dy, du, dqkv = s.dz[q], s.dy[q], s.du[q], s.dqkv[q]
-            dzl = s.dzm[0][q] if p_blk > 0 else dz      # what net[3] saw: mask * dz / (1 - p)
+            masked, r_l = self._masked(s, l), s.r_path[l]
+            dzl = s.dzm[0][q] if masked else dz      # what net[3] saw: s * mask * dz / (1 - p)
             # ---- feed-forward branch: x[l+1] = y + drop(W2 drop(gelu(W1 ln2(y) + b1)) + b2)
             e['ff2'] = wgrad(d, mlp, M, dzl, d, 0, s.h[l], mlp, 0, EPI_ATOMIC_F32, gr[p + 'ff2.w'], mlp, split_k=0)
             before_overwrite(old.get('ff1'))   # du of this parity
@@ -516,10 +553,10 @@ class StepEngine:
             e['ff1'] = wgrad(mlp, d, M, du, mlp, 0, s.ln2[l], d, 0, EPI_ATOMIC_F32, gr[p + 'ff1.w'], d, split_k=0)
             self._gemm(M, d, mlp, du, mlp, 1, wt[p + 'ff1.w'], d, 0, EPI_STORE, s.dln, d)
             before_overwrite(old.get('out'))   # dy / its masked copy of this parity
-            dyl = s.dzm[1][q] if p_blk > 0 else dy
+            dyl = s.dzm[1][q] if masked else dy
             layernorm_bwd(0, s.dln, s.y[l], pf[p + 'ln2.w'], s.stat2[l], dz, dy, gr[p + 'ln2.w'], gr[p + 'ln2.b'],
-                          gr[p + 'out.b'], dyl if p_blk > 0 else None, p_blk, s_out)
-            # ---- attention branch: y = x + drop(Wo attn(Wqkv ln1(x)) + bo); dyl = mask * dy / (1 - p)
+                          gr[p + 'out.b'], dyl if masked else None, p_blk, s_out, r_l, s.path_site + 2 * l)
+            # ---- attention branch: y = x + s * drop(Wo attn(Wqkv ln1(x)) + bo); dyl = s * mask * dy / (1 - p)
             e['out'] = wgrad(d, inner, M, dyl, d, 0, s.o[l], inner, 0, EPI_ATOMIC_F32, gr[p + 'out.w'], inner, split_k=0)
             self._gemm(M, inner, d, dyl, d, 1, wt[p + 'out.w'], inner, 0, EPI_STORE, s.d_o, inner)
             before_overwrite(old.get('qkv'))   # dqkv of this parity
@@ -531,12 +568,14 @@ class StepEngine:
                              split_k=0)
             self._gemm(M, d, 3 * inner, dqkv, 3 * inner, 1, wt[p + 'qkv.w'], d, 0, EPI_STORE, s.dln, d)
             below_bias = gr[f'{s.prefix}{l - 1}.ff2.b'] if l > 0 else None
-            drop_below = p_blk > 0 and l > 0
+            drop_below = l > 0 and self._masked(s, l - 1)
+            r_below = s.r_path[l - 1] if l > 0 else 0.0
             # LayerNorm' writes the input gradient of layer l - 1 into the OTHER parity, last read by the ff2 weight
             # gradient of layer l + 1
             before_overwrite(evs.get(l + 1, {}).get('ff2'))
             layernorm_bwd(1, s.dln, s.x[l], pf[p + 'ln1.w'], s.stat1[l], dy, s.dz[qn], gr[p + 'ln1.w'], gr[p + 'ln1.b'],
-                          below_bias, s.dzm[0][qn] if drop_below else None, p_blk if drop_below else 0.0, s_ff2 - 4)
+                          below_bias, s.dzm[0][qn] if drop_below else None, p_blk if drop_below else 0.0, s_ff2 - 4,
+                          r_below if drop_below else 0.0, s.path_site + 2 * (l - 1) + 1)
             if s.hooks and m._after_layer_backward is not None:
                 # the gradient bucket of layer l is complete once its side-stream wgrads AND everything the main stream
                 # has issued so far (LayerNorm / bias gradients) are done.  The collective is therefore issued from the

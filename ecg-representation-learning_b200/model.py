@@ -16,7 +16,7 @@ import torch
 from torch import nn
 
 from . import _lib
-from .config import EcgVitConfig
+from .config import EcgVitConfig, check_drop_path_rate
 from .engine import StepEngine, MaskedPatchEngine, MaskedAutoencoderEngine
 
 ModelOutput = namedtuple('ModelOutput', ['loss', 'logits'])  # reference: util/models.py:3
@@ -154,6 +154,12 @@ class _EcgVitFunction(torch.autograd.Function):
         return (None, None, None) + (None,) * len(params)
 
 
+def _draws_masks(config):
+    """whether a training forward of this config draws dropout masks or drop-path keeps"""
+    return (config.hidden_dropout_prob > 0 or config.attention_probs_dropout_prob > 0 or
+            float(getattr(config, 'drop_path_rate', 0.0)) > 0)
+
+
 class EcgVit(nn.Module):
     _classification_head = True   # ViT container with `mlp_head`
     _encoder_mask_token = False   # ... and without `mask_token`
@@ -169,6 +175,7 @@ class EcgVit(nn.Module):
             raise ValueError(f"pool must be 'cls' or 'mean', got {pool!r}")
         # only the classification head pools; the pre-training heads read every patch token and ignore `pool`
         self._mean_pool = pool == 'mean' and self._classification_head
+        check_drop_path_rate(getattr(config, 'drop_path_rate', 0.0))
         self.config = config
         self.num_class = num_class  # the reference builds the head from the ctor arg, not config.num_class (:105)
         self.vit = ViT(signal_length=config.max_signal_length, patch_size=config.patch_size, num_classes=num_class,
@@ -253,8 +260,8 @@ class EcgVit(nn.Module):
         return ModelOutput(loss=loss, logits=logits)
 
     def _draws_step_seed(self):
-        """whether a training forward needs a fresh device seed (dropout masks)"""
-        return self.training and (self.config.hidden_dropout_prob > 0 or self.config.attention_probs_dropout_prob > 0)
+        """whether a training forward needs a fresh device seed (dropout masks, drop-path keeps)"""
+        return self.training and _draws_masks(self.config)
 
     # ---- flat storage ------------------------------------------------------------------------------
     def _param_list(self):
@@ -573,7 +580,7 @@ class Recorder(nn.Module):
         model = self.vit._owner()
         assert img.dim() == 4 and img.shape[2] == 1, 'expected [B, C, 1, L] (height axis of 1, ecg_vit.py:141)'
         model._prepare(img.device)
-        if model.training and (model.config.hidden_dropout_prob > 0 or model.config.attention_probs_dropout_prob > 0):
+        if model.training and _draws_masks(model.config):
             model._engine.new_dropout_seed()
         with torch.no_grad():
             _, logits = model._engine.forward(img.squeeze(2), None, model.loss_reduction, record_attention=True)

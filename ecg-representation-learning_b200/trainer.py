@@ -346,11 +346,12 @@ class FusedTrainer:
         pipe = self.model.input_pipeline
         cfg = self.model.config
         # everything the capture bakes in: shapes, loss weighting / reduction, train vs eval (dropout on or off and its
-        # probabilities), the input pipeline, and the flat buffers the kernels point at
+        # probabilities, the drop-path rates), the input pipeline, and the flat buffers the kernels point at
         # (a masked-patch model: no labels, and its mask ratio sets how many patches the captured mask draw takes)
         key = (tuple(sample_values.shape), None if labels is None else tuple(labels.shape),
                tuple(float(v) for v in lw) if lw else None,
                self.model.training, float(cfg.hidden_dropout_prob), float(cfg.attention_probs_dropout_prob),
+               float(getattr(cfg, 'drop_path_rate', 0.0)),
                self.model.loss_reduction, self.model._flat_p.data_ptr(),
                None if pipe is None else (id(pipe), pipe.pad, pipe.timeout), getattr(self.model, 'mask_ratio', None),
                None if self.param_groups is None else (tuple(self._group_names), self._gmap.data_ptr()))

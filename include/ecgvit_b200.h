@@ -193,6 +193,14 @@ int ecgvit_layernorm_bwd(const void *dy, const void *x, const float *gamma, cons
                          const uint32_t *dropout_seed, int M, int d, int defer_finalize, int dtype, void *stream);
 int ecgvit_layernorm_bwd_finalize(const float *scratch, float *dgamma, float *dbeta, float *dcolsum, int M, int d,
                                   void *stream);
+/* ecgvit_layernorm_bwd when dx feeds a Linear through element dropout (p >= 0) and drop path (see ecgvit_gemm_drop_path):
+ * dxm = s[row / rows_per_record] * mask * dx (mask all ones when dropout_p = 0; fp32 before rounding) is written, dxm
+ * must not be NULL, and dcolsum += colsum(dxm). */
+int ecgvit_layernorm_bwd_drop_path(const void *dy, const void *x, const float *gamma, const float *mean,
+                                   const float *rstd, const void *dres, void *dx, float *dgamma, float *dbeta,
+                                   float *dcolsum, float *scratch, void *dxm, float dropout_p, int dropout_stream,
+                                   const uint32_t *dropout_seed, int M, int d, int defer_finalize, int dtype,
+                                   float path_p, int path_stream, int rows_per_record, void *stream);
 
 /* ---- dense contraction  C[m,n] = sum_k A(m,k) * B(n,k)  with fused epilogue.
  *      Replaces nn.Linear forward / its autograd dgrad / wgrad (vit_pytorch Attention.to_qkv, to_out[0],
@@ -223,6 +231,20 @@ typedef struct ecgvit_gemm_args {
     const uint32_t *dropout_seed;
 } ecgvit_gemm_args;
 int ecgvit_gemm(const ecgvit_gemm_args *g, void *stream);
+
+/* ---- drop path (stochastic depth, timm's DropPath): a residual branch is kept or dropped per RECORD.
+ *      Added in ABI version 7 without changing any earlier entry point, so the version number stays 7.
+ *
+ *      Token row `row` of a [B * rows_per_record, d] matrix belongs to record b = row / rows_per_record, whose factor is
+ *      s[b] = 1 / (1 - path_p) when the 16 bits of the dropout counter hash (see "dropout" below) that site `path_stream`
+ *      assigns to element index b are >= round(path_p * 65536), else 0.  The rate is therefore quantised to a multiple of
+ *      1/65536, as dropout's is.  The seed is the dropout seed of the call (g->dropout_seed / dropout_seed), which must
+ *      be set when path_p > 0 even if dropout_p = 0 (element dropout off).  path_p = 0 makes every call below exactly its
+ *      plain counterpart.  path_p outside [0, 1) and rows_per_record <= 0 are rejected before any launch.
+ *
+ *      GEMM: only with ECGVIT_EPI_BIAS_RES / ECGVIT_EPI_BIAS_RES_F32 (K-major A and B): out = s[row / rows_per_record] *
+ *      drop(acc + bias) + aux.  Other epilogues with path_p > 0 are rejected. */
+int ecgvit_gemm_drop_path(const ecgvit_gemm_args *g, float path_p, int path_stream, int rows_per_record, void *stream);
 
 /* ---- softmax attention on the packed projection: replaces chunk(3) + rearrange + q k^T * scale +
  *      Softmax + attn v + rearrange back (vit_pytorch Attention.forward).
@@ -295,6 +317,10 @@ int ecgvit_eval_metrics(const float *preds, const float *labels, int64_t n_rows,
  *      dym = mask * dy / (1 - p) (operand of the Linear's dgrad / wgrad), dcolsum += colsum(dym) (its bias gradient). */
 int ecgvit_dropout_bwd_copy(const void *dy, void *dym, float *dcolsum, int M, int N, int64_t ld, float dropout_p,
                             int dropout_stream, const uint32_t *dropout_seed, int dtype, void *stream);
+/* the same copy with drop path (see ecgvit_gemm_drop_path): dym = s[row / rows_per_record] * mask * dy; dropout_p may be 0 */
+int ecgvit_dropout_bwd_copy_drop_path(const void *dy, void *dym, float *dcolsum, int M, int N, int64_t ld,
+                                      float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int dtype,
+                                      float path_p, int path_stream, int rows_per_record, void *stream);
 
 /* ---- column sum  out[n] += sum_m x[m, n]   (bias gradients) */
 int ecgvit_colsum(const void *x, float *out, int M, int N, int64_t ld, int dtype, void *stream);
