@@ -54,9 +54,9 @@ int make_tmap(CUtensorMap *tm, const void *base, uint64_t inner, uint64_t outer,
     return 0;
 }
 
-// CTA pairs the persistent GEMM grid may use: all of them (SMs / 2) unless ecgvit_set_gemm_sm_budget() or the environment
-// variable ECGVIT_GEMM_CLUSTERS lowered it (data-parallel runs leave a few SMs to NCCL's collective kernels: a persistent
-// grid that cannot place its last CTAs runs a second, nearly empty wave)
+// CTA pairs the persistent GEMM grid may use: all of them (SMs / 2) unless the environment variable ECGVIT_GEMM_CLUSTERS,
+// read once at the first launch, lowered it (data-parallel runs leave a few SMs to NCCL's collective kernels: a
+// persistent grid that cannot place its last CTAs runs a second, nearly empty wave)
 int g_gemm_clusters = -1;
 int gemm_clusters() {
     if (g_gemm_clusters < 0) {
