@@ -97,6 +97,7 @@ SIGNATURES = {
     'ecgvit_token_mean_bwd': [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
     'ecgvit_colsum': [c_void_p, c_void_p, c_int, c_int, c_int64, c_int, c_void_p],
     'ecgvit_grad_sumsq': [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p],
+    'ecgvit_grad_sumsq_grouped': [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p, c_void_p],
     'ecgvit_grad_sumsq_partial': [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_int, c_int, c_void_p],
     'ecgvit_grad_sumsq_finalize': [c_void_p, c_int, c_void_p],
     'ecgvit_adamw_step': [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int,
@@ -135,7 +136,7 @@ def last_error():
 
 
 # kernels launched per successful entry-point call (memsets are not kernels); feeds bench.py's `gpu_launches`
-KERNELS_PER_CALL = {'layernorm_patch_bwd': 3, 'attention_bwd_flash': 3, 'head_fwd': 2, 'head_bwd': 3, 'layernorm_bwd': 2, 'layernorm_bwd_partial': 1, 'grad_sumsq': 2, 'eval_metrics': 3,
+KERNELS_PER_CALL = {'layernorm_patch_bwd': 3, 'attention_bwd_flash': 3, 'head_fwd': 2, 'head_bwd': 3, 'layernorm_bwd': 2, 'layernorm_bwd_partial': 1, 'grad_sumsq': 2, 'grad_sumsq_grouped': 2, 'eval_metrics': 3,
                     'embed_assemble_visible_bwd': 3, 'mae_unshuffle_bwd': 3}
 launch_counter = [0]
 

@@ -29,14 +29,21 @@ __device__ __forceinline__ float4 load_grad4(const bf16 *g, int64_t i) {
     return v;
 }
 
-template <typename TG>
+// group id of the 64-element blocks that neither count in the norm nor get updated (frozen / in no group)
+constexpr uint8_t ADAMW_UNGROUPED = 255;
+
+// kGrouped: gmap holds one group id per 64-element block of g (n is then a multiple of 64); blocks with id
+// ADAMW_UNGROUPED contribute nothing.  The partials and their order are those of the plain kernel.
+template <typename TG, bool kGrouped = false>
 __global__ void __launch_bounds__(256) grad_sumsq_kernel(const TG *__restrict__ g, int64_t n,
-                                                          const float *__restrict__ hyper, float *__restrict__ stats) {
+                                                          const float *__restrict__ hyper, float *__restrict__ stats,
+                                                          const uint8_t *__restrict__ gmap = nullptr) {
     __shared__ float red[8];
     const float gs = hyper[H_GSCALE];
     const int64_t n4 = n / 4;
     float s = 0.f;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+        if (kGrouped && __ldg(gmap + (i >> 4)) == ADAMW_UNGROUPED) continue;   // 16 float4 = one 64-element block
         const float4 v = load_grad4(g, i);
         const float a = v.x * gs, b = v.y * gs, c = v.z * gs, d = v.w * gs;
         s = fmaf(a, a, s); s = fmaf(b, b, s); s = fmaf(c, c, s); s = fmaf(d, d, s);
@@ -82,7 +89,6 @@ __device__ __forceinline__ float clip_coef_from(const float *hyper, const float 
 // flat buffers (every tensor starts on a 64-element boundary); gtable[2 * id] = 1 - lr_g * wd_g and
 // gtable[2 * id + 1] = lr_g / (1 - beta1^t) replace hyper's decay / step size; id ADAMW_UNGROUPED leaves p, m, v and
 // the shadow untouched.  Everything else (clip, skip, the non-finite counter, the update itself) is shared.
-constexpr uint8_t ADAMW_UNGROUPED = 255;
 
 template <bool kShadow, typename TG, bool kGrouped = false>
 __global__ void __launch_bounds__(256) adamw_kernel(float *__restrict__ p, float *__restrict__ m,
@@ -182,6 +188,26 @@ int ecgvit_grad_sumsq(const void *g, int grad_dtype, int64_t n, const float *hyp
     else
         grad_sumsq_kernel<bf16><<<grid, 256, 0, as_stream(stream)>>>((const bf16 *)g, n, hyper, stats);
     int rc = check_launch("grad_sumsq");
+    if (rc) return rc;
+    grad_sumsq_finalize_kernel<<<1, 256, 0, as_stream(stream)>>>(stats, grid);
+    return check_launch("grad_sumsq_finalize");
+}
+
+int ecgvit_grad_sumsq_grouped(const void *g, int grad_dtype, int64_t n, const uint8_t *group_map, const float *hyper,
+                              float *stats, void *stream) {
+    ECGVIT_REQUIRE(g && group_map && hyper && stats && n > 0, "grad_sumsq_grouped: bad arguments");
+    ECGVIT_REQUIRE(n % 64 == 0, "grad_sumsq_grouped: length %lld must be a multiple of 64 (one group id per 64 elements)",
+                   (long long)n);
+    ECGVIT_REQUIRE((reinterpret_cast<uintptr_t>(g) & 15) == 0, "grad_sumsq_grouped: g must be 16-byte aligned");
+    ECGVIT_REQUIRE(grad_dtype == ECGVIT_F32 || grad_dtype == ECGVIT_BF16, "grad_sumsq_grouped: unknown gradient dtype %d",
+                   grad_dtype);
+    int grid = flat_grid(n);
+    if (grid > SUMSQ_MAX_BLOCKS) grid = SUMSQ_MAX_BLOCKS;
+    if (grad_dtype == ECGVIT_F32)
+        grad_sumsq_kernel<float, true><<<grid, 256, 0, as_stream(stream)>>>((const float *)g, n, hyper, stats, group_map);
+    else
+        grad_sumsq_kernel<bf16, true><<<grid, 256, 0, as_stream(stream)>>>((const bf16 *)g, n, hyper, stats, group_map);
+    int rc = check_launch("grad_sumsq_grouped");
     if (rc) return rc;
     grad_sumsq_finalize_kernel<<<1, 256, 0, as_stream(stream)>>>(stats, grid);
     return check_launch("grad_sumsq_finalize");

@@ -47,6 +47,7 @@ class StepEngine:
         self.device = model._flat_p.device
         self._lw_key = self._lw_table = None
         self._spans = {}
+        self._frozen = frozenset()   # flat-buffer keys of the frozen parameters during a backward pass
         self.rng = torch.zeros(2, device=self.device, dtype=torch.int32)
         # Weight-gradient GEMMs do not feed the backward chain: issued on a side stream they become a parallel branch of
         # the step graph and fill the SMs that the chain's kernels leave idle (partial last waves, launch ramps,
@@ -109,13 +110,17 @@ class StepEngine:
             _lib.check(self.lib.ecgvit_gemm(ctypes.byref(g), self._stream), 'gemm')
 
     def workspace(self, B, L, n_vis=None):
-        """activations of one (batch, length) shape; n_vis: the patches the encoder sees per record (all when None)"""
-        key = (B, L, n_vis)
+        """activations of one (batch, length) shape; n_vis: the patches the encoder sees per record (all when None).
+        The encoder blocks below the lowest trainable one (`EcgVit.trainable_span`) share one activation set: backward
+        never reads them"""
+        m = self.model
+        c = m.config
+        lowest = m.trainable_span().lowest
+        n_frozen = c.num_hidden_layers if lowest is None else max(0, lowest)
+        key = (B, L, n_vis, n_frozen)
         w = self.ws.get(key)
         if w is not None:
             return w
-        m = self.model
-        c = m.config
         dev = m._flat_p.device
         T = m._act_dtype
         P, C, d, mlp = c.patch_size, c.num_channels, c.hidden_size, c.intermediate_size
@@ -150,7 +155,7 @@ class StepEngine:
         # and is recomputed from x[l] in backward.  Two sets, so that the weight-gradient GEMMs of layer l (side stream)
         # can still read their operands while layer l - 1 is being recomputed into the other set.
         ckpt = bool(getattr(c, 'activation_checkpointing', False)) and depth > 2
-        self._alloc_stack(w, 'l', B, N, d, mlp, H, depth, ckpt)
+        self._alloc_stack(w, 'l', B, N, d, mlp, H, depth, ckpt, n_frozen)
         # head
         n_class = m.num_class
         w.xn = buf(B, d, dtype=torch.float32)
@@ -167,10 +172,11 @@ class StepEngine:
         self.ws[key] = w
         return w
 
-    def _alloc_stack(self, s, prefix, B, N, d, mlp, H, depth, ckpt):
+    def _alloc_stack(self, s, prefix, B, N, d, mlp, H, depth, ckpt, n_frozen=0):
         """a block stack on the object s: `depth` blocks of width d over B sequences of N tokens, parameters keyed
-        `{prefix}{l}.`, its dims, activations and backward scratch.  Only the encoder stack (prefix 'l') calls the layer
-        hooks; p_blk is its block dropout probability and r_path its per-block drop-path rates, both set by the forward
+        `{prefix}{l}.`, its dims, activations and backward scratch.  Blocks l < n_frozen are never visited by backward:
+        they run through one shared activation set and two alternating inputs x[l], and only x[n_frozen] persists.  Only
+        the encoder stack (prefix 'l') calls the layer hooks; p_blk is its block dropout probability and r_path its per-block drop-path rates, both set by the forward
         pass (the encoder's; a decoder keeps zeros).  Drop-path site of branch j (0 attention, 1 feed-forward) of block l:
         path_site + 2 * l + j, after the dropout sites 0 .. 4 * depth and the mask site 4 * depth + 1."""
         m = self.model
@@ -188,12 +194,17 @@ class StepEngine:
             return torch.empty(*shape, device=dev, dtype=dtype)
 
         RT = m._res_dtype  # residual stream: fp32 for deep models in bf16 mode (config.residual_dtype)
-        s.x = [buf(M, d, dtype=RT) for _ in range(depth + 1)]  # x[l] = input of block l; x[depth] = stack output
-        n_sets = 2 if ckpt else depth
+        # x[l] = input of block l; x[depth] = stack output
+        xf = [buf(M, d, dtype=RT) for _ in range(min(n_frozen, 2))]
+        s.x = [xf[l % 2] for l in range(n_frozen)] + [buf(M, d, dtype=RT) for _ in range(n_frozen, depth + 1)]
+        shared = 1 if n_frozen > 0 and not ckpt else 0   # the set of the frozen blocks (checkpointing has two sets anyway)
+        n_sets = 2 if ckpt else depth - n_frozen + shared
 
         def per_layer(make):
             sets = [make() for _ in range(n_sets)]
-            return [sets[l % n_sets] for l in range(depth)]
+            if ckpt:
+                return [sets[l % 2] for l in range(depth)]
+            return [sets[0] if l < n_frozen else sets[l - n_frozen + shared] for l in range(depth)]
 
         s.ln1 = per_layer(lambda: buf(M, d))
         s.ln2 = per_layer(lambda: buf(M, d))
@@ -241,6 +252,7 @@ class StepEngine:
         pipe = m.input_pipeline
         L = L_in if pipe is None else pipe.padded_length(L_in)  # TimeEndPad happens inside the gather
         w = self.workspace(B, L)
+        w.span = m.trainable_span()   # what this pass's backward has to produce
         self._cur = w
         self._fwd_id += 1
         w.fwd_id = self._fwd_id   # a later forward through the same workspace invalidates this one's backward
@@ -409,8 +421,13 @@ class StepEngine:
         B, d = w.B, c.hidden_size
         depth = c.num_hidden_layers
         gr = m._grads_f32()
+        # frozen parameters (requires_grad=False): backward stops at the lowest trainable encoder position and skips the
+        # weight-gradient GEMMs of frozen weights; gradients outside [lo, n) are neither zeroed nor read
+        span = w.span
+        lowest = depth if span.lowest is None else span.lowest
+        self._frozen = span.frozen
         if zero_grads:
-            m._flat_g.zero_()
+            (m._flat_g if span.lo == 0 else m._flat_g[span.lo:]).zero_()
         last = f'l{depth - 1}.'
         top = (depth - 1) & 1
         # with dropout or drop path between net[3] / to_out[0] and the residual add, the Linear sees s * mask * dz / (1 - p):
@@ -418,12 +435,21 @@ class StepEngine:
         # gradient
         self._head_backward(w, w.dz[top], None if self._masked(w, depth - 1) else gr[last + 'ff2.b'], grad_scale,
                             grad_scale_dev)
-        self._stack_backward(w)
+        if lowest == depth:
+            # linear probe: the head's backward ends the chain (its gradient of the encoder output goes unused)
+            if m._after_layer_backward is not None:
+                m._after_layer_backward(depth)
+            return
+        self._stack_backward(w, max(lowest, 0))
+        if lowest > -1:
+            return
         dz = w.dz[(-1) & 1]   # gradient w.r.t. the token matrix (input of block 0)
         # ---- embedding: tok = [cls | a_emb We^T + be] + pos
         self._assemble_backward(w, dz)
         rows = B * w.n_vis
-        if w.Kp == w.K:
+        if 'embed.w' in self._frozen:
+            pass   # its weight-gradient GEMM is the only thing that reads `de` here
+        elif w.Kp == w.K:
             self._gemm(d, w.K, rows, w.de, d, 0, w.a_emb, w.K, 0, EPI_ATOMIC_F32, gr['embed.w'], w.K, split_k=0)
         else:
             w.embed_gpad.zero_()
@@ -439,10 +465,12 @@ class StepEngine:
         Linears then read a masked copy of the residual-stream gradient"""
         return s.p_blk > 0 or s.r_path[l] > 0
 
-    def _stack_backward(self, s):
-        """backward through the blocks of the stack s, from the gradient of its output in s.dz[(depth - 1) & 1] (its
-        column sum already added to the top ff2 bias gradient when the top block is not masked) to that of its input in
-        s.dz[1]; the weight gradients run on the side stream, which is joined at the end"""
+    def _stack_backward(self, s, l0=0):
+        """backward through the blocks l0 .. depth - 1 of the stack s, from the gradient of its output in
+        s.dz[(depth - 1) & 1] (its column sum already added to the top ff2 bias gradient when the top block is not masked)
+        to that of the input of block l0 in s.dz[(l0 - 1) & 1]; the weight gradients run on the side stream, which is
+        joined at the end.  The weight-gradient GEMMs (and FF1's bias column sum) of the parameters in self._frozen are
+        skipped."""
         m, lib, st = self.model, self.lib, self._stream
         dt = m._dtype_code
         rdt = m._res_code
@@ -474,6 +502,9 @@ class StepEngine:
                 done = torch.cuda.Event()
                 done.record(side)
             return done
+
+        def trains(key):
+            return key not in self._frozen
 
         def before_overwrite(ev):
             """the main stream may not overwrite a scratch buffer that a side-stream GEMM is still reading"""
@@ -521,7 +552,7 @@ class StepEngine:
                            'dropout_bwd_copy')
             else:
                 _lib.check(lib.ecgvit_dropout_bwd_copy(*args, st), 'dropout_bwd_copy')
-        for l in range(depth - 1, -1, -1):
+        for l in range(depth - 1, l0 - 1, -1):
             p = f'{s.prefix}{l}.'
             q, qn = l & 1, (l - 1) & 1      # buffer parity of this layer / of the layer below
             s_att, s_out, s_act, s_ff2 = 1 + 4 * l, 2 + 4 * l, 3 + 4 * l, 4 + 4 * l
@@ -536,12 +567,15 @@ class StepEngine:
             masked, r_l = self._masked(s, l), s.r_path[l]
             dzl = s.dzm[0][q] if masked else dz      # what net[3] saw: s * mask * dz / (1 - p)
             # ---- feed-forward branch: x[l+1] = y + drop(W2 drop(gelu(W1 ln2(y) + b1)) + b2)
-            e['ff2'] = wgrad(d, mlp, M, dzl, d, 0, s.h[l], mlp, 0, EPI_ATOMIC_F32, gr[p + 'ff2.w'], mlp, split_k=0)
+            if trains(p + 'ff2.w'):
+                e['ff2'] = wgrad(d, mlp, M, dzl, d, 0, s.h[l], mlp, 0, EPI_ATOMIC_F32, gr[p + 'ff2.w'], mlp, split_k=0)
             before_overwrite(old.get('ff1'))   # du of this parity
             self._gemm(M, mlp, d, dzl, d, 1, wt[p + 'ff2.w'], mlp, 0, EPI_DGELU, du, mlp, aux=s.u[l], drop=(p_blk, s_act))
             # FF1's bias gradient (column sums of du) feeds nothing in the chain: it rides on the side stream in front of
             # FF1's weight gradient (same operand, so the event that guards `du` covers both)
-            if side is None:
+            if not trains(p + 'ff1.b'):
+                pass
+            elif side is None:
                 _lib.check(lib.ecgvit_colsum(du.data_ptr(), gr[p + 'ff1.b'].data_ptr(), M, mlp, mlp, dt, st), 'colsum')
             else:
                 ready = torch.cuda.Event()
@@ -550,26 +584,31 @@ class StepEngine:
                 with torch.cuda.stream(side):
                     _lib.check(lib.ecgvit_colsum(du.data_ptr(), gr[p + 'ff1.b'].data_ptr(), M, mlp, mlp, dt,
                                                  side.cuda_stream), 'colsum')
-            e['ff1'] = wgrad(mlp, d, M, du, mlp, 0, s.ln2[l], d, 0, EPI_ATOMIC_F32, gr[p + 'ff1.w'], d, split_k=0)
+            if trains(p + 'ff1.w'):
+                e['ff1'] = wgrad(mlp, d, M, du, mlp, 0, s.ln2[l], d, 0, EPI_ATOMIC_F32, gr[p + 'ff1.w'], d, split_k=0)
             self._gemm(M, d, mlp, du, mlp, 1, wt[p + 'ff1.w'], d, 0, EPI_STORE, s.dln, d)
             before_overwrite(old.get('out'))   # dy / its masked copy of this parity
             dyl = s.dzm[1][q] if masked else dy
             layernorm_bwd(0, s.dln, s.y[l], pf[p + 'ln2.w'], s.stat2[l], dz, dy, gr[p + 'ln2.w'], gr[p + 'ln2.b'],
                           gr[p + 'out.b'], dyl if masked else None, p_blk, s_out, r_l, s.path_site + 2 * l)
             # ---- attention branch: y = x + s * drop(Wo attn(Wqkv ln1(x)) + bo); dyl = s * mask * dy / (1 - p)
-            e['out'] = wgrad(d, inner, M, dyl, d, 0, s.o[l], inner, 0, EPI_ATOMIC_F32, gr[p + 'out.w'], inner, split_k=0)
+            if trains(p + 'out.w'):
+                e['out'] = wgrad(d, inner, M, dyl, d, 0, s.o[l], inner, 0, EPI_ATOMIC_F32, gr[p + 'out.w'], inner,
+                                 split_k=0)
             self._gemm(M, inner, d, dyl, d, 1, wt[p + 'out.w'], inner, 0, EPI_STORE, s.d_o, inner)
             before_overwrite(old.get('qkv'))   # dqkv of this parity
             _lib.check(lib.ecgvit_attention_bwd(s.qkv[l].data_ptr(), s.o[l].data_ptr(), s.d_o.data_ptr(),
                                                 s.lse[l].data_ptr(), dqkv.data_ptr(), _lib.ptr(s.attn_scratch), B, N,
                                                 H, dh, scale, p_blk, s_att, blk_seed, dt, st),
                        'attention_bwd' if s.attn_scratch is None else 'attention_bwd_flash')
-            e['qkv'] = wgrad(3 * inner, d, M, dqkv, 3 * inner, 0, s.ln1[l], d, 0, EPI_ATOMIC_F32, gr[p + 'qkv.w'], d,
-                             split_k=0)
+            if trains(p + 'qkv.w'):
+                e['qkv'] = wgrad(3 * inner, d, M, dqkv, 3 * inner, 0, s.ln1[l], d, 0, EPI_ATOMIC_F32, gr[p + 'qkv.w'], d,
+                                 split_k=0)
             self._gemm(M, d, 3 * inner, dqkv, 3 * inner, 1, wt[p + 'qkv.w'], d, 0, EPI_STORE, s.dln, d)
-            below_bias = gr[f'{s.prefix}{l - 1}.ff2.b'] if l > 0 else None
-            drop_below = l > 0 and self._masked(s, l - 1)
-            r_below = s.r_path[l - 1] if l > 0 else 0.0
+            # the block below l0 gets no gradient: no bias pre-sum and no masked copy for it
+            below_bias = gr[f'{s.prefix}{l - 1}.ff2.b'] if l > l0 else None
+            drop_below = l > l0 and self._masked(s, l - 1)
+            r_below = s.r_path[l - 1] if l > l0 else 0.0
             # LayerNorm' writes the input gradient of layer l - 1 into the OTHER parity, last read by the ff2 weight
             # gradient of layer l + 1
             before_overwrite(evs.get(l + 1, {}).get('ff2'))

@@ -24,6 +24,24 @@ MaskedPatchOutput = namedtuple('MaskedPatchOutput', ['loss', 'reconstruction', '
 
 _ALIGN = 64  # elements: every tensor starts on a 256-byte boundary of the flat buffers
 
+# The trainable part of a model, derived from the `requires_grad` flags (`EcgVit.trainable_span`):
+#   lowest        lowest forward position holding a trainable parameter: -1 = patch embedding / pos / cls / mask token,
+#                 0 .. depth - 1 = encoder block, depth = everything above the encoder; None when nothing is trainable
+#   lo            flat offset of the first trainable tensor (the flat length when nothing is trainable)
+#   frozen_inside whether a frozen tensor lies in [lo, flat length)
+#   frozen        flat-buffer keys of the frozen tensors
+#   key           the flags themselves, in `named_parameters()` order (cache and graph key)
+TrainableSpan = namedtuple('TrainableSpan', ['lowest', 'lo', 'frozen_inside', 'frozen', 'key'])
+
+
+def _forward_position(key, depth):
+    """forward position of the flat-buffer key `key` (see TrainableSpan.lowest)"""
+    if key in ('pos', 'cls', 'mask') or key.startswith('embed.'):
+        return -1
+    if key[0] == 'l' and key[1].isdigit():
+        return int(key[1:key.index('.')])
+    return depth
+
 
 class _Slot(nn.Module):
     """parameter-free placeholder keeping vit_pytorch's child indices (Rearrange, GELU, Dropout...)"""
@@ -137,8 +155,8 @@ class _EcgVitFunction(torch.autograd.Function):
         # Gradients are produced straight into the flat fp32 buffer and `.grad` is pointed at its views, so the
         # clip / AdamW kernels later see one contiguous array (no per-tensor copies through AccumulateGrad).
         params, views = model._param_list(), model._grad_views()
-        # frozen parameters (requires_grad=False) never get a .grad, as with autograd; the kernels still write their slot
-        # of the flat buffer, which the optimizer front end ignores for them
+        # frozen parameters (requires_grad=False) never get a .grad, as with autograd; backward skips what only they need
+        # (trainable_span), and whatever a fused kernel still writes into their slot the optimizer front end ignores
         live = [(p, v) for p, v in zip(params, views) if p.requires_grad]
         ours = [p.grad is not None and p.grad.data_ptr() == v.data_ptr() for p, v in live]
         if all(ours):
@@ -373,6 +391,28 @@ class EcgVit(nn.Module):
     def _grad_views(self):
         names = self._short_names()
         return [self._views_g[k] for k in names.values()]
+
+    def trainable_span(self):
+        """`TrainableSpan` of the current `requires_grad` flags: what backward, the optimizers and the gradient exchange
+        have to cover.  The encoder is the bottom of every model, and the flat buffers follow forward order, so every
+        trainable tensor lies in [lo, flat length) and backward can stop at the lowest trainable encoder position."""
+        flags = tuple(p.requires_grad for p in self.parameters())
+        span = getattr(self, '_span_cache', None)
+        if span is not None and span.key == flags:
+            return span
+        layout, total = (self._layout, self._flat_p.numel()) if self._layout is not None else self._flat_layout()
+        keys = list(layout)
+        first = next((i for i, trains in enumerate(flags) if trains), None)
+        if first is None:
+            lowest, lo = None, total
+        else:
+            lo = layout[keys[first]][0]
+            lowest = _forward_position(keys[first], self.config.num_hidden_layers)
+        span = TrainableSpan(lowest=lowest, lo=lo,
+                             frozen_inside=first is not None and not all(flags[first:]),
+                             frozen=frozenset(k for k, trains in zip(keys, flags) if not trains), key=flags)
+        self._span_cache = span
+        return span
 
 
 def _recon_patch_dim(c):

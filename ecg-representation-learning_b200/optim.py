@@ -165,8 +165,9 @@ class FusedAdamW(torch.optim.Optimizer):
     not updated.  All groups share the constructor's betas and eps (a group with others raises `ValueError`).
 
     `state_dict()` / `load_state_dict()` carry the moments and the step count (as flat tensors under `state['flat']`),
-    so the usual `torch.save(optimizer.state_dict())` checkpoint resumes exactly.  Parameters whose `.grad` is None are
-    left untouched (value and moments), as torch.optim.AdamW leaves them."""
+    so the usual `torch.save(optimizer.state_dict())` checkpoint resumes exactly.  Parameters whose `.grad` is None
+    (frozen ones: requires_grad=False) are left untouched (value and moments), as torch.optim.AdamW leaves them: the
+    grouped kernel's map gives them id 255."""
 
     def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, param_groups=None):
         self.model = model
@@ -207,22 +208,19 @@ class FusedAdamW(torch.optim.Optimizer):
         loss = closure() if closure is not None else None
         model = self.model
         model._prepare(next(model.parameters()).device)
-        # parameters without a gradient keep their value and moments (torch skips them); they are rare (frozen tensors)
-        frozen = [k for (k, _), p in zip(model._layout.items(), model._param_list()) if p.grad is None]
+        # parameters without a gradient (frozen tensors) keep their value and moments, as torch skips them: the grouped
+        # kernel leaves them out through its map (one group when no groups were given)
+        no_grad = frozenset(name for name, p in model.named_parameters() if p.grad is None)
         g = _flat_grads(model)
         n = g.numel()
         self._ensure_moments(g)
-        keep = []
-        for k in frozen:
-            o, cnt, _, _ = model._layout[k]
-            keep.append((o, cnt, model._flat_p[o:o + cnt].clone(), self._m[o:o + cnt].clone(), self._v[o:o + cnt].clone()))
         grp = self.param_groups[0]
         self._step += 1
         hyper, stats = _scratch(model)
         b1, b2 = grp['betas']
         st = torch.cuda.current_stream().cuda_stream
-        if self._grouped:
-            self._grouped_step(g, stats, st)
+        if self._grouped or no_grad:
+            self._grouped_step(g, stats, st, no_grad)
         else:
             # max_norm 0: clipping is a separate call in the reference loop
             _upload(model, hyper, _lib.adamw_hyper(grp['lr'], b1, b2, grp['eps'], grp['weight_decay'], self._step, 0.0,
@@ -231,20 +229,16 @@ class FusedAdamW(torch.optim.Optimizer):
             _lib.check(_lib.load().ecgvit_adamw_step(model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(),
                                                      g.data_ptr(), _lib.F32, _lib.ptr(model._shadow), n,
                                                      hyper.data_ptr(), stats.data_ptr(), 0, st), 'adamw_step')
-        for o, cnt, p0, m0, v0 in keep:
-            model._flat_p[o:o + cnt].copy_(p0)
-            self._m[o:o + cnt].copy_(m0)
-            self._v[o:o + cnt].copy_(v0)
-        if keep:
-            model.sync_shadow(force=True)
         return loss
 
-    def _grouped_step(self, g, stats, st):
-        """ecgvit_adamw_step_grouped with every group's current lr / weight decay; the group map is rebuilt when the
-        membership or the flat layout changes"""
+    def _grouped_step(self, g, stats, st, no_grad):
+        """ecgvit_adamw_step_grouped with every group's current lr / weight decay and the parameters named in `no_grad`
+        at id 255; the group map is rebuilt when the membership, the parameters without a gradient or the flat layout
+        change"""
         model = self.model
         self._check_groups()
-        names = group_names(model, self.param_groups)
+        names = group_names(model, self.param_groups) if self._grouped else [tuple(n for n, _ in model.named_parameters())]
+        names = [tuple(n for n in row if n not in no_grad) for row in names]
         key = (tuple(names), model._flat_p.data_ptr())
         if self._gmap_key != key:
             self._gmap = group_map(model, names).to(model._flat_p.device)

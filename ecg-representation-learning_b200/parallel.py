@@ -13,22 +13,26 @@ import torch
 import torch.distributed as dist
 
 
-def bucket_slices(layer_offsets, total, depth, bucket_layers):
+def bucket_slices(layer_offsets, total, depth, bucket_layers, lowest=-1, span_lo=0):
     """[(trigger_layer, lo, hi)] in the order backward completes them.
 
     layer_offsets[l] = first element of layer l's parameters in the flat buffer (forward order); everything before
     layer 0 (pos, cls, patch embedding) belongs to trigger -1, everything after the last layer (head) to the first
-    bucket."""
+    bucket.  (lowest, span_lo): the trainable span (`EcgVit.trainable_span`); the buckets cover [span_lo, total) and
+    every trigger is a position that backward visits, the head's backward (trigger `depth`) when no encoder or
+    embedding parameter is trainable."""
     out = []
     hi = total
     l = depth
-    while l > 0:
-        lo_layer = max(0, l - bucket_layers)
-        lo = layer_offsets[lo_layer]
+    bottom = max(lowest, 0)
+    while l > bottom:
+        lo_layer = max(bottom, l - bucket_layers)
+        lo = max(span_lo, layer_offsets[lo_layer])
         out.append((lo_layer, lo, hi))
         hi = lo
         l = lo_layer
-    out.append((-1, 0, hi))
+    if lowest in (-1, depth):   # the embedding's bucket, or the head's alone
+        out.append((lowest, span_lo, hi))
     return [(t, lo, hi) for (t, lo, hi) in out if hi > lo]
 
 
@@ -37,14 +41,23 @@ class BucketedGradReducer:
         """bf16=True: every bucket is cast to bf16 (a contiguous slice of `flat_g16`) right before its all-reduce and the
         optimizer kernels read the reduced bf16 image; the fp32 buffer keeps receiving the split-K partial sums."""
         self.group = group
+        span = None
         if model is not None:
             flat_g = model._flat_g
             depth = model.config.num_hidden_layers
             layer_offsets = [model._layout[f'l{l}.ln1.w'][0] for l in range(depth)]
             model._after_layer_backward = self.on_layer_done
+            span = model.trainable_span()
+        self.span_key = None if span is None else span.key
         self.flat_g = flat_g
         self.flat_g16 = torch.empty(flat_g.numel(), device=flat_g.device, dtype=torch.bfloat16) if bf16 else None
-        self.slices = bucket_slices(layer_offsets, flat_g.numel(), depth, bucket_layers)
+        if span is None:
+            self.slices = bucket_slices(layer_offsets, flat_g.numel(), depth, bucket_layers)
+        else:
+            # buckets over the trainable span; a bucket that holds no trainable tensor is not exchanged
+            self.slices = bucket_slices(layer_offsets, flat_g.numel(), depth, bucket_layers, span.lowest, span.lo)
+            live = [o for k, (o, _, _, _) in model._layout.items() if k not in span.frozen]
+            self.slices = [(t, lo, hi) for (t, lo, hi) in self.slices if any(lo <= o < hi for o in live)]
         self.by_trigger = {t: (lo, hi) for (t, lo, hi) in self.slices}
         self.works = []
 

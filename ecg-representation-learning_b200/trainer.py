@@ -84,6 +84,10 @@ class FusedTrainer:
         self._reducer = None
         self.launches_per_step = None
         self._step_done = collections.deque(maxlen=2)
+        # the trainable span of the current step (`EcgVit.trainable_span`), and whether it runs the grouped kernels
+        self._span = None
+        self._grouped = param_groups is not None
+        self._gmap = self._gmap_key = None
         # param_groups (e.g. `param_groups_lrd(model)`): per group lr = learning_rate * schedule * lr_scale and its own
         # weight decay (the trainer's when the group has none); parameters in no group are not updated.  Without groups
         # the step issues exactly the ungrouped kernels
@@ -115,13 +119,11 @@ class FusedTrainer:
         if old is not None:
             self.exp_avg.copy_(old[0])
             self.exp_avg_sq.copy_(old[1])
-        # with groups, the group table sits right behind the 16-float hyper block: one upload per step feeds both
-        n_hyper = 16 + (2 * len(self.param_groups) if self.param_groups is not None else 0)
+        # with groups (or frozen tensors among the trainable ones: one group), the group table sits right behind the
+        # 16-float hyper block: one upload per step feeds both
+        n_hyper = 16 + 2 * (len(self.param_groups) if self.param_groups is not None else 1)
         self.hyper = torch.zeros(n_hyper, device=device, dtype=torch.float32)
-        self._gmap = None
-        if self.param_groups is not None:
-            from .optim import group_map
-            self._gmap = group_map(m, self._group_names).to(device)   # once per flat layout
+        self._gmap = self._gmap_key = None   # built per flat layout and requires_grad flags (`_plan`)
         self.stats = torch.zeros(_lib.STATS_FLOATS, device=device, dtype=torch.float32)
         self._flat_ptr = m._flat_p.data_ptr()
         self._graph = None   # a captured graph points at the old flat buffers
@@ -158,6 +160,28 @@ class FusedTrainer:
             m.sync_shadow(force=True)
         self._state_ready = True
 
+    def _plan(self):
+        """read the requires_grad flags: the trainable span and, when the grouped kernels run, the group map with the
+        frozen tensors at id 255 (no groups: one group at the trainer's lr / weight decay)"""
+        m = self.model
+        span = m.trainable_span()
+        if span.lowest is None:
+            raise ValueError('FusedTrainer: every parameter has requires_grad=False, there is nothing to train')
+        if span.frozen and self.defer_optimizer:
+            raise ValueError('FusedTrainer: defer_optimizer=True does not support frozen parameters '
+                             '(requires_grad=False); use the default defer_optimizer=False')
+        self._span = span
+        self._grouped = self.param_groups is not None or span.frozen_inside
+        if self._grouped and self._gmap_key != (span.key, self._flat_ptr):
+            from .optim import group_map
+            names = self._group_names if self.param_groups is not None else [tuple(v[3] for v in m._layout.values())]
+            frozen = {m._layout[k][3] for k in span.frozen}
+            self._gmap = group_map(m, [tuple(n for n in g if n not in frozen) for g in names]).to(m._flat_p.device)
+            self._gmap_key = (span.key, self._flat_ptr)
+        if self._reducer is not None and self._reducer.span_key != span.key:
+            from .parallel import BucketedGradReducer
+            self._reducer = BucketedGradReducer(m, self.group, self.bucket_layers, bf16=self._reducer.flat_g16 is not None)
+
     def current_lr(self):
         return self.lr * lr_multiplier(self.schedule, self.step_count, self.n_warmup, self.n_step)
 
@@ -166,23 +190,23 @@ class FusedTrainer:
         calls optimizer.step() for the t-th time); t None = nothing to apply (skip flag)"""
         b1, b2 = self.betas
         mg = self.max_grad_norm if self.max_grad_norm is not None else 0.0
+        groups = self.param_groups if self.param_groups is not None else [{'lr_scale': 1.0, 'weight_decay': None}]
         if t is None:
             vals = _lib.adamw_hyper(0.0, b1, b2, self.eps, self.wd, 1, mg, 1.0 / self.world, skip=True)
-            return vals if self.param_groups is None else vals + [1.0, 0.0] * len(self.param_groups)
+            return vals if not self._grouped else vals + [1.0, 0.0] * len(groups)
         lr = self.lr * lr_multiplier(self.schedule, t - 1, self.n_warmup, self.n_step)
         vals = _lib.adamw_hyper(lr, b1, b2, self.eps, self.wd, t, mg, 1.0 / self.world)
-        if self.param_groups is None:
+        if not self._grouped:
             return vals
         from .optim import group_table
-        return vals + group_table([lr * g['lr_scale'] for g in self.param_groups],
-                                  [self.wd if g['weight_decay'] is None else g['weight_decay'] for g in self.param_groups],
-                                  b1, t)
+        return vals + group_table([lr * g['lr_scale'] for g in groups],
+                                  [self.wd if g['weight_decay'] is None else g['weight_decay'] for g in groups], b1, t)
 
     def _adamw(self, p, m, v, g, g_code, shadow, lo, n, flags, stream):
         """AdamW over [lo, lo + n) of the flat buffers (the base pointers are passed; the slice offsets them)"""
         esz = 4 if g_code == _lib.F32 else 2
         args = (p + 4 * lo, m + 4 * lo, v + 4 * lo, g + esz * lo, g_code, None if shadow is None else shadow + 2 * lo, n)
-        if self.param_groups is None:
+        if not self._grouped:
             _lib.check(self.lib.ecgvit_adamw_step(*args, self.hyper.data_ptr(), self.stats.data_ptr(), flags, stream),
                        'adamw_step')
         else:
@@ -194,14 +218,14 @@ class FusedTrainer:
     def _upload_hyper(self):
         # immediate mode: this replay applies update step_count + 1; deferred mode: it applies the PENDING update (or none)
         vals = self._hyper_values(self._pending_step if self.defer_optimizer else self.step_count + 1)
-        if self._hyper_ring is None:
+        if self._hyper_ring is None or self._hyper_ring.bufs[0].numel() != len(vals):
             self._hyper_ring = _lib.PinnedRing(len(vals), torch.float32)
-        self._hyper_ring.upload(self.hyper, vals)  # asynchronous: the host keeps queueing steps ahead of the device
+        self._hyper_ring.upload(self.hyper[:len(vals)], vals)  # asynchronous: the host keeps queueing steps ahead of the device
 
     def _slice_norm(self, layer):
         """engine hook: the gradients of `layer` (and of everything above it) are final on the current stream"""
         s = self._norm_slices.get(layer)
-        if s is None:
+        if s is None or self._span.frozen:   # the sliced norm covers the whole buffer: off while anything is frozen
             return
         lo, hi, first, per = s
         m = self.model
@@ -214,6 +238,8 @@ class FusedTrainer:
         m, st = self.model, torch.cuda.current_stream().cuda_stream
         eng = m._engine
         side = eng.side_stream
+        # with a frozen prefix the memset, the norm and AdamW cover [lo, n) only
+        lo = self._span.lo
         if side is not None:
             # the 342 MB gradient memset does not depend on the forward pass: on the side stream it becomes a parallel
             # branch of the step graph and disappears behind the (tensor-bound) forward kernels
@@ -223,7 +249,7 @@ class FusedTrainer:
             side.wait_event(fork)  # after the previous step's AdamW / all-reduce, which read the gradients
             if not self.defer_optimizer:
                 with torch.cuda.stream(side):
-                    m._flat_g.zero_()
+                    (m._flat_g if lo == 0 else m._flat_g[lo:]).zero_()
                     zeroed = torch.cuda.Event()
                     zeroed.record(side)
         if self.defer_optimizer:
@@ -242,18 +268,25 @@ class FusedTrainer:
         # all-reduce ran in bf16
         g, g_code = (m._flat_g, _lib.F32) if self._reducer is None or self._reducer.flat_g16 is None \
             else (self._reducer.flat_g16, _lib.BF16)
-        if self._norm_slices is not None:
+        esz = 4 if g_code == _lib.F32 else 2
+        if self._norm_slices is not None and not self._span.frozen:
             if side is not None:   # the slice partials were issued on the side stream
                 done = torch.cuda.Event()
                 done.record(side)
                 main.wait_event(done)
             _lib.check(self.lib.ecgvit_grad_sumsq_finalize(self.stats.data_ptr(), self._norm_blocks, st), 'grad_sumsq_finalize')
+        elif self._grouped and self._span.frozen:
+            # frozen tensors (id 255 in the map) do not count in the norm
+            from .model import _ALIGN
+            _lib.check(self.lib.ecgvit_grad_sumsq_grouped(g.data_ptr() + esz * lo, g_code, n - lo,
+                                                          self._gmap.data_ptr() + lo // _ALIGN, self.hyper.data_ptr(),
+                                                          self.stats.data_ptr(), st), 'grad_sumsq_grouped')
         else:
-            _lib.check(self.lib.ecgvit_grad_sumsq(g.data_ptr(), g_code, n, self.hyper.data_ptr(), self.stats.data_ptr(), st),
-                       'grad_sumsq')
+            _lib.check(self.lib.ecgvit_grad_sumsq(g.data_ptr() + esz * lo, g_code, n - lo, self.hyper.data_ptr(),
+                                                  self.stats.data_ptr(), st), 'grad_sumsq')
         if not self.defer_optimizer:
             self._adamw(m._flat_p.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), g.data_ptr(), g_code,
-                        _lib.ptr(m._shadow), 0, n, 0, st)
+                        _lib.ptr(m._shadow), lo, n - lo, 0, st)
         return loss, logits
 
     # ---- deferred optimizer --------------------------------------------------------------------------------------
@@ -307,7 +340,8 @@ class FusedTrainer:
         if not self.defer_optimizer or self._pending_step is None or not self._state_ready:
             return
         t, self._pending_step = self._pending_step, None
-        self._hyper_ring.upload(self.hyper, self._hyper_values(t))
+        vals = self._hyper_values(t)
+        self._hyper_ring.upload(self.hyper[:len(vals)], vals)
         self._apply_update(torch.cuda.current_stream())
 
     def step(self, sample_values, labels=None, time_out_spans=None):
@@ -320,6 +354,7 @@ class FusedTrainer:
         if (labels is None) != pretrain:
             raise ValueError('a masked-patch model trains without labels' if pretrain else 'EcgVit.step needs labels')
         self._ensure_state(sample_values.device)
+        self._plan()
         self._upload_hyper()
         pipe = self.model.input_pipeline
         if pipe is not None and pipe.timeout is not None and self.model.training:
@@ -347,14 +382,16 @@ class FusedTrainer:
         cfg = self.model.config
         # everything the capture bakes in: shapes, loss weighting / reduction, train vs eval (dropout on or off and its
         # probabilities, the drop-path rates), the input pipeline, and the flat buffers the kernels point at
-        # (a masked-patch model: no labels, and its mask ratio sets how many patches the captured mask draw takes)
-        key = (tuple(sample_values.shape), None if labels is None else tuple(labels.shape),
+        # (a masked-patch model: no labels, and its mask ratio sets how many patches the captured mask draw takes) and the
+        # requires_grad flags (which backward kernels run, and over which span the optimizer does)
+        key = (self._span.key, tuple(sample_values.shape), None if labels is None else tuple(labels.shape),
                tuple(float(v) for v in lw) if lw else None,
                self.model.training, float(cfg.hidden_dropout_prob), float(cfg.attention_probs_dropout_prob),
                float(getattr(cfg, 'drop_path_rate', 0.0)),
                self.model.loss_reduction, self.model._flat_p.data_ptr(),
                None if pipe is None else (id(pipe), pipe.pad, pipe.timeout), getattr(self.model, 'mask_ratio', None),
-               None if self.param_groups is None else (tuple(self._group_names), self._gmap.data_ptr()))
+               None if self.param_groups is None else tuple(self._group_names),
+               None if self._gmap is None else self._gmap.data_ptr())
         if self._graph is None or self._graph_key != key:
             self._static_x = torch.empty_like(sample_values)
             self._static_y = None if labels is None else \

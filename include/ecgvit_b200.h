@@ -341,6 +341,11 @@ int ecgvit_colsum(const void *x, float *out, int M, int N, int64_t ld, int dtype
 /* `g` is the flat gradient buffer in `grad_dtype`: ECGVIT_F32, or ECGVIT_BF16 when a data-parallel run all-reduced the
  * gradients in bf16 (half the NVLink bytes; the moments and parameters stay fp32 either way). */
 int ecgvit_grad_sumsq(const void *g, int grad_dtype, int64_t n, const float *hyper, float *stats, void *stream);
+/* The same norm over the 64-element blocks whose id in group_map (device uint8[n / 64], the map of
+ * ecgvit_adamw_step_grouped) is not 255: frozen parameters and parameters in no group do not count.  n must be a
+ * multiple of 64; a slice offsets group_map by its first element / 64.  Same partials, finalize and determinism. */
+int ecgvit_grad_sumsq_grouped(const void *g, int grad_dtype, int64_t n, const uint8_t *group_map, const float *hyper,
+                              float *stats, void *stream);
 /* The same norm, slice by slice: every call reduces one slice of the gradient buffer into its own `n_blocks` partial
  * slots [first_block, first_block + n_blocks) of the stats scratch (2048 slots in all) and may run as soon as that slice
  * is final -- e.g. per layer beside the rest of backward -- in any order and on any stream; ecgvit_grad_sumsq_finalize
