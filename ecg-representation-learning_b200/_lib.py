@@ -104,8 +104,11 @@ SIGNATURES = {
                           c_void_p],
     'ecgvit_adamw_step_grouped': [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int64, c_void_p, c_void_p,
                                   c_void_p, c_void_p, c_int, c_void_p],
+    'ecgvit_adamw_step_ema': [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int64, c_void_p,
+                              c_void_p, c_void_p, c_void_p, c_int, c_void_p],
     'ecgvit_grad_scale_by_clip': [c_void_p, c_int64, c_void_p, c_void_p, c_void_p],
     'ecgvit_cast_f32_to_bf16': [c_void_p, c_void_p, c_int64, c_void_p],
+    'ecgvit_swap_f32_cast': [c_void_p, c_void_p, c_void_p, c_int64, c_void_p],
 }
 _RESTYPES = {'ecgvit_last_error': c_char_p, 'ecgvit_layernorm_bwd_scratch_floats': c_int64,
              'ecgvit_eval_metrics_scratch_bytes': c_int64, 'ecgvit_attention_bwd_scratch_floats': c_int64}
@@ -211,13 +214,13 @@ def mpm_mask(seed, B, n, k, site):
 ADAMW_SLICE, ADAMW_FIRST_SLICE = 1, 2
 
 
-def adamw_hyper(lr, beta1, beta2, eps, weight_decay, step, max_norm, grad_scale, skip=False):
-    """the 16-float `hyper` block of ecgvit_grad_sumsq / ecgvit_adamw_step (include/ecgvit_b200.h); derived scalars
-    are evaluated in double precision here, exactly where torch.optim.AdamW evaluates them"""
+def adamw_hyper(lr, beta1, beta2, eps, weight_decay, step, max_norm, grad_scale, skip=False, ema_rate=0.0):
+    """the 16-float `hyper` block of ecgvit_grad_sumsq / ecgvit_adamw_step[_ema] (include/ecgvit_b200.h); derived
+    scalars are evaluated in double precision here, exactly where torch.optim.AdamW evaluates them; `ema_rate` = 1 - d_t
+    of the weight moving average (slot 15, read by ecgvit_adamw_step_ema only)"""
     bc1, bc2 = 1.0 - beta1 ** step, 1.0 - beta2 ** step
-    vals = [lr, beta1, beta2, eps, weight_decay, bc1, bc2, max_norm, grad_scale,
-            1.0 - beta1, 1.0 - beta2, 1.0 - lr * weight_decay, lr / bc1, bc2 ** 0.5, 1.0 if skip else 0.0]
-    return vals + [0.0] * (16 - len(vals))
+    return [lr, beta1, beta2, eps, weight_decay, bc1, bc2, max_norm, grad_scale,
+            1.0 - beta1, 1.0 - beta2, 1.0 - lr * weight_decay, lr / bc1, bc2 ** 0.5, 1.0 if skip else 0.0, ema_rate]
 
 
 class PinnedRing:

@@ -844,6 +844,28 @@ __global__ void cast_f32_bf16_kernel(const float *__restrict__ src, bf16 *__rest
         for (int64_t i = n8 * 8; i < n; ++i) dst[i] = __float2bfloat16_rn(src[i]);
 }
 
+// a <-> b in place (the fp32 master weights and their moving average) and, when shadow is given, shadow = bf16(new a)
+// with the rounding of cast_f32_bf16_kernel, so swapping twice restores a, b and the shadow bit for bit
+__global__ void swap_f32_cast_kernel(float *__restrict__ a, float *__restrict__ b, bf16 *__restrict__ shadow,
+                                     int64_t n) {
+    const int64_t n8 = n / 8;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
+        float va[8], vb[8];
+        load8(a + i * 8, va);
+        load8(b + i * 8, vb);
+        store8(a + i * 8, vb);
+        store8(b + i * 8, va);
+        if (shadow) store8(shadow + i * 8, vb);
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0)
+        for (int64_t i = n8 * 8; i < n; ++i) {
+            const float t = a[i];
+            a[i] = b[i];
+            b[i] = t;
+            if (shadow) shadow[i] = __float2bfloat16_rn(a[i]);
+        }
+}
+
 inline int grid_for(int64_t work_items, int threads, int max_blocks_per_sm = 8) {
     int64_t g = (work_items + threads - 1) / threads;
     const int64_t cap = (int64_t)sm_count() * max_blocks_per_sm;
@@ -1402,6 +1424,17 @@ int ecgvit_cast_f32_to_bf16(const float *src, void *dst, int64_t n, void *stream
     const int grid = grid_for(n / 8 + 1, 256);
     cast_f32_bf16_kernel<<<grid, 256, 0, as_stream(stream)>>>(src, (bf16 *)dst, n);
     return check_launch("cast_f32_to_bf16");
+}
+
+int ecgvit_swap_f32_cast(float *a, float *b, void *shadow_bf16, int64_t n, void *stream) {
+    ECGVIT_REQUIRE(a && b && n >= 0, "swap_f32_cast: bad arguments");
+    ECGVIT_REQUIRE(((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) |
+                     reinterpret_cast<uintptr_t>(shadow_bf16)) & 15) == 0,
+                   "swap_f32_cast: a, b and the shadow must be 16-byte aligned");
+    if (n == 0) return 0;
+    const int grid = grid_for(n / 8 + 1, 256);
+    swap_f32_cast_kernel<<<grid, 256, 0, as_stream(stream)>>>(a, b, (bf16 *)shadow_bf16, n);
+    return check_launch("swap_f32_cast");
 }
 
 }  // extern "C"

@@ -2,7 +2,8 @@
 // live in one contiguous allocation, so "multi-tensor" is a single launch).
 // Replaces nn.utils.clip_grad_norm_(params, 1.0, error_if_nonfinite=True) (~300 launches) and
 // torch.optim.AdamW.step (~1.1 k launches) of /root/reference/ecg_transformer/models/train.py:281-282.
-// HBM-bound: 28 B/param algorithmic (p, m, v read+write, g read) + 2 B/param for the bf16 weight shadow.
+// HBM-bound: 28 B/param algorithmic (p, m, v read+write, g read) + 2 B/param for the bf16 weight shadow
+// (+ 8 B/param for the fused weight EMA: read + write).
 #include "common.cuh"
 
 namespace ecgvit {
@@ -10,7 +11,7 @@ namespace ecgvit {
 namespace {
 
 enum { H_LR = 0, H_BETA1, H_BETA2, H_EPS, H_WD, H_BC1, H_BC2, H_MAXNORM, H_GSCALE,
-       H_ONE_MINUS_B1, H_ONE_MINUS_B2, H_DECAY, H_STEP_SIZE, H_BC2_SQRT, H_SKIP };
+       H_ONE_MINUS_B1, H_ONE_MINUS_B2, H_DECAY, H_STEP_SIZE, H_BC2_SQRT, H_SKIP, H_EMA_RATE };
 enum { S_SUMSQ = 0, S_NONFINITE, S_NORM, S_SKIPPED };
 
 // Stage 1: one partial sum of squares per CTA (fixed grid-stride order inside the CTA).
@@ -89,14 +90,18 @@ __device__ __forceinline__ float clip_coef_from(const float *hyper, const float 
 // flat buffers (every tensor starts on a 64-element boundary); gtable[2 * id] = 1 - lr_g * wd_g and
 // gtable[2 * id + 1] = lr_g / (1 - beta1^t) replace hyper's decay / step size; id ADAMW_UNGROUPED leaves p, m, v and
 // the shadow untouched.  Everything else (clip, skip, the non-finite counter, the update itself) is shared.
+// kEma: after the update, ema += hyper[H_EMA_RATE] * (p_new - ema) from the registers holding p_new (the rate 1 - d_t
+// is derived by the host in double precision).  Whatever leaves p untouched (skip, non-finite norm, id 255) leaves the
+// EMA untouched too.
 
-template <bool kShadow, typename TG, bool kGrouped = false>
+template <bool kShadow, typename TG, bool kGrouped = false, bool kEma = false>
 __global__ void __launch_bounds__(256) adamw_kernel(float *__restrict__ p, float *__restrict__ m,
                                                      float *__restrict__ v, const TG *__restrict__ g,
                                                      bf16 *__restrict__ shadow, int64_t n,
                                                      const float *__restrict__ hyper, float *__restrict__ stats,
                                                      bool count_skips, const uint8_t *__restrict__ gmap = nullptr,
-                                                     const float *__restrict__ gtable = nullptr) {
+                                                     const float *__restrict__ gtable = nullptr,
+                                                     float *__restrict__ ema = nullptr) {
     if (hyper[H_SKIP] != 0.f) return;   // a deferred-update slot with nothing pending (first step, or just flushed)
     float total_norm;
     const float clip = clip_coef_from(hyper, stats, total_norm);
@@ -113,6 +118,7 @@ __global__ void __launch_bounds__(256) adamw_kernel(float *__restrict__ p, float
     const float one_m_b1 = hyper[H_ONE_MINUS_B1], one_m_b2 = hyper[H_ONE_MINUS_B2];
     float decay = hyper[H_DECAY], step_size = hyper[H_STEP_SIZE];
     const float bc2_sqrt = hyper[H_BC2_SQRT];
+    const float ema_rate = kEma ? hyper[H_EMA_RATE] : 0.f;
     const float gmul = hyper[H_GSCALE] * clip;
     const int64_t n4 = n / 4;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
@@ -145,7 +151,31 @@ __global__ void __launch_bounds__(256) adamw_kernel(float *__restrict__ p, float
             u.y = pack_bf16x2(pp[2], pp[3]);
             reinterpret_cast<uint2 *>(shadow)[i] = u;
         }
+        if (kEma) {
+            float4 e4 = reinterpret_cast<float4 *>(ema)[i];
+            e4.x = fmaf(ema_rate, pp[0] - e4.x, e4.x);
+            e4.y = fmaf(ema_rate, pp[1] - e4.y, e4.y);
+            e4.z = fmaf(ema_rate, pp[2] - e4.z, e4.z);
+            e4.w = fmaf(ema_rate, pp[3] - e4.w, e4.w);
+            reinterpret_cast<float4 *>(ema)[i] = e4;
+        }
     }
+}
+
+template <bool kShadow, typename TG, bool kGrouped>
+void launch_adamw_ema(int grid, cudaStream_t s, float *p, float *m, float *v, const void *g, void *shadow, int64_t n,
+                      const float *hyper, float *stats, bool count, const uint8_t *gmap, const float *gtable,
+                      float *ema) {
+    adamw_kernel<kShadow, TG, kGrouped, true><<<grid, 256, 0, s>>>(p, m, v, (const TG *)g, (bf16 *)shadow, n, hyper,
+                                                                    stats, count, gmap, gtable, ema);
+}
+
+template <bool kShadow, typename TG>
+void launch_adamw_ema(bool grouped, int grid, cudaStream_t s, float *p, float *m, float *v, const void *g, void *shadow,
+                      int64_t n, const float *hyper, float *stats, bool count, const uint8_t *gmap, const float *gtable,
+                      float *ema) {
+    if (grouped) launch_adamw_ema<kShadow, TG, true>(grid, s, p, m, v, g, shadow, n, hyper, stats, count, gmap, gtable, ema);
+    else launch_adamw_ema<kShadow, TG, false>(grid, s, p, m, v, g, shadow, n, hyper, stats, count, nullptr, nullptr, ema);
 }
 
 __global__ void __launch_bounds__(256) grad_scale_kernel(float *__restrict__ g, int64_t n,
@@ -288,6 +318,36 @@ int ecgvit_adamw_step_grouped(float *p, float *m, float *v, const void *g, int g
         else adamw_kernel<false, bf16, true><<<grid, 256, 0, s>>>(p, m, v, (const bf16 *)g, nullptr, n, hyper, stats, count, gm, gt);
     }
     return check_launch("adamw_step_grouped");
+}
+
+int ecgvit_adamw_step_ema(float *p, float *m, float *v, const void *g, int grad_dtype, void *shadow_bf16, float *ema,
+                          int64_t n, const uint8_t *group_map, const float *group_table, const float *hyper,
+                          float *stats, int flags, void *stream) {
+    const bool grouped = group_map != nullptr;
+    ECGVIT_REQUIRE(p && m && v && g && ema && hyper && stats && n > 0, "adamw_step_ema: bad arguments");
+    ECGVIT_REQUIRE(!grouped || group_table, "adamw_step_ema: a group map needs a group table");
+    ECGVIT_REQUIRE(n % (grouped ? 64 : 4) == 0, "adamw_step_ema: length %lld must be a multiple of %d%s", (long long)n,
+                   grouped ? 64 : 4, grouped ? " (one group id per 64 elements)" : " (pad the flat buffer)");
+    ECGVIT_REQUIRE(((reinterpret_cast<uintptr_t>(p) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(v) |
+                     reinterpret_cast<uintptr_t>(g) | reinterpret_cast<uintptr_t>(ema)) & 15) == 0,
+                   "adamw_step_ema: buffers must be 16-byte aligned");
+    ECGVIT_REQUIRE(grad_dtype == ECGVIT_F32 || grad_dtype == ECGVIT_BF16, "adamw_step_ema: unknown gradient dtype %d",
+                   grad_dtype);
+    cudaStream_t s = as_stream(stream);
+    const bool slice = (flags & ECGVIT_ADAMW_SLICE) != 0;
+    const bool count = !slice || (flags & ECGVIT_ADAMW_FIRST_SLICE) != 0;
+    const int grid = slice ? (int)((n / 4 + 255) / 256) : flat_grid(n);
+    void *sh = shadow_bf16;
+    const uint8_t *gm = group_map;
+    const float *gt = group_table;
+    if (grad_dtype == ECGVIT_F32) {
+        if (sh) launch_adamw_ema<true, float>(grouped, grid, s, p, m, v, g, sh, n, hyper, stats, count, gm, gt, ema);
+        else launch_adamw_ema<false, float>(grouped, grid, s, p, m, v, g, nullptr, n, hyper, stats, count, gm, gt, ema);
+    } else {
+        if (sh) launch_adamw_ema<true, bf16>(grouped, grid, s, p, m, v, g, sh, n, hyper, stats, count, gm, gt, ema);
+        else launch_adamw_ema<false, bf16>(grouped, grid, s, p, m, v, g, nullptr, n, hyper, stats, count, gm, gt, ema);
+    }
+    return check_launch("adamw_step_ema");
 }
 
 int ecgvit_grad_scale_by_clip(float *g, int64_t n, const float *hyper, float *stats, void *stream) {

@@ -8,7 +8,9 @@
 
 keeps working unchanged while each of clip / step is one or two kernel launches instead of ~1.4 k.
 """
+import contextlib
 import math
+from collections import OrderedDict
 
 import torch
 
@@ -100,6 +102,99 @@ def group_table(lrs, weight_decays, beta1, step):
     return out
 
 
+class WeightEma:
+    """The exponential moving average of a model's weights that `FusedTrainer` and `FusedAdamW` update inside their AdamW
+    kernel (`ecgvit_adamw_step_ema`): a flat fp32 buffer shaped like `model._flat_p`.  After the AdamW update of
+    optimizer step t (1-based, the step of AdamW's bias correction) has written p_t,
+
+        ema <- ema + (1 - d_t) * (p_t - ema),    d_t = decay,  or with warmup  d_t = min(decay, (1 + t) / (10 + t))
+
+    (the `num_updates` form of TensorFlow's `ExponentialMovingAverage`).  The buffer starts as a copy of the weights
+    when the optimizer state is created (the first step).  Exactly the elements the step updates are averaged: frozen
+    tensors and skipped updates leave it untouched."""
+
+    def __init__(self, decay, warmup=False):
+        if warmup and decay is None:
+            raise ValueError('ema_warmup=True needs ema_decay')
+        if not 0.0 < float(decay) < 1.0:
+            raise ValueError(f'ema_decay must lie in (0, 1), got {decay!r}')
+        self.decay, self.warmup = float(decay), bool(warmup)
+        self.buf = None
+        self.active = False    # inside `weights()`
+        self.swapped = False   # ... and the model holds the average, `buf` the trained weights
+
+    @classmethod
+    def create(cls, decay, warmup):
+        """None without EMA (`ema_decay=None`); raises on a decay outside (0, 1) or a warm-up without a decay"""
+        if decay is None and not warmup:
+            return None
+        return cls(decay, warmup)
+
+    def decay_at(self, t):
+        return min(self.decay, (1.0 + t) / (10.0 + t)) if self.warmup else self.decay
+
+    def rate(self, t):
+        """hyper[15] of optimizer step t: 1 - d_t in double precision"""
+        return 1.0 - self.decay_at(t)
+
+    def ensure(self, flat_p):
+        """create the buffer from the weights (first step), or move it to the weights' device; keeps a buffer of the same
+        length (loaded before the first step, or the model re-flattened its parameters)"""
+        if self.buf is not None and self.buf.numel() == flat_p.numel() and self.buf.device == flat_p.device:
+            return
+        old = self.buf
+        self.buf = flat_p.detach().clone()
+        if old is not None and old.numel() == flat_p.numel():
+            self.buf.copy_(old)
+
+    def check_inactive(self, what):
+        if self.active:
+            raise RuntimeError(f'{what} inside ema_weights(): leave the context first')
+
+    def average(self, model):
+        """the flat tensor that holds the average right now (None before the first step)"""
+        return model._flat_p if self.swapped else self.buf
+
+    @contextlib.contextmanager
+    def weights(self, model):
+        """the model's weights (fp32 master and bf16 shadow) are the average inside the context, and bit-identical to
+        before on exit; `ecgvit_swap_f32_cast` exchanges the two buffers in place and re-casts the shadow in one pass.
+        Before the first step the average is the weights themselves and nothing is swapped."""
+        if self.active:
+            raise RuntimeError('ema_weights() is already active: it does not nest')
+        swap = self.buf is not None
+        if swap:
+            self._swap(model)
+        self.active, self.swapped = True, swap
+        try:
+            yield
+        finally:
+            if swap:
+                self._swap(model)
+            self.active = self.swapped = False
+
+    def _swap(self, model):
+        _lib.check(_lib.load().ecgvit_swap_f32_cast(model._flat_p.data_ptr(), self.buf.data_ptr(), _lib.ptr(model._shadow),
+                                                    self.buf.numel(), torch.cuda.current_stream().cuda_stream),
+                   'swap_f32_cast')
+
+    def state_dict(self, model):
+        """the average in the model's own `state_dict()` keys (loads with strict=True into the same model class)"""
+        sd = model.state_dict()
+        avg = self.average(model)
+        if avg is None or self.swapped:
+            return OrderedDict((k, v.detach().clone()) for k, v in sd.items())
+        for o, n, shape, name in model._layout.values():
+            sd[name] = avg[o:o + n].view(shape).clone()
+        return sd
+
+    def load(self, model, flat):
+        """the buffer from a checkpoint's flat tensor, or from the current weights when the checkpoint has none"""
+        self.check_inactive('loading a checkpoint')
+        self.ensure(model._flat_p)
+        self.buf.copy_(model._flat_p if flat is None else flat)
+
+
 def _flat_grads(model):
     """make `model._flat_g` hold the current `.grad` of every parameter and return it"""
     views = model._grad_views()
@@ -167,9 +262,16 @@ class FusedAdamW(torch.optim.Optimizer):
     `state_dict()` / `load_state_dict()` carry the moments and the step count (as flat tensors under `state['flat']`),
     so the usual `torch.save(optimizer.state_dict())` checkpoint resumes exactly.  Parameters whose `.grad` is None
     (frozen ones: requires_grad=False) are left untouched (value and moments), as torch.optim.AdamW leaves them: the
-    grouped kernel's map gives them id 255."""
+    grouped kernel's map gives them id 255.
 
-    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, param_groups=None):
+    `ema_decay` (in (0, 1); None = no average) keeps an exponential moving average of the weights, updated by the AdamW
+    kernel itself (`WeightEma`: ema <- ema + (1 - d_t) * (p_t - ema), d_t = ema_decay, or with `ema_warmup=True`
+    min(ema_decay, (1 + t) / (10 + t))).  `ema_weights()` puts it into the model for evaluation or saving,
+    `ema_state_dict()` returns it in the model's keys, and `state_dict()['flat']['ema']` carries it."""
+
+    def __init__(self, model, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2, param_groups=None,
+                 ema_decay=None, ema_warmup=False):
+        self.ema = WeightEma.create(ema_decay, ema_warmup)
         self.model = model
         self._grouped = param_groups is not None
         params = model.parameters()
@@ -205,6 +307,8 @@ class FusedAdamW(torch.optim.Optimizer):
 
     @torch.no_grad()
     def step(self, closure=None):
+        if self.ema is not None:
+            self.ema.check_inactive('step()')
         loss = closure() if closure is not None else None
         model = self.model
         model._prepare(next(model.parameters()).device)
@@ -214,6 +318,8 @@ class FusedAdamW(torch.optim.Optimizer):
         g = _flat_grads(model)
         n = g.numel()
         self._ensure_moments(g)
+        if self.ema is not None:
+            self.ema.ensure(model._flat_p)
         grp = self.param_groups[0]
         self._step += 1
         hyper, stats = _scratch(model)
@@ -224,12 +330,20 @@ class FusedAdamW(torch.optim.Optimizer):
         else:
             # max_norm 0: clipping is a separate call in the reference loop
             _upload(model, hyper, _lib.adamw_hyper(grp['lr'], b1, b2, grp['eps'], grp['weight_decay'], self._step, 0.0,
-                                                   1.0))
+                                                   1.0, ema_rate=self._ema_rate()))
             stats.zero_()
-            _lib.check(_lib.load().ecgvit_adamw_step(model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(),
-                                                     g.data_ptr(), _lib.F32, _lib.ptr(model._shadow), n,
-                                                     hyper.data_ptr(), stats.data_ptr(), 0, st), 'adamw_step')
+            args = (model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(), g.data_ptr(), _lib.F32,
+                    _lib.ptr(model._shadow))
+            if self.ema is None:
+                _lib.check(_lib.load().ecgvit_adamw_step(*args, n, hyper.data_ptr(), stats.data_ptr(), 0, st),
+                           'adamw_step')
+            else:
+                _lib.check(_lib.load().ecgvit_adamw_step_ema(*args, self.ema.buf.data_ptr(), n, None, None,
+                                                             hyper.data_ptr(), stats.data_ptr(), 0, st), 'adamw_step_ema')
         return loss
+
+    def _ema_rate(self):
+        return 0.0 if self.ema is None else self.ema.rate(self._step)
 
     def _grouped_step(self, g, stats, st, no_grad):
         """ecgvit_adamw_step_grouped with every group's current lr / weight decay and the parameters named in `no_grad`
@@ -244,7 +358,7 @@ class FusedAdamW(torch.optim.Optimizer):
             self._gmap = group_map(model, names).to(model._flat_p.device)
             self._gmap_key = key
         b1, b2 = self.defaults['betas']
-        vals = _lib.adamw_hyper(0.0, b1, b2, self.defaults['eps'], 0.0, self._step, 0.0, 1.0)
+        vals = _lib.adamw_hyper(0.0, b1, b2, self.defaults['eps'], 0.0, self._step, 0.0, 1.0, ema_rate=self._ema_rate())
         vals += group_table([grp['lr'] for grp in self.param_groups], [grp['weight_decay'] for grp in self.param_groups],
                             b1, self._step)
         if self._ghyper is None or self._ghyper.numel() != len(vals) or self._ghyper.device != g.device:
@@ -252,10 +366,24 @@ class FusedAdamW(torch.optim.Optimizer):
             self._gring = _lib.PinnedRing(len(vals), torch.float32)
         self._gring.upload(self._ghyper, vals)   # hyper block, then the group table right behind it
         stats.zero_()
-        _lib.check(_lib.load().ecgvit_adamw_step_grouped(
-            model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(), g.data_ptr(), _lib.F32,
-            _lib.ptr(model._shadow), g.numel(), self._gmap.data_ptr(), self._ghyper.data_ptr() + 64,
-            self._ghyper.data_ptr(), stats.data_ptr(), 0, st), 'adamw_step_grouped')
+        args = (model._flat_p.data_ptr(), self._m.data_ptr(), self._v.data_ptr(), g.data_ptr(), _lib.F32,
+                _lib.ptr(model._shadow))
+        tail = (g.numel(), self._gmap.data_ptr(), self._ghyper.data_ptr() + 64, self._ghyper.data_ptr(),
+                stats.data_ptr(), 0, st)
+        if self.ema is None:
+            _lib.check(_lib.load().ecgvit_adamw_step_grouped(*args, *tail), 'adamw_step_grouped')
+        else:
+            _lib.check(_lib.load().ecgvit_adamw_step_ema(*args, self.ema.buf.data_ptr(), *tail), 'adamw_step_ema')
+
+    # ---- the weight moving average ----
+    def ema_weights(self):
+        """context manager: inside it the model's weights are the moving average (`WeightEma.weights`); `step()`
+        inside it and nesting it raise `RuntimeError`"""
+        return _require_ema(self.ema).weights(self.model)
+
+    def ema_state_dict(self):
+        """the moving average in the model's `state_dict()` keys"""
+        return _require_ema(self.ema).state_dict(self.model)
 
     # ---- checkpointing: torch.optim.Optimizer.state is empty here (the moments are flat), so carry them explicitly ----
     def state_dict(self):
@@ -263,6 +391,9 @@ class FusedAdamW(torch.optim.Optimizer):
         sd['flat'] = {'step': self._step,
                       'exp_avg': None if self._m is None else self._m.detach().clone(),
                       'exp_avg_sq': None if self._v is None else self._v.detach().clone()}
+        if self.ema is not None:
+            avg = self.ema.average(self.model)
+            sd['flat']['ema'] = None if avg is None else avg.detach().clone()
         return sd
 
     def load_state_dict(self, state_dict):
@@ -277,3 +408,17 @@ class FusedAdamW(torch.optim.Optimizer):
                 self._v = flat['exp_avg_sq'].detach().to(device=dev, dtype=torch.float32).clone()
             else:
                 self._m = self._v = None
+            if self.ema is not None:
+                self.ema.check_inactive('load_state_dict()')
+                ema = flat.get('ema')
+                if ema is not None:
+                    self.ema.buf = ema.detach().to(device=next(self.model.parameters()).device,
+                                                   dtype=torch.float32).clone()
+                elif self.ema.buf is not None:   # no average in the checkpoint: start it from the loaded weights
+                    self.ema.load(self.model, None)
+
+
+def _require_ema(ema):
+    if ema is None:
+        raise ValueError('the optimizer keeps no weight moving average: pass ema_decay=...')
+    return ema

@@ -12,12 +12,14 @@ flag polled on request.  With `world_size > 1` gradients are summed over NCCL in
 stream while backward is still running (`parallel.py`).
 """
 import collections
+import contextlib
 import math
 import os
 
 import torch
 
 from . import _lib
+from .optim import WeightEma
 
 
 
@@ -47,10 +49,17 @@ def get_train_args(args=None, n_train=None):
 
 
 class FusedTrainer:
+    """`ema_decay` (in (0, 1); None = no average) keeps an exponential moving average of the weights, updated inside
+    the AdamW kernel after every update (`optim.WeightEma`): ema <- ema + (1 - d_t) * (p_t - ema) with d_t = ema_decay,
+    or with `ema_warmup=True` d_t = min(ema_decay, (1 + t) / (10 + t)), t the 1-based optimizer step.  `ema_weights()`
+    evaluates or saves it, `fit` evaluates it next to the weights (`eval_ema/*`) and `save()` writes
+    `model_ema - <tag>.pt`."""
+
     def __init__(self, model, learning_rate=3e-4, weight_decay=1e-2, betas=(0.9, 0.999), eps=1e-8,
                  schedule='constant', n_warmup=0, n_step=1 << 30, max_grad_norm=1.0, process_group=None,
                  bucket_layers=1, use_cuda_graph=False, data_parallel=True, grad_reduce_dtype='auto',
-                 defer_optimizer=False, param_groups=None):
+                 defer_optimizer=False, param_groups=None, ema_decay=None, ema_warmup=False):
+        self.ema = WeightEma.create(ema_decay, ema_warmup)
         self.model = model
         self._flat_ptr = None
         self.lr, self.wd, self.betas, self.eps = learning_rate, weight_decay, betas, eps
@@ -119,6 +128,8 @@ class FusedTrainer:
         if old is not None:
             self.exp_avg.copy_(old[0])
             self.exp_avg_sq.copy_(old[1])
+        if self.ema is not None:
+            self.ema.ensure(m._flat_p)   # first use: the average starts from the weights
         # with groups (or frozen tensors among the trainable ones: one group), the group table sits right behind the
         # 16-float hyper block: one upload per step feeds both
         n_hyper = 16 + 2 * (len(self.param_groups) if self.param_groups is not None else 1)
@@ -152,7 +163,7 @@ class FusedTrainer:
             # replicas must start from the same weights and optimizer state whatever each rank's RNG or checkpoint did
             # (torch DDP broadcasts at construction too): rank 0 wins
             src = dist.get_global_rank(self.group, 0) if self.group is not None else 0
-            for t in (m._flat_p, self.exp_avg, self.exp_avg_sq):
+            for t in (m._flat_p, self.exp_avg, self.exp_avg_sq) + (() if self.ema is None else (self.ema.buf,)):
                 dist.broadcast(t, src=src, group=self.group)
             cnt = torch.tensor([self.step_count], device=device, dtype=torch.int64)
             dist.broadcast(cnt, src=src, group=self.group)
@@ -195,7 +206,8 @@ class FusedTrainer:
             vals = _lib.adamw_hyper(0.0, b1, b2, self.eps, self.wd, 1, mg, 1.0 / self.world, skip=True)
             return vals if not self._grouped else vals + [1.0, 0.0] * len(groups)
         lr = self.lr * lr_multiplier(self.schedule, t - 1, self.n_warmup, self.n_step)
-        vals = _lib.adamw_hyper(lr, b1, b2, self.eps, self.wd, t, mg, 1.0 / self.world)
+        vals = _lib.adamw_hyper(lr, b1, b2, self.eps, self.wd, t, mg, 1.0 / self.world,
+                                ema_rate=0.0 if self.ema is None else self.ema.rate(t))
         if not self._grouped:
             return vals
         from .optim import group_table
@@ -206,7 +218,13 @@ class FusedTrainer:
         """AdamW over [lo, lo + n) of the flat buffers (the base pointers are passed; the slice offsets them)"""
         esz = 4 if g_code == _lib.F32 else 2
         args = (p + 4 * lo, m + 4 * lo, v + 4 * lo, g + esz * lo, g_code, None if shadow is None else shadow + 2 * lo, n)
-        if not self._grouped:
+        if self.ema is not None:
+            from .model import _ALIGN
+            gm, gt = (self._gmap.data_ptr() + lo // _ALIGN, self.hyper.data_ptr() + 64) if self._grouped else (None, None)
+            _lib.check(self.lib.ecgvit_adamw_step_ema(*args[:6], self.ema.buf.data_ptr() + 4 * lo, n, gm, gt,
+                                                      self.hyper.data_ptr(), self.stats.data_ptr(), flags, stream),
+                       'adamw_step_ema')
+        elif not self._grouped:
             _lib.check(self.lib.ecgvit_adamw_step(*args, self.hyper.data_ptr(), self.stats.data_ptr(), flags, stream),
                        'adamw_step')
         else:
@@ -350,6 +368,8 @@ class FusedTrainer:
         The returned tensors are views of workspace buffers: valid until the next step.  With an `input_pipeline` on
         the model, `sample_values` are raw records; `time_out_spans` as in `EcgVit.forward`.
         An `EcgVitForMaskedPatchModeling` takes no labels (its masks are drawn on the device) and returns (loss, None)."""
+        if self.ema is not None:
+            self.ema.check_inactive('step()')
         pretrain = getattr(self.model, 'mask_ratio', None) is not None
         if (labels is None) != pretrain:
             raise ValueError('a masked-patch model trains without labels' if pretrain else 'EcgVit.step needs labels')
@@ -403,13 +423,16 @@ class FusedTrainer:
             # parameters/optimizer state are snapshotted so the warm-up does not count as a step
             self.flush()   # the warm-up below must not apply a pending update twice
             self._upload_hyper()
-            snap = (self.model._flat_p.clone(), self.exp_avg.clone(), self.exp_avg_sq.clone())
+            snap = (self.model._flat_p.clone(), self.exp_avg.clone(), self.exp_avg_sq.clone(),
+                    None if self.ema is None else self.ema.buf.clone())
             s = torch.cuda.Stream()
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
                 self._device_step(self._static_x, self._static_y)
             torch.cuda.current_stream().wait_stream(s)
             self.model._flat_p.copy_(snap[0]); self.exp_avg.copy_(snap[1]); self.exp_avg_sq.copy_(snap[2])
+            if self.ema is not None:
+                self.ema.buf.copy_(snap[3])
             self.model.sync_shadow(force=True)
             g = torch.cuda.CUDAGraph()
             n0 = _lib.launch_counter[0]
@@ -478,7 +501,9 @@ class FusedTrainer:
                 'dropout_counter': eng._seed_counter, 'dropout_base_seed': eng.base_seed,  # rank-independent
                 'schedule': self.schedule, 'n_warmup': self.n_warmup, 'n_step': self.n_step, 'lr': self.lr,
                 'weight_decay': self.wd, 'betas': tuple(self.betas), 'eps': self.eps, 'max_grad_norm': self.max_grad_norm,
-                **({} if self.param_groups is None else {'param_groups': self._groups_state()})}
+                **({} if self.param_groups is None else {'param_groups': self._groups_state()}),
+                **({} if self.ema is None else {'ema': self.ema.average(self.model).clone(), 'ema_decay': self.ema.decay,
+                                                'ema_warmup': self.ema.warmup})}
 
     def _groups_state(self):
         """the groups as [(parameter names, lr_scale, weight_decay)]"""
@@ -491,6 +516,8 @@ class FusedTrainer:
         if theirs != mine:
             raise ValueError('FusedTrainer.load_state_dict: the checkpoint\'s parameter groups differ from this '
                              'trainer\'s (build the trainer with the same param_groups)')
+        if self.ema is not None:
+            self.ema.check_inactive('load_state_dict()')
         self._ensure_state(next(self.model.parameters()).device)
         self._pending_step = None
         self.step_count = sd['step']
@@ -503,7 +530,37 @@ class FusedTrainer:
                         ('weight_decay', 'wd'), ('betas', 'betas'), ('eps', 'eps'), ('max_grad_norm', 'max_grad_norm')):
             if k in sd:
                 setattr(self, attr, sd[k])
+        if self.ema is not None:
+            # a checkpoint without an average (written without EMA): the average starts from the loaded weights
+            self.ema.load(self.model, sd.get('ema'))
+            if 'ema_decay' in sd:
+                self.ema.decay, self.ema.warmup = float(sd['ema_decay']), bool(sd['ema_warmup'])
         self.model.sync_shadow(force=True)
+
+    # ---- the weight moving average -------------------------------------------------------------------------
+    @contextlib.contextmanager
+    def ema_weights(self):
+        """Inside this context the model's weights (fp32 master and bf16 shadow) ARE the moving average: `model(...)`,
+        `evaluate`, `Recorder`, `state_dict()` and `encoder_state_dict()` all see it; on exit the weights and the shadow
+        are restored bit for bit.  A pending deferred update is applied first.  `step()` inside it and nesting it raise
+        `RuntimeError`; without `ema_decay` it raises `ValueError`."""
+        ema = self._require_ema()
+        self._ensure_state(next(self.model.parameters()).device)
+        self.flush()
+        with ema.weights(self.model):
+            yield
+
+    def ema_state_dict(self):
+        """the moving average in the model's own `state_dict()` keys (loads with strict=True into the model's class and
+        into the oracle)"""
+        ema = self._require_ema()
+        self._ensure_state(next(self.model.parameters()).device)
+        return ema.state_dict(self.model)
+
+    def _require_ema(self):
+        if self.ema is None:
+            raise ValueError('the trainer keeps no weight moving average: build it with ema_decay=...')
+        return self.ema
 
 
     # ---- the reference's outer loop (MyTrainer.train, train.py:263-319), re-hosted -------------------------------------
@@ -579,9 +636,14 @@ class FusedTrainer:
             if do_eval and eval_data is not None:
                 ebsz = eval_batch_size or bsz
                 xe, ye = eval_data
-                d = evaluate(self.model, ({'sample_values': xe[j:j + ebsz], 'labels': ye[j:j + ebsz]}
-                                          for j in range(0, xe.shape[0], ebsz)))
+                batches_eval = lambda: ({'sample_values': xe[j:j + ebsz], 'labels': ye[j:j + ebsz]}
+                                        for j in range(0, xe.shape[0], ebsz))
+                d = evaluate(self.model, batches_eval())
                 rec = dict(epoch=epoch, step=self.step_count, **d)
+                if self.ema is not None:   # the moving average next to the weights; patience watches eval/loss
+                    with self.ema_weights():
+                        d_ema = evaluate(self.model, batches_eval())
+                    rec.update({'eval_ema/' + k[len('eval/'):]: v for k, v in d_ema.items()})
                 logs.append(rec)
                 emit(rec)
                 if d['eval/loss'] < best_eval:   # train.py:304-314
@@ -597,11 +659,16 @@ class FusedTrainer:
 
     def save(self, output_dir, tag):
         """`model - <tag>.pt` = `model.state_dict()` as the reference saves it (train.py:297-300,319; loadable by its
-        `load_trained`), `trainer - <tag>.pt` = optimizer / schedule / dropout-stream state"""
+        `load_trained`), `trainer - <tag>.pt` = optimizer / schedule / dropout-stream state (and the moving average),
+        with EMA `model_ema - <tag>.pt` = `ema_state_dict()` in the format of `model - <tag>.pt`"""
+        if self.ema is not None:
+            self.ema.check_inactive('save()')
         os.makedirs(output_dir, exist_ok=True)
         torch.cuda.synchronize()
         torch.save(self.model.state_dict(), os.path.join(output_dir, f'model - {tag}.pt'))
         torch.save(self.state_dict(), os.path.join(output_dir, f'trainer - {tag}.pt'))
+        if self.ema is not None:
+            torch.save(self.ema_state_dict(), os.path.join(output_dir, f'model_ema - {tag}.pt'))
 
     def resume(self, output_dir, tag):
         self.model.load_state_dict(torch.load(os.path.join(output_dir, f'model - {tag}.pt'), map_location='cpu'), strict=True)

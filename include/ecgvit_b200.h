@@ -332,6 +332,8 @@ int ecgvit_colsum(const void *x, float *out, int M, int N, int64_t ld, int dtype
  *        [9] 1-beta1  [10] 1-beta2  [11] 1-lr*weight_decay  [12] lr/(1-beta1^t)  [13] sqrt(1-beta2^t)
  *        ([9..13] are derived by the host in double precision, as torch.optim.AdamW derives them)
  *        [14] skip: non-zero makes ecgvit_adamw_step a no-op
+ *        [15] 1 - d_t, the averaging rate of ecgvit_adamw_step_ema (derived by the host in double precision: 1 minus
+ *             fp32(0.9999) in fp32 is 1.7e-4 off relative); unused by every other entry point
  *      stats (device, fp32[ECGVIT_STATS_FLOATS]): [0] sum of squares of (grad_scale*g)  [1] non-finite flag
  *        [2] total_norm (written by grad_sumsq, adamw and grad_scale_by_clip)  [3] updates SKIPPED because the norm was non-finite
  *        (incremented by adamw, never cleared by the library: `error_if_nonfinite` for a host that polls every k steps)
@@ -371,11 +373,25 @@ int ecgvit_adamw_step(float *p, float *m, float *v, const void *g, int grad_dtyp
 int ecgvit_adamw_step_grouped(float *p, float *m, float *v, const void *g, int grad_dtype, void *shadow_bf16, int64_t n,
                               const uint8_t *group_map, const float *group_table, const float *hyper, float *stats,
                               int flags, void *stream);
+/* ecgvit_adamw_step (group_map NULL) or ecgvit_adamw_step_grouped (group_map and group_table given; n a multiple of
+ * 64) followed, per element the update writes, by the weight moving average
+ *      ema = ema + hyper[15] * (p_new - ema)          (ema: device fp32[n], 16-byte aligned, offset like p by a slice)
+ * computed from the p it has just written.  Same flags, hyper, stats and validation as those two entry points; what
+ * they leave untouched (hyper[14] skip, a non-finite norm, group id 255) keeps its ema value too.
+ *      Added in ABI version 7 without changing any earlier entry point, so the version number stays 7. */
+int ecgvit_adamw_step_ema(float *p, float *m, float *v, const void *g, int grad_dtype, void *shadow_bf16, float *ema,
+                          int64_t n, const uint8_t *group_map, const float *group_table, const float *hyper,
+                          float *stats, int flags, void *stream);
 /* in-place  g *= clip_coef  for API-compatible clip_grad_norm_ on a flat buffer */
 int ecgvit_grad_scale_by_clip(float *g, int64_t n, const float *hyper, float *stats, void *stream);
 
 /* ---- fp32 -> bf16 cast of a flat buffer (weight shadows) */
 int ecgvit_cast_f32_to_bf16(const float *src, void *dst, int64_t n, void *stream);
+/* a <-> b in place over n floats and, when shadow_bf16 is not NULL, shadow = bf16(new a) with the rounding of
+ * ecgvit_cast_f32_to_bf16 (one pass, no temporary: swaps the master weights with their moving average, shadow
+ * included; a second call restores all three bit for bit).  a, b and the shadow must be 16-byte aligned.
+ *      Added in ABI version 7 without changing any earlier entry point, so the version number stays 7. */
+int ecgvit_swap_f32_cast(float *a, float *b, void *shadow_bf16, int64_t n, void *stream);
 
 #ifdef __cplusplus
 }
