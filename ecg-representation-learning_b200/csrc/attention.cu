@@ -142,7 +142,8 @@ int ecgvit_attention_bwd(const void *qkv, const void *o, const void *d_o, const 
     if (dtype == ECGVIT_BF16 && attention_mma_supported(N, dh))
         return attention_bwd_mma(qkv, o, d_o, lse, dqkv, B, N, H, dh, scale, drop, as_stream(stream));
     if (dtype == ECGVIT_BF16 && attention_flash_supported(N, dh)) {
-        ECGVIT_REQUIRE(scratch != nullptr, "attention_bwd: N=%d needs the scratch of ecgvit_attention_bwd_scratch_floats", N);
+        ECGVIT_REQUIRE(scratch != nullptr && (reinterpret_cast<uintptr_t>(scratch) & 15) == 0,
+                       "attention_bwd: N=%d needs the (16-byte aligned) scratch of ecgvit_attention_bwd_scratch_floats", N);
         return attention_bwd_flash(qkv, o, d_o, lse, dqkv, scratch, B, N, H, dh, scale, drop, as_stream(stream));
     }
     return attention_bwd_simt(qkv, o, d_o, lse, dqkv, B, N, H, dh, scale, dtype, drop, as_stream(stream));

@@ -67,8 +67,9 @@ __global__ void __launch_bounds__(128) flash_fwd_kernel(const bf16 *__restrict__
     typedef typename FlashSmem<DH>::Tile Tile;
     Tile sQ = reinterpret_cast<Tile>(smem_raw);
     Tile sK0 = sQ + TILE, sV0 = sQ + 3 * TILE;  // two buffers each: [buf * TILE]
-    const int q0 = blockIdx.x * TILE;
-    const int bh = blockIdx.y, h = bh % H, b = bh / H;
+    // grid: one flat x over (b*H + h, query tile), query tile fastest (B * H may exceed the 65535 of grid.y)
+    const int bh = (int)(blockIdx.x / ((N + TILE - 1) / TILE)), h = bh % H, b = bh / H;
+    const int q0 = (int)(blockIdx.x - bh * ((N + TILE - 1) / TILE)) * TILE;
     const int inner = H * DH;
     const int64_t ld = 3 * (int64_t)inner;
     const bf16 *base = qkv + (int64_t)b * N * ld + h * DH;
@@ -207,8 +208,8 @@ __global__ void __launch_bounds__(128) flash_bwd_dq_kernel(const bf16 *__restric
     Tile sQ = reinterpret_cast<Tile>(smem_raw);
     Tile sdO = sQ + TILE;
     Tile sK0 = sQ + 2 * TILE, sV0 = sQ + 4 * TILE;  // two buffers each: [buf * TILE]
-    const int q0 = blockIdx.x * TILE;
-    const int bh = blockIdx.y, h = bh % H, b = bh / H;
+    const int bh = (int)(blockIdx.x / ((N + TILE - 1) / TILE)), h = bh % H, b = bh / H;  // grid as in flash_fwd_kernel
+    const int q0 = (int)(blockIdx.x - bh * ((N + TILE - 1) / TILE)) * TILE;
     const int inner = H * DH;
     const int64_t ld = 3 * (int64_t)inner;
     const bf16 *base = qkv + (int64_t)b * N * ld + h * DH;
@@ -291,8 +292,8 @@ __global__ void __launch_bounds__(128) flash_bwd_dkv_kernel(const bf16 *__restri
     Tile sQ0 = sK + 2 * TILE, sdO0 = sK + 4 * TILE;  // two buffers each: [buf * TILE]
     float *sL = reinterpret_cast<float *>(sK + 6 * TILE);  // [2][TILE] lse * log2(e) of the query tile
     float *sD = sL + 2 * TILE;                             // [2][TILE]
-    const int k0 = blockIdx.x * TILE;
-    const int bh = blockIdx.y, h = bh % H, b = bh / H;
+    const int bh = (int)(blockIdx.x / ((N + TILE - 1) / TILE)), h = bh % H, b = bh / H;  // grid as in flash_fwd_kernel
+    const int k0 = (int)(blockIdx.x - bh * ((N + TILE - 1) / TILE)) * TILE;
     const int inner = H * DH;
     const int64_t ld = 3 * (int64_t)inner;
     const bf16 *base = qkv + (int64_t)b * N * ld + h * DH;
@@ -383,7 +384,7 @@ int flash_fwd(const void *qkv, void *o, float *lse, int B, int N, int H, float s
         if (rc) return rc;
         attr_set = true;
     }
-    dim3 grid((N + TILE - 1) / TILE, B * H);
+    const unsigned grid = (unsigned)((N + TILE - 1) / TILE) * (unsigned)(B * H);
     flash_fwd_kernel<DH><<<grid, 128, smem, stream>>>((const bf16 *)qkv, (bf16 *)o, lse, N, H, scale, drop);
     return check_launch("attention_flash_fwd");
 }
@@ -406,7 +407,7 @@ int flash_bwd(const void *qkv, const void *o, const void *d_o, const float *lse,
                                                                                B, N, H);
     int rc = check_launch("attention_flash_bwd_dot");
     if (rc) return rc;
-    dim3 grid((N + TILE - 1) / TILE, B * H);
+    const unsigned grid = (unsigned)((N + TILE - 1) / TILE) * (unsigned)(B * H);   // flat, as in flash_fwd
     flash_bwd_dq_kernel<DH><<<grid, 128, smem_dq, stream>>>((const bf16 *)qkv, (const bf16 *)d_o, lse, dscratch,
                                                              (bf16 *)dqkv, N, H, scale, drop);
     rc = check_launch("attention_flash_bwd_dq");

@@ -252,8 +252,10 @@ int ecgvit_gemm_drop_path(const ecgvit_gemm_args *g, float path_p, int path_stre
 int ecgvit_attention_fwd(const void *qkv, void *o, float *lse, int B, int N, int H, int dh, float scale,
                          float dropout_p, int dropout_stream, const uint32_t *dropout_seed, int dtype,
                          void *stream);
-/* scratch: fp32 workspace of ecgvit_attention_bwd_scratch_floats(...) elements (rowsum(dO * O) of the tiled kernels
- * that serve N > 64 in bf16; 0 -> may be NULL) */
+/* scratch: fp32 workspace of ecgvit_attention_bwd_scratch_floats(...) elements, 16-byte aligned (rowsum(dO * O) of
+ * the tiled kernels that serve N > 64 in bf16; 0 -> may be NULL).  Its contents on entry do not matter.
+ * `o` is the forward's output, read for D = rowsum(dO * O) -- except on the tcgen05 path for N <= 64 (bf16, dh 64),
+ * which forms D from its own recomputed probabilities and never reads `o`. */
 int64_t ecgvit_attention_bwd_scratch_floats(int B, int N, int H, int dh, int dtype);
 int ecgvit_attention_bwd(const void *qkv, const void *o, const void *d_o, const float *lse, void *dqkv,
                          float *scratch, int B, int N, int H, int dh, float scale, float dropout_p,
