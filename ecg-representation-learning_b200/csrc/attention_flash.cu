@@ -1,6 +1,6 @@
-// Tiled ("flash") softmax attention for sequences longer than one 64-token tile: BASELINE.json configs[3] (12x5000,
-// patch 25, per-lead tokens -> N = 2401, attention = 34 % of the step's FLOPs).  bf16 operands, fp32 statistics,
-// mma.sync m16n8k16; 64 queries x 64 keys per inner step, K / V (or Q / dO) tiles double-buffered with cp.async.
+// Tiled ("flash") softmax attention for sequences longer than one 64-token tile with head dim 32 (head dim 64 runs on
+// the tcgen05 kernels of attention_tc.cu).  bf16 operands, fp32 statistics, mma.sync m16n8k16; 64 queries x 64 keys
+// per inner step, K / V (or Q / dO) tiles double-buffered with cp.async.
 //
 // Nothing of size N x N is ever written: forward keeps a running (max, sum) per query row and saves the log-sum-exp;
 // backward recomputes the probabilities from it in two kernels that need no atomics:
@@ -419,17 +419,17 @@ int flash_bwd(const void *qkv, const void *o, const void *d_o, const float *lse,
 
 }  // namespace
 
-bool attention_flash_supported(int N, int dh) { return N > NMAX && (dh == 32 || dh == 64); }
+bool attention_flash_supported(int N, int dh) { return N > NMAX && dh == 32; }
 
 int attention_fwd_flash(const void *qkv, void *o, float *lse, int B, int N, int H, int dh, float scale,
                         DropoutParams drop, cudaStream_t stream) {
-    if (dh == 64) return flash_fwd<64>(qkv, o, lse, B, N, H, scale, drop, stream);
+    ECGVIT_REQUIRE(dh == 32, "attention_fwd_flash: head dim %d (only 32)", dh);
     return flash_fwd<32>(qkv, o, lse, B, N, H, scale, drop, stream);
 }
 
 int attention_bwd_flash(const void *qkv, const void *o, const void *d_o, const float *lse, void *dqkv, float *dscratch,
                         int B, int N, int H, int dh, float scale, DropoutParams drop, cudaStream_t stream) {
-    if (dh == 64) return flash_bwd<64>(qkv, o, d_o, lse, dqkv, dscratch, B, N, H, scale, drop, stream);
+    ECGVIT_REQUIRE(dh == 32, "attention_bwd_flash: head dim %d (only 32)", dh);
     return flash_bwd<32>(qkv, o, d_o, lse, dqkv, dscratch, B, N, H, scale, drop, stream);
 }
 

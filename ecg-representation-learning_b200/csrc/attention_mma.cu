@@ -1,12 +1,10 @@
-// Tensor-core softmax attention for short sequences (N <= 64 tokens: the 12x2500 / patch-50 geometry has N = 51),
-// bf16 operands, fp32 softmax statistics.  One CTA (4 warps) per (batch, head); each warp owns 16 query rows.
+// Tensor-core softmax attention for short sequences (N <= 64 tokens) with head dim 16 or 32, bf16 operands, fp32
+// softmax statistics (head dim 64 runs on the tcgen05 kernels of attention_tc.cu).  One CTA (4 warps) per
+// (batch, head); each warp owns 16 query rows, with warp-level mma.sync m16n8k16 (HMMA).
 //
 // The whole (b,h) problem lives in shared memory / registers, so the forward never materialises the [B,H,N,N]
 // probability tensor that vit_pytorch's Attention.forward writes, and the backward recomputes P from the saved
 // log-sum-exp.  q | k | v are read in place from the packed projection (no chunk / rearrange copies).
-//
-// At N = 51 attention is 1.1 % of the step's FLOPs (BASELINE.md section 3): a 51-row problem cannot fill a 128-row
-// tcgen05 tile, so this kernel uses warp-level mma.sync m16n8k16 (HMMA); the tcgen05 budget goes to the GEMMs.
 #include "common.cuh"
 
 namespace ecgvit {
@@ -265,7 +263,7 @@ int launch_fwd(const void *qkv, void *o, float *lse, int B, int N, int H, float 
 
 }  // namespace
 
-bool attention_mma_supported(int N, int dh) { return N <= NMAX && (dh == 16 || dh == 32 || dh == 64); }
+bool attention_mma_supported(int N, int dh) { return N <= NMAX && (dh == 16 || dh == 32); }
 
 // the number of 16-key tiles is a template parameter so the inner loops carry no runtime predicates
 #define ECGVIT_ATTN_DISPATCH(FN, ...)                                                     \
@@ -280,10 +278,6 @@ bool attention_mma_supported(int N, int dh) { return N <= NMAX && (dh == 16 || d
             case 32 * 8 + 2: return FN<32, 2>(__VA_ARGS__);                               \
             case 32 * 8 + 3: return FN<32, 3>(__VA_ARGS__);                               \
             case 32 * 8 + 4: return FN<32, 4>(__VA_ARGS__);                               \
-            case 64 * 8 + 1: return FN<64, 1>(__VA_ARGS__);                               \
-            case 64 * 8 + 2: return FN<64, 2>(__VA_ARGS__);                               \
-            case 64 * 8 + 3: return FN<64, 3>(__VA_ARGS__);                               \
-            case 64 * 8 + 4: return FN<64, 4>(__VA_ARGS__);                               \
             default: return fail(-1, "attention_mma: unsupported head dim %d / length %d", dh, N); \
         }                                                                                 \
     } while (0)

@@ -25,7 +25,6 @@
 #include "ptx.cuh"
 
 #include <cudaTypedefs.h>
-#include <stdlib.h>
 
 namespace ecgvit {
 
@@ -150,19 +149,9 @@ __device__ __forceinline__ uint32_t sw128_offset(int r, int j) {
 template <bool kPacked>
 __global__ void __launch_bounds__(384, 1)
 attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_o,
-                   float *__restrict__ lse, int B, int N, int H, float scale, DropoutParams drop,
-                   long long *__restrict__ timeline) {
+                   float *__restrict__ lse, int B, int N, int H, float scale, DropoutParams drop) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    // debug timeline (ECGVIT_ATTN_TIMELINE): CTA 0 records clock64() at its hand-over points, 64 slots per role
-    int tl_n = 0;
-    auto stamp = [&](int role, int tag) {
-        if (timeline != nullptr && blockIdx.x == 0 && (threadIdx.x & 31) == 0 && tl_n < 64) {
-            timeline[(role * 64 + tl_n) * 2] = clock64();
-            timeline[(role * 64 + tl_n) * 2 + 1] = tag;
-            ++tl_n;
-        }
-    };
     FwdBars *bars = reinterpret_cast<FwdBars *>(smem + F_BAR_OFF);
 
     pdl_launch_dependents();
@@ -345,10 +334,8 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                     // ---- the successor step's scores
                     const bool more_blocks = j + 1 < nkb;
                     if (more_blocks || nxt.valid[t]) {
-                        stamp(0, 10 + t);
                         ptx::mbar_wait(&bars->s_free[t], fph[t]);   // S_t is in the warpgroup's registers
                         fph[t] ^= 1;
-                        stamp(0, 20 + t);
                         if (more_blocks) {
                             if (t == 0) st_shared = take_kv();      // tile 0 exists whenever tile 1 does
                             issue_qk(t, slot_cur[t], st_shared, j + 2 == nkb);
@@ -359,12 +346,9 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                         }
                     }
                     // ---- this step's output product
-                    stamp(0, 30 + t);
                     ptx::mbar_wait(&bars->p_full[t], pph[t]);
                     pph[t] ^= 1;
-                    stamp(0, 40 + t);
                     issue_pv(t, st_cur[t], j > 0, kPacked || !it.valid[1] || t == 1);
-                    stamp(0, 50 + t);
                     st_cur[t] = st_next[t];
                 }
             }
@@ -441,11 +425,9 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
             for (int j = 0; j < nkb; ++j) {
                 const int nvalid = kPacked ? N : min(TN, N - j * TN);  // valid keys of this block (>= 1)
                 const bool partial = nvalid < NCH * 32;                // CTA-uniform
-                if (q == 0) stamp(1 + t, 1);
                 ptx::mbar_wait(&bars->s_full[t], sph);
                 sph ^= 1;
                 ptx::tcgen05_fence_after();
-                if (q == 0) stamp(1 + t, 2);
                 // ---- the whole row of scores into registers, then hand S_t back to the tensor core
                 uint32_t s[NCH][32];
 #pragma unroll
@@ -455,7 +437,6 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 ptx::tcgen05_fence_before();
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(&bars->s_free[t]);
-                if (q == 0) stamp(1 + t, 3);
                 // ---- running max
                 float mx4[4] = {m, m, m, m};
 #pragma unroll
@@ -501,16 +482,13 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 ptx::tcgen05_fence_before();
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(&bars->p_full[t]);
-                if (q == 0) stamp(1 + t, 4);
             }
             // ---- epilogue: O / l -> bf16 -> swizzled staging tile -> TMA store; log-sum-exp of the scaled scores
             ptx::mbar_wait(&bars->pv_done[t], dph);
             dph ^= 1;
             ptx::tcgen05_fence_after();
-            if (q == 0) stamp(1 + t, 5);
             ptx::mbar_wait(&bars->out_free[t], oph ^ 1);   // warp 3's previous store of this tile has read `ost`
             oph ^= 1;
-            if (q == 0) stamp(1 + t, 7);
             const float inv_l = drop.scale / l;   // drop.scale = 1 / (1 - p) of the attention dropout (1 when off)
 #pragma unroll 1
             for (int c = 0; c < DH / 32; ++c) {
@@ -528,12 +506,10 @@ attn_tc_fwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 }
             }
             ptx::tcgen05_fence_before();   // O_t has been read: the next item's first P V may overwrite it
-            if (q == 0) stamp(1 + t, 8);
             if (qrow < N && prob < B * H) lse[static_cast<int64_t>(prob) * N + qrow] = m * scale + __logf(l);
             ptx::fence_proxy_async_smem();
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(&bars->out_full[t]);   // warp 3 issues the TMA store
-            if (q == 0) stamp(1 + t, 6);
         }
     }
 
@@ -574,31 +550,6 @@ int make_tmap3(CUtensorMap *tm, const void *base, int cols, int N, int B, int64_
     return 0;
 }
 
-// debug only: <env>=<file> dumps CTA 0's clock64() stamps (3 roles x 64 x (clock, tag)) after a synchronous copy
-long long *timeline_begin(const char *env) {
-    if (getenv(env) == nullptr) return nullptr;
-    long long *tl = nullptr;
-    cudaMalloc(&tl, 3 * 64 * 2 * sizeof(long long));
-    cudaMemset(tl, 0, 3 * 64 * 2 * sizeof(long long));
-    return tl;
-}
-void timeline_end(long long *tl, const char *env) {
-    if (tl == nullptr) return;
-    long long host[3 * 64 * 2];
-    cudaMemcpy(host, tl, sizeof(host), cudaMemcpyDeviceToHost);
-    cudaFree(tl);
-    long long t0 = 0;
-    for (int i = 0; i < 3 * 64; ++i)
-        if (host[2 * i + 1] != 0 && (t0 == 0 || host[2 * i] < t0)) t0 = host[2 * i];
-    if (FILE *f = fopen(getenv(env), "w")) {
-        for (int r = 0; r < 3; ++r)
-            for (int i = 0; i < 64; ++i)
-                if (host[(r * 64 + i) * 2 + 1] != 0)
-                    fprintf(f, "%d %d %lld %lld\n", r, i, host[(r * 64 + i) * 2] - t0, host[(r * 64 + i) * 2 + 1]);
-        fclose(f);
-    }
-}
-
 template <bool kPacked>
 int launch_fwd(const void *qkv, void *o, float *lse, int B, int N, int H, float scale, DropoutParams drop,
                cudaStream_t stream) {
@@ -618,10 +569,8 @@ int launch_fwd(const void *qkv, void *o, float *lse, int B, int N, int H, float 
     if (kPacked) items = (B * H + 1) >> 1;
     else items = B * H * ((((N + TM - 1) / TM) + 1) >> 1);
     const int grid = items < sm_count() ? items : sm_count();
-    long long *tl = timeline_begin("ECGVIT_ATTN_TIMELINE");
-    cudaError_t le = launch_pdl(kern, dim3(grid), dim3(384), F_SMEM_BYTES, stream, tq, to, lse, B, N, H, scale, drop, tl);
+    cudaError_t le = launch_pdl(kern, dim3(grid), dim3(384), F_SMEM_BYTES, stream, tq, to, lse, B, N, H, scale, drop);
     if (le != cudaSuccess) return fail((int)le, "attn_tc_fwd launch: %s", cudaGetErrorString(le));
-    timeline_end(tl, "ECGVIT_ATTN_TIMELINE");
     return check_launch("attn_tc_fwd");
 }
 
@@ -700,16 +649,8 @@ __global__ void __launch_bounds__(384, 1)
 attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_constant__ CUtensorMap tm_do,
                    const __grid_constant__ CUtensorMap tm_out, const __grid_constant__ CUtensorMap tm_acc,
                    const float *__restrict__ lse, const float *__restrict__ Drow, int B, int N, int H, float scale,
-                   DropoutParams drop, long long *__restrict__ timeline) {
+                   DropoutParams drop) {
     extern __shared__ __align__(1024) uint8_t smem[];
-    int tl_n = 0;   // debug timeline (ECGVIT_ATTN_TIMELINE), see the forward kernel
-    auto stamp = [&](int role, int tag) {
-        if (timeline != nullptr && blockIdx.x == 0 && (threadIdx.x & 31) == 0 && tl_n < 64) {
-            timeline[(role * 64 + tl_n) * 2] = clock64();
-            timeline[(role * 64 + tl_n) * 2 + 1] = tag;
-            ++tl_n;
-        }
-    };
     if ((ptx::smem_u32(smem) & 1023u) != 0) asm volatile("trap;");   // SWIZZLE_128B tiles need the declared alignment
     using Map = BwdMap<kPacked>;
     constexpr int G_KV_OFF = Map::KV_OFF, G_QD_OFF = Map::QD_OFF, G_PD_OFF = Map::PD_OFF, G_DS_OFF = Map::DS_OFF,
@@ -894,22 +835,17 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 const bool last = i + 1 == nsteps;
                 int kv_next = kv_cur, st_next = 0;
                 if (!last || nxt.valid) {
-                    stamp(0, 10);
                     ptx::mbar_wait(&bars->sdp_free, fph);   // S and dP are in the compute warps' registers
                     fph ^= 1;
-                    stamp(0, 11);
                     // (issuing this step's second group of products first whenever the next operands are still in flight
                     // was measured slower: 43.1 vs 41.1 us at cfg2 -- the next S / dP then arrive late for the warps)
                     if (last) kv_next = wait_kv();
                     st_next = wait_qd();
                     mma1(kv_next, st_next);
                 }
-                stamp(0, 12);
                 ptx::mbar_wait(&bars->pds_full, pph);       // Pd_s / dS_s written, previous outputs drained
                 pph ^= 1;
-                stamp(0, 13);
                 mma2(kv_cur, st_cur, i > 0, last);
-                stamp(0, 14);
                 kv_cur = kv_next;
                 st_cur = st_next;
             }
@@ -926,7 +862,6 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
             for (int i = 0; i < nsteps; ++i) {
                 ptx::mbar_wait(&bars->out_full, oph);
                 oph ^= 1;
-                stamp(2, 30);
                 if (ptx::elect_one()) {
                     if (kPacked) {
 #pragma unroll
@@ -947,7 +882,6 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                     ptx::mbar_arrive(&bars->out_free);
                 }
                 __syncwarp();
-                stamp(2, 31);
                 if (!kPacked && i + 1 == nsteps) {
                     ptx::mbar_wait(&bars->out_full, oph);
                     oph ^= 1;
@@ -1024,9 +958,7 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
             ptx::mbar_wait(&bars->mma2_done, dph);
             dph ^= 1;
             ptx::tcgen05_fence_after();
-            if (warp == 4) stamp(1, 7);
             wait_out_free();
-            if (warp == 4) stamp(1, 8);
             if (kPacked) {
                 stage_bf16(G_TM_DQ, out, scale);
                 stage_bf16(G_TM_DK, out + TILE_BYTES, scale);
@@ -1080,11 +1012,9 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 float D = D_next;
                 if (i + 1 < nsteps) row_stats(kk, i + 1, lse_next, D_next);
                 else row_stats(kk + 1, 0, lse_next, D_next);
-                if (warp == 4) stamp(1, 1);
                 ptx::mbar_wait(&bars->sdp_full, sph);
                 sph ^= 1;
                 ptx::tcgen05_fence_after();
-                if (warp == 4) stamp(1, 2);
                 uint32_t s[NCH][32], dp[NCH][32];
 #pragma unroll
                 for (int c = 0; c < NCH; ++c) ptx::tmem_ld_32x32(lane_addr + G_TM_S + cbase + 32 * c, s[c]);
@@ -1098,7 +1028,6 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 ptx::tcgen05_fence_before();
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(&bars->sdp_free);
-                if (warp == 4) stamp(1, 3);
                 // ---- P = exp2(S sl2 - lse log2e), t = dP * mask, Pd = P * mask, dS' = P (t - D)   (packed fp32x2 math;
                 //      the softmax scale of dS is applied when dQ / dK leave TMEM)
                 const float nl2 = -lse_r * LOG2E_F;   // -inf for rows that do not exist: P = 0
@@ -1171,9 +1100,7 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                     }
                 }
                 // ---- the previous step's outputs leave TMEM before the tensor core may overwrite them
-                if (warp == 4) stamp(1, 4);
                 if (have_prev) drain();
-                if (warp == 4) stamp(1, 5);
                 // ---- Pd_s / dS_s rows (swizzled 16-byte pieces), then hand over to the tensor core
 #pragma unroll
                 for (int c = 0; c < NCH; ++c)
@@ -1189,7 +1116,6 @@ attn_tc_bwd_kernel(const __grid_constant__ CUtensorMap tm_qkv, const __grid_cons
                 ptx::tcgen05_fence_before();
                 __syncwarp();
                 if (lane == 0) ptx::mbar_arrive(&bars->pds_full);
-                if (warp == 4) stamp(1, 6);
                 have_prev = true;
                 prev_last = i + 1 == nsteps;
             }
@@ -1261,27 +1187,15 @@ int launch_bwd(const void *qkv, const void *d_o, const float *lse, const float *
     }
     const int items = kPacked ? (B * H + 1) >> 1 : B * H * ((N + TN - 1) / TN);
     const int grid = items < sm_count() ? items : sm_count();
-    long long *tl = timeline_begin("ECGVIT_ATTN_TIMELINE_BWD");
     cudaError_t le = launch_pdl(kern, dim3(grid), dim3(384), BwdMap<kPacked>::SMEM_BYTES, stream, tq, td, tout, tacc, lse,
-                                Drow, B, N, H, scale, drop, tl);
+                                Drow, B, N, H, scale, drop);
     if (le != cudaSuccess) return fail((int)le, "attn_tc_bwd launch: %s", cudaGetErrorString(le));
-    timeline_end(tl, "ECGVIT_ATTN_TIMELINE_BWD");
     return check_launch("attn_tc_bwd");
 }
 
 }  // namespace
 
-// ECGVIT_ATTN=mma keeps the warp-level mma.sync kernels (A/B measurements)
-bool attention_tc_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("ECGVIT_ATTN");
-        v = (e != nullptr && e[0] == 'm') ? 0 : 1;
-    }
-    return v == 1;
-}
-
-bool attention_tc_supported(int N, int dh) { return attention_tc_enabled() && dh == DH && N >= 1; }
+bool attention_tc_supported(int N, int dh) { return dh == DH && N >= 1; }
 
 int attention_fwd_tc(const void *qkv, void *o, float *lse, int B, int N, int H, int dh, float scale, DropoutParams drop,
                      cudaStream_t stream) {

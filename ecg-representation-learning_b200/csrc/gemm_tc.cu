@@ -11,7 +11,6 @@
 #include "ptx.cuh"
 
 #include <cudaTypedefs.h>
-#include <stdlib.h>
 
 namespace ecgvit {
 
@@ -54,19 +53,8 @@ int make_tmap(CUtensorMap *tm, const void *base, uint64_t inner, uint64_t outer,
     return 0;
 }
 
-// CTA pairs the persistent GEMM grid may use: all of them (SMs / 2) unless the environment variable ECGVIT_GEMM_CLUSTERS,
-// read once at the first launch, lowered it (data-parallel runs leave a few SMs to NCCL's collective kernels: a
-// persistent grid that cannot place its last CTAs runs a second, nearly empty wave)
-int g_gemm_clusters = -1;
-int gemm_clusters() {
-    if (g_gemm_clusters < 0) {
-        const char *e = getenv("ECGVIT_GEMM_CLUSTERS");
-        const int all = sm_count() / 2;
-        int v = e != nullptr ? atoi(e) : all;
-        g_gemm_clusters = (v >= 1 && v <= all) ? v : all;
-    }
-    return g_gemm_clusters;
-}
+// CTA pairs of the persistent GEMM grid: one per pair of SMs
+int gemm_clusters() { return sm_count() / 2; }
 
 // Counters of the in-kernel unit scheduler: one (next unit, clusters done) pair per launch, taken round-robin from a static
 // array.  A kernel leaves its pair at zero when its last cluster runs dry, so a slot can be re-used by any later launch
@@ -127,11 +115,10 @@ int launch_pair(const ecgvit_gemm_args *g, int split_k, cudaStream_t stream, con
     static_cast<EpiParams &>(ep) =
         EpiParams{g->out, g->out2, g->aux, g->bias, g->ldo, make_dropout(g->dropout_p, g->dropout_stream, g->dropout_seed)};
     if constexpr (kPath) ep.path = *path;
-    static const int dynamic = [] { const char *e = getenv("ECGVIT_GEMM_DYNAMIC"); return e == nullptr || atoi(e) != 0; }();
     int *sched = next_sched_slot();
     if (sched == nullptr) return fail(-4, "gemm_tc2: cannot resolve the scheduler counters");
     cudaError_t le = launch_pdl(kern, dim3(grid), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, stream, ta, tb, to, to2, tx, g->M,
-                                g->N, g->K, split_k, ep, sched, dynamic);
+                                g->N, g->K, split_k, ep, sched);
     if (le != cudaSuccess) return fail((int)le, "gemm_tc2 launch: %s", cudaGetErrorString(le));
     return check_launch("gemm_tc2");
 }
@@ -226,10 +213,6 @@ int gemm_bf16_tc(const ecgvit_gemm_args *g, cudaStream_t stream, const PathParam
         return (double)waves * bn / eff;
     };
     const bool wide_ok = g->epilogue != ECGVIT_EPI_BIAS_RES_F32;   // see dispatch_pair
-    static const int forced_bn = [] { const char *e = getenv("ECGVIT_GEMM_BN"); return e != nullptr ? atoi(e) : 0; }();
-    if (forced_bn == 128) return dispatch_pair<128>(g, split_k, stream, path);   // experiments only
-    if (forced_bn == 192) return dispatch_pair<192>(g, split_k, stream, path);
-    if (forced_bn == 256 && wide_ok) return dispatch_pair<256>(g, split_k, stream, path);
     const double s256 = wide_ok ? score(256, 1.0) : 1e30, s192 = score(192, b_kmajor_eff(g->b_kmajor)), s128 = score(128, 0.67);
     if (g->N <= 128 || (s128 < s256 && s128 < s192)) return dispatch_pair<128>(g, split_k, stream, path);
     if (s192 < s256) return dispatch_pair<192>(g, split_k, stream, path);

@@ -180,7 +180,7 @@ __launch_bounds__(PairCfgFor<BN, B_MN, MODE>::THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                 const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_out2,
                 const __grid_constant__ CUtensorMap tmap_aux, int M, int N, int K, int split_k, EpiParamsFor<kPath> ep,
-                int *__restrict__ sched_ctr, int dynamic) {
+                int *__restrict__ sched_ctr) {
     constexpr bool kWide = MODE == ECGVIT_EPI_BIAS_RES_F32;   // (the split-K epilogue has its own fp32 path below)
     using Cfg = PairCfgFor<BN, B_MN, MODE>;
     constexpr bool kRowSq = MODE == ECGVIT_EPI_BIAS_SUB_ROWSQ;
@@ -345,8 +345,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
             for (int k = 0;; ++k) {
                 const int slot = k % Cfg::SCHED_SLOTS;
                 ptx::mbar_wait(&sched_empty[slot], ((k / Cfg::SCHED_SLOTS) & 1) ^ 1);
-                // (dynamic == 0: the static round-robin deal, for A/B measurements)
-                int u = dynamic ? num_clusters + atomicAdd(&sched_ctr[0], 1) : cluster_id + (k + 1) * num_clusters;
+                int u = num_clusters + atomicAdd(&sched_ctr[0], 1);
                 if (u >= num_units) u = kNoUnit;
                 sched_unit[slot] = u;
                 ptx::mbar_arrive(&sched_full[slot]);
@@ -357,7 +356,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constan
             }
             // the last cluster to run dry re-arms the counters for the next launch that uses this slot
             __threadfence();
-            if (dynamic && atomicAdd(&sched_ctr[1], 1) == num_clusters - 1) {
+            if (atomicAdd(&sched_ctr[1], 1) == num_clusters - 1) {
                 sched_ctr[0] = 0;
                 sched_ctr[1] = 0;
                 __threadfence();

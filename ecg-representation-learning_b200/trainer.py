@@ -138,22 +138,6 @@ class FusedTrainer:
         self.stats = torch.zeros(_lib.STATS_FLOATS, device=device, dtype=torch.float32)
         self._flat_ptr = m._flat_p.data_ptr()
         self._graph = None   # a captured graph points at the old flat buffers
-        self._norm_slices = None
-        if (self.world == 1 and not self.defer_optimizer and m._engine.side_stream is not None
-                and os.environ.get('ECGVIT_SLICE_NORM', '0') == '1'):
-            # experiment (off by default): reduce the gradient norm slice by slice beside backward (a layer's slice is
-            # final -- and still in L2 -- the moment its weight-gradient GEMMs finish) so that only a one-CTA fold sits
-            # between backward and AdamW instead of a 342 MB pass.  Measured on B200: 9.18 vs 9.00 ms per step -- the
-            # per-layer join of the side stream with the main chain and the extra kernels beside the persistent GEMMs
-            # cost more than the 66 us pass they hide.
-            from .parallel import bucket_slices
-            depth = m.config.num_hidden_layers
-            offs = [m._layout[f'l{l}.ln1.w'][0] for l in range(depth)]
-            slices = bucket_slices(offs, n, depth, 1)
-            per = max(1, min(148, _lib.SUMSQ_MAX_BLOCKS // len(slices)))
-            self._norm_slices = {t: (lo, hi, i * per, per) for i, (t, lo, hi) in enumerate(slices)}
-            self._norm_blocks = per * len(slices)
-            m._after_layer_backward = self._slice_norm
         if self.world > 1:
             from .parallel import BucketedGradReducer
             dist = torch.distributed
@@ -240,17 +224,6 @@ class FusedTrainer:
             self._hyper_ring = _lib.PinnedRing(len(vals), torch.float32)
         self._hyper_ring.upload(self.hyper[:len(vals)], vals)  # asynchronous: the host keeps queueing steps ahead of the device
 
-    def _slice_norm(self, layer):
-        """engine hook: the gradients of `layer` (and of everything above it) are final on the current stream"""
-        s = self._norm_slices.get(layer)
-        if s is None or self._span.frozen:   # the sliced norm covers the whole buffer: off while anything is frozen
-            return
-        lo, hi, first, per = s
-        m = self.model
-        _lib.check(self.lib.ecgvit_grad_sumsq_partial(m._flat_g.data_ptr() + 4 * lo, _lib.F32, hi - lo, self.hyper.data_ptr(),
-                                                      self.stats.data_ptr(), first, per,
-                                                      torch.cuda.current_stream().cuda_stream), 'grad_sumsq_partial')
-
     # ---- the step ----------------------------------------------------------------------------------
     def _device_step(self, sample_values, labels):
         m, st = self.model, torch.cuda.current_stream().cuda_stream
@@ -287,13 +260,7 @@ class FusedTrainer:
         g, g_code = (m._flat_g, _lib.F32) if self._reducer is None or self._reducer.flat_g16 is None \
             else (self._reducer.flat_g16, _lib.BF16)
         esz = 4 if g_code == _lib.F32 else 2
-        if self._norm_slices is not None and not self._span.frozen:
-            if side is not None:   # the slice partials were issued on the side stream
-                done = torch.cuda.Event()
-                done.record(side)
-                main.wait_event(done)
-            _lib.check(self.lib.ecgvit_grad_sumsq_finalize(self.stats.data_ptr(), self._norm_blocks, st), 'grad_sumsq_finalize')
-        elif self._grouped and self._span.frozen:
+        if self._grouped and self._span.frozen:
             # frozen tensors (id 255 in the map) do not count in the norm
             from .model import _ALIGN
             _lib.check(self.lib.ecgvit_grad_sumsq_grouped(g.data_ptr() + esz * lo, g_code, n - lo,

@@ -1,7 +1,6 @@
 #!/usr/bin/env python
 """Times the attention kernels alone (CUDA events, rotating over `layers` distinct buffers like the real step so that
-consecutive launches do not hit in L2) at the cfg2 (B=256, N=51) and cfg4 (B=32, N=2401) shapes.
-ECGVIT_ATTN=mma selects the warp-level mma.sync kernels for comparison."""
+consecutive launches do not hit in L2) at the cfg2 (B=256, N=51) and cfg4 (B=32, N=2401) shapes."""
 import os
 import sys
 import json

@@ -9,8 +9,6 @@ run n1 python $B --gpus 1
 run n8_default $TR --nproc-per-node 8 --master-port 29701 $B --gpus 8
 run n8_ctas4 $TR --nproc-per-node 8 --master-port 29702 $B --gpus 8 --nccl-max-ctas 4
 run n8_ctas8 $TR --nproc-per-node 8 --master-port 29703 $B --gpus 8 --nccl-max-ctas 8
-ECGVIT_GEMM_CLUSTERS=70 run n8_ctas8_cl70 $TR --nproc-per-node 8 --master-port 29704 $B --gpus 8 --nccl-max-ctas 8
-ECGVIT_GEMM_CLUSTERS=72 run n8_ctas4_cl72 $TR --nproc-per-node 8 --master-port 29705 $B --gpus 8 --nccl-max-ctas 4
 run n8_bucket3 $TR --nproc-per-node 8 --master-port 29706 $B --gpus 8 --bucket-layers 3
 python scripts/ddp_timeline.py gpurun_out/tl_n1.json > gpurun_out/tl_n1.log 2>&1
 $TR --nproc-per-node 8 --master-port 29707 scripts/ddp_timeline.py gpurun_out/tl_n8.json > gpurun_out/tl_n8.log 2>&1

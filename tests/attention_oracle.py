@@ -52,8 +52,8 @@ from ecg_b200 import _lib as L
 
 NMAX = 64                  # Np granularity of the dropout counter, and the longest sequence of the mma kernels
 TC_DH = 64                 # the tcgen05 kernels serve head dim 64 only
-FLASH_DHS = (32, 64)
-MMA_DHS = (16, 32, 64)
+FLASH_DHS = (32,)
+MMA_DHS = (16, 32)
 SIMT_SMEM_MAX = 227 * 1024
 
 U_BF16 = 2.0 ** -8
@@ -91,12 +91,11 @@ def simt_max_len(dh, bwd):
     return N
 
 
-def plan(dtype, N, dh, attn_env=None, B=1, H=1):
-    """which kernels `ecgvit_attention_fwd` / `_bwd` launch for (dtype, N, dh) with ECGVIT_ATTN = attn_env (None: unset)
-    and how many scratch floats backward needs at (B, H) (`ecgvit_attention_bwd_scratch_floats`).  Kernel names are
-    'base<args>' with the template arguments written as in the source (bf16 / float, true / false, no spaces)."""
-    tc_on = not (attn_env and attn_env[0] == 'm')
-    if dtype == L.BF16 and tc_on and dh == TC_DH and N >= 1:
+def plan(dtype, N, dh, B=1, H=1):
+    """which kernels `ecgvit_attention_fwd` / `_bwd` launch for (dtype, N, dh) and how many scratch floats backward
+    needs at (B, H) (`ecgvit_attention_bwd_scratch_floats`).  Kernel names are 'base<args>' with the template arguments
+    written as in the source (bf16 / float, true / false, no spaces)."""
+    if dtype == L.BF16 and dh == TC_DH and N >= 1:
         if N <= NMAX:
             return Plan('tc_packed', ('true',), ['attn_tc_fwd_kernel<true>'], ['attn_tc_bwd_kernel<true>'], 0)
         d_floats = cdiv(B * H * N, 64) * 64
@@ -114,18 +113,17 @@ def plan(dtype, N, dh, attn_env=None, B=1, H=1):
 
 
 def all_kernels():
-    """the 44 attention kernels the library compiles: (name, reachable only with ECGVIT_ATTN=mma)"""
-    ks = [('attn_tc_fwd_kernel<true>', False), ('attn_tc_fwd_kernel<false>', False), ('attn_tc_bwd_kernel<true>', False),
-          ('attn_tc_bwd_kernel<false>', False), ('attn_tc_dot_kernel', False), ('attn_tc_dq_convert_kernel', False)]
+    """the 32 attention kernels the library compiles"""
+    ks = ['attn_tc_fwd_kernel<true>', 'attn_tc_fwd_kernel<false>', 'attn_tc_bwd_kernel<true>', 'attn_tc_bwd_kernel<false>',
+          'attn_tc_dot_kernel', 'attn_tc_dq_convert_kernel']
     for dh in MMA_DHS:
         for nt in range(1, 5):
-            ks += [(f'attention_fwd_mma_kernel<{dh},{nt}>', dh == 64), (f'attention_bwd_mma_kernel<{dh},{nt}>', dh == 64)]
+            ks += [f'attention_fwd_mma_kernel<{dh},{nt}>', f'attention_bwd_mma_kernel<{dh},{nt}>']
     for dh in FLASH_DHS:
-        ks += [(f'{k}<{dh}>', dh == 64) for k in ('flash_fwd_kernel', 'flash_bwd_dot_kernel', 'flash_bwd_dq_kernel',
-                                                   'flash_bwd_dkv_kernel')]
+        ks += [f'{k}<{dh}>' for k in ('flash_fwd_kernel', 'flash_bwd_dot_kernel', 'flash_bwd_dq_kernel',
+                                      'flash_bwd_dkv_kernel')]
     for t in ('bf16', 'float'):
-        ks += [(f'attention_fwd_simt_kernel<{t}>', False), (f'attention_bwd_simt_kernel<{t}>', False),
-               (f'attention_probs_kernel<{t}>', False)]
+        ks += [f'attention_fwd_simt_kernel<{t}>', f'attention_bwd_simt_kernel<{t}>', f'attention_probs_kernel<{t}>']
     return ks
 
 
@@ -155,7 +153,7 @@ class Case:
     """one attention problem [B, N, H, dh] in one dtype with its device buffers: qkv / d_o inputs (random unless set),
     NaN-filled o / lse / dqkv with GUARD NaN elements after each, and NaN-filled scratch of the planned size."""
 
-    def __init__(self, B, N, H, dh, dtype, scale=None, p=0.0, site=0, seed=0, attn_env=None, amp=1.0,
+    def __init__(self, B, N, H, dh, dtype, scale=None, p=0.0, site=0, seed=0, amp=1.0,
                  device='cuda', null_seed=False):
         self.B, self.N, self.H, self.dh, self.dtype = B, N, H, dh, dtype
         self.inner = H * dh
@@ -165,7 +163,7 @@ class Case:
         self.null_seed = null_seed
         self.device = device
         self.td = torch.bfloat16 if dtype == L.BF16 else torch.float32
-        self.plan = plan(dtype, N, dh, attn_env, B, H)
+        self.plan = plan(dtype, N, dh, B, H)
         g = torch.Generator(device=device).manual_seed(2000 + seed)
         n_qkv, n_o = B * N * 3 * self.inner, B * N * self.inner
         self.qkv_buf, q = guarded(n_qkv, self.td, device)

@@ -54,33 +54,28 @@ def test_plan_model_shapes():
     assert O.plan(F32, 51, 64).family == 'simt' and O.plan(F32, 2401, 32).family == 'simt'
 
 
-def test_plan_under_ecgvit_attn_mma():
-    assert O.plan(BF, 51, 64, 'mma') == O.Plan('mma', (64, 4), ['attention_fwd_mma_kernel<64,4>'],
-                                               ['attention_bwd_mma_kernel<64,4>'], 0)
-    assert O.plan(BF, 2401, 64, 'mma').targs == (64,) and O.plan(BF, 2401, 64, 'mma').family == 'flash'
-    assert O.plan(BF, 51, 64, 'tc').family == 'tc_packed'     # only a value starting with 'm' switches
+def test_plan_bf16_dh64_is_tcgen05_at_every_length():
+    for N in range(1, 2402):
+        assert O.plan(BF, N, 64).family == ('tc_packed' if N <= 64 else 'tc_long'), N
 
 
 @pytest.mark.parametrize('N,nt', [(1, 1), (16, 1), (17, 2), (32, 2), (33, 3), (48, 3), (49, 4), (64, 4)])
 def test_plan_nt_boundaries(N, nt):
     for dh in (16, 32):
         assert O.plan(BF, N, dh).targs == (dh, nt)
-    assert O.plan(BF, N, 64, 'mma').targs == (64, nt)
     assert O.plan(BF, N, 64).family == 'tc_packed'
     assert O.plan(BF, N, 64, B=7, H=3).scratch_floats == 0
 
 
 def test_kernel_inventory():
     ks = O.all_kernels()
-    assert len(ks) == 44 and len({k for k, _ in ks}) == 44
-    assert sum(m for _, m in ks) == 12
-    names = {k for k, _ in ks}
+    assert len(ks) == 32 and len(set(ks)) == 32
+    names = set(ks)
     for dt in (BF, F32):
         for N in (1, 17, 64, 65, 300, 2401):
             for dh in (8, 16, 24, 32, 64):
-                for env in (None, 'mma'):
-                    p = O.plan(dt, N, dh, env)
-                    assert set(p.fwd + p.bwd) <= names, (dt, N, dh, env)
+                p = O.plan(dt, N, dh)
+                assert set(p.fwd + p.bwd) <= names, (dt, N, dh)
 
 
 def test_simt_length_limit():
